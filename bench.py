@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s (primary + shadow + reflection) and frames/s of the render path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one frame of the workload.  The default workload is BASELINE.json configs[4]
 (synth256_8k_d10: the mirror-heavy 256-sphere scene at 7680x4320, depth 10) — the largest config, it fits
@@ -59,6 +59,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (which may be read-only)
 
 # name -> (scene, W, H, depth): BASELINE.json configs[0..4] (+ the reference's SCENE 2, + reduced copies)
 WORKLOADS = {
@@ -79,6 +80,7 @@ METRIC = "Mrays/s (primary+shadow+reflection)"
 CAPTURE_OF = {"synth256_8k_d10": "synth256_1080p_d10", "synth1024_4k_d50": "synth1024_1080p_d50"}
 NCU_METRICS = os.path.join(ROOT, "profiles", "ncu_metrics_r2.json")
 GOLDEN_COLUMNS = os.path.join(ROOT, "tests", "golden", "bench_columns.json")
+DUMP_BYTES = 48 << 20    # --dump-outputs: pixel bytes at most; with the column indices and counters well under 64 MB
 
 
 # ---- clocks during the timed region (NVML) ---------------------------------------------------------
@@ -367,11 +369,44 @@ class Dist:
     def gather(self, v):
         return self.D.gather_floats(v, self.tdev)
 
+    def gather_objects(self, obj):
+        """Every rank's object on rank 0, in rank order (None on the other ranks); over gloo, outside timed regions."""
+        if self.world == 1:
+            return [obj]
+        import torch.distributed as dist
+
+        out = [None] * self.world if self.rank == 0 else None
+        dist.gather_object(obj, out, dst=0, group=self.cpu_group)
+        return out
+
     def bcast(self, obj):
         return self.D.broadcast_object(obj)
 
 
-def run_workload(ctx, dist, args, name, steps, warmup, inproc, sample_clocks=False, host=None):
+def dump_outputs(ctx, dist, out_dir, params, x0, x1, st):
+    """--dump-outputs: what the last timed step computed, as its caller receives it: the band tcrt_render_device left
+    on the device (fetched with tcrt_download) and the ray counters of its tcrt_stats.  A frame larger than DUMP_BYTES
+    is sampled by whole columns whose x positions come from a fixed seed, so two runs with the same arguments (and two
+    builds of the project) write the same pixels.
+      image.npy          float32 [columns, height, 3]: the sampled columns, x-major like the frame
+      image_columns.npy  float64 [columns]: the x of each of them
+      rays.npy           float64 [3]: primary, shadow and reflection rays of the whole frame"""
+    import numpy as np
+
+    w, h = params.width, params.height
+    band = ctx.download(np.empty((x1 - x0, h, 3), np.float32))
+    k = min(w, DUMP_BYTES // (h * 3 * 4))
+    cols = np.arange(w) if k == w else np.sort(np.random.default_rng(0).choice(w, k, replace=False))
+    parts = dist.gather_objects(band[cols[(cols >= x0) & (cols < x1)] - x0])
+    rays = [dist.sum(v) for v in (st.rays_primary, st.rays_shadow, st.rays_reflect)]
+    if dist.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "image.npy"), np.concatenate(parts, 0))
+        np.save(os.path.join(out_dir, "image_columns.npy"), cols.astype(np.float64))
+        np.save(os.path.join(out_dir, "rays.npy"), np.array(rays, np.float64))
+
+
+def run_workload(ctx, dist, args, name, steps, warmup, inproc, sample_clocks=False, host=None, dump_dir=None):
     """Kernel-only and end-to-end measurement of one workload at this N, plus its parity verdict."""
     import numpy as np
 
@@ -423,6 +458,8 @@ def run_workload(ctx, dist, args, name, steps, warmup, inproc, sample_clocks=Fal
             launches += st.gpu_launches
     wall = time.perf_counter() - wall0
     dist.barrier()
+    if dump_dir is not None:
+        dump_outputs(ctx, dist, dump_dir, params, x0, x1, st)
     t_rank_ms = sum(kernel_ms)
     t_ms = dist.max(t_rank_ms)                         # slowest rank, device time
     rank_ms = [t / steps for t in dist.gather(t_rank_ms)]
@@ -679,7 +716,8 @@ def run_ours(args):
     ctx = api.Context(list(range(args.gpus)) if inproc else [local])
     t_start = time.perf_counter()
 
-    head = run_workload(ctx, dist, args, args.workload, args.steps, args.warmup, inproc, sample_clocks=True)
+    head = run_workload(ctx, dist, args, args.workload, args.steps, args.warmup, inproc, sample_clocks=True,
+                        dump_dir=args.dump_outputs)
     params, x0, x1, out, flat, camx, hb = head.pop("_ctx_state")
     scene_name, w, h, depth = WORKLOADS[args.workload]
     line = {
@@ -825,7 +863,14 @@ def main():
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline workload only (developer loop)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step (a seeded column sample when large) and its ray "
+                         "counters to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 path computed; --impl reference has no such frame")
     quiet_stdout()
     if args.impl == "reference":
         # the prebuilt oracle/_ref travels with the repo; built here only where /root/reference exists

@@ -328,7 +328,7 @@ def test_synth256_8k_sampled_parity(gpu_ctx):
 
 # ---- error behaviour of the boundary -------------------------------------------------------------------
 
-def test_error_codes(gpu_ctx):
+def test_error_codes(gpu_ctx, tmp_path):
     fresh = api.Context([0])
     p = api.default_params(8, 8, 2)
     with pytest.raises(api.TcrtError) as e:
@@ -351,11 +351,12 @@ def test_error_codes(gpu_ctx):
     assert e.value.code == _ffi.TCRT_ERR_INVALID
     fresh.render_device(p, 2, 6)
     with pytest.raises(api.TcrtError) as e:
-        fresh.write_txt(p, "/tmp/should_not_exist.txt")       # band, not the whole image
+        fresh.write_txt(p, str(tmp_path / "should_not_exist.txt"))       # band, not the whole image
     assert e.value.code == _ffi.TCRT_ERR_INVALID
+    assert not (tmp_path / "should_not_exist.txt").exists()
     fresh.render_device(p)
     with pytest.raises(api.TcrtError) as e:
-        fresh.write_txt(p, "/nonexistent_dir/x/raytracer_screen.txt")
+        fresh.write_txt(p, str(tmp_path / "nonexistent_dir" / "x" / "raytracer_screen.txt"))
     assert e.value.code == _ffi.TCRT_ERR_IO
     with pytest.raises(api.TcrtError) as e:
         api.Context([99])
@@ -477,6 +478,28 @@ def test_cpp_host_program_is_a_drop_in(golden, tmp_path):
     assert r.returncode == 0, r.stdout + r.stderr
     txt = (tmp_path / "raytracer_screen.txt").read_bytes()
     assert pixel_md5(txt) == golden["md5"]["two_mirrors_500x504_d50"]["pixel_md5"]
+
+
+def test_bench_dump_outputs_are_the_timed_frame(golden, tmp_path):
+    """bench.py --dump-outputs: on the reference's own configuration (small enough to be written whole) the dumped
+    frame carries the reference program's pixel lines, and the dumped counters are that frame's rays."""
+    import json
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "default_500x504_d50", "--steps", "2",
+                        "--warmup", "1", "--quick", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                       cwd=tmp_path, capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads(r.stdout)
+    assert line["steps"] == 2
+    img, cols, rays = (np.load(out / f) for f in ("image.npy", "image_columns.npy", "rays.npy"))
+    assert img.dtype == np.float32 and img.shape == (500, 504, 3)
+    assert np.array_equal(cols, np.arange(500))
+    assert pixel_md5(O.format_txt(img)) == golden["md5"]["default_500x504_d50"]["pixel_md5"]
+    assert rays.tolist() == [252000, 963640, 230689] and line["rays_per_frame"] == rays.sum()
 
 
 # ---- round 2: the sphere BVH that collapses into one leaf, text scenes ---------------------------------

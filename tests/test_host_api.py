@@ -1,9 +1,9 @@
 """CPU tests: the host construction API (include/CelioRayTracer.hpp, tcrt_host.h) and the
 C-ABI surface of libtcrt.so.  No compute calls: there is no GPU here and no CPU fallback."""
-import ctypes as C
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -53,18 +53,29 @@ def test_library_is_sm100a_only_and_has_no_oracle_dependency():
     assert "tcrt_oracle_render" not in strings
 
 
+NO_DEVICE_CHECK = """
+import ctypes as C, sys
+sys.path.insert(0, %r)
+from tilecoderaytracer_b200 import _ffi, api
+lib = _ffi.load()
+n = lib.tcrt_device_count()
+assert n in (_ffi.TCRT_ERR_NO_DEVICE, 0), n
+h = C.c_void_p()
+rc = lib.tcrt_create(C.byref(h), None, 1)
+assert rc == _ffi.TCRT_ERR_NO_DEVICE and not h.value, rc
+assert b"CUDA" in lib.tcrt_last_error(None) or b"device" in lib.tcrt_last_error(None)
+try:
+    api.Context([0])
+except api.TcrtError:
+    print("NO_DEVICE_OK")
+""" % ROOT
+
+
 def test_no_gpu_means_loud_failure_not_fallback():
-    lib = _ffi.load()
-    n = lib.tcrt_device_count()
-    if n > 0:
-        pytest.skip("a GPU is visible here")
-    assert n in (_ffi.TCRT_ERR_NO_DEVICE, 0)
-    h = C.c_void_p()
-    rc = lib.tcrt_create(C.byref(h), None, 1)
-    assert rc == _ffi.TCRT_ERR_NO_DEVICE and not h.value
-    assert b"CUDA" in lib.tcrt_last_error(None) or b"device" in lib.tcrt_last_error(None)
-    with pytest.raises(api.TcrtError):
-        api.Context([0])
+    """In a process that sees no CUDA device (CUDA_VISIBLE_DEVICES empty, so that this runs on a GPU machine too)."""
+    r = subprocess.run([sys.executable, "-c", NO_DEVICE_CHECK], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True)
+    assert r.returncode == 0 and "NO_DEVICE_OK" in r.stdout, r.stdout + r.stderr
 
 
 def test_abi_version_and_default_params():

@@ -59,6 +59,16 @@ public:
         run_time_s_ = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         return rc_;
     }
+    // the same frame quantised to 8 bits on the GPU: pixels_xmajor_rgb8[(x*H + z)*3 + c] = floor(clamp(c,0,1)*255 + 0.5);
+    // the float frame stays the last render (printPixelsToLog writes it)
+    int renderRGB8(const RenderSettings& rs, unsigned char* pixels_xmajor_rgb8, tcrt_stats* stats = NULL) {
+        settings_ = rs;
+        tcrt_params p = rs.params();
+        std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+        rc_ = tcrt_render_rgb8(ctx_, &p, pixels_xmajor_rgb8, stats);
+        run_time_s_ = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        return rc_;
+    }
     // init_log + printPixelsToLog (RayTracer.cpp:2022-2061,1574-1626)
     int printPixelsToLog(const char* path = LOG_FILE_NAME) {
         tcrt_params p = settings_.params();

@@ -135,12 +135,13 @@ typedef struct tcrt_stats {
     int n_devices;
     int col_begin[TCRT_MAX_DEVICES]; /* band [col_begin, col_end) rendered by each device */
     int col_end[TCRT_MAX_DEVICES];
-    double render_ms[TCRT_MAX_DEVICES]; /* kernel time, CUDA events on the launching stream */
+    double render_ms[TCRT_MAX_DEVICES]; /* kernel time, CUDA events on the launching stream (RGB8 frames: render +
+                                           quantisation) */
     double d2h_ms[TCRT_MAX_DEVICES];    /* copy-back time of the band (0 if none) */
     unsigned long long rays_primary[TCRT_MAX_DEVICES];
     unsigned long long rays_shadow[TCRT_MAX_DEVICES];
     unsigned long long rays_reflect[TCRT_MAX_DEVICES];
-    unsigned long long gpu_launches;    /* kernels launched by this call */
+    unsigned long long gpu_launches;    /* kernels launched by this call (RGB8 frames: the quantisation launches too) */
 } tcrt_stats;
 
 /* ---- context ------------------------------------------------------------------- */
@@ -201,6 +202,18 @@ int tcrt_download(tcrt_ctx* ctx, float* host_rgb_band);
  * "last render" the synchronous calls refer to (tcrt_download, tcrt_write_*) is the last frame WAITED for. */
 int tcrt_render_async(tcrt_ctx* ctx, const tcrt_params* params, int x0, int x1, float* host_rgb_band, int* ticket);
 int tcrt_wait(tcrt_ctx* ctx, int ticket, tcrt_stats* stats);
+/* 8-bit frames: tcrt_render, tcrt_render_columns and tcrt_render_async with 3 bytes per pixel crossing the bus instead of
+ * 12.  x-major like tcrt_render: byte (x*height + z)*3 + c, q(c) = floor(clamp(c,0,1)*255 + 0.5) (NaN -> 0), the
+ * quantisation of tcrt_write_ppm; a column band is one contiguous slice.  Each column chunk is quantised on the device
+ * by one more launch behind its render launch; the float frame stays on the device and remains "the last render" of
+ * tcrt_download, tcrt_device_frame and the writers.  Pinned and pageable destinations as in tcrt_render.  A NULL
+ * destination is TCRT_ERR_INVALID (the device-only call is tcrt_render_device).  RGB8 and float frames share tcrt_wait
+ * and the two frames in flight.  Image rows (top row first) are the free view transpose(1,0,2)[::-1] of the array. */
+int tcrt_render_rgb8(tcrt_ctx* ctx, const tcrt_params* params, unsigned char* host_rgb8, tcrt_stats* stats);
+int tcrt_render_columns_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int x0, int x1, unsigned char* host_rgb8_band,
+                             tcrt_stats* stats);
+int tcrt_render_async_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int x0, int x1, unsigned char* host_rgb8_band,
+                           int* ticket);
 /* Device address of a device's band of the last render (for zero-copy consumers, e.g. a
  * torch tensor view); floats = (col_end-col_begin)*height*3. */
 int tcrt_device_frame(tcrt_ctx* ctx, int device_slot, void** dev_ptr, size_t* n_floats);

@@ -92,6 +92,11 @@ SIGNATURES = {
     "tcrt_download": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tcrt_render_async": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
     "tcrt_wait": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(TcrtStats)]),
+    "tcrt_render_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_void_p, C.POINTER(TcrtStats)]),
+    "tcrt_render_columns_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p,
+                                           C.POINTER(TcrtStats)]),
+    "tcrt_render_async_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p,
+                                         C.POINTER(C.c_int)]),
     "tcrt_device_frame": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),

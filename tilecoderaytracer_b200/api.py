@@ -315,6 +315,29 @@ class Context:
                                              out.ctypes.data_as(C.c_void_p) if out is not None else None, C.byref(t)))
         return t.value
 
+    def render_rgb8(self, params: TcrtParams, x0: int = 0, x1: Optional[int] = None, out: Optional[np.ndarray] = None):
+        """Columns [x0,x1) quantised to 8 bits on the GPU (q(c) = floor(clamp(c,0,1)*255 + 0.5)), 3 bytes per pixel to
+        host memory; returns (array[x1-x0, H, 3] uint8, RenderStats).  x-major like render(): image rows (top row
+        first) are a.transpose(1, 0, 2)[::-1].  The float frame stays on the device as the last render."""
+        x1 = params.width if x1 is None else x1
+        shape = (x1 - x0, params.height, 3)
+        if out is None:
+            out = np.empty(shape, dtype=np.uint8)
+        assert out.dtype == np.uint8 and out.size == int(np.prod(shape)) and out.flags["C_CONTIGUOUS"]
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_columns_rgb8(self._h, C.byref(params), x0, x1, out.ctypes.data_as(C.c_void_p),
+                                                    C.byref(st)))
+        return out.reshape(shape), RenderStats.from_c(st)
+
+    def render_async_rgb8(self, params: TcrtParams, x0: int, x1: int, out: np.ndarray) -> int:
+        """render_async() of an 8-bit frame into `out` (uint8, pinned host memory: HostBuffer.array(np.uint8, ...));
+        wait(ticket) completes it."""
+        assert out.dtype == np.uint8 and out.size == (x1 - x0) * params.height * 3 and out.flags["C_CONTIGUOUS"]
+        t = C.c_int(-1)
+        self._ck(self._lib.tcrt_render_async_rgb8(self._h, C.byref(params), x0, x1, out.ctypes.data_as(C.c_void_p),
+                                                  C.byref(t)))
+        return t.value
+
     def wait(self, ticket: int) -> RenderStats:
         st = TcrtStats()
         self._ck(self._lib.tcrt_wait(self._h, ticket, C.byref(st)))

@@ -39,6 +39,8 @@ constexpr int kChunkStreams = TCRT_CHUNK_STREAMS;   // streams their launches al
 struct FrameRes {
     float* frame = nullptr;                   // the band, (x1-x0)*height*3 floats, x-major
     size_t frame_cap = 0;                     // floats
+    unsigned char* frame8 = nullptr;          // the band quantised to 8 bits, (x1-x0)*height*3 bytes, x-major (RGB8 frames)
+    size_t frame8_cap = 0;                    // bytes
     int x0 = 0, x1 = 0, height = 0;
     unsigned char* ctl = nullptr;             // queue head @0, ray counters @8..31, queue heads of the column chunks @64 (kMaxChunks x u32)
     unsigned long long* h_counters = nullptr; // pinned, 4 x u64 (slot 0 unused)
@@ -187,6 +189,7 @@ void free_device(DeviceState& d) {
     cudaFree(d.scene_mem);
     for (FrameRes& f : d.res) {
         cudaFree(f.frame);
+        cudaFree(f.frame8);
         cudaFree(f.ctl);
         cudaFreeHost(f.h_counters);
         if (f.ev_start) cudaEventDestroy(f.ev_start);
@@ -868,7 +871,15 @@ static int ensure_row_order(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p,
 // asynchronous).  kCopyStaged: chunked launches and their events only — the caller moves the chunks out afterwards
 // (copy_out_staged: pageable destinations).  Ignored without host_band.
 enum { kCopyDirect = 0, kCopyStaged = 1 };
-static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, float* host_band, int set, int copies = kCopyDirect) {
+// What crosses the bus: the float32 frame, or (tcrt_render_rgb8) each chunk quantised by one more launch on its stream into
+// the device's byte buffer.  The float frame stays the "last render" either way.
+enum FrameFormat { kFloat32 = 0, kRGB8 = 1 };
+static size_t bytes_per_px(FrameFormat fmt) { return fmt == kRGB8 ? 3 : 3 * sizeof(float); }
+static const char* frame_src(const FrameRes& f, FrameFormat fmt) {
+    return fmt == kRGB8 ? reinterpret_cast<const char*>(f.frame8) : reinterpret_cast<const char*>(f.frame);
+}
+static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, int set, int copies = kCopyDirect,
+                         FrameFormat fmt = kFloat32) {
     if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
     if (!valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
     if (x0 < 0 || x1 > p->width || x0 >= x1) return fail(ctx, TCRT_ERR_INVALID, "bad column range [%d,%d)", x0, x1);
@@ -917,6 +928,10 @@ static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, fl
             const size_t n_floats = (size_t)(d.fr().x1 - d.fr().x0) * p->height * 3;
             int rc = ensure(ctx, d.fr().frame, d.fr().frame_cap, n_floats);
             if (rc) return rc;
+            if (fmt == kRGB8 && host_band) {
+                rc = ensure(ctx, d.fr().frame8, d.fr().frame8_cap, n_floats);
+                if (rc) return rc;
+            }
             CK(ctx, cudaMemsetAsync(d.fr().ctl, 0, 64, d.stream));
             // With a host destination the band is rendered as up to kMaxChunks column chunks; chunk k is copied back on
             // the copy stream while the next chunks render (the output is x-major: a chunk is one contiguous slice).
@@ -970,13 +985,18 @@ static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, fl
                 }
                 if (rc) return rc;
                 if (host_band) {
-                    const size_t off = (size_t)(cx0 - d.fr().x0) * p->height * 3;
+                    const size_t off = (size_t)(cx0 - d.fr().x0) * p->height * 3;     // channels into the band
                     const size_t cnt = (size_t)(cx1 - cx0) * p->height * 3;
+                    if (fmt == kRGB8) {
+                        CK(ctx, tcrt_launch_quantize8(d.fr().frame + off, cnt / 3, d.fr().frame8 + off, ks));
+                        launches++;
+                    }
                     CK(ctx, cudaEventRecord(d.fr().ev_chunk[k], ks));
                     if (copies == kCopyDirect) {
+                        const size_t bpc = bytes_per_px(fmt) / 3;                      // bytes per channel
                         CK(ctx, cudaStreamWaitEvent(d.copy_stream, d.fr().ev_chunk[k], 0));
-                        CK(ctx, cudaMemcpyAsync(host_band + (size_t)(d.fr().x0 - x0) * p->height * 3 + off, d.fr().frame + off,
-                                                cnt * sizeof(float), cudaMemcpyDeviceToHost, d.copy_stream));
+                        CK(ctx, cudaMemcpyAsync(static_cast<char*>(host_band) + ((size_t)(d.fr().x0 - x0) * p->height * 3 + off) * bpc,
+                                                frame_src(d.fr(), fmt) + off * bpc, cnt * bpc, cudaMemcpyDeviceToHost, d.copy_stream));
                     }
                 }
             }
@@ -1063,9 +1083,10 @@ static int render_finish(tcrt_ctx* ctx, int set, tcrt_stats* stats) {
     return TCRT_OK;
 }
 
-static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, float* host_band);
+static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, void* host_band, FrameFormat fmt);
 
-static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, float* host_band, tcrt_stats* stats) {
+static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, tcrt_stats* stats,
+                       FrameFormat fmt = kFloat32) {
     if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
     const int set = ctx->devs[0].cur;
     // A pageable destination (a plain malloc'd / std::vector / numpy buffer): cudaMemcpyAsync would block the calling
@@ -1081,10 +1102,10 @@ static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, floa
             staged = at.type == cudaMemoryTypeUnregistered;
         }
     }
-    int rc = render_submit(ctx, p, x0, x1, host_band, set, staged ? kCopyStaged : kCopyDirect);
+    int rc = render_submit(ctx, p, x0, x1, host_band, set, staged ? kCopyStaged : kCopyDirect, fmt);
     if (rc) return rc;
     if (staged) {
-        rc = copy_out_staged(ctx, p, x0, host_band);
+        rc = copy_out_staged(ctx, p, x0, host_band, fmt);
         if (rc) {
             render_finish(ctx, set, nullptr);
             return rc;
@@ -1181,18 +1202,38 @@ int tcrt_render_device(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, tcrt
     return render_impl(ctx, p, x0, x1, nullptr, stats);
 }
 
-int tcrt_render_async(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, float* host_rgb_band, int* ticket) {
+static int render_async_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, int* ticket, FrameFormat fmt) {
     if (!ctx || !ticket) return fail(ctx, TCRT_ERR_INVALID, "null argument");
     // the set that is not pending; with none pending, the one the last frame did not use (its band may still be wanted)
     int set = ctx->pend[0].active ? 1 : (ctx->pend[1].active ? 0 : 1 - ctx->devs[0].cur);
     if (ctx->pend[set].active) return fail(ctx, TCRT_ERR_INVALID, "two frames are already in flight: tcrt_wait for one first");
     const int keep = ctx->devs[0].cur;
-    int rc = render_submit(ctx, p, x0, x1, host_rgb_band, set);
+    int rc = render_submit(ctx, p, x0, x1, host_band, set, kCopyDirect, fmt);
     if (rc) return rc;
     // the "last frame" of the synchronous calls (tcrt_download, the writers) stays what it was until tcrt_wait
     for (auto& d : ctx->devs) d.cur = keep;
     *ticket = set;
     return TCRT_OK;
+}
+
+int tcrt_render_async(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, float* host_rgb_band, int* ticket) {
+    return render_async_impl(ctx, p, x0, x1, host_rgb_band, ticket, kFloat32);
+}
+
+// ---- 8-bit frames: the same calls, each column chunk quantised on the device before it crosses the bus --------------
+int tcrt_render_rgb8(tcrt_ctx* ctx, const tcrt_params* p, unsigned char* host_rgb8, tcrt_stats* stats) {
+    if (!host_rgb8) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
+    if (!p) return fail(ctx, TCRT_ERR_INVALID, "null params");
+    return render_impl(ctx, p, 0, p->width, host_rgb8, stats, kRGB8);
+}
+int tcrt_render_columns_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, unsigned char* host_rgb8_band,
+                             tcrt_stats* stats) {
+    if (!host_rgb8_band) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
+    return render_impl(ctx, p, x0, x1, host_rgb8_band, stats, kRGB8);
+}
+int tcrt_render_async_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, unsigned char* host_rgb8_band, int* ticket) {
+    if (!host_rgb8_band) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
+    return render_async_impl(ctx, p, x0, x1, host_rgb8_band, ticket, kRGB8);
 }
 
 int tcrt_wait(tcrt_ctx* ctx, int ticket, tcrt_stats* stats) {
@@ -1216,7 +1257,7 @@ int tcrt_download(tcrt_ctx* ctx, float* host_band) {
         if (pageable) {
             tcrt_params p{};
             p.height = ctx->frame_h;
-            return copy_out_staged(ctx, &p, ctx->frame_x0, host_band);
+            return copy_out_staged(ctx, &p, ctx->frame_x0, host_band, kFloat32);
         }
     }
     for (auto& d : ctx->devs) {
@@ -1846,8 +1887,10 @@ int n_txt_workers() {
 
 // The band of the frame just submitted with kCopyStaged -> pageable host memory: chunk after chunk (as their kernels
 // finish) into the pinned staging slots of the .txt writer at bus speed, from there by worker threads into host_band.
-static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, float* host_band) {
+// fmt picks the device buffer (float frame or its 8-bit copy) and the bytes per pixel.
+static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, void* host_band, FrameFormat fmt) {
     const size_t slot_bytes = kTxtChunkPx * kTxtLine;
+    const size_t bpp = bytes_per_px(fmt);
     if (!ctx->copy_pipe) {      // the workers live as long as the ctx: starting eight threads costs as much as a 1080p frame
         ctx->copy_sink = new TxtSink();
         ctx->copy_pipe = new TxtPipe();
@@ -1876,21 +1919,23 @@ static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, float* h
         const int n_chunks = std::max(1, f.n_chunks);
         for (int k = 0; k < n_chunks && e == cudaSuccess; k++) {
             const int cx0 = f.n_chunks ? f.chunk_x[k] : f.x0, cx1 = f.n_chunks ? f.chunk_x[k + 1] : f.x1;
-            const size_t c0 = (size_t)(cx0 - f.x0) * p->height * 12, c1 = (size_t)(cx1 - f.x0) * p->height * 12;
+            const size_t c0 = (size_t)(cx0 - f.x0) * p->height * bpp, c1 = (size_t)(cx1 - f.x0) * p->height * bpp;
             if (c1 <= c0) continue;
-            if (f.n_chunks > 1) e = cudaStreamWaitEvent(d.copy_stream, f.ev_chunk[k], 0);
+            // every chunk, the only one of a band too (a device band of a multi-device frame can be a single chunk although
+            // the frame is large enough to be staged): the copy stream is not ordered behind the render streams otherwise
+            if (f.n_chunks) e = cudaStreamWaitEvent(d.copy_stream, f.ev_chunk[k], 0);
             for (size_t b = c0; b < c1 && e == cudaSuccess; b += slot_bytes, piece++) {
                 const int slot = (int)(piece % kTxtSlots);
                 const size_t n = std::min(slot_bytes, c1 - b);
                 pipe.wait_slot(&slot_busy[slot]);
                 char* stage = d.txt_stage + slot * slot_bytes;
-                e = cudaMemcpyAsync(stage, reinterpret_cast<const char*>(f.frame) + b, n, cudaMemcpyDeviceToHost, d.copy_stream);
+                e = cudaMemcpyAsync(stage, frame_src(f, fmt) + b, n, cudaMemcpyDeviceToHost, d.copy_stream);
                 if (e == cudaSuccess) e = cudaEventRecord(d.ev_txt[slot], d.copy_stream);
                 if (e != cudaSuccess) break;
                 const int parts = n >= (size_t)kTxtParts * 65536 ? kTxtParts : 1;
                 slot_busy[slot] = 1;
                 left[slot].store(parts);
-                const size_t dst = (size_t)(f.x0 - x0) * p->height * 12 + b;
+                const size_t dst = (size_t)(f.x0 - x0) * p->height * bpp + b;
                 for (int q = 0; q < parts; q++) {
                     const size_t b0 = n * q / parts, b1 = n * (q + 1) / parts;
                     pipe.push({d.dev, d.ev_txt[slot], stage + b0, dst + b0, b1 - b0, &left[slot], &slot_busy[slot]});

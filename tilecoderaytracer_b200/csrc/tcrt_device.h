@@ -162,6 +162,9 @@ cudaError_t tcrt_launch_txt_general(const float* rgb, size_t n_pixels, const uns
                                     const unsigned long long* block_offs, char* text, cudaStream_t stream);
 // 8-bit quantisation + transposition of an x-major band (cols x height) into image rows (top row first, cols pixels each)
 cudaError_t tcrt_launch_quantize8_image(const float* rgb, int cols, int height, unsigned char* out, cudaStream_t stream);
+// 8-bit quantisation in place order (the RGB8 frames of tcrt_render_rgb8): byte j of out = q(rgb[j]), j < 3*n_pixels.
+// Any start address of either buffer.
+cudaError_t tcrt_launch_quantize8(const float* rgb, size_t n_pixels, unsigned char* out, cudaStream_t stream);
 cudaError_t tcrt_launch_l2_flush(void* scratch, size_t bytes, cudaStream_t stream);
 // 8 independent chains per thread, `iters` rounds: 8*iters FFMA, or 8*iters FMUL + 8*iters FADD
 cudaError_t tcrt_launch_fp32_peak(bool fma, float* scratch, int grid, int iters, cudaStream_t stream);

@@ -14,6 +14,8 @@
 //           a two-level exclusive scan, then byte stores at the scanned offsets.
 #include "tcrt_device.h"
 
+#include <algorithm>
+
 namespace {
 
 constexpr int kFmtBlock = 256;
@@ -335,6 +337,44 @@ __global__ void __launch_bounds__(256) quantize8_image_kernel(const float* __res
     }
 }
 }  // namespace
+
+// Element-wise q(c) of a run of floats into as many bytes: float j -> byte j, so an x-major band stays x-major (3 bytes a
+// pixel).  `head` scalar elements bring rgb to 16 bytes and out to 4 bytes; the body is one float4 in, one u32 out per
+// thread and step; the rest is the scalar tail.
+__global__ void __launch_bounds__(256) tcrt_quantize8_kernel(const float* __restrict__ rgb, size_t n, size_t head,
+                                                             size_t n_vec, unsigned char* __restrict__ out) {
+    const size_t tid = blockIdx.x * (size_t)blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
+    const float4* in4 = reinterpret_cast<const float4*>(rgb + head);
+    unsigned int* out4 = reinterpret_cast<unsigned int*>(out + head);
+    for (size_t i = tid; i < n_vec; i += stride) {
+        const float4 v = in4[i];
+        out4[i] = (unsigned int)quant8(v.x) | (unsigned int)quant8(v.y) << 8 | (unsigned int)quant8(v.z) << 16 |
+                  (unsigned int)quant8(v.w) << 24;
+    }
+    const size_t tail0 = head + 4 * n_vec;
+    for (size_t i = tid; i < head + (n - tail0); i += stride) {
+        const size_t j = i < head ? i : tail0 + (i - head);
+        out[j] = quant8(rgb[j]);
+    }
+}
+
+cudaError_t tcrt_launch_quantize8(const float* rgb, size_t n_pixels, unsigned char* out, cudaStream_t stream) {
+    if (n_pixels == 0) return cudaSuccess;
+    const size_t n = 3 * n_pixels;
+    // the first element at which both pointers are aligned; a pair that never is (not the case of the frame buffers,
+    // which sit at the same pixel offset of two cudaMalloc blocks) takes the scalar loop alone
+    size_t head = n, n_vec = 0;
+    for (size_t h = 0; h < 4 && h < n; h++)
+        if (((uintptr_t)(rgb + h) & 15) == 0 && ((uintptr_t)(out + h) & 3) == 0) {
+            head = h;
+            n_vec = (n - h) / 4;
+            break;
+        }
+    const size_t work = std::max(n_vec, head + (n - head - 4 * n_vec));
+    const int grid = (int)std::min<size_t>((work + 255) / 256, (size_t)148 * 8);
+    tcrt_quantize8_kernel<<<grid, 256, 0, stream>>>(rgb, n, head, n_vec, out);
+    return cudaGetLastError();
+}
 
 cudaError_t tcrt_launch_quantize8_image(const float* rgb, int cols, int height, unsigned char* out, cudaStream_t stream) {
     if (cols <= 0 || height <= 0) return cudaSuccess;

@@ -136,12 +136,13 @@ typedef struct tcrt_stats {
     int col_begin[TCRT_MAX_DEVICES]; /* band [col_begin, col_end) rendered by each device */
     int col_end[TCRT_MAX_DEVICES];
     double render_ms[TCRT_MAX_DEVICES]; /* kernel time, CUDA events on the launching stream (RGB8 frames: render +
-                                           quantisation) */
+                                           quantisation; supersampled frames: render + resolve) */
     double d2h_ms[TCRT_MAX_DEVICES];    /* copy-back time of the band (0 if none) */
     unsigned long long rays_primary[TCRT_MAX_DEVICES];
     unsigned long long rays_shadow[TCRT_MAX_DEVICES];
     unsigned long long rays_reflect[TCRT_MAX_DEVICES];
-    unsigned long long gpu_launches;    /* kernels launched by this call (RGB8 frames: the quantisation launches too) */
+    unsigned long long gpu_launches;    /* kernels launched by this call (RGB8 frames: the quantisation launches too;
+                                           supersampled frames: the resolve launches too) */
 } tcrt_stats;
 
 /* ---- context ------------------------------------------------------------------- */
@@ -214,6 +215,29 @@ int tcrt_render_columns_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int x0, i
                              tcrt_stats* stats);
 int tcrt_render_async_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int x0, int x1, unsigned char* host_rgb8_band,
                            int* ticket);
+/* Supersampled (anti-aliased) frames: ss x ss samples per pixel, ss = samples per axis, 1 <= ss <= 8.  Sample (i, j),
+ * 0 <= i, j < ss, of output pixel (x, z) is the reference's pixel (ss*x + i, ss*z + j) of the same scene, camera and
+ * params at (ss*width, ss*height): every sample is a value the reference computes, so the grid is anchored at the
+ * pixel's corner as the reference's rays are, and an ss > 1 image is shifted by (ss-1)/(2*ss) pixel against the ss = 1
+ * image.  Resolve, in binary32, in exactly this order: acc = sample(0,0); acc += sample(i,j) for i = 0..ss-1 (outer),
+ * j = 0..ss-1 (inner), skipping (0,0); out = acc / (float)(ss*ss) (IEEE division; no FMA, no pairwise tree; NaN and inf
+ * propagate).  ss = 1 is the plain frame, bit for bit.  ss < 1: TCRT_ERR_INVALID; ss > 8, or ss*width or ss*height above
+ * 2^24 (where (float)x stops being exact): TCRT_ERR_UNSUPPORTED, as is a frame whose column chunks would exceed the
+ * kernels' index range (ss*ss*height*columns of a chunk above 2^31/3 sample channels).
+ * The output is the W x H frame, x-major like tcrt_render, a column band [x0,x1) one contiguous slice; host_rgb_band NULL
+ * leaves it on the device (tcrt_render_device).  The RGB8 forms carry quant8 of the resolved floats (not the mean of
+ * quantised samples); their destination must not be NULL.  The resolved float frame becomes the last render of
+ * tcrt_download, tcrt_device_frame and the writers.  Stats: rays_* count the rays of the whole sample frame,
+ * col_begin/col_end are output columns, render_ms and gpu_launches include the resolve launches.  Pinned and pageable
+ * destinations, multi-device contexts, tcrt_wait and the two frames in flight as in tcrt_render / tcrt_render_async. */
+int tcrt_render_columns_ss(tcrt_ctx* ctx, const tcrt_params* params, int ss, int x0, int x1, float* host_rgb_band,
+                           tcrt_stats* stats);
+int tcrt_render_columns_ss_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int ss, int x0, int x1,
+                                unsigned char* host_rgb8_band, tcrt_stats* stats);
+int tcrt_render_async_ss(tcrt_ctx* ctx, const tcrt_params* params, int ss, int x0, int x1, float* host_rgb_band,
+                         int* ticket);
+int tcrt_render_async_ss_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int ss, int x0, int x1,
+                              unsigned char* host_rgb8_band, int* ticket);
 /* Device address of a device's band of the last render (for zero-copy consumers, e.g. a
  * torch tensor view); floats = (col_end-col_begin)*height*3. */
 int tcrt_device_frame(tcrt_ctx* ctx, int device_slot, void** dev_ptr, size_t* n_floats);

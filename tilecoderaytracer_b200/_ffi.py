@@ -97,6 +97,14 @@ SIGNATURES = {
                                            C.POINTER(TcrtStats)]),
     "tcrt_render_async_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p,
                                          C.POINTER(C.c_int)]),
+    "tcrt_render_columns_ss": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                         C.POINTER(TcrtStats)]),
+    "tcrt_render_columns_ss_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                              C.POINTER(TcrtStats)]),
+    "tcrt_render_async_ss": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                       C.POINTER(C.c_int)]),
+    "tcrt_render_async_ss_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                            C.POINTER(C.c_int)]),
     "tcrt_device_frame": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),

@@ -338,6 +338,62 @@ class Context:
                                                   C.byref(t)))
         return t.value
 
+    def render_ss(self, params: TcrtParams, ss: int, x0: int = 0, x1: Optional[int] = None,
+                  out: Optional[np.ndarray] = None):
+        """Columns [x0,x1) of the supersampled frame: every pixel the mean of its ss x ss samples, sample (i, j) of pixel
+        (x, z) being the reference's pixel (ss*x+i, ss*z+j) at (ss*W, ss*H), summed in the order of tcrt.h and resolved
+        on the GPU.  Returns (array[x1-x0, H, 3] float32, RenderStats); the stats count the rays of the sample frame.
+        The resolved frame becomes the last render."""
+        x1 = params.width if x1 is None else x1
+        shape = (x1 - x0, params.height, 3)
+        if out is None:
+            out = np.empty(shape, dtype=np.float32)
+        assert out.dtype == np.float32 and out.size == int(np.prod(shape)) and out.flags["C_CONTIGUOUS"]
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_columns_ss(self._h, C.byref(params), ss, x0, x1, out.ctypes.data_as(C.c_void_p),
+                                                  C.byref(st)))
+        return out.reshape(shape), RenderStats.from_c(st)
+
+    def render_ss_rgb8(self, params: TcrtParams, ss: int, x0: int = 0, x1: Optional[int] = None,
+                       out: Optional[np.ndarray] = None):
+        """render_ss() quantised to 8 bits on the GPU in the resolve pass (quant8 of the resolved floats); returns
+        (array[x1-x0, H, 3] uint8, RenderStats).  The resolved float frame stays on the device as the last render."""
+        x1 = params.width if x1 is None else x1
+        shape = (x1 - x0, params.height, 3)
+        if out is None:
+            out = np.empty(shape, dtype=np.uint8)
+        assert out.dtype == np.uint8 and out.size == int(np.prod(shape)) and out.flags["C_CONTIGUOUS"]
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_columns_ss_rgb8(self._h, C.byref(params), ss, x0, x1,
+                                                       out.ctypes.data_as(C.c_void_p), C.byref(st)))
+        return out.reshape(shape), RenderStats.from_c(st)
+
+    def render_ss_device(self, params: TcrtParams, ss: int, x0: int = 0, x1: Optional[int] = None) -> RenderStats:
+        """render_ss() left in device memory (download() fetches it), like render_device()."""
+        x1 = params.width if x1 is None else x1
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_columns_ss(self._h, C.byref(params), ss, x0, x1, None, C.byref(st)))
+        return RenderStats.from_c(st)
+
+    def render_async_ss(self, params: TcrtParams, ss: int, x0: int = 0, x1: Optional[int] = None,
+                        out: Optional[np.ndarray] = None) -> int:
+        """render_async() of a supersampled frame (into `out`, pinned host memory, when given)."""
+        x1 = params.width if x1 is None else x1
+        if out is not None:
+            assert out.dtype == np.float32 and out.size == (x1 - x0) * params.height * 3 and out.flags["C_CONTIGUOUS"]
+        t = C.c_int(-1)
+        self._ck(self._lib.tcrt_render_async_ss(self._h, C.byref(params), ss, x0, x1,
+                                                out.ctypes.data_as(C.c_void_p) if out is not None else None, C.byref(t)))
+        return t.value
+
+    def render_async_ss_rgb8(self, params: TcrtParams, ss: int, x0: int, x1: int, out: np.ndarray) -> int:
+        """render_async() of a supersampled 8-bit frame into `out` (uint8, pinned host memory)."""
+        assert out.dtype == np.uint8 and out.size == (x1 - x0) * params.height * 3 and out.flags["C_CONTIGUOUS"]
+        t = C.c_int(-1)
+        self._ck(self._lib.tcrt_render_async_ss_rgb8(self._h, C.byref(params), ss, x0, x1,
+                                                     out.ctypes.data_as(C.c_void_p), C.byref(t)))
+        return t.value
+
     def wait(self, ticket: int) -> RenderStats:
         st = TcrtStats()
         self._ck(self._lib.tcrt_wait(self._h, ticket, C.byref(st)))

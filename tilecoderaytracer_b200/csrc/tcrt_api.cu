@@ -94,6 +94,11 @@ struct DeviceState {
     // L2 flush scratch
     void* flush = nullptr;
     size_t flush_bytes = 0;
+    // supersampled frames: the sample columns of one column chunk, one buffer per render stream (0 = `stream`, then
+    // chunk_stream[]).  The chunk's render launch and its resolve launch run on that stream, and so does every later
+    // chunk that reuses the buffer, so both frame sets share it.
+    float* ss_scratch[kChunkStreams] = {};
+    size_t ss_scratch_cap[kChunkStreams] = {};     // floats
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -209,6 +214,7 @@ void free_device(DeviceState& d) {
     cudaFree(d.row_order);
     cudaFree(d.col_cost);
     cudaFree(d.wave_mem);
+    for (float* s : d.ss_scratch) cudaFree(s);
     cudaFreeHost(d.h_txt);
     cudaFreeHost(d.txt_stage);
     for (auto& e : d.ev_txt)
@@ -860,9 +866,42 @@ int tcrt_rebalance_columns(const int* bounds, const double* ms, int n_bands, int
     return tcrt_bands_from_costs(cost.data(), width, width, n_bands, new_bounds);
 }
 
-static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, unsigned int* col_cost,
+static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, float* out, unsigned int* col_cost,
                        int* launches, cudaStream_t stream = nullptr, unsigned int* queue = nullptr);
 static int ensure_row_order(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, bool pre_pass, const int** out);
+
+// Samples per axis of a supersampled frame (tcrt_render_columns_ss).  At 8 the widest column chunk of a 7680x4320 frame
+// needs 2.2 GB of sample scratch per render stream (DESIGN.md §4.3).
+constexpr int kMaxSS = 8;
+
+// The column chunks of a device band [f.x0, f.x1) -> f.n_chunks, f.chunk_x.  px_per_col: pixels traced per column of the
+// band (ss*ss*height for a supersampled frame).  Unchunked: one launch.  Chunked (a host destination, or a supersampled
+// frame): up to kMaxChunks column chunks.  Chunk k of a band that goes to host memory is copied back on the copy stream
+// while the next chunks render (the output is x-major: a chunk is one contiguous slice).  The chunks are separate launches
+// on kChunkStreams streams, round robin: a launch ends in a tail of half-empty SMs (its deepest paths: 0.13-0.25 ms per
+// launch measured), and with the next chunks' launches already queued on the other streams their CTAs move in as this
+// one's retire.
+static void plan_chunks(FrameRes& f, long long px_per_col, bool chunked) {
+    const int w = f.x1 - f.x0;
+    int n_chunks = 1;
+    if (chunked) {
+        // 256 K pixels (3 MB) or more per chunk: a 1080p frame is 7 chunks (0.56 ms end to end; 3 chunks 0.61 ms,
+        // 15 chunks 0.57 ms), larger frames kMaxChunks
+        const long long chunk_px = 256 * 1024;
+        n_chunks = (int)std::min<long long>(std::min<long long>(kMaxChunks, w), std::max<long long>(1, w * px_per_col / chunk_px));
+    }
+    // chunk boundaries on tile boundaries, so that every chunk of a tileable band is tileable.  With the full
+    // number of chunks the first and the last ones are narrow: the copies start after the first chunk's kernel
+    // and the frame ends with the last chunk's copy, neither of which anything hides.
+    static const int kChunkWeight[kMaxChunks + 1] = {0, 1, 2, 4, 8, 12, 16, 20, 24, 28, 32, 36, 40, 42, 44, 45, 46};
+    for (int j = 0; j <= n_chunks; j++) {
+        int c = n_chunks == kMaxChunks ? (int)((long long)w * kChunkWeight[j] / kChunkWeight[kMaxChunks])
+                                       : (int)((long long)w * j / n_chunks);
+        if (j < n_chunks && w % TCRT_TILE_W == 0) c -= c % TCRT_TILE_W;
+        f.chunk_x[j] = f.x0 + c;
+    }
+    f.n_chunks = n_chunks;
+}
 
 // One frame = submit (everything is queued on the devices' streams, nothing waits) + finish (waits for this
 // frame's events only, reads its timings and ray counters).  `set` picks which of the two FrameRes sets of
@@ -878,8 +917,11 @@ static size_t bytes_per_px(FrameFormat fmt) { return fmt == kRGB8 ? 3 : 3 * size
 static const char* frame_src(const FrameRes& f, FrameFormat fmt) {
     return fmt == kRGB8 ? reinterpret_cast<const char*>(f.frame8) : reinterpret_cast<const char*>(f.frame);
 }
+// ss > 1: a supersampled frame (tcrt_render_columns_ss).  Chunk k of output columns [c0, c1) is one render launch over
+// sample columns [ss*c0, ss*c1) of the sample frame (ss*width x ss*height) into the scratch buffer of its stream, then one
+// resolve launch on that stream into the band's frame (and, for RGB8, its byte buffer).  The caller has checked ss.
 static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, int set, int copies = kCopyDirect,
-                         FrameFormat fmt = kFloat32) {
+                         FrameFormat fmt = kFloat32, int ss = 1) {
     if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
     if (!valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
     if (x0 < 0 || x1 > p->width || x0 >= x1) return fail(ctx, TCRT_ERR_INVALID, "bad column range [%d,%d)", x0, x1);
@@ -913,12 +955,26 @@ static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, vo
         cut = ctx->cut;
     }
     const int prev_cur = ctx->devs[0].cur;
+    const bool super = ss > 1;
+    tcrt_params sp = *p;                // the frame the render launches trace: for a supersampled frame, its sample frame
+    sp.width = ss * p->width;
+    sp.height = ss * p->height;
+    const long long spc = (long long)ss * sp.height;     // pixels traced per output column
     for (int i = 0; i < nd; i++) {
         DeviceState& d = ctx->devs[i];
         d.cur = set;
         d.fr().x0 = cut[i];
         d.fr().x1 = cut[i + 1];
         d.fr().height = p->height;
+        if (d.fr().x1 <= d.fr().x0) continue;
+        plan_chunks(d.fr(), spc, host_band != nullptr || super);
+        // the render kernels index the pixels of a launch with ints (3 floats each)
+        for (int k = 0; super && k < d.fr().n_chunks; k++)
+            if ((long long)(d.fr().chunk_x[k + 1] - d.fr().chunk_x[k]) * spc > 0x7fffffffLL / 3) {
+                for (auto& dd : ctx->devs) dd.cur = prev_cur;
+                return fail(ctx, TCRT_ERR_UNSUPPORTED, "%d x %d at %d x %d samples: a column chunk of the sample frame exceeds "
+                            "the kernels' index range", p->width, p->height, ss, ss);
+            }
     }
     auto submit_all = [&]() -> int {
         for (int i = 0; i < nd; i++) {
@@ -933,36 +989,29 @@ static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, vo
                 if (rc) return rc;
             }
             CK(ctx, cudaMemsetAsync(d.fr().ctl, 0, 64, d.stream));
-            // With a host destination the band is rendered as up to kMaxChunks column chunks; chunk k is copied back on
-            // the copy stream while the next chunks render (the output is x-major: a chunk is one contiguous slice).
-            // The chunks are separate launches on kChunkStreams streams, round robin: a launch ends in a tail of half-empty
-            // SMs (its deepest paths: 0.13-0.25 ms per launch measured), and with the next chunks' launches already queued
-            // on the other streams their CTAs move in as this one's retire.  Without a host destination, a single launch.
-            int n_chunks = 1;
-            if (host_band) {
-                const long long px = (long long)(d.fr().x1 - d.fr().x0) * p->height;
-                // 256 K pixels (3 MB) or more per chunk: a 1080p frame is 7 chunks (0.56 ms end to end; 3 chunks 0.61 ms,
-                // 15 chunks 0.57 ms), larger frames kMaxChunks
-                const long long chunk_px = 256 * 1024;
-                n_chunks = (int)std::min<long long>(std::min<long long>(kMaxChunks, d.fr().x1 - d.fr().x0), std::max<long long>(1, px / chunk_px));
-            }
-            // chunk boundaries on tile boundaries, so that every chunk of a tileable band is tileable.  With the full
-            // number of chunks the first and the last ones are narrow: the copies start after the first chunk's kernel
-            // and the frame ends with the last chunk's copy, neither of which anything hides.
-            static const int kChunkWeight[kMaxChunks + 1] = {0, 1, 2, 4, 8, 12, 16, 20, 24, 28, 32, 36, 40, 42, 44, 45, 46};
-            auto chunk_start = [&](int j) {
-                const int w = d.fr().x1 - d.fr().x0;
-                int c = n_chunks == kMaxChunks ? (int)((long long)w * kChunkWeight[j] / kChunkWeight[kMaxChunks])
-                                               : (int)((long long)w * j / n_chunks);
-                if (j < n_chunks && w % TCRT_TILE_W == 0) c -= c % TCRT_TILE_W;
-                return d.fr().x0 + c;
-            };
+            const int n_chunks = d.fr().n_chunks;
+            const int* chunk_x = d.fr().chunk_x;
             const bool two_streams = n_chunks > 1 && !ctx->one_stream;   // (several streams)
+            if (super) {       // sample scratch for the widest chunk, on every stream the chunks use
+                int widest = 0;
+                for (int k = 0; k < n_chunks; k++) widest = std::max(widest, chunk_x[k + 1] - chunk_x[k]);
+                const size_t need = (size_t)widest * spc * 3;
+                const int n_bufs = two_streams ? std::min(kChunkStreams, n_chunks) : 1;
+                for (int si = 0; si < n_bufs; si++)     // a buffer about to be replaced may still serve the other frame set
+                    if (need > d.ss_scratch_cap[si]) {
+                        CK(ctx, cudaDeviceSynchronize());
+                        break;
+                    }
+                for (int si = 0; si < n_bufs; si++) {
+                    rc = ensure(ctx, d.ss_scratch[si], d.ss_scratch_cap[si], need);
+                    if (rc) return rc;
+                }
+            }
             if (two_streams) {
                 // everything the launches on the second stream read must be in place: queue heads, counters, row order
                 CK(ctx, cudaMemsetAsync(d.fr().ctl + 64, 0, kMaxChunks * sizeof(unsigned int), d.stream));
                 const int* unused = nullptr;
-                rc = ensure_row_order(ctx, d, p, chunk_start(0), chunk_start(1), false, &unused);
+                rc = ensure_row_order(ctx, d, &sp, ss * chunk_x[0], ss * chunk_x[1], false, &unused);
                 if (rc) return rc;
                 CK(ctx, cudaEventRecord(d.fr().ev_start, d.stream));
                 for (auto& cs : d.chunk_stream) CK(ctx, cudaStreamWaitEvent(cs, d.fr().ev_start, 0));
@@ -971,28 +1020,35 @@ static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, vo
             int last_on[kChunkStreams];
             for (int& l : last_on) l = -1;
             for (int k = 0; k < n_chunks; k++) {
-                const int cx0 = chunk_start(k), cx1 = chunk_start(k + 1);
+                const int cx0 = chunk_x[k], cx1 = chunk_x[k + 1];
                 if (cx1 <= cx0) continue;
+                const size_t off = (size_t)(cx0 - d.fr().x0) * p->height * 3;     // channels into the band
+                const size_t cnt = (size_t)(cx1 - cx0) * p->height * 3;
                 cudaStream_t ks = d.stream;
+                const int si = two_streams ? k % kChunkStreams : 0;
+                float* out = super ? d.ss_scratch[si] : d.fr().frame + off;
                 if (two_streams) {
-                    const int si = k % kChunkStreams;
                     if (si > 0) ks = d.chunk_stream[si - 1];
                     last_on[si] = k;
-                    rc = launch_band(ctx, d, p, cx0, cx1, nullptr, &launches, ks, reinterpret_cast<unsigned int*>(d.fr().ctl + 64) + k);
+                    rc = launch_band(ctx, d, &sp, ss * cx0, ss * cx1, out, nullptr, &launches, ks,
+                                     reinterpret_cast<unsigned int*>(d.fr().ctl + 64) + k);
                 } else {
                     if (k > 0) CK(ctx, cudaMemsetAsync(d.fr().ctl, 0, 4, d.stream));   // queue head only; ray counters accumulate
-                    rc = launch_band(ctx, d, p, cx0, cx1, nullptr, &launches);
+                    rc = launch_band(ctx, d, &sp, ss * cx0, ss * cx1, out, nullptr, &launches);
                 }
                 if (rc) return rc;
-                if (host_band) {
-                    const size_t off = (size_t)(cx0 - d.fr().x0) * p->height * 3;     // channels into the band
-                    const size_t cnt = (size_t)(cx1 - cx0) * p->height * 3;
-                    if (fmt == kRGB8) {
+                if (super) {
+                    CK(ctx, tcrt_launch_resolve_ss(out, cx1 - cx0, p->height, ss, d.fr().frame + off,
+                                                   fmt == kRGB8 && host_band ? d.fr().frame8 + off : nullptr, ks));
+                    launches++;
+                }
+                if (host_band || super) {
+                    if (host_band && fmt == kRGB8 && !super) {
                         CK(ctx, tcrt_launch_quantize8(d.fr().frame + off, cnt / 3, d.fr().frame8 + off, ks));
                         launches++;
                     }
                     CK(ctx, cudaEventRecord(d.fr().ev_chunk[k], ks));
-                    if (copies == kCopyDirect) {
+                    if (host_band && copies == kCopyDirect) {
                         const size_t bpc = bytes_per_px(fmt) / 3;                      // bytes per channel
                         CK(ctx, cudaStreamWaitEvent(d.copy_stream, d.fr().ev_chunk[k], 0));
                         CK(ctx, cudaMemcpyAsync(static_cast<char*>(host_band) + ((size_t)(d.fr().x0 - x0) * p->height * 3 + off) * bpc,
@@ -1000,8 +1056,6 @@ static int render_submit(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, vo
                     }
                 }
             }
-            d.fr().n_chunks = n_chunks;
-            for (int k = 0; k <= n_chunks; k++) d.fr().chunk_x[k] = chunk_start(k);
             for (int si = 1; si < kChunkStreams; si++)      // the frame ends on d.stream
                 if (last_on[si] >= 0) CK(ctx, cudaStreamWaitEvent(d.stream, d.fr().ev_chunk[last_on[si]], 0));
             CK(ctx, cudaEventRecord(d.fr().ev_k1, d.stream));
@@ -1086,7 +1140,7 @@ static int render_finish(tcrt_ctx* ctx, int set, tcrt_stats* stats) {
 static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, void* host_band, FrameFormat fmt);
 
 static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, tcrt_stats* stats,
-                       FrameFormat fmt = kFloat32) {
+                       FrameFormat fmt = kFloat32, int ss = 1) {
     if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
     const int set = ctx->devs[0].cur;
     // A pageable destination (a plain malloc'd / std::vector / numpy buffer): cudaMemcpyAsync would block the calling
@@ -1102,7 +1156,7 @@ static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void
             staged = at.type == cudaMemoryTypeUnregistered;
         }
     }
-    int rc = render_submit(ctx, p, x0, x1, host_band, set, staged ? kCopyStaged : kCopyDirect, fmt);
+    int rc = render_submit(ctx, p, x0, x1, host_band, set, staged ? kCopyStaged : kCopyDirect, fmt, ss);
     if (rc) return rc;
     if (staged) {
         rc = copy_out_staged(ctx, p, x0, host_band, fmt);
@@ -1114,9 +1168,9 @@ static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void
     return render_finish(ctx, set, stats);
 }
 
-// Columns [cx0, cx1) of device d's band [d.fr().x0, d.fr().x1) of the frame `p`, into the band's frame buffer.
-// The caller has sized the buffer and zeroed the queue head.
-static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, unsigned int* col_cost,
+// Columns [cx0, cx1) of the frame `p` into out[(cx1-cx0)*p->height*3] (a slice of the band's frame buffer, or the sample
+// scratch of a supersampled frame, whose `p` is then the sample frame).  The caller has sized out and zeroed the queue head.
+static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, float* out, unsigned int* col_cost,
                        int* launches, cudaStream_t stream, unsigned int* queue) {
     if (!stream) stream = d.stream;
     RenderLaunch rl{};
@@ -1134,7 +1188,7 @@ static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int 
     rl.null_b = p->null_color[2];
     rl.far_dist = p->far_dist;
     rl.n_objects = ctx->n_objects;
-    rl.out = d.fr().frame + (size_t)(cx0 - d.fr().x0) * p->height * 3;
+    rl.out = out;
     rl.queue = queue ? queue : reinterpret_cast<unsigned int*>(d.fr().ctl);
     rl.counters = reinterpret_cast<unsigned long long*>(d.fr().ctl + 8);
     rl.col_cost = col_cost;
@@ -1202,13 +1256,14 @@ int tcrt_render_device(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, tcrt
     return render_impl(ctx, p, x0, x1, nullptr, stats);
 }
 
-static int render_async_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, int* ticket, FrameFormat fmt) {
+static int render_async_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void* host_band, int* ticket, FrameFormat fmt,
+                             int ss = 1) {
     if (!ctx || !ticket) return fail(ctx, TCRT_ERR_INVALID, "null argument");
     // the set that is not pending; with none pending, the one the last frame did not use (its band may still be wanted)
     int set = ctx->pend[0].active ? 1 : (ctx->pend[1].active ? 0 : 1 - ctx->devs[0].cur);
     if (ctx->pend[set].active) return fail(ctx, TCRT_ERR_INVALID, "two frames are already in flight: tcrt_wait for one first");
     const int keep = ctx->devs[0].cur;
-    int rc = render_submit(ctx, p, x0, x1, host_band, set, kCopyDirect, fmt);
+    int rc = render_submit(ctx, p, x0, x1, host_band, set, kCopyDirect, fmt, ss);
     if (rc) return rc;
     // the "last frame" of the synchronous calls (tcrt_download, the writers) stays what it was until tcrt_wait
     for (auto& d : ctx->devs) d.cur = keep;
@@ -1234,6 +1289,39 @@ int tcrt_render_columns_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1
 int tcrt_render_async_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, unsigned char* host_rgb8_band, int* ticket) {
     if (!host_rgb8_band) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
     return render_async_impl(ctx, p, x0, x1, host_rgb8_band, ticket, kRGB8);
+}
+
+// ---- supersampled frames: ss x ss samples of the reference's frame at (ss*width, ss*height) per pixel, box-filtered ------
+// ss = 1 is the plain frame through the plain path.
+static int check_ss(tcrt_ctx* ctx, const tcrt_params* p, int ss) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
+    if (ss < 1) return fail(ctx, TCRT_ERR_INVALID, "samples per axis %d < 1", ss);
+    if (ss > kMaxSS) return fail(ctx, TCRT_ERR_UNSUPPORTED, "samples per axis %d > %d", ss, kMaxSS);
+    // the kernels map sample column x to (float)x / (float)(ss*width): exact up to 2^24
+    if (p && ((long long)ss * p->width > (1LL << 24) || (long long)ss * p->height > (1LL << 24)))
+        return fail(ctx, TCRT_ERR_UNSUPPORTED, "sample frame %lld x %lld: above 2^24 columns or rows",
+                    (long long)ss * p->width, (long long)ss * p->height);
+    return TCRT_OK;
+}
+int tcrt_render_columns_ss(tcrt_ctx* ctx, const tcrt_params* p, int ss, int x0, int x1, float* host_rgb_band, tcrt_stats* stats) {
+    const int rc = check_ss(ctx, p, ss);
+    return rc ? rc : render_impl(ctx, p, x0, x1, host_rgb_band, stats, kFloat32, ss);
+}
+int tcrt_render_columns_ss_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int ss, int x0, int x1, unsigned char* host_rgb8_band,
+                                tcrt_stats* stats) {
+    if (!host_rgb8_band) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
+    const int rc = check_ss(ctx, p, ss);
+    return rc ? rc : render_impl(ctx, p, x0, x1, host_rgb8_band, stats, kRGB8, ss);
+}
+int tcrt_render_async_ss(tcrt_ctx* ctx, const tcrt_params* p, int ss, int x0, int x1, float* host_rgb_band, int* ticket) {
+    const int rc = check_ss(ctx, p, ss);
+    return rc ? rc : render_async_impl(ctx, p, x0, x1, host_rgb_band, ticket, kFloat32, ss);
+}
+int tcrt_render_async_ss_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int ss, int x0, int x1, unsigned char* host_rgb8_band,
+                              int* ticket) {
+    if (!host_rgb8_band) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
+    const int rc = check_ss(ctx, p, ss);
+    return rc ? rc : render_async_impl(ctx, p, x0, x1, host_rgb8_band, ticket, kRGB8, ss);
 }
 
 int tcrt_wait(tcrt_ctx* ctx, int ticket, tcrt_stats* stats) {
@@ -1338,7 +1426,7 @@ int tcrt_balance_columns(tcrt_ctx* ctx, const tcrt_params* p, int n_bands, int* 
     cudaError_t e = cudaMemsetAsync(col_cost, 0, sizeof(unsigned int) * n_cost, d.stream);
     if (e == cudaSuccess) rc = ensure(ctx, d.fr().frame, d.fr().frame_cap, (size_t)lp.width * lp.height * 3);
     if (e == cudaSuccess && rc == TCRT_OK) e = cudaMemsetAsync(d.fr().ctl, 0, 64, d.stream);
-    if (e == cudaSuccess && rc == TCRT_OK) rc = launch_band(ctx, d, &lp, 0, lp.width, col_cost, &launches);
+    if (e == cudaSuccess && rc == TCRT_OK) rc = launch_band(ctx, d, &lp, 0, lp.width, d.fr().frame, col_cost, &launches);
     if (e == cudaSuccess && rc == TCRT_OK)
         e = cudaMemcpyAsync(h.data(), col_cost, sizeof(unsigned int) * n_cost, cudaMemcpyDeviceToHost, d.stream);
     if (e == cudaSuccess && rc == TCRT_OK) e = cudaStreamSynchronize(d.stream);

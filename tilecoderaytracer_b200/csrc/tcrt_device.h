@@ -165,6 +165,11 @@ cudaError_t tcrt_launch_quantize8_image(const float* rgb, int cols, int height, 
 // 8-bit quantisation in place order (the RGB8 frames of tcrt_render_rgb8): byte j of out = q(rgb[j]), j < 3*n_pixels.
 // Any start address of either buffer.
 cudaError_t tcrt_launch_quantize8(const float* rgb, size_t n_pixels, unsigned char* out, cudaStream_t stream);
+// Supersampled frames (tcrt_render_columns_ss): cols x height output pixels, x-major, each the mean of its ss x ss samples
+// in `samples` (ss*cols x ss*height sample pixels, x-major, 1 <= ss <= 8) summed in the order of tcrt.h; out8 (nullable)
+// gets the same pixels quantised to 8 bits in the same pass.  samples must be 16-byte aligned.
+cudaError_t tcrt_launch_resolve_ss(const float* samples, int cols, int height, int ss, float* out, unsigned char* out8,
+                                   cudaStream_t stream);
 cudaError_t tcrt_launch_l2_flush(void* scratch, size_t bytes, cudaStream_t stream);
 // 8 independent chains per thread, `iters` rounds: 8*iters FFMA, or 8*iters FMUL + 8*iters FADD
 cudaError_t tcrt_launch_fp32_peak(bool fma, float* scratch, int grid, int iters, cudaStream_t stream);

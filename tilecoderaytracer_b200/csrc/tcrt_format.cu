@@ -376,6 +376,72 @@ cudaError_t tcrt_launch_quantize8(const float* rgb, size_t n_pixels, unsigned ch
     return cudaGetLastError();
 }
 
+// ---- supersampled frames: the box filter over SS x SS samples per pixel -------------------------------------------------
+// samples: SS*cols sample columns of SS*height sample rows, x-major; sample (i, j) of output pixel (x, z) is sample pixel
+// (SS*x + i, SS*z + j).  For fixed i the SS samples of a pixel are one run of 3*SS contiguous floats, and the run of pixel
+// z+1 follows it: one thread per output pixel with z fastest makes a warp read 32 consecutive runs.  The runs are loaded
+// as float4 (SS % 4 == 0) or float2 (SS even) — every run and every sample column then starts at a multiple of that
+// width — and as floats otherwise.  The sum is the contract of tcrt_render_columns_ss: acc = sample (0,0), then += in
+// i-major, j-minor order, then one IEEE division by SS*SS.  out8 (optional) gets quant8 of the resolved floats.
+namespace {
+template <int SS>
+__global__ void __launch_bounds__(256) resolve_ss_kernel(const float* __restrict__ samples, int cols, int height,
+                                                         float* __restrict__ out, unsigned char* __restrict__ out8) {
+    constexpr int V = SS % 4 == 0 ? 4 : (SS % 2 == 0 ? 2 : 1);     // floats per load
+    constexpr int R = 3 * SS;                                      // floats per run
+    const long long px = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (px >= (long long)cols * height) return;
+    const int x = (int)(px / height), z = (int)(px - (long long)x * height);
+    const size_t col = (size_t)SS * height * 3;                    // floats per sample column
+    const float* s = samples + (size_t)SS * x * col + (size_t)R * z;
+    float acc[3] = {0.f, 0.f, 0.f};    // set to sample (0,0) below
+#pragma unroll
+    for (int i = 0; i < SS; i++) {
+        float run[R];
+#pragma unroll
+        for (int k = 0; k < R; k += V) {
+            if constexpr (V == 4) {
+                const float4 v = __ldg(reinterpret_cast<const float4*>(s + i * col + k));
+                run[k] = v.x; run[k + 1] = v.y; run[k + 2] = v.z; run[k + 3] = v.w;
+            } else if constexpr (V == 2) {
+                const float2 v = __ldg(reinterpret_cast<const float2*>(s + i * col + k));
+                run[k] = v.x; run[k + 1] = v.y;
+            } else {
+                run[k] = __ldg(s + i * col + k);
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < SS; j++)
+#pragma unroll
+            for (int c = 0; c < 3; c++) acc[c] = (i == 0 && j == 0) ? run[c] : __fadd_rn(acc[c], run[3 * j + c]);
+    }
+#pragma unroll
+    for (int c = 0; c < 3; c++) {
+        const float v = __fdiv_rn(acc[c], (float)(SS * SS));
+        out[px * 3 + c] = v;
+        if (out8) out8[px * 3 + c] = quant8(v);
+    }
+}
+}  // namespace
+
+cudaError_t tcrt_launch_resolve_ss(const float* samples, int cols, int height, int ss, float* out, unsigned char* out8,
+                                   cudaStream_t stream) {
+    if (cols <= 0 || height <= 0) return cudaSuccess;
+    const int grid = (int)(((long long)cols * height + 255) / 256);
+    switch (ss) {
+        case 1: resolve_ss_kernel<1><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 2: resolve_ss_kernel<2><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 3: resolve_ss_kernel<3><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 4: resolve_ss_kernel<4><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 5: resolve_ss_kernel<5><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 6: resolve_ss_kernel<6><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 7: resolve_ss_kernel<7><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        case 8: resolve_ss_kernel<8><<<grid, 256, 0, stream>>>(samples, cols, height, out, out8); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
 cudaError_t tcrt_launch_quantize8_image(const float* rgb, int cols, int height, unsigned char* out, cudaStream_t stream) {
     if (cols <= 0 || height <= 0) return cudaSuccess;
     const long long tiles = (long long)((cols + 31) / 32) * ((height + 31) / 32);

@@ -75,6 +75,21 @@ public:
         run_time_s_ = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         return rc_;
     }
+    // what is at each pixel of the frame rs describes (tcrt_hit_buffers), x-major like render: obj[x*H + z] the object
+    // index of the primary ray's nearest hit (-1: miss), dist[x*H + z] its distance, normal[(x*H + z)*3 + c] its normal;
+    // a NULL pointer is not copied back.  The last render is not touched.  Not for rs.samples != 1.
+    int hitBuffers(const RenderSettings& rs, int* obj, float* dist, float* normal, tcrt_stats* stats = NULL) {
+        if (rs.samples != 1) return rc_ = TCRT_ERR_UNSUPPORTED;
+        tcrt_params p = rs.params();
+        return rc_ = tcrt_hit_buffers(ctx_, &p, 0, p.width, obj, dist, normal, stats);
+    }
+    // the object under pixel (x, z) (tcrt_pick), its distance and normal (3 floats); any pointer may be NULL
+    int pick(const RenderSettings& rs, int x, int z, int* obj, float* dist = NULL, float* normal3 = NULL) {
+        if (rs.samples != 1) return rc_ = TCRT_ERR_UNSUPPORTED;
+        tcrt_params p = rs.params();
+        const int xz[2] = {x, z};
+        return rc_ = tcrt_pick(ctx_, &p, 1, xz, obj, dist, normal3);
+    }
     // init_log + printPixelsToLog (RayTracer.cpp:2022-2061,1574-1626)
     int printPixelsToLog(const char* path = LOG_FILE_NAME) {
         tcrt_params p = settings_.params();

@@ -241,6 +241,40 @@ int tcrt_render_async_ss_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int ss, 
 /* Device address of a device's band of the last render (for zero-copy consumers, e.g. a
  * torch tensor view); floats = (col_end-col_begin)*height*3. */
 int tcrt_device_frame(tcrt_ctx* ctx, int device_slot, void** dev_ptr, size_t* n_floats);
+/* Primary-hit buffers: what is at each pixel.  For pixel (x, z) of the params.width x params.height frame:
+ *   - primary ray: the ray the render traces (Camera::createEyeRay at x / W, z / H);
+ *   - nearest hit: the reference's getCollision (RayTracer.cpp:50-89), lexicographic on (distance, object index); hits at
+ *     or beyond far_dist are invisible; lights are objects like any other;
+ *   - object (int32): the object index of the nearest hit (its position in the scene's list, as in tcrt_scene), -1 on
+ *     a miss;
+ *   - distance (float32): the winning primitive's distance exactly as the reference computes it; negative when the eye
+ *     is inside a sphere (SceneSphere.cpp:139); far_dist on a miss;
+ *   - normal (3 x float32): the direction of the hit's normal ray (CollisionObject, SceneObject.h:47-105): the
+ *     primitive's normal re-normalised by Ray(point, normal), for planes the side facing the ray (computeNormal);
+ *     (+0, +0, +0) on a miss.
+ * The result does not depend on max_depth, shadows_on, reflections_on or null_color.  Layout x-major like frames:
+ * object[(x-x0)*H + z], distance[(x-x0)*H + z], normal[((x-x0)*H + z)*3 + c]; a column band is one contiguous slice of
+ * each buffer.  Supersampled hit buffers do not exist.
+ *
+ * tcrt_hit_buffers: columns [x0, x1).  All three buffers are computed on the device (20 B per pixel); a NULL host pointer
+ * is not copied back, all three NULL leaves them on the device only (tcrt_device_hit_buffers).  Pinned and pageable
+ * destinations as in tcrt_render.  A multi-device ctx computes one band of equal width per device.  Stats: col_begin /
+ * col_end per device, render_ms = kernel time, d2h_ms as for frames, rays_primary = pixels, no shadow or reflection
+ * rays, gpu_launches = kernel launches.  Errors as for frames.
+ * tcrt_device_hit_buffers: device addresses of a device's band of the last tcrt_hit_buffers call, n_pixels per buffer
+ * (normal holds 3 * n_pixels floats); TCRT_ERR_NO_FRAME before the first call.
+ * tcrt_pick: the hits of n pixels xz[2i] = x, xz[2i+1] = z on device slot 0, into object[i], distance[i],
+ * normal[3i..3i+2]; each output pointer may be NULL.  n = 0 launches nothing.  A pixel outside the frame is
+ * TCRT_ERR_INVALID and nothing is written.
+ * None of these calls changes the last render (tcrt_download, tcrt_device_frame, the writers), the multi-device cut or
+ * cost map, or a frame in flight: they have buffers of their own, may be called while two frames are in flight and do
+ * not count as one.  They trace with the camera of tcrt_set_camera, like frames. */
+int tcrt_hit_buffers(tcrt_ctx* ctx, const tcrt_params* params, int x0, int x1, int* host_object, float* host_distance,
+                     float* host_normal, tcrt_stats* stats);
+int tcrt_device_hit_buffers(tcrt_ctx* ctx, int device_slot, int** object, float** distance, float** normal,
+                            size_t* n_pixels);
+int tcrt_pick(tcrt_ctx* ctx, const tcrt_params* params, int n, const int* xz, int* object, float* distance,
+              float* normal);
 /* Cost-balanced column bands (replaces the equal z-bands of the reference's strategy 1,
  * RayTracer.cpp:904-906, whose load imbalance strategies 2-7 and PixelQueue were written to fix).
  * Renders a low-resolution copy of the frame on device slot 0 in which every finished pixel adds its

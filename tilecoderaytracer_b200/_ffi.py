@@ -106,6 +106,11 @@ SIGNATURES = {
     "tcrt_render_async_ss_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_void_p,
                                             C.POINTER(C.c_int)]),
     "tcrt_device_frame": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
+    "tcrt_hit_buffers": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.POINTER(TcrtStats)]),
+    "tcrt_device_hit_buffers": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
+                                          C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
+    "tcrt_pick": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),
     "tcrt_bands_from_costs": (C.c_int, [C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),

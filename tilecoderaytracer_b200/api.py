@@ -403,6 +403,56 @@ class Context:
         self._ck(self._lib.tcrt_download(self._h, out.ctypes.data_as(C.c_void_p)))
         return out
 
+    HIT_BUFFERS = (("object", np.int32, ()), ("distance", np.float32, ()), ("normal", np.float32, (3,)))
+
+    def hit_buffers(self, params: TcrtParams, x0: int = 0, x1: Optional[int] = None, out: Optional[dict] = None):
+        """What is at each pixel of columns [x0,x1), computed on the GPU (tcrt_hit_buffers): "object" (cols, H) int32, the
+        object index of the primary ray's nearest hit or -1; "distance" (cols, H) float32, its distance (far_dist on a
+        miss); "normal" (cols, H, 3) float32, its normal ray's direction ((0,0,0) on a miss).  x-major like render().
+        `out` maps some of these names to C-contiguous destinations (pinned or pageable); only those are copied back and
+        returned.  Returns (dict, RenderStats).  The last render is not touched."""
+        x1 = params.width if x1 is None else x1
+        cols, h = x1 - x0, params.height
+        if out is None:
+            out = {name: np.empty((cols, h) + tail, dtype) for name, dtype, tail in self.HIT_BUFFERS}
+        ptrs = []
+        for name, dtype, tail in self.HIT_BUFFERS:
+            a = out.get(name)
+            if a is not None:
+                assert a.dtype == dtype and a.size == cols * h * int(np.prod(tail)) and a.flags["C_CONTIGUOUS"], name
+            ptrs.append(a.ctypes.data_as(C.c_void_p) if a is not None else None)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_hit_buffers(self._h, C.byref(params), x0, x1, *ptrs, C.byref(st)))
+        res = {name: out[name].reshape((cols, h) + tail) for name, _, tail in self.HIT_BUFFERS if out.get(name) is not None}
+        return res, RenderStats.from_c(st)
+
+    def hit_buffers_device(self, params: TcrtParams, x0: int = 0, x1: Optional[int] = None) -> RenderStats:
+        """hit_buffers() left in device memory (device_hit_buffers() gives their addresses)."""
+        x1 = params.width if x1 is None else x1
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_hit_buffers(self._h, C.byref(params), x0, x1, None, None, None, C.byref(st)))
+        return RenderStats.from_c(st)
+
+    def device_hit_buffers(self, slot: int = 0):
+        """Device addresses (object, distance, normal) of device `slot`'s band of the last hit_buffers() call and the
+        pixels in it: (int, int, int, n_pixels).  normal holds 3 * n_pixels floats."""
+        o, d, n = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        cnt = C.c_size_t()
+        self._ck(self._lib.tcrt_device_hit_buffers(self._h, slot, C.byref(o), C.byref(d), C.byref(n), C.byref(cnt)))
+        return o.value or 0, d.value or 0, n.value or 0, cnt.value
+
+    def pick(self, params: TcrtParams, xs, zs):
+        """The hits under pixels (xs[i], zs[i]) of the frame, on device slot 0 (tcrt_pick): (object (n,) int32,
+        distance (n,) float32, normal (n, 3) float32), each equal to hit_buffers() at that pixel."""
+        xz = np.ascontiguousarray(np.stack([np.asarray(xs, np.int32).ravel(), np.asarray(zs, np.int32).ravel()], axis=1))
+        n = xz.shape[0]
+        obj = np.empty(n, np.int32)
+        dist = np.empty(n, np.float32)
+        normal = np.empty((n, 3), np.float32)
+        self._ck(self._lib.tcrt_pick(self._h, C.byref(params), n, xz.ctypes.data_as(C.c_void_p), obj.ctypes.data_as(C.c_void_p),
+                                     dist.ctypes.data_as(C.c_void_p), normal.ctypes.data_as(C.c_void_p)))
+        return obj, dist, normal
+
     def balance_columns(self, params: TcrtParams, n_bands: int) -> list[tuple[int, int]]:
         """Cost-balanced column bands of the frame (low-resolution pre-pass on device slot 0):
         [(x0, x1)] * n_bands tiling [0, width).  A measurement: compute it once and share it."""

@@ -99,6 +99,18 @@ struct DeviceState {
     // chunk that reuses the buffer, so both frame sets share it.
     float* ss_scratch[kChunkStreams] = {};
     size_t ss_scratch_cap[kChunkStreams] = {};     // floats
+    // primary-hit buffers (tcrt_hit_buffers) and picks (tcrt_pick): buffers, queue head and events of their own, so that
+    // neither touches the last render or a frame in flight.  hit_mem holds the band of the last tcrt_hit_buffers call:
+    // n = (hit_x1 - hit_x0) * hit_h object indices, then n distances, then 3n normal components.  pick_mem: the 2n
+    // coordinates of a pick, then its 5n result words in the same layout.
+    float* hit_mem = nullptr;
+    size_t hit_mem_cap = 0;                       // 4-byte words
+    int hit_x0 = 0, hit_x1 = 0, hit_h = 0;
+    int* pick_mem = nullptr;
+    size_t pick_mem_cap = 0;                      // 4-byte words
+    unsigned int* hit_queue = nullptr;            // device, 16 B
+    cudaEvent_t ev_h0 = nullptr, ev_h1 = nullptr; // around the hit kernel (render stream)
+    cudaEvent_t ev_hc = nullptr;                  // the direct copies of the hit buffers are in host memory (copy stream)
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -115,6 +127,7 @@ struct tcrt_ctx {
     std::string err;
     bool has_scene = false;
     bool has_frame = false;
+    bool has_hits = false;       // a tcrt_hit_buffers call has completed (tcrt_device_hit_buffers)
     bool txt_prepared = false;
     int frame_x0 = 0, frame_x1 = 0, frame_h = 0;
     tcrt_camera cam{};           // passed by value with every launch
@@ -215,6 +228,11 @@ void free_device(DeviceState& d) {
     cudaFree(d.col_cost);
     cudaFree(d.wave_mem);
     for (float* s : d.ss_scratch) cudaFree(s);
+    cudaFree(d.hit_mem);
+    cudaFree(d.pick_mem);
+    cudaFree(d.hit_queue);
+    for (cudaEvent_t e : {d.ev_h0, d.ev_h1, d.ev_hc})
+        if (e) cudaEventDestroy(e);
     cudaFreeHost(d.h_txt);
     cudaFreeHost(d.txt_stage);
     for (auto& e : d.ev_txt)
@@ -377,6 +395,10 @@ int tcrt_create(tcrt_ctx** out, const int* device_ids, int n_devices) {
         }
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d.ev_scene, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaMalloc((void**)&d.flag, 16);
+        if (e == cudaSuccess) e = cudaMalloc((void**)&d.hit_queue, 16);
+        if (e == cudaSuccess) e = cudaEventCreate(&d.ev_h0);
+        if (e == cudaSuccess) e = cudaEventCreate(&d.ev_h1);
+        if (e == cudaSuccess) e = cudaEventCreate(&d.ev_hc);
         if (e == cudaSuccess) e = cudaHostAlloc((void**)&d.h_txt, 64, cudaHostAllocPortable);
         if (e != cudaSuccess) {
             std::string msg = cudaGetErrorString(e);
@@ -1971,37 +1993,84 @@ int n_txt_workers() {
     return (int)std::max(2u, std::min(16u, hc ? hc : 4u));
 }
 
+// The pinned staging slots of one device that a staged copy cycles through, and which of them still hold bytes on their way
+// to the destination.
+struct StageSlots {
+    int busy[kTxtSlots] = {};
+    std::atomic<int> left[kTxtSlots];
+    size_t piece = 0;
+    StageSlots() {
+        for (auto& l : left) l.store(0);
+    }
+    void drain(TxtPipe& pipe) {
+        for (int sl = 0; sl < kTxtSlots; sl++) pipe.wait_slot(&busy[sl]);
+    }
+};
+
+// Device d's pinned staging slots (shared with the .txt writer), allocated at first use.
+cudaError_t ensure_stage(DeviceState& d) {
+    cudaError_t e = cudaSuccess;
+    if (!d.txt_stage) {
+        e = cudaHostAlloc((void**)&d.txt_stage, kTxtSlots * kTxtChunkPx * kTxtLine, cudaHostAllocPortable);
+        for (auto& ev : d.ev_txt)
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    }
+    return e;
+}
+
+// n bytes of device memory at src -> byte dst of the copy sink: on d's copy stream once `ready` has completed (nullptr: the
+// bytes are complete already), slot by slot into d's pinned staging at bus speed, from there by the pipe's worker threads.
+// The caller has called cudaSetDevice(d.dev) and ensure_stage(d), and drains `slots` before the destination may be read.
+cudaError_t stage_out(TxtPipe& pipe, DeviceState& d, StageSlots& slots, const char* src, size_t n, size_t dst, cudaEvent_t ready) {
+    const size_t slot_bytes = kTxtChunkPx * kTxtLine;
+    cudaError_t e = ready ? cudaStreamWaitEvent(d.copy_stream, ready, 0) : cudaSuccess;
+    for (size_t b = 0; b < n && e == cudaSuccess; b += slot_bytes, slots.piece++) {
+        const int slot = (int)(slots.piece % kTxtSlots);
+        const size_t m = std::min(slot_bytes, n - b);
+        pipe.wait_slot(&slots.busy[slot]);
+        char* stage = d.txt_stage + slot * slot_bytes;
+        e = cudaMemcpyAsync(stage, src + b, m, cudaMemcpyDeviceToHost, d.copy_stream);
+        if (e == cudaSuccess) e = cudaEventRecord(d.ev_txt[slot], d.copy_stream);
+        if (e != cudaSuccess) break;
+        const int parts = m >= (size_t)kTxtParts * 65536 ? kTxtParts : 1;
+        slots.busy[slot] = 1;
+        slots.left[slot].store(parts);
+        for (int q = 0; q < parts; q++) {
+            const size_t b0 = m * q / parts, b1 = m * (q + 1) / parts;
+            pipe.push({d.dev, d.ev_txt[slot], stage + b0, dst + b + b0, b1 - b0, &slots.left[slot], &slots.busy[slot]});
+        }
+    }
+    return e;
+}
+
 }  // namespace
 
-// The band of the frame just submitted with kCopyStaged -> pageable host memory: chunk after chunk (as their kernels
-// finish) into the pinned staging slots of the .txt writer at bus speed, from there by worker threads into host_band.
-// fmt picks the device buffer (float frame or its 8-bit copy) and the bytes per pixel.
-static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, void* host_band, FrameFormat fmt) {
-    const size_t slot_bytes = kTxtChunkPx * kTxtLine;
-    const size_t bpp = bytes_per_px(fmt);
+// The staged copy's worker threads, now writing into host (their sink).
+static TxtPipe& copy_pipe_to(tcrt_ctx* ctx, void* host) {
     if (!ctx->copy_pipe) {      // the workers live as long as the ctx: starting eight threads costs as much as a 1080p frame
         ctx->copy_sink = new TxtSink();
         ctx->copy_pipe = new TxtPipe();
         ctx->copy_pipe->start(ctx->copy_sink, std::min(8, n_txt_workers()));
     }
-    TxtPipe& pipe = *ctx->copy_pipe;
-    ctx->copy_sink->map = reinterpret_cast<char*>(host_band);     // the workers are idle between calls
-    pipe.io_error = false;
+    ctx->copy_sink->map = reinterpret_cast<char*>(host);     // the workers are idle between calls
+    ctx->copy_pipe->io_error = false;
+    return *ctx->copy_pipe;
+}
+
+// The band of the frame just submitted with kCopyStaged -> pageable host memory: chunk after chunk (as their kernels
+// finish) into the pinned staging slots of the .txt writer at bus speed, from there by worker threads into host_band.
+// fmt picks the device buffer (float frame or its 8-bit copy) and the bytes per pixel.
+static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, void* host_band, FrameFormat fmt) {
+    const size_t bpp = bytes_per_px(fmt);
+    TxtPipe& pipe = copy_pipe_to(ctx, host_band);
     int rc = TCRT_OK;
     std::string err;
     for (auto& d : ctx->devs) {
         FrameRes& f = d.fr();
         if (f.x1 <= f.x0 || rc) continue;
         cudaError_t e = cudaSetDevice(d.dev);
-        if (e == cudaSuccess && !d.txt_stage) {
-            e = cudaHostAlloc((void**)&d.txt_stage, kTxtSlots * slot_bytes, cudaHostAllocPortable);
-            for (auto& ev : d.ev_txt)
-                if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-        }
-        int slot_busy[kTxtSlots] = {};
-        std::atomic<int> left[kTxtSlots];
-        for (auto& l : left) l.store(0);
-        size_t piece = 0;
+        if (e == cudaSuccess) e = ensure_stage(d);
+        StageSlots slots;
         // chunk k may leave once its kernel has finished (a frame that is already complete — tcrt_download — has no chunk
         // events of its own: older ones have long completed, and the render call has waited for the frame)
         const int n_chunks = std::max(1, f.n_chunks);
@@ -2011,26 +2080,10 @@ static int copy_out_staged(tcrt_ctx* ctx, const tcrt_params* p, int x0, void* ho
             if (c1 <= c0) continue;
             // every chunk, the only one of a band too (a device band of a multi-device frame can be a single chunk although
             // the frame is large enough to be staged): the copy stream is not ordered behind the render streams otherwise
-            if (f.n_chunks) e = cudaStreamWaitEvent(d.copy_stream, f.ev_chunk[k], 0);
-            for (size_t b = c0; b < c1 && e == cudaSuccess; b += slot_bytes, piece++) {
-                const int slot = (int)(piece % kTxtSlots);
-                const size_t n = std::min(slot_bytes, c1 - b);
-                pipe.wait_slot(&slot_busy[slot]);
-                char* stage = d.txt_stage + slot * slot_bytes;
-                e = cudaMemcpyAsync(stage, frame_src(f, fmt) + b, n, cudaMemcpyDeviceToHost, d.copy_stream);
-                if (e == cudaSuccess) e = cudaEventRecord(d.ev_txt[slot], d.copy_stream);
-                if (e != cudaSuccess) break;
-                const int parts = n >= (size_t)kTxtParts * 65536 ? kTxtParts : 1;
-                slot_busy[slot] = 1;
-                left[slot].store(parts);
-                const size_t dst = (size_t)(f.x0 - x0) * p->height * bpp + b;
-                for (int q = 0; q < parts; q++) {
-                    const size_t b0 = n * q / parts, b1 = n * (q + 1) / parts;
-                    pipe.push({d.dev, d.ev_txt[slot], stage + b0, dst + b0, b1 - b0, &left[slot], &slot_busy[slot]});
-                }
-            }
+            e = stage_out(pipe, d, slots, frame_src(f, fmt) + c0, c1 - c0, (size_t)(f.x0 - x0) * p->height * bpp + c0,
+                          f.n_chunks ? f.ev_chunk[k] : nullptr);
         }
-        for (int sl = 0; sl < kTxtSlots; sl++) pipe.wait_slot(&slot_busy[sl]);
+        slots.drain(pipe);
         if (e != cudaSuccess) {
             err = cudaGetErrorString(e);
             rc = TCRT_ERR_CUDA;
@@ -2052,6 +2105,183 @@ static void destroy_copy_pipe(tcrt_ctx* ctx) {
         ctx->copy_sink = nullptr;
     }
 }
+
+// ---- primary-hit buffers and picking (tcrt_hits.cu) -------------------------------------------------------------------
+// What the hit kernel needs of the frame p over columns [cx0, cx1) of device d: its rays are the render's primary rays.
+static HitLaunch hit_launch(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, unsigned int* queue) {
+    HitLaunch hl{};
+    RenderLaunch& rl = hl.rl;
+    rl.scene = d.ds;
+    rl.cam = ctx->cam;
+    rl.width = p->width;
+    rl.height = p->height;
+    rl.x0 = cx0;
+    rl.x1 = cx1;
+    rl.far_dist = p->far_dist;
+    rl.n_objects = ctx->n_objects;
+    rl.queue = queue;
+    return hl;
+}
+
+// A plain malloc'd / numpy destination, which cudaMemcpyAsync copies into at the driver's staging rate (render_impl).
+static bool host_pageable(const void* p) {
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+        cudaGetLastError();
+        return true;
+    }
+    return at.type == cudaMemoryTypeUnregistered;
+}
+
+extern "C" {
+
+int tcrt_hit_buffers(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, int* host_object, float* host_distance,
+                     float* host_normal, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
+    if (!valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
+    if (x0 < 0 || x1 > p->width || x0 >= x1) return fail(ctx, TCRT_ERR_INVALID, "bad column range [%d,%d)", x0, x1);
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    const int nd = (int)ctx->devs.size();
+    const int h = p->height;
+    // one band of equal width per device: every pixel costs one sweep, so there is nothing to balance
+    std::vector<int> cut(nd + 1);
+    for (int i = 0; i <= nd; i++) cut[i] = x0 + (int)((long long)(x1 - x0) * i / nd);
+    // the three buffers: destination, bytes per pixel, word offset per pixel of the band in hit_mem
+    char* host[3] = {reinterpret_cast<char*>(host_object), reinterpret_cast<char*>(host_distance),
+                     reinterpret_cast<char*>(host_normal)};
+    const size_t bpp[3] = {4, 4, 12}, word_off[3] = {0, 1, 2};
+    // pageable destinations of at least 512 K pixels go through the pinned staging, as frames do (render_impl)
+    const bool big = (long long)(x1 - x0) * h >= 512 * 1024;
+    bool staged[3], any_direct = false;
+    for (int k = 0; k < 3; k++) {
+        staged[k] = host[k] && big && host_pageable(host[k]);
+        any_direct = any_direct || (host[k] && !staged[k]);
+    }
+    ctx->has_hits = false;
+    int launches = 0;
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        d.hit_x0 = cut[i];
+        d.hit_x1 = cut[i + 1];
+        d.hit_h = h;
+        if (d.hit_x1 <= d.hit_x0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        const size_t n = (size_t)(d.hit_x1 - d.hit_x0) * h;
+        const int rc = ensure(ctx, d.hit_mem, d.hit_mem_cap, 5 * n);
+        if (rc) return rc;
+        HitLaunch hl = hit_launch(ctx, d, p, d.hit_x0, d.hit_x1, d.hit_queue);
+        hl.object = reinterpret_cast<int*>(d.hit_mem);
+        hl.distance = d.hit_mem + n;
+        hl.normal = d.hit_mem + 2 * n;
+        // on the render stream, behind whatever is queued there (a scene upload, frames in flight)
+        CK(ctx, cudaMemsetAsync(d.hit_queue, 0, 4, d.stream));
+        CK(ctx, cudaEventRecord(d.ev_h0, d.stream));
+        CK(ctx, tcrt_launch_hits(hl, d.sm_count, d.stream));
+        launches++;
+        CK(ctx, cudaEventRecord(d.ev_h1, d.stream));
+        if (any_direct) {
+            CK(ctx, cudaStreamWaitEvent(d.copy_stream, d.ev_h1, 0));
+            for (int k = 0; k < 3; k++)
+                if (host[k] && !staged[k])
+                    CK(ctx, cudaMemcpyAsync(host[k] + (size_t)(d.hit_x0 - x0) * h * bpp[k], d.hit_mem + word_off[k] * n,
+                                            n * bpp[k], cudaMemcpyDeviceToHost, d.copy_stream));
+            CK(ctx, cudaEventRecord(d.ev_hc, d.copy_stream));
+        }
+    }
+    for (int k = 0; k < 3; k++) {
+        if (!staged[k]) continue;
+        TxtPipe& pipe = copy_pipe_to(ctx, host[k]);
+        cudaError_t e = cudaSuccess;
+        for (auto& d : ctx->devs) {
+            if (d.hit_x1 <= d.hit_x0) continue;
+            const size_t n = (size_t)(d.hit_x1 - d.hit_x0) * h;
+            e = cudaSetDevice(d.dev);
+            if (e == cudaSuccess) e = ensure_stage(d);
+            StageSlots slots;
+            if (e == cudaSuccess)
+                e = stage_out(pipe, d, slots, reinterpret_cast<const char*>(d.hit_mem + word_off[k] * n), n * bpp[k],
+                              (size_t)(d.hit_x0 - x0) * h * bpp[k], d.ev_h1);
+            slots.drain(pipe);
+            if (e != cudaSuccess) break;
+        }
+        if (e != cudaSuccess || pipe.io_error)
+            return fail(ctx, TCRT_ERR_CUDA, "staged copy-out of a hit buffer: %s",
+                        e != cudaSuccess ? cudaGetErrorString(e) : "a chunk did not arrive");
+    }
+    if (stats) memset(stats, 0, sizeof(*stats));
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        if (stats) {
+            stats->col_begin[i] = d.hit_x0;
+            stats->col_end[i] = d.hit_x1;
+        }
+        if (d.hit_x1 <= d.hit_x0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaEventSynchronize(d.ev_h1));
+        if (any_direct) CK(ctx, cudaEventSynchronize(d.ev_hc));
+        if (stats) {
+            float ms = 0.f;
+            CK(ctx, cudaEventElapsedTime(&ms, d.ev_h0, d.ev_h1));
+            stats->render_ms[i] = ms;
+            if (any_direct) CK(ctx, cudaEventElapsedTime(&ms, d.ev_h1, d.ev_hc));
+            stats->d2h_ms[i] = any_direct ? std::max(ms, 0.f) : 0.0;   // copy time not hidden behind the kernel
+            stats->rays_primary[i] = (unsigned long long)(d.hit_x1 - d.hit_x0) * h;
+        }
+    }
+    if (stats) {
+        stats->n_devices = nd;
+        stats->gpu_launches = (unsigned long long)launches;
+    }
+    ctx->has_hits = true;
+    return TCRT_OK;
+}
+
+int tcrt_device_hit_buffers(tcrt_ctx* ctx, int slot, int** object, float** distance, float** normal, size_t* n_pixels) {
+    if (!ctx || slot < 0 || slot >= (int)ctx->devs.size() || !object || !distance || !normal || !n_pixels)
+        return fail(ctx, TCRT_ERR_INVALID, "bad argument");
+    if (!ctx->has_hits) return fail(ctx, TCRT_ERR_NO_FRAME, "no hit buffers computed yet");
+    DeviceState& d = ctx->devs[slot];
+    const size_t n = d.hit_x1 > d.hit_x0 ? (size_t)(d.hit_x1 - d.hit_x0) * d.hit_h : 0;
+    *object = n ? reinterpret_cast<int*>(d.hit_mem) : nullptr;
+    *distance = n ? d.hit_mem + n : nullptr;
+    *normal = n ? d.hit_mem + 2 * n : nullptr;
+    *n_pixels = n;
+    return TCRT_OK;
+}
+
+int tcrt_pick(tcrt_ctx* ctx, const tcrt_params* p, int n, const int* xz, int* object, float* distance, float* normal) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
+    if (!valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
+    if (n < 0 || (n > 0 && !xz)) return fail(ctx, TCRT_ERR_INVALID, "bad pixel list");
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    for (int i = 0; i < n; i++)
+        if (xz[2 * i] < 0 || xz[2 * i] >= p->width || xz[2 * i + 1] < 0 || xz[2 * i + 1] >= p->height)
+            return fail(ctx, TCRT_ERR_INVALID, "pick %d: pixel (%d, %d) outside the %dx%d frame", i, xz[2 * i], xz[2 * i + 1],
+                        p->width, p->height);
+    if (n == 0) return TCRT_OK;
+    DeviceState& d = ctx->devs[0];
+    CK(ctx, cudaSetDevice(d.dev));
+    const size_t m = (size_t)n;
+    const int rc = ensure(ctx, d.pick_mem, d.pick_mem_cap, 7 * m);
+    if (rc) return rc;
+    HitLaunch hl = hit_launch(ctx, d, p, 0, p->width, d.hit_queue + 1);
+    hl.xz = d.pick_mem;
+    hl.n_list = n;
+    hl.object = d.pick_mem + 2 * m;
+    hl.distance = reinterpret_cast<float*>(d.pick_mem + 3 * m);
+    hl.normal = reinterpret_cast<float*>(d.pick_mem + 4 * m);
+    CK(ctx, cudaMemcpyAsync(d.pick_mem, xz, 2 * m * sizeof(int), cudaMemcpyHostToDevice, d.stream));
+    CK(ctx, cudaMemsetAsync(d.hit_queue + 1, 0, 4, d.stream));
+    CK(ctx, tcrt_launch_hits(hl, d.sm_count, d.stream));
+    if (object) CK(ctx, cudaMemcpyAsync(object, hl.object, m * sizeof(int), cudaMemcpyDeviceToHost, d.stream));
+    if (distance) CK(ctx, cudaMemcpyAsync(distance, hl.distance, m * sizeof(float), cudaMemcpyDeviceToHost, d.stream));
+    if (normal) CK(ctx, cudaMemcpyAsync(normal, hl.normal, 3 * m * sizeof(float), cudaMemcpyDeviceToHost, d.stream));
+    CK(ctx, cudaEventRecord(d.ev_h1, d.stream));
+    CK(ctx, cudaEventSynchronize(d.ev_h1));
+    return TCRT_OK;
+}
+
+}  // extern "C"
 
 namespace {
 

@@ -118,6 +118,18 @@ struct RenderLaunch {
     int tiled;               // queue positions map to 4x8-pixel tiles (band width % 4 == 0, height % 8 == 0)
 };
 
+// Primary-hit launch (tcrt_hits.cu): rl describes the frame, the band [x0, x1) and the scene; out of rl the kernel uses the
+// camera, width, height, x0, x1, far_dist, queue and n_objects.  Band mode (xz == nullptr): every pixel of the band, x-major
+// like frames.  List mode: entry i is pixel (xz[2i], xz[2i+1]) of the frame (rl.x0 == 0), and output i is its hit.
+struct HitLaunch {
+    RenderLaunch rl;
+    const int* xz;
+    int n_list;
+    int* object;       // per pixel: object index of the nearest hit, -1 on a miss
+    float* distance;   // its distance (far_dist on a miss)
+    float* normal;     // 3 per pixel: its normal ray's direction ((0,0,0) on a miss)
+};
+
 // host builder of the box clusters (tcrt_cluster.cpp).  Face f = 2*axis + k; an absent face has
 // c = NaN and plane = -1; `plane` indexes the caller's list.
 struct TcrtBoxCluster {
@@ -149,6 +161,9 @@ cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count
 cudaError_t tcrt_launch_render_pool(const RenderLaunch& rl, int fm, int sm_count, size_t smem_scene, cudaStream_t stream);
 // n random (a.xyz, b) cases: div3 (shared-reciprocal division of the render kernel) vs __fdiv_rn; *bad += mismatches
 cudaError_t tcrt_launch_div3_check(unsigned long long n, unsigned seed, unsigned long long* bad, cudaStream_t stream);   // dynamic shared memory the kernel may opt in to
+
+// primary-hit buffers and picks (tcrt_hits.cu): one launch, nothing when there are no pixels
+cudaError_t tcrt_launch_hits(const HitLaunch& hl, int sm_count, cudaStream_t stream);
 
 // txt formatter (tcrt_format.cu)
 // fixed path: 31-byte lines; general path: per-pixel lengths -> two-level exclusive scan

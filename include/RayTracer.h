@@ -23,6 +23,8 @@ struct RenderSettings {
     bool shadows = true;      // SHADOWS_ON
     bool reflections = true;  // REFLECTIONS_ON
     int samples = 1;          // samples per axis: > 1 renders the anti-aliased frame of tcrt_render_columns_ss
+    int contrast = -1;        // with samples > 1: >= 0 supersamples only the pixels at quant8 contrast edges above this
+                              // (tcrt_render_columns_adaptive); -1 supersamples every pixel
     tcrt_params params() const {
         tcrt_params p;
         tcrt_default_params(&p);
@@ -51,12 +53,15 @@ public:
         return rc_ = tcrt_upload_scene(ctx_, &s, &c);
     }
     // the pixel loop (RayTracer.cpp:911-923): pixels[x][z] -> pixels_xmajor[(x*H + z)*3 + c]; with rs.samples > 1 each
-    // pixel is the mean of rs.samples x rs.samples samples (tcrt_render_columns_ss)
+    // pixel is the mean of rs.samples x rs.samples samples (tcrt_render_columns_ss), with rs.contrast >= 0 only the pixels
+    // at contrast edges (tcrt_render_columns_adaptive)
     int render(const RenderSettings& rs, float* pixels_xmajor, tcrt_stats* stats = NULL) {
         settings_ = rs;
         tcrt_params p = rs.params();
         std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
-        if (rs.samples != 1)
+        if (rs.samples != 1 && rs.contrast >= 0)
+            rc_ = tcrt_render_columns_adaptive(ctx_, &p, rs.samples, rs.contrast, 0, p.width, pixels_xmajor, NULL, NULL, stats);
+        else if (rs.samples != 1)
             rc_ = tcrt_render_columns_ss(ctx_, &p, rs.samples, 0, p.width, pixels_xmajor, stats);
         else
             rc_ = pixels_xmajor ? tcrt_render(ctx_, &p, pixels_xmajor, stats)
@@ -70,8 +75,12 @@ public:
         settings_ = rs;
         tcrt_params p = rs.params();
         std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
-        rc_ = rs.samples != 1 ? tcrt_render_columns_ss_rgb8(ctx_, &p, rs.samples, 0, p.width, pixels_xmajor_rgb8, stats)
-                              : tcrt_render_rgb8(ctx_, &p, pixels_xmajor_rgb8, stats);
+        if (rs.samples != 1 && rs.contrast >= 0)
+            rc_ = tcrt_render_columns_adaptive_rgb8(ctx_, &p, rs.samples, rs.contrast, 0, p.width, pixels_xmajor_rgb8, NULL,
+                                                    NULL, stats);
+        else
+            rc_ = rs.samples != 1 ? tcrt_render_columns_ss_rgb8(ctx_, &p, rs.samples, 0, p.width, pixels_xmajor_rgb8, stats)
+                                  : tcrt_render_rgb8(ctx_, &p, pixels_xmajor_rgb8, stats);
         run_time_s_ = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         return rc_;
     }

@@ -238,6 +238,36 @@ int tcrt_render_async_ss(tcrt_ctx* ctx, const tcrt_params* params, int ss, int x
                          int* ticket);
 int tcrt_render_async_ss_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int ss, int x0, int x1,
                               unsigned char* host_rgb8_band, int* ticket);
+/* Adaptive anti-aliasing: the samples of tcrt_render_columns_ss traced only where the plain frame shows contrast.  For
+ * params p (W x H), ss (1 <= ss <= 8) and contrast (-1 <= contrast <= 255):
+ *   - P is the plain frame, exactly what tcrt_render returns for p; q(c) is the quant8 above;
+ *   - pixel (x, z) is refined when contrast < 0, or when some neighbour (x', z') != (x, z) with |x'-x| <= 1 and
+ *     |z'-z| <= 1 inside [0, W) x [0, H) has max over c of |q(P(x,z)_c) - q(P(x',z')_c)| > contrast.  Neighbours are
+ *     taken from the frame, not from the requested band: a band's result does not depend on where the band is cut;
+ *   - output pixel (x, z) is exactly the pixel of tcrt_render_columns_ss at the same ss where refined, exactly P(x, z)
+ *     otherwise.  The RGB8 form carries quant8 of that float.
+ * So contrast -1 gives the tcrt_render_columns_ss frame, contrast 255 and ss = 1 the plain frame (the mask is still
+ * computed: an edge preview).  A refined pixel is resolved from the plain pixel, which is its sample (0,0) bit for bit
+ * (the quotient x/W is the same at ss*W), and its ss*ss-1 other samples, in the order and arithmetic of
+ * tcrt_render_columns_ss.
+ * host_mask (may be NULL): one byte per pixel of the band, 1 refined / 0 not, x-major: host_mask[(x-x0)*H + z].
+ * n_refined (may be NULL): the refined pixels of the band, over all devices.  host_rgb_band NULL leaves the frame on the
+ * device (float form only; the RGB8 destination must not be NULL).  Pinned and pageable destinations as in tcrt_render.
+ * Errors: ss < 1 or contrast outside [-1, 255]: TCRT_ERR_INVALID; ss > 8, or ss*W or ss*H above 2^24:
+ * TCRT_ERR_UNSUPPORTED.  A long list of refined pixels is traced in pieces, never refused.
+ * The call is synchronous: it renders the plain frame over the band and one halo column each side, classifies and
+ * compacts the band on the device, reads the list's length (4 bytes), then traces and resolves the list's samples.  The
+ * resolved frame becomes the last render (tcrt_download, tcrt_device_frame, the writers); with frames in flight the
+ * rules of tcrt_render_columns_ss apply.  A multi-device ctx renders bands of equal width and neither reads nor updates
+ * the balanced cut or its cost map.  Stats: col_begin/col_end per device; render_ms from the first launch to the last
+ * (it includes the wait for the list's length); gpu_launches every launch; rays_* every ray traced, rays_primary =
+ * (band + halo columns)*H + (ss*ss-1)*n_refined. */
+int tcrt_render_columns_adaptive(tcrt_ctx* ctx, const tcrt_params* params, int ss, int contrast, int x0, int x1,
+                                 float* host_rgb_band, unsigned char* host_mask, unsigned long long* n_refined,
+                                 tcrt_stats* stats);
+int tcrt_render_columns_adaptive_rgb8(tcrt_ctx* ctx, const tcrt_params* params, int ss, int contrast, int x0, int x1,
+                                      unsigned char* host_rgb8_band, unsigned char* host_mask,
+                                      unsigned long long* n_refined, tcrt_stats* stats);
 /* Device address of a device's band of the last render (for zero-copy consumers, e.g. a
  * torch tensor view); floats = (col_end-col_begin)*height*3. */
 int tcrt_device_frame(tcrt_ctx* ctx, int device_slot, void** dev_ptr, size_t* n_floats);

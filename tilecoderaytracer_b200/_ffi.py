@@ -105,6 +105,10 @@ SIGNATURES = {
                                        C.POINTER(C.c_int)]),
     "tcrt_render_async_ss_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_void_p,
                                             C.POINTER(C.c_int)]),
+    "tcrt_render_columns_adaptive": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_void_p, C.c_void_p, C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
+    "tcrt_render_columns_adaptive_rgb8": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_int, C.c_int,
+                                                    C.c_void_p, C.c_void_p, C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
     "tcrt_device_frame": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]),
     "tcrt_hit_buffers": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.POINTER(TcrtStats)]),

@@ -394,6 +394,44 @@ class Context:
                                                      out.ctypes.data_as(C.c_void_p), C.byref(t)))
         return t.value
 
+    def _adaptive(self, fn, dtype, params: TcrtParams, ss: int, contrast: int, x0: int, x1: Optional[int], out, mask,
+                  device_only: bool = False):
+        x1 = params.width if x1 is None else x1
+        shape = (x1 - x0, params.height, 3)
+        if out is None and not device_only:
+            out = np.empty(shape, dtype=dtype)
+        if out is not None:
+            assert out.dtype == dtype and out.size == int(np.prod(shape)) and out.flags["C_CONTIGUOUS"]
+        if mask is not None:
+            assert mask.dtype == np.uint8 and mask.size == (x1 - x0) * params.height and mask.flags["C_CONTIGUOUS"]
+        n = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(fn(self._h, C.byref(params), ss, contrast, x0, x1, out.ctypes.data_as(C.c_void_p) if out is not None else None,
+                    mask.ctypes.data_as(C.c_void_p) if mask is not None else None, C.byref(n), C.byref(st)))
+        frame = out.reshape(shape) if out is not None else None
+        m = mask.reshape(shape[:2]) if mask is not None else None
+        return frame, m, int(n.value), RenderStats.from_c(st)
+
+    def render_adaptive(self, params: TcrtParams, ss: int, contrast: int, x0: int = 0, x1: Optional[int] = None,
+                        out: Optional[np.ndarray] = None, mask: Optional[np.ndarray] = None):
+        """Columns [x0,x1) of the adaptively anti-aliased frame (tcrt_render_columns_adaptive): the render_ss() pixel where
+        the plain frame's 3x3 neighbourhood (quant8, max over channels) differs by more than `contrast` (-1: everywhere),
+        the render() pixel elsewhere.  `mask` (uint8, (cols, H), optional) receives 1 for every refined pixel.  Returns
+        (array[x1-x0, H, 3] float32, mask or None, n_refined, RenderStats).  The frame becomes the last render."""
+        return self._adaptive(self._lib.tcrt_render_columns_adaptive, np.float32, params, ss, contrast, x0, x1, out, mask)
+
+    def render_adaptive_rgb8(self, params: TcrtParams, ss: int, contrast: int, x0: int = 0, x1: Optional[int] = None,
+                             out: Optional[np.ndarray] = None, mask: Optional[np.ndarray] = None):
+        """render_adaptive() quantised to 8 bits on the GPU: (array[x1-x0, H, 3] uint8, mask or None, n_refined,
+        RenderStats).  The float frame stays on the device as the last render."""
+        return self._adaptive(self._lib.tcrt_render_columns_adaptive_rgb8, np.uint8, params, ss, contrast, x0, x1, out, mask)
+
+    def render_adaptive_device(self, params: TcrtParams, ss: int, contrast: int, x0: int = 0, x1: Optional[int] = None):
+        """render_adaptive() left in device memory (download() fetches it): (n_refined, RenderStats)."""
+        _, _, n, st = self._adaptive(self._lib.tcrt_render_columns_adaptive, np.float32, params, ss, contrast, x0, x1,
+                                     None, None, device_only=True)
+        return n, st
+
     def wait(self, ticket: int) -> RenderStats:
         st = TcrtStats()
         self._ck(self._lib.tcrt_wait(self._h, ticket, C.byref(st)))

@@ -111,6 +111,17 @@ struct DeviceState {
     unsigned int* hit_queue = nullptr;            // device, 16 B
     cudaEvent_t ev_h0 = nullptr, ev_h1 = nullptr; // around the hit kernel (render stream)
     cudaEvent_t ev_hc = nullptr;                  // the direct copies of the hit buffers are in host memory (copy stream)
+    // adaptive frames (tcrt_render_columns_adaptive): the plain frame over the band and its halo columns, the band's mask,
+    // the classify pass's per-CTA counts (then their exclusive scan and the total), the list of refined pixels.  The call
+    // is synchronous: nothing else uses them while it runs.
+    float* ad_plain = nullptr;
+    size_t ad_plain_cap = 0;                      // floats
+    unsigned char* ad_mask = nullptr;
+    size_t ad_mask_cap = 0;
+    unsigned int* ad_counts = nullptr;
+    size_t ad_counts_cap = 0;
+    int* ad_list = nullptr;
+    size_t ad_list_cap = 0;
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -231,6 +242,10 @@ void free_device(DeviceState& d) {
     cudaFree(d.hit_mem);
     cudaFree(d.pick_mem);
     cudaFree(d.hit_queue);
+    cudaFree(d.ad_plain);
+    cudaFree(d.ad_mask);
+    cudaFree(d.ad_counts);
+    cudaFree(d.ad_list);
     for (cudaEvent_t e : {d.ev_h0, d.ev_h1, d.ev_hc})
         if (e) cudaEventDestroy(e);
     cudaFreeHost(d.h_txt);
@@ -1190,11 +1205,10 @@ static int render_impl(tcrt_ctx* ctx, const tcrt_params* p, int x0, int x1, void
     return render_finish(ctx, set, stats);
 }
 
-// Columns [cx0, cx1) of the frame `p` into out[(cx1-cx0)*p->height*3] (a slice of the band's frame buffer, or the sample
-// scratch of a supersampled frame, whose `p` is then the sample frame).  The caller has sized out and zeroed the queue head.
-static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, float* out, unsigned int* col_cost,
-                       int* launches, cudaStream_t stream, unsigned int* queue) {
-    if (!stream) stream = d.stream;
+// The launch of columns [cx0, cx1) of the frame `p` into `out`, with queue head `queue` (nullptr: the frame set's) and the
+// frame set's ray counters; no row order, no cost map.
+static RenderLaunch band_launch(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, float* out,
+                                unsigned int* queue) {
     RenderLaunch rl{};
     rl.scene = d.ds;
     rl.cam = ctx->cam;
@@ -1213,6 +1227,15 @@ static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int 
     rl.out = out;
     rl.queue = queue ? queue : reinterpret_cast<unsigned int*>(d.fr().ctl);
     rl.counters = reinterpret_cast<unsigned long long*>(d.fr().ctl + 8);
+    return rl;
+}
+
+// Columns [cx0, cx1) of the frame `p` into out[(cx1-cx0)*p->height*3] (a slice of the band's frame buffer, or the sample
+// scratch of a supersampled frame, whose `p` is then the sample frame).  The caller has sized out and zeroed the queue head.
+static int launch_band(tcrt_ctx* ctx, DeviceState& d, const tcrt_params* p, int cx0, int cx1, float* out, unsigned int* col_cost,
+                       int* launches, cudaStream_t stream, unsigned int* queue) {
+    if (!stream) stream = d.stream;
+    RenderLaunch rl = band_launch(ctx, d, p, cx0, cx1, out, queue);
     rl.col_cost = col_cost;
     int rc_ro = ensure_row_order(ctx, d, p, cx0, cx1, col_cost != nullptr, &rl.row_order);
     if (rc_ro) return rc_ro;
@@ -2279,6 +2302,261 @@ int tcrt_pick(tcrt_ctx* ctx, const tcrt_params* p, int n, const int* xz, int* ob
     CK(ctx, cudaEventRecord(d.ev_h1, d.stream));
     CK(ctx, cudaEventSynchronize(d.ev_h1));
     return TCRT_OK;
+}
+
+}  // extern "C"
+
+// ---- adaptive frames (tcrt_adaptive.cu): supersample only the pixels at contrast edges ------------------------------------
+// Samples traced per piece of the refined list: 4 M samples = 48 MB of sample scratch per render stream, far inside the
+// kernels' int index range at every ss.
+constexpr long long kPieceSamples = 1LL << 22;
+
+// Per device band [bx0, bx1) (equal widths; the balancer's cut and cost map are neither read nor updated):
+//   1. the plain frame over [bx0 - 1, bx1 + 1) clipped to the frame, column chunks round robin over the render streams;
+//   2. classify + scan + compact on the render stream: mask, the plain pixels copied into the band's frame, the list;
+//   3. the list's length to the host (it sizes step 4): one 4-byte copy and a wait;
+//   4. pieces of the list round robin over the render streams, each one list-mode render launch of samples 1 .. ss*ss-1
+//      into the stream's sample scratch and one resolve launch into the frame;
+//   5. RGB8: one quantisation launch over the band; then the band and the mask to the host.
+// Steps 1-2 run on all devices before any waits in step 3, and step 4 on all before any waits in step 5.
+static int render_adaptive(tcrt_ctx* ctx, const tcrt_params* p, int ss, int contrast, int x0, int x1, void* host_band,
+                           FrameFormat fmt, unsigned char* host_mask, unsigned long long* n_refined, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
+    if (ss < 1) return fail(ctx, TCRT_ERR_INVALID, "samples per axis %d < 1", ss);
+    if (contrast < -1 || contrast > 255) return fail(ctx, TCRT_ERR_INVALID, "contrast %d outside [-1, 255]", contrast);
+    int rc = check_ss(ctx, p, ss);
+    if (rc) return rc;
+    if (!valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
+    if (x0 < 0 || x1 > p->width || x0 >= x1) return fail(ctx, TCRT_ERR_INVALID, "bad column range [%d,%d)", x0, x1);
+    if (p->max_depth > TCRT_MAX_DEPTH)
+        return fail(ctx, TCRT_ERR_UNSUPPORTED, "max_depth %d > TCRT_MAX_DEPTH %d", p->max_depth, TCRT_MAX_DEPTH);
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    const int set = ctx->devs[0].cur;
+    if (ctx->pend[set].active)
+        return fail(ctx, TCRT_ERR_INVALID, "a frame submitted with tcrt_render_async is still pending in this slot: tcrt_wait first");
+    const int nd = (int)ctx->devs.size();
+    const int W = p->width, H = p->height;
+    const int m = ss * ss - 1;                           // samples traced per refined pixel
+    tcrt_params sp = *p;                                 // the sample frame the list-mode launches trace
+    sp.width = ss * W;
+    sp.height = ss * H;
+    std::vector<int> cut(nd + 1);
+    for (int i = 0; i <= nd; i++) cut[i] = x0 + (int)((long long)(x1 - x0) * i / nd);
+    // pageable destinations of at least 512 K pixels go through the pinned staging, as frames do (render_impl)
+    const bool big = (long long)(x1 - x0) * H >= 512 * 1024;
+    const bool staged_frame = host_band && big && host_pageable(host_band);
+    const bool staged_mask = host_mask && big && host_pageable(host_mask);
+    const bool any_direct = (host_band && !staged_frame) || (host_mask && !staged_mask);
+    const size_t bpp = bytes_per_px(fmt);
+    ctx->has_frame = false;
+    ctx->txt_prepared = false;
+    int launches = 0;
+    auto queue_of = [](DeviceState& d, int si) { return reinterpret_cast<unsigned int*>(d.fr().ctl + 64) + si; };
+    auto stream_of = [](DeviceState& d, int si) { return si == 0 ? d.stream : d.chunk_stream[si - 1]; };
+    // the render streams 1.. join the render stream: ev_chunk[si] marks stream si's last launch
+    auto join = [&](DeviceState& d, int n_streams) -> int {
+        for (int si = 1; si < n_streams; si++) {
+            CK(ctx, cudaEventRecord(d.fr().ev_chunk[si], stream_of(d, si)));
+            CK(ctx, cudaStreamWaitEvent(d.stream, d.fr().ev_chunk[si], 0));
+        }
+        return TCRT_OK;
+    };
+    // ...and wait for what the render stream has queued so far (ev_start)
+    auto fork = [&](DeviceState& d, int n_streams) -> int {
+        CK(ctx, cudaEventRecord(d.fr().ev_start, d.stream));
+        for (int si = 1; si < n_streams; si++) CK(ctx, cudaStreamWaitEvent(stream_of(d, si), d.fr().ev_start, 0));
+        return TCRT_OK;
+    };
+    // ---- 1-2: plain pass and classification ----------------------------------------------------------------------------------
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        FrameRes& f = d.fr();
+        f.x0 = cut[i];
+        f.x1 = cut[i + 1];
+        f.height = H;
+        f.n_chunks = 0;      // the band has no chunk events: the whole band is complete when the call returns
+        if (f.x1 <= f.x0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        const int bx0 = f.x0, bx1 = f.x1, hx0 = std::max(0, bx0 - 1), hx1 = std::min(W, bx1 + 1);
+        const size_t n_px = (size_t)(bx1 - bx0) * H;
+        const size_t nb = (n_px + 255) / 256;
+        rc = ensure(ctx, f.frame, f.frame_cap, 3 * n_px);
+        if (!rc && fmt == kRGB8) rc = ensure(ctx, f.frame8, f.frame8_cap, 3 * n_px);
+        if (!rc) rc = ensure(ctx, d.ad_plain, d.ad_plain_cap, (size_t)(hx1 - hx0) * H * 3);
+        if (!rc) rc = ensure(ctx, d.ad_mask, d.ad_mask_cap, n_px);
+        if (!rc) rc = ensure(ctx, d.ad_counts, d.ad_counts_cap, nb + 1);
+        if (!rc) rc = ensure(ctx, d.ad_list, d.ad_list_cap, n_px);
+        if (rc) return rc;
+        CK(ctx, cudaMemsetAsync(f.ctl, 0, 64 + kMaxChunks * sizeof(unsigned int), d.stream));
+        CK(ctx, cudaEventRecord(f.ev_k0, d.stream));
+        // column chunks of the halo band as plain frames are chunked (plan_chunks)
+        FrameRes plan;
+        plan.x0 = hx0;
+        plan.x1 = hx1;
+        plan_chunks(plan, H, true);
+        const int n_streams = ctx->one_stream ? 1 : std::min(kChunkStreams, plan.n_chunks);
+        rc = fork(d, n_streams);
+        if (rc) return rc;
+        for (int k = 0; k < plan.n_chunks; k++) {
+            const int cx0 = plan.chunk_x[k], cx1 = plan.chunk_x[k + 1];
+            if (cx1 <= cx0) continue;
+            const int si = k % n_streams;
+            const cudaStream_t ks = stream_of(d, si);
+            CK(ctx, cudaMemsetAsync(queue_of(d, si), 0, sizeof(unsigned int), ks));
+            const RenderLaunch rl = band_launch(ctx, d, p, cx0, cx1, d.ad_plain + (size_t)(cx0 - hx0) * H * 3, queue_of(d, si));
+            CK(ctx, tcrt_launch_render(rl, d.sm_count, ks, &launches, nullptr, 0));
+        }
+        rc = join(d, n_streams);
+        if (rc) return rc;
+        CK(ctx, tcrt_launch_adaptive_classify(d.ad_plain, hx0, W, H, bx0, bx1, contrast, f.frame, d.ad_mask, d.ad_counts,
+                                              d.ad_list, d.stream));
+        launches += 3;
+        f.h_counters[0] = 0;     // slot 0 of the counters is free: the list's length goes there
+        CK(ctx, cudaMemcpyAsync(f.h_counters, d.ad_counts + nb, sizeof(unsigned int), cudaMemcpyDeviceToHost, d.stream));
+        CK(ctx, cudaEventRecord(f.ev_done, d.stream));
+    }
+    // ---- 3: the lists' lengths -------------------------------------------------------------------------------------------------
+    std::vector<long long> n_list(nd, 0);
+    unsigned long long total = 0;
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        if (d.fr().x1 <= d.fr().x0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaEventSynchronize(d.fr().ev_done));
+        n_list[i] = (long long)(d.fr().h_counters[0] & 0xffffffffull);
+        total += (unsigned long long)n_list[i];
+    }
+    // ---- 4: sample pass --------------------------------------------------------------------------------------------------------
+    const long long per_piece = std::max(1LL, kPieceSamples / std::max(1, m));    // list entries per piece
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        FrameRes& f = d.fr();
+        if (f.x1 <= f.x0 || ss == 1 || n_list[i] == 0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        const int n_pieces = (int)((n_list[i] + per_piece - 1) / per_piece);
+        const int n_streams = ctx->one_stream ? 1 : std::min(kChunkStreams, n_pieces);
+        const size_t need = (size_t)std::min(n_list[i], per_piece) * m * 3;
+        for (int si = 0; si < n_streams; si++)     // a buffer about to be replaced may still serve a frame in flight
+            if (need > d.ss_scratch_cap[si]) {
+                CK(ctx, cudaDeviceSynchronize());
+                break;
+            }
+        for (int si = 0; si < n_streams; si++) {
+            rc = ensure(ctx, d.ss_scratch[si], d.ss_scratch_cap[si], need);
+            if (rc) return rc;
+        }
+        rc = fork(d, n_streams);
+        if (rc) return rc;
+        for (int k = 0; k < n_pieces; k++) {
+            const long long e0 = (long long)k * per_piece, cnt = std::min(per_piece, n_list[i] - e0);
+            const int si = k % n_streams;
+            const cudaStream_t ks = stream_of(d, si);
+            CK(ctx, cudaMemsetAsync(queue_of(d, si), 0, sizeof(unsigned int), ks));
+            RenderLaunch rl = band_launch(ctx, d, &sp, 0, sp.width, d.ss_scratch[si], queue_of(d, si));
+            rl.list = d.ad_list + e0;
+            rl.list_n = (int)(cnt * m);
+            rl.list_ss = ss;
+            CK(ctx, tcrt_launch_render_list(rl, d.sm_count, ks));
+            CK(ctx, tcrt_launch_adaptive_resolve(d.ad_list, (int)e0, (int)cnt, f.x0, H, ss, d.ss_scratch[si], f.frame, ks));
+            launches += 2;
+        }
+        rc = join(d, n_streams);
+        if (rc) return rc;
+    }
+    // ---- 5: output -------------------------------------------------------------------------------------------------------------
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        FrameRes& f = d.fr();
+        if (f.x1 <= f.x0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        const size_t n_px = (size_t)(f.x1 - f.x0) * H;
+        if (fmt == kRGB8) {
+            CK(ctx, tcrt_launch_quantize8(f.frame, n_px, f.frame8, d.stream));
+            launches++;
+        }
+        CK(ctx, cudaEventRecord(f.ev_k1, d.stream));
+        CK(ctx, cudaMemcpyAsync(f.h_counters, f.ctl, 32, cudaMemcpyDeviceToHost, d.stream));
+        CK(ctx, cudaEventRecord(f.ev_done, d.stream));
+        if (any_direct) {
+            CK(ctx, cudaStreamWaitEvent(d.copy_stream, f.ev_k1, 0));
+            if (host_band && !staged_frame)
+                CK(ctx, cudaMemcpyAsync(static_cast<char*>(host_band) + (size_t)(f.x0 - x0) * H * bpp, frame_src(f, fmt),
+                                        n_px * bpp, cudaMemcpyDeviceToHost, d.copy_stream));
+            if (host_mask && !staged_mask)
+                CK(ctx, cudaMemcpyAsync(host_mask + (size_t)(f.x0 - x0) * H, d.ad_mask, n_px, cudaMemcpyDeviceToHost,
+                                        d.copy_stream));
+            CK(ctx, cudaEventRecord(f.ev_c1, d.copy_stream));
+        }
+    }
+    // pageable destinations: through the pinned staging slots and the copy workers, band after band
+    for (int k = 0; k < 2; k++) {
+        if (!(k == 0 ? staged_frame : staged_mask)) continue;
+        const size_t b = k == 0 ? bpp : 1;
+        TxtPipe& pipe = copy_pipe_to(ctx, k == 0 ? host_band : host_mask);
+        cudaError_t e = cudaSuccess;
+        for (auto& d : ctx->devs) {
+            FrameRes& f = d.fr();
+            if (f.x1 <= f.x0) continue;
+            const char* src = k == 0 ? frame_src(f, fmt) : reinterpret_cast<const char*>(d.ad_mask);
+            e = cudaSetDevice(d.dev);
+            if (e == cudaSuccess) e = ensure_stage(d);
+            StageSlots slots;
+            if (e == cudaSuccess) e = stage_out(pipe, d, slots, src, (size_t)(f.x1 - f.x0) * H * b, (size_t)(f.x0 - x0) * H * b, f.ev_k1);
+            slots.drain(pipe);
+            if (e != cudaSuccess) break;
+        }
+        if (e != cudaSuccess || pipe.io_error)
+            return fail(ctx, TCRT_ERR_CUDA, "staged copy-out of an adaptive %s: %s", k == 0 ? "frame" : "mask",
+                        e != cudaSuccess ? cudaGetErrorString(e) : "a chunk did not arrive");
+    }
+    if (stats) memset(stats, 0, sizeof(*stats));
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        FrameRes& f = d.fr();
+        if (stats) {
+            stats->col_begin[i] = f.x0;
+            stats->col_end[i] = f.x1;
+        }
+        if (f.x1 <= f.x0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaEventSynchronize(f.ev_done));
+        if (any_direct) CK(ctx, cudaEventSynchronize(f.ev_c1));
+        if (stats) {
+            float ms = 0.f;
+            CK(ctx, cudaEventElapsedTime(&ms, f.ev_k0, f.ev_k1));
+            stats->render_ms[i] = ms;
+            if (any_direct) CK(ctx, cudaEventElapsedTime(&ms, f.ev_k1, f.ev_c1));
+            stats->d2h_ms[i] = any_direct ? std::max(ms, 0.f) : 0.0;
+            stats->rays_primary[i] = f.h_counters[1];
+            stats->rays_shadow[i] = f.h_counters[2];
+            stats->rays_reflect[i] = f.h_counters[3];
+        }
+    }
+    if (stats) {
+        stats->n_devices = nd;
+        stats->gpu_launches = (unsigned long long)launches;
+    }
+    if (n_refined) *n_refined = total;
+    ctx->has_frame = true;
+    ctx->txt_prepared = false;
+    ctx->frame_x0 = x0;
+    ctx->frame_x1 = x1;
+    ctx->frame_h = H;
+    return TCRT_OK;
+}
+
+extern "C" {
+
+int tcrt_render_columns_adaptive(tcrt_ctx* ctx, const tcrt_params* p, int ss, int contrast, int x0, int x1, float* host_rgb_band,
+                                 unsigned char* host_mask, unsigned long long* n_refined, tcrt_stats* stats) {
+    return render_adaptive(ctx, p, ss, contrast, x0, x1, host_rgb_band, kFloat32, host_mask, n_refined, stats);
+}
+
+int tcrt_render_columns_adaptive_rgb8(tcrt_ctx* ctx, const tcrt_params* p, int ss, int contrast, int x0, int x1,
+                                      unsigned char* host_rgb8_band, unsigned char* host_mask, unsigned long long* n_refined,
+                                      tcrt_stats* stats) {
+    if (!host_rgb8_band) return fail(ctx, TCRT_ERR_INVALID, "null output buffer");
+    return render_adaptive(ctx, p, ss, contrast, x0, x1, host_rgb8_band, kRGB8, host_mask, n_refined, stats);
 }
 
 }  // extern "C"

@@ -116,6 +116,12 @@ struct RenderLaunch {
     int n_objects;           // objects of the scene (checked builds verify table indices against it)
     int refill_min;          // idle lanes a warp waits for before it takes new pixels (1..32)
     int tiled;               // queue positions map to 4x8-pixel tiles (band width % 4 == 0, height % 8 == 0)
+    // list mode (tcrt_launch_render_list, adaptive frames): width x height is the ss*W x ss*H sample frame, x0 == 0, and
+    // queue position q traces sample 1 + q % (ss*ss-1) of frame pixel list[q / (ss*ss-1)] (x*H + z of the W x H frame)
+    // into out[3q..3q+2] (list_to_sample, tcrt_render_common.cuh).  Band mode ignores these.
+    const int* list;
+    int list_n;              // queue positions: list entries * (ss*ss - 1)
+    int list_ss;
 };
 
 // Primary-hit launch (tcrt_hits.cu): rl describes the frame, the band [x0, x1) and the scene; out of rl the kernel uses the
@@ -156,7 +162,10 @@ cudaError_t tcrt_launch_render_wave(const RenderLaunch& rl, int fm, int sm_count
                                     cudaStream_t stream, int* launches);
 size_t tcrt_render_max_smem();
 // kernel for scenes whose spheres sit in a uniform grid (tcrt_render_grid.cu); smem = bytes of the staged blob
-cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream);
+cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream,
+                                    bool list = false);
+// list-mode render launch (adaptive frames, RenderLaunch::list): the render or grid kernel's list-mode twin, one launch
+cudaError_t tcrt_launch_render_list(const RenderLaunch& rl, int sm_count, cudaStream_t stream);
 // experimental task-pool kernel for sphere-BVH scenes (tcrt_render_pool.cu, developer builds only); smem_scene = bytes of the staged blob
 cudaError_t tcrt_launch_render_pool(const RenderLaunch& rl, int fm, int sm_count, size_t smem_scene, cudaStream_t stream);
 // n random (a.xyz, b) cases: div3 (shared-reciprocal division of the render kernel) vs __fdiv_rn; *bad += mismatches
@@ -185,6 +194,17 @@ cudaError_t tcrt_launch_quantize8(const float* rgb, size_t n_pixels, unsigned ch
 // gets the same pixels quantised to 8 bits in the same pass.  samples must be 16-byte aligned.
 cudaError_t tcrt_launch_resolve_ss(const float* samples, int cols, int height, int ss, float* out, unsigned char* out8,
                                    cudaStream_t stream);
+// Adaptive frames (tcrt_adaptive.cu).  classify: for band [bx0, bx1) of the width x height frame, from the plain frame's
+// columns [px0, ...) (the band and its in-frame halo columns): mask[p] (1 = refined, contrast < 0 refines every pixel),
+// frame[p] = the plain pixel, then the refined pixels' x*height + z, x-major, into list and their number into
+// block_counts[ceil(band pixels / 256)] (block_counts holds that many + 1 words).  Three launches.
+cudaError_t tcrt_launch_adaptive_classify(const float* plain, int px0, int width, int height, int bx0, int bx1, int contrast,
+                                          float* frame, unsigned char* mask, unsigned int* block_counts, int* list,
+                                          cudaStream_t stream);
+// resolve of list entries [e0, e0 + n): samples 1 .. ss*ss-1 of entry e0 + t are scratch[(t*(ss*ss-1) + s-1)*3 ..] (the
+// list-mode render launch's output), sample 0 is the band's frame pixel; the mean, in tcrt.h's order, replaces it.
+cudaError_t tcrt_launch_adaptive_resolve(const int* list, int e0, int n, int bx0, int height, int ss, const float* scratch,
+                                         float* frame, cudaStream_t stream);
 cudaError_t tcrt_launch_l2_flush(void* scratch, size_t bytes, cudaStream_t stream);
 // 8 independent chains per thread, `iters` rounds: 8*iters FFMA, or 8*iters FMUL + 8*iters FADD
 cudaError_t tcrt_launch_fp32_peak(bool fma, float* scratch, int grid, int iters, cudaStream_t stream);

@@ -37,8 +37,10 @@
 
 namespace {
 
-template <int CAP, int SBVH, int FM>
-__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_kernel(const __grid_constant__ RenderLaunch rl) {
+// The kernel body.  LIST = false: the pixels of the band [rl.x0, rl.x1) (render_kernel).  LIST = true: the samples of a
+// pixel list (render_list_kernel, adaptive frames; RenderLaunch::list): only the refill block and the output slot differ.
+template <int CAP, int SBVH, int FM, bool LIST>
+__device__ __forceinline__ void render_body(const RenderLaunch& rl) {
     extern __shared__ float4 smem4[];
     const DeviceScene& sc = rl.scene;
     // ---- stage the sweep blob: coalesced 16-byte loads, once per CTA ------------------------
@@ -59,7 +61,7 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
 
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned total = (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = LIST ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     const V3 null_color = mk(rl.null_r, rl.null_g, rl.null_b);
 
     float stack[CAP * 7];   // per level: local rgb, k, object rgb (local memory, touched only on reflective hits)
@@ -100,9 +102,10 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
             if (ln.pix < 0 && rank < avail) {
                 int xc, z;
                 TCRT_CHECK(wcur + rank < total, kChkQueue);
-                queue_to_pixel(rl, (int)(wcur + rank), xc, z);
+                if (LIST) list_to_sample(rl, (int)(wcur + rank), xc, z);
+                else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
                 TCRT_CHECK(xc >= 0 && xc < rl.x1 - rl.x0 && z >= 0 && z < rl.height, kChkQueue);
-                ln.pix = xc * rl.height + z;
+                ln.pix = LIST ? (int)(wcur + rank) : xc * rl.height + z;
                 ln.level = 0;
                 primary_ray(rl, xc, z, ln.O, ln.D);
             }
@@ -295,7 +298,7 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
                 o[1] = tail.y;
                 o[2] = tail.z;
                 // cost estimate for the band balancer's pre-pass: bounces of this pixel, per column
-                if (rl.col_cost != nullptr) {
+                if (!LIST && rl.col_cost != nullptr) {
                     const int xc = ln.pix / rl.height;
                     atomicAdd(rl.col_cost + xc, (unsigned)(ln.level + 1));
                     atomicAdd(rl.col_cost + (rl.x1 - rl.x0) + (ln.pix - xc * rl.height), (unsigned)(ln.level + 1));
@@ -315,6 +318,16 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
 }
 
 template <int CAP, int SBVH, int FM>
+__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_body<CAP, SBVH, FM, false>(rl);
+}
+
+template <int CAP, int SBVH, int FM>
+__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_list_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_body<CAP, SBVH, FM, true>(rl);
+}
+
+template <int CAP, int SBVH, int FM>
 cudaError_t launch_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
     cudaError_t e = cudaFuncSetAttribute(render_kernel<CAP, SBVH, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);
@@ -329,6 +342,27 @@ cudaError_t launch_cap(const RenderLaunch& rl, int grid, size_t smem, cudaStream
     const int fm = rl.scene.bvh_fin != nullptr ? 2 : (rl.scene.n_fin == 0 ? 0 : (rl.scene.n_clu > 0 ? 1 : 3));
 #define TCRT_CASE(SB, FMV) \
     if (sb == SB && fm == FMV) return launch_one<CAP, SB, FMV>(rl, grid, smem, stream);
+    TCRT_CASE(0, 0) TCRT_CASE(0, 1) TCRT_CASE(0, 2) TCRT_CASE(0, 3)
+    TCRT_CASE(1, 0) TCRT_CASE(1, 1) TCRT_CASE(1, 2) TCRT_CASE(1, 3)
+#undef TCRT_CASE
+    return cudaErrorInvalidValue;
+}
+
+template <int CAP, int SBVH, int FM>
+cudaError_t launch_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
+    cudaError_t e = cudaFuncSetAttribute(render_list_kernel<CAP, SBVH, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
+    if (e != cudaSuccess) return e;
+    render_list_kernel<CAP, SBVH, FM><<<grid, kBlock, smem, stream>>>(rl);
+    return cudaGetLastError();
+}
+
+template <int CAP>
+cudaError_t launch_list_cap(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
+    const int sb = rl.scene.bvh_sph == nullptr ? 0 : 1;
+    const int fm = rl.scene.bvh_fin != nullptr ? 2 : (rl.scene.n_fin == 0 ? 0 : (rl.scene.n_clu > 0 ? 1 : 3));
+#define TCRT_CASE(SB, FMV) \
+    if (sb == SB && fm == FMV) return launch_list_one<CAP, SB, FMV>(rl, grid, smem, stream);
     TCRT_CASE(0, 0) TCRT_CASE(0, 1) TCRT_CASE(0, 2) TCRT_CASE(0, 3)
     TCRT_CASE(1, 0) TCRT_CASE(1, 1) TCRT_CASE(1, 2) TCRT_CASE(1, 3)
 #undef TCRT_CASE
@@ -488,4 +522,30 @@ cudaError_t tcrt_launch_render(const RenderLaunch& rl_in, int sm_count, cudaStre
     else e = launch_cap<256>(rl, grid, smem, stream);
     if (launches) *launches += 1;
     return e;
+}
+
+// List mode (adaptive frames): the same kernels with the list refill, grid-sized and dispatched as tcrt_launch_render
+// does, never the developer builds' pool or wavefront paths.  One launch; nothing when the list is empty.
+cudaError_t tcrt_launch_render_list(const RenderLaunch& rl_in, int sm_count, cudaStream_t stream) {
+    RenderLaunch rl = rl_in;
+    if (rl.list_n <= 0) return cudaSuccess;
+    const size_t smem = (size_t)std::max(1, rl.scene.blob_f4 - rl.scene.stage_off) * sizeof(float4);
+    if (smem > tcrt_render_max_smem()) return cudaErrorInvalidValue;
+    const int fm = finite_mode(rl.scene);
+    rl.tiled = 0;
+    rl.row_order = nullptr;
+    rl.col_cost = nullptr;
+    rl.refill_min = 32;
+    if (rl.scene.grid_cells != nullptr && rl.scene.bvh_sph != nullptr && (fm == 0 || fm == 3))
+        return tcrt_launch_render_grid(rl, fm, sm_count, smem, stream, true);
+    int ctas_per_sm = (rl.scene.bvh_sph != nullptr && rl.scene.n_fin == 0) ? kMinBlocksBvh : kMinBlocks;
+    while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;
+    // persistent grid, but no more CTAs than there are claims of 32 queue positions per warp
+    const long long need = ((long long)rl.list_n + kBlock - 1) / kBlock;
+    const int grid = (int)std::min<long long>((long long)sm_count * ctas_per_sm, need);
+    const int levels = rl.max_depth + 1;
+    if (levels <= 8) return launch_list_cap<8>(rl, grid, smem, stream);
+    if (levels <= 16) return launch_list_cap<16>(rl, grid, smem, stream);
+    if (levels <= 64) return launch_list_cap<64>(rl, grid, smem, stream);
+    return launch_list_cap<256>(rl, grid, smem, stream);
 }

@@ -28,8 +28,10 @@ namespace {
 constexpr int kGridBlock = TCRT_GRID_BLOCK;
 constexpr int kGridMinBlocks = TCRT_GRID_MIN_BLOCKS;      // the walk waits on cell and sphere loads: 4 CTAs/SM at 64 registers
 
-template <int CAP, int FM>
-__global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel(const __grid_constant__ RenderLaunch rl) {
+// The kernel body.  LIST = false: the pixels of the band (render_grid_kernel); LIST = true: the samples of a pixel list
+// (render_grid_list_kernel, adaptive frames; RenderLaunch::list): only the refill block and the output slot differ.
+template <int CAP, int FM, bool LIST>
+__device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
     extern __shared__ float4 smem4[];
     const DeviceScene& sc = rl.scene;
     // ---- stage the sweep blob (the grid-covered spheres in front of stage_off stay in global memory) ----------------
@@ -49,7 +51,7 @@ __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel
 
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned total = (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = LIST ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     const V3 null_color = mk(rl.null_r, rl.null_g, rl.null_b);
 
     float stack[CAP * 7];   // per level: local rgb, k, object rgb (local memory, touched only on reflective hits)
@@ -85,8 +87,9 @@ __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel
             if (ln.pix < 0 && rank < avail) {
                 int xc, z;
                 TCRT_CHECK(wcur + rank < total, kChkQueue);
-                queue_to_pixel(rl, (int)(wcur + rank), xc, z);
-                ln.pix = xc * rl.height + z;
+                if (LIST) list_to_sample(rl, (int)(wcur + rank), xc, z);
+                else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
+                ln.pix = LIST ? (int)(wcur + rank) : xc * rl.height + z;
                 ln.level = 0;
                 primary_ray(rl, xc, z, ln.O, ln.D);
             }
@@ -383,7 +386,7 @@ __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel
                 o[1] = tail.y;
                 o[2] = tail.z;
                 // cost estimate for the band balancer's pre-pass: bounces of this pixel, per column
-                if (rl.col_cost != nullptr) {
+                if (!LIST && rl.col_cost != nullptr) {
                     const int xc = ln.pix / rl.height;
                     atomicAdd(rl.col_cost + xc, (unsigned)(ln.level + 1));
                     atomicAdd(rl.col_cost + (rl.x1 - rl.x0) + (ln.pix - xc * rl.height), (unsigned)(ln.level + 1));
@@ -403,6 +406,16 @@ __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel
 }
 
 template <int CAP, int FM>
+__global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_grid_body<CAP, FM, false>(rl);
+}
+
+template <int CAP, int FM>
+__global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_list_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_grid_body<CAP, FM, true>(rl);
+}
+
+template <int CAP, int FM>
 cudaError_t launch_grid_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
     cudaError_t e = cudaFuncSetAttribute(render_grid_kernel<CAP, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -410,8 +423,17 @@ cudaError_t launch_grid_one(const RenderLaunch& rl, int grid, size_t smem, cudaS
     return cudaGetLastError();
 }
 
+template <int CAP, int FM>
+cudaError_t launch_grid_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
+    cudaError_t e = cudaFuncSetAttribute(render_grid_list_kernel<CAP, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    render_grid_list_kernel<CAP, FM><<<grid, kGridBlock, smem, stream>>>(rl);
+    return cudaGetLastError();
+}
+
 template <int CAP>
-cudaError_t launch_grid_cap(const RenderLaunch& rl, int fm, int grid, size_t smem, cudaStream_t stream) {
+cudaError_t launch_grid_cap(const RenderLaunch& rl, int fm, int grid, size_t smem, cudaStream_t stream, bool list) {
+    if (list) return fm == 0 ? launch_grid_list_one<CAP, 0>(rl, grid, smem, stream) : launch_grid_list_one<CAP, 3>(rl, grid, smem, stream);
     return fm == 0 ? launch_grid_one<CAP, 0>(rl, grid, smem, stream) : launch_grid_one<CAP, 3>(rl, grid, smem, stream);
 }
 
@@ -429,14 +451,16 @@ extern "C" int tcrt_dev_lane_stats_grid(unsigned long long* out16, int reset) {
 }
 #endif
 
-// fm: 0 no finite planes, 3 a handful swept linearly; rl.scene.grid_cells != nullptr (tcrt_upload_scene built a grid)
-cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream) {
+// fm: 0 no finite planes, 3 a handful swept linearly; rl.scene.grid_cells != nullptr (tcrt_upload_scene built a grid).
+// list: the list-mode kernels (tcrt_launch_render_list), with no more CTAs than there are claims.
+cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream, bool list) {
     int ctas_per_sm = kGridMinBlocks;
     while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;
-    const int grid = sm_count * ctas_per_sm;
+    int grid = sm_count * ctas_per_sm;
+    if (list) grid = (int)std::min<long long>(grid, ((long long)rl.list_n + kGridBlock - 1) / kGridBlock);
     const int levels = rl.max_depth + 1;
-    if (levels <= 8) return launch_grid_cap<8>(rl, fm, grid, smem, stream);
-    if (levels <= 16) return launch_grid_cap<16>(rl, fm, grid, smem, stream);
-    if (levels <= 64) return launch_grid_cap<64>(rl, fm, grid, smem, stream);
-    return launch_grid_cap<256>(rl, fm, grid, smem, stream);
+    if (levels <= 8) return launch_grid_cap<8>(rl, fm, grid, smem, stream, list);
+    if (levels <= 16) return launch_grid_cap<16>(rl, fm, grid, smem, stream, list);
+    if (levels <= 64) return launch_grid_cap<64>(rl, fm, grid, smem, stream, list);
+    return launch_grid_cap<256>(rl, fm, grid, smem, stream, list);
 }

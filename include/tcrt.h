@@ -180,6 +180,12 @@ int tcrt_plan_scene(const tcrt_scene* scene, int info[8], int grid_dims[3]);
  * (optional): the fattening up to which a ray may use the grid. */
 int tcrt_plan_grid_cells(const tcrt_scene* scene, const float* points, int n_points, int* objects, int cap, int* counts,
                          float* grid_margin);
+/* Host only: *prune = 1 when renders of the scene with params may skip the shading of reflection levels whose colour the
+ * reference multiplies by zero (the path's every channel has met a zero object colour above them; sphere-grid scenes,
+ * DESIGN.md 4.1c) — when a bound on every colour the reference forms on the way is finite and far from overflow.  The
+ * result is the same either way; 0 where a zero could meet an overflowed colour and make NaN, which is then rendered.
+ * Bad params: TCRT_ERR_INVALID; max_depth above TCRT_MAX_DEPTH: TCRT_ERR_UNSUPPORTED, as for renders. */
+int tcrt_plan_dead_paths(const tcrt_scene* scene, const tcrt_params* params, int* prune);
 
 /* ---- render (replaces the pixel loop RayTracer.cpp:911-923) ----------------------- */
 /* Whole image -> host_rgb[width*height*3], x-major, z fastest, (r,g,b) float32: the layout

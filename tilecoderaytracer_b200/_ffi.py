@@ -85,6 +85,7 @@ SIGNATURES = {
     "tcrt_scene_structures": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "tcrt_plan_scene": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "tcrt_plan_grid_cells": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_float)]),
+    "tcrt_plan_dead_paths": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.POINTER(C.c_int)]),
     "tcrt_render": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_void_p, C.POINTER(TcrtStats)]),
     "tcrt_render_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_int, C.c_void_p,
                                       C.POINTER(TcrtStats)]),

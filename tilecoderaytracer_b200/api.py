@@ -227,6 +227,17 @@ def plan_grid_cells(flat, points, cap: int = 32):
     return [set(int(v) for v in objs[i, :counts[i]]) for i in range(len(pts))], float(margin.value)
 
 
+def plan_dead_paths(flat, params: TcrtParams) -> bool:
+    """Whether renders of the flattened scene with params may skip the shading of dead reflection levels
+    (tcrt_plan_dead_paths, host only)."""
+    lib = _ffi.load()
+    prune = C.c_int(0)
+    rc = lib.tcrt_plan_dead_paths(C.byref(flat), C.byref(params), C.byref(prune))
+    if rc != 0:
+        raise TcrtError(rc, (lib.tcrt_last_error(None) or b"").decode())
+    return bool(prune.value)
+
+
 class HostBuffer:
     """Pinned host memory (tcrt_alloc_host) viewed as a numpy array."""
 

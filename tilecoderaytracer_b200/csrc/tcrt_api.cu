@@ -127,6 +127,16 @@ struct DeviceState {
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
 struct TxtSink;
 
+// Bounds on the colours a scene's paths form (DESIGN.md §4.1c), from its materials alone; dead_paths_prunable adds the
+// launch's depth and NULL_COLOR.
+struct DeadPathBound {
+    bool finite = false;   // every colour, factor, intensity and texture colour is finite
+    double local = 0.0;    // |local| of any level: every light's diffuse and specular terms, clamps ignored
+    double leaf = 0.0;     // |tail| of a light hit or of a non-reflective hit (local)
+    double obj = 0.0;      // largest |object colour| component, textures included
+    double kref = 0.0;     // largest reflective factor
+};
+
 }  // namespace
 
 static void destroy_copy_pipe(tcrt_ctx* ctx);
@@ -172,6 +182,7 @@ struct tcrt_ctx {
     DeviceScene scene_ds{};
     size_t scene_off[9] = {};       // surface, material, normals, frame, tex, bvh_s, bvh_f, grid cells, grid items
     bool scene_bvh_s = false, scene_bvh_f = false, scene_grid = false;
+    DeadPathBound scene_dead;
 };
 
 namespace {
@@ -463,6 +474,82 @@ static int validate_scene(tcrt_ctx* ctx, const tcrt_scene* s) {
         if (s->light_obj[i] < 0 || s->light_obj[i] >= n) return fail(ctx, TCRT_ERR_INVALID, "light_obj out of range");
     for (int i = 0; i < n; i++)
         if (s->obj_info[4 * i + 3] >= s->n_textures) return fail(ctx, TCRT_ERR_INVALID, "texture id out of range");
+    return TCRT_OK;
+}
+
+// The grid kernel skips the shading of a level once every channel has met a zero object colour above it: that is exact
+// only if every tail the reference forms (and k * tail) is finite, so that the zero turns it into +-0 and not into NaN
+// (DESIGN.md §4.1c).  A bound in double: |dot| <= 1.001 for the unit vectors of the light loop (a cosine and the (V.R)
+// of the specular term, whose 20th power is then <= 1.001^20), clamps ignored, leaf tails the NULL_COLOR, a light's
+// colour (texture included) times its intensity, or a local colour; each stacked level adds its local colour to
+// kref * obj * its child's.  The float arithmetic's relative error over a whole path stays below 1 %, far inside the
+// margin to FLT_MAX that dead_paths_prunable keeps.
+static DeadPathBound dead_path_bound(const tcrt_scene* s) {
+    DeadPathBound b;
+    const int n = s->n_objects;
+    bool finite = true;
+    auto fin = [&](float v) {
+        finite = finite && std::isfinite(v);
+        return fabs((double)v);
+    };
+    auto tex_max = [&](int t) {   // largest |component| of texture t's two colours
+        double m = 0.0;
+        for (int k = 0; k < 3; k++) m = std::max({m, fin(s->textures[8 * t + k]), fin(s->textures[8 * t + 4 + k])});
+        return m;
+    };
+    double diffuse = 0.0, specular = 0.0, light_leaf = 0.0;
+    for (int i = 0; i < n; i++) {
+        double col = 0.0;
+        for (int k = 0; k < 3; k++) col = std::max(col, fin(s->obj_surface[4 * i + k]));
+        const int tex = s->obj_info[4 * i + 3];
+        if (tex >= 0) col = std::max(col, tex_max(tex));
+        b.obj = std::max(b.obj, col);
+        diffuse = std::max(diffuse, fin(s->obj_surface[4 * i + 3]));
+        specular = std::max(specular, fin(s->obj_material[4 * i]));
+        b.kref = std::max(b.kref, fin(s->obj_material[4 * i + 1]));
+        const double inten = fin(s->obj_material[4 * i + 2]);
+        if (s->obj_info[4 * i + 2]) light_leaf = std::max(light_leaf, col * inten);
+    }
+    const double dot = 1.001, pw = pow(dot, 20.0);
+    for (int l = 0; l < s->n_lights; l++) {
+        const int lo = s->light_obj[l];
+        double lc = 0.0;
+        for (int k = 0; k < 3; k++) lc = std::max(lc, fabs((double)s->obj_surface[4 * lo + k]));
+        // every factor taken as at least 1: then each partial product the light loop forms on the way — c * diffuse,
+        // * intensity, * object colour (f * color * lc), and pw * specular — stays below its term as well, so no
+        // intermediate can overflow to inf (and turn into NaN at a zero colour) while the bound stays small
+        auto at_least_1 = [](double v) { return std::max(v, 1.0); };
+        const double inten = fabs((double)s->obj_material[4 * lo + 2]);
+        b.local += dot * at_least_1(diffuse) * at_least_1(inten) * at_least_1(b.obj) * at_least_1(lc) +
+                   at_least_1(lc) * pw * at_least_1(specular);
+    }
+    b.leaf = std::max(light_leaf, b.local);
+    b.finite = finite && std::isfinite(b.local);
+    return b;
+}
+
+// Whether launches of `p` may skip dead levels: the scene's bound is finite and, over max_depth + 1 stacked levels below
+// a leaf, every tail and every k * tail stays below 1e30 (FLT_MAX is 3.4e38).
+static bool dead_paths_prunable(const DeadPathBound& b, const tcrt_params* p) {
+    if (!b.finite) return false;
+    double tail = 0.0;
+    for (int k = 0; k < 3; k++) {
+        if (!std::isfinite(p->null_color[k])) return false;
+        tail = std::max(tail, fabs((double)p->null_color[k]));
+    }
+    tail = std::max(tail, b.leaf);
+    const double limit = 1e30;
+    for (int level = p->max_depth; level >= 0 && tail <= limit && b.kref * tail <= limit; level--)
+        tail = b.local + b.kref * b.obj * tail;
+    return tail <= limit && b.kref * tail <= limit;
+}
+
+int tcrt_plan_dead_paths(const tcrt_scene* s, const tcrt_params* p, int* prune) {
+    if (!s || !p || !prune) return fail(nullptr, TCRT_ERR_INVALID, "null argument");
+    if (!valid_params(p)) return fail(nullptr, TCRT_ERR_INVALID, "bad params");
+    if (p->max_depth > TCRT_MAX_DEPTH) return fail(nullptr, TCRT_ERR_UNSUPPORTED, "max_depth too large");
+    if (int rc = validate_scene(nullptr, s)) return rc;
+    *prune = dead_paths_prunable(dead_path_bound(s), p) ? 1 : 0;
     return TCRT_OK;
 }
 
@@ -851,6 +938,7 @@ static int build_scene_blob(tcrt_ctx* ctx, const tcrt_scene* s) {
     ctx->scene_grid = b.grid;
     ctx->scene_bvh_s = b.bvh_s;
     ctx->scene_bvh_f = b.bvh_f;
+    ctx->scene_dead = dead_path_bound(s);
     return TCRT_OK;
 }
 
@@ -1223,6 +1311,7 @@ static RenderLaunch band_launch(tcrt_ctx* ctx, DeviceState& d, const tcrt_params
     rl.null_g = p->null_color[1];
     rl.null_b = p->null_color[2];
     rl.far_dist = p->far_dist;
+    rl.prune_dead = dead_paths_prunable(ctx->scene_dead, p) ? 1 : 0;
     rl.n_objects = ctx->n_objects;
     rl.out = out;
     rl.queue = queue ? queue : reinterpret_cast<unsigned int*>(d.fr().ctl);

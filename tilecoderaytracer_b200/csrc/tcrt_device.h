@@ -116,6 +116,8 @@ struct RenderLaunch {
     int n_objects;           // objects of the scene (checked builds verify table indices against it)
     int refill_min;          // idle lanes a warp waits for before it takes new pixels (1..32)
     int tiled;               // queue positions map to 4x8-pixel tiles (band width % 4 == 0, height % 8 == 0)
+    int prune_dead;          // every colour the reference forms is finite: the grid kernel may skip the shading of levels
+                             // whose contribution is multiplied by a zero object colour (dead_path_bound, tcrt_api.cu)
     // list mode (tcrt_launch_render_list, adaptive frames): width x height is the ss*W x ss*H sample frame, x0 == 0, and
     // queue position q traces sample 1 + q % (ss*ss-1) of frame pixel list[q / (ss*ss-1)] (x*H + z of the W x H frame)
     // into out[3q..3q+2] (list_to_sample, tcrt_render_common.cuh).  Band mode ignores these.

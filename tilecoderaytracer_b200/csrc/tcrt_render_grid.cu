@@ -27,6 +27,15 @@ namespace {
 #endif
 constexpr int kGridBlock = TCRT_GRID_BLOCK;
 constexpr int kGridMinBlocks = TCRT_GRID_MIN_BLOCKS;      // the walk waits on cell and sphere loads: 4 CTAs/SM at 64 registers
+// Lane::level packs, so that dead paths (DESIGN.md §4.1c) cost no register: bits 0-7 the recursion level, bits 8-16 the
+// level records stacked when the path died, bits 20-22 the channels that have met a zero object colour on a stacked
+// level.  A path with all three is dead: nothing of its level or any deeper one can reach the pixel.
+constexpr int kLevelMask = 0xff;
+constexpr int kRecShift = 8;
+constexpr int kRecMask = 0x1ff;
+constexpr int kZeroShift = 20;
+constexpr int kDead = 7 << kZeroShift;
+static_assert(TCRT_MAX_DEPTH < kLevelMask, "levels and level records have to fit their fields");
 
 // The kernel body.  LIST = false: the pixels of the band (render_grid_kernel); LIST = true: the samples of a pixel list
 // (render_grid_list_kernel, adaptive frames; RenderLaunch::list): only the refill block and the output slot differ.
@@ -99,6 +108,7 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
         }
         if (idle == kFull) break;
         const bool active = ln.pix >= 0;
+        const bool dead = ln.level >= kDead;   // traced for the reference's ray counts only: no shading, no record
 
         // ---- one bounce = passes around ONE walk: pass 0 the ray, pass l the shadow ray to light l - 1 ---------------------
         V3 P = ln.O, n2 = mk(0.f, 0.f, 1.f), N = n2, refl = ln.D, color = null_color;
@@ -125,7 +135,6 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                 rD = div3(dir, best);
                 want = shade;
                 if (rl.shadows_on) {
-                    n_shadow += (unsigned)__popc(__ballot_sync(kFull, shade));
                     // The answer only matters if this light can change `local`: a positive cosine term, the clamp of
                     // cosineShade (which runs for every unshadowed light once local > 1), or a positive specular dot
                     // product.  Otherwise the ray is counted (the reference casts it) but not traced.
@@ -251,7 +260,7 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                     kref = mat.y;
                     inten = mat.z;
                     is_light = flags < 0;
-                    const int tex = (flags & 0x7fffffff) - 1;
+                    const int tex = dead ? -1 : (flags & 0x7fffffff) - 1;   // a dead level's colour is not used
                     V3 n1;
                     const V3 Pp = scale(ln.D, best) + ln.O;   // t*D + O  (SceneSphere.cpp:122, SceneFinitePlane.cpp:108)
                     if (bkey < sc.n_sph) {
@@ -296,7 +305,21 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                         refl = normalize(mk(-2.0f * n1.x * ndi + ln.D.x, -2.0f * n1.y * ndi + ln.D.y, -2.0f * n1.z * ndi + ln.D.z));
                     }
                 }
-                shade = hit && !is_light;
+                // the reference casts a shadow ray per light from every non-light hit; the light passes trace the ones
+                // that can change the pixel, and a warp without a live lane to shade skips them altogether
+                if (rl.shadows_on) n_shadow += (unsigned)sc.n_lights * (unsigned)__popc(__ballot_sync(kFull, hit && !is_light));
+#ifdef TCRT_LANE_STATS
+                {   // light passes dropped at dead levels: slot 6 warp-passes skipped whole (no live lane left to shade),
+                    // slot 7 lane-passes (shadow rays counted, not traced)
+                    const unsigned dead_shade = __ballot_sync(kFull, hit && !is_light && dead);
+                    const bool none_live = !__any_sync(kFull, hit && !is_light && !dead);
+                    if (lane == 0 && rl.shadows_on && dead_shade != 0u) {
+                        if (none_live) atomicAdd(&g_lane_stats[6], (unsigned long long)sc.n_lights);
+                        atomicAdd(&g_lane_stats[7], (unsigned long long)__popc(dead_shade) * (unsigned long long)sc.n_lights);
+                    }
+                }
+#endif
+                shade = hit && !is_light && !dead;
             } else if (shade && (!rl.shadows_on || (want && !found))) {
                 // ---- light pass - 1 reaches the hit (RayTracer.cpp:548-588); rD is the light ray ---------------------------------
                 // (a light whose answer did not matter adds nothing and leaves `local` as it is: skipping it is exact)
@@ -342,19 +365,28 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
         if (active) {
             V3 tail;
             bool done = true;
-            int n_stacked = ln.level;
+            // every level below this one stacked a record, up to the one where the path died
+            int n_stacked = dead ? (ln.level >> kRecShift) & kRecMask : ln.level & kLevelMask;
             if (!hit) {
                 tail = null_color;                        // :507-509
             } else if (is_light) {
                 tail = scale(color, inten);               // :520-527
             } else if (rl.reflections_on && kref > 0.0f) {   // :595-604
-                TCRT_CHECK(ln.level >= 0 && ln.level < CAP, kChkLevelStack);
-                float* rec = stack + 7 * ln.level;   // every level below this one stacked a record
-                rec[0] = local.x; rec[1] = local.y; rec[2] = local.z;
-                rec[3] = kref;
-                rec[4] = color.x; rec[5] = color.y; rec[6] = color.z;
-                ++n_stacked;
-                if (ln.level + 1 > rl.max_depth) {
+                if (!dead) {
+                    TCRT_CHECK(n_stacked >= 0 && n_stacked < CAP, kChkLevelStack);
+                    float* rec = stack + 7 * n_stacked;
+                    rec[0] = local.x; rec[1] = local.y; rec[2] = local.z;
+                    rec[3] = kref;
+                    rec[4] = color.x; rec[5] = color.y; rec[6] = color.z;
+                    ++n_stacked;
+                    // (k * child) * obj.c is +-0 for a finite child when obj.c == +-0: channel c of the pixel no longer
+                    // depends on anything deeper.  rl.prune_dead: every child the reference forms is finite.
+                    if (rl.prune_dead) {
+                        ln.level |= ((color.x == 0.0f ? 1 : 0) | (color.y == 0.0f ? 2 : 0) | (color.z == 0.0f ? 4 : 0)) << kZeroShift;
+                        if (ln.level >= kDead) ln.level |= n_stacked << kRecShift;
+                    }
+                }
+                if ((ln.level & kLevelMask) + 1 > rl.max_depth) {
                     tail = null_color;                    // the child returns NULL_COLOR (:454-455)
                 } else {
                     reflected = true;
@@ -367,6 +399,7 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                 tail = local;
             }
             if (done) {
+                if (dead) tail = mk(0.f, 0.f, 0.f);   // the deepest record's child: any finite colour gives the same pixel
                 // final += (k * child) * obj, deepest level first (:601)
                 TCRT_UNROLL_LOOP
                 for (int i = n_stacked - 1; i >= 0; --i) {
@@ -388,8 +421,9 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                 // cost estimate for the band balancer's pre-pass: bounces of this pixel, per column
                 if (!LIST && rl.col_cost != nullptr) {
                     const int xc = ln.pix / rl.height;
-                    atomicAdd(rl.col_cost + xc, (unsigned)(ln.level + 1));
-                    atomicAdd(rl.col_cost + (rl.x1 - rl.x0) + (ln.pix - xc * rl.height), (unsigned)(ln.level + 1));
+                    const unsigned bounces = (unsigned)((ln.level & kLevelMask) + 1);
+                    atomicAdd(rl.col_cost + xc, bounces);
+                    atomicAdd(rl.col_cost + (rl.x1 - rl.x0) + (ln.pix - xc * rl.height), bounces);
                 }
                 ln.pix = -1;
             }

@@ -43,3 +43,5 @@ for name in [a for a in sys.argv[1:] if not a.startswith("--")] or ["synth256_10
     if "--grid" in sys.argv:
         print(f"  shadow walks of a bounce: sum over passes of the longest walk {out[4]}, longest per-lane sum {out[5]} "
               f"({out[5] / max(out[4], 1):.3f})")
+        print(f"  light passes at dead levels (DESIGN.md §4.1c): warp-passes skipped whole {out[6]}, lane-passes {out[7]} "
+              f"({out[7] / max(st.rays_shadow, 1):.3f} of the {st.rays_shadow} shadow rays counted)")

@@ -473,6 +473,19 @@ cudaError_t launch_grid_cap(const RenderLaunch& rl, int fm, int grid, size_t sme
 
 }  // namespace
 
+#ifdef TCRT_CHECKED
+// the checked build's flags of this translation unit (tcrt_dev_check_flags reads those of tcrt_render.cu)
+extern "C" int tcrt_dev_grid_check_flags(unsigned int* flags, int reset) {
+    cudaDeviceSynchronize();
+    if (flags && cudaMemcpyFromSymbol(flags, g_check_flags, sizeof(unsigned int)) != cudaSuccess) return -1;
+    if (reset) {
+        const unsigned int z = 0;
+        if (cudaMemcpyToSymbol(g_check_flags, &z, sizeof z) != cudaSuccess) return -1;
+    }
+    return 0;
+}
+#endif
+
 #ifdef TCRT_LANE_STATS
 extern "C" int tcrt_dev_lane_stats_grid(unsigned long long* out16, int reset) {
     cudaDeviceSynchronize();

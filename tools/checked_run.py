@@ -1,26 +1,56 @@
 #!/usr/bin/env python
 """Sanitizer substitute (compute-sanitizer is closed on the GPU pool): renders the parity scenes with a -DTCRT_CHECKED
 library — every index range-checked, the level stack poisoned and checked for reads of unwritten records — compares
-every frame with the oracle bit for bit, and reports the check flags (0 = nothing fired).
-usage: TCRT_LIB=.../libtcrt_checked.so python tools/checked_run.py"""
+every frame with the oracle bit for bit, and reports the check flags (0 = nothing fired).  Then the same for every
+dispatch class of tests/test_kernel_variants.py at the boundary depths of each level stack: band kernels (a tiled and an
+untiled frame, a band from an odd column), list kernels (adaptive frames refining every pixel) and hit kernels.  The
+flags are read from each translation unit that launches a kernel: render, grid and hits.
+usage: python -c "from tilecoderaytracer_b200 import build; build.build_lib(defines=('TCRT_CHECKED',), out=LIB)"
+       TCRT_LIB=LIB python tools/checked_run.py"""
 import ctypes as C
 import os
+import subprocess
 import sys
+import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np  # noqa: E402
 
 from oracle import oracle_py as O  # noqa: E402
 from tilecoderaytracer_b200 import _ffi, api  # noqa: E402
+import test_kernel_variants as V  # noqa: E402
+from test_hit_buffers import assert_hits_equal, primary_hits  # noqa: E402
 
 NAMES = ["pixel store", "level stack index", "BVH stack pointer", "primitive key", "object index", "leaf range", "node index",
          "read of an unwritten level record", "cluster face slot", "queue position"]
 lib = _ffi.load()
 print("lib:", os.path.basename(_ffi.LIB_PATH), flush=True)
+READERS = [lib.tcrt_dev_check_flags, lib.tcrt_dev_grid_check_flags, lib.tcrt_dev_hits_check_flags]
 ctx = api.Context([0])
 flags = C.c_uint(0)
-lib.tcrt_dev_check_flags(C.byref(flags), 1)
+
+
+def fired():
+    """Names of the checks that fired since the last call, in any translation unit; resets the flags."""
+    bits = 0
+    for read in READERS:
+        if read(C.byref(flags), 1) != 0:
+            raise RuntimeError("cannot read the check flags")
+        bits |= flags.value
+    return [NAMES[b] for b in range(len(NAMES)) if bits >> b & 1]
+
+
+def n_bad(img, ref):
+    return int((img.view(np.uint32) != ref.view(np.uint32)).any(-1).sum())
+
+
+def counters_differ(st, cnt):
+    return int((st.rays_primary, st.rays_shadow, st.rays_reflect) != (cnt["rays_primary"], cnt["rays_shadow"], cnt["rays_reflect"]))
+
+
+fired()
 bad_total = 0
 CASES = [("default", 160, 128, 50), ("boxes:3:14", 128, 96, 12), ("synth256", 160, 128, 10), ("two_mirrors", 96, 80, 50),
          ("synth1024", 160, 128, 50), ("random:24:200", 112, 80, 9), ("random:27:1500", 64, 48, 6), ("random:7:120", 120, 96, 9),
@@ -32,9 +62,56 @@ for name, w, h, d in CASES:
     p = api.default_params(w, h, d)
     img, st = ctx.render(p)
     ref, cnt = O.render(sc.flatten(), cam.export(), p)
-    bad = int((img.view(np.uint32) != ref.view(np.uint32)).any(-1).sum())
-    lib.tcrt_dev_check_flags(C.byref(flags), 1)
-    fired = [NAMES[b] for b in range(len(NAMES)) if flags.value >> b & 1]
-    bad_total += bad + len(fired)
-    print(f"{name:16s} {w}x{h} d{d}: mismatching pixels {bad}, finite {bool(np.isfinite(img).all())}, checks fired: {fired or 'none'}", flush=True)
+    bad = n_bad(img, ref)
+    f = fired()
+    bad_total += bad + len(f)
+    print(f"{name:16s} {w}x{h} d{d}: mismatching pixels {bad}, finite {bool(np.isfinite(img).all())}, checks fired: {f or 'none'}", flush=True)
+
+# ---- every dispatch class at the boundary depths of the level stacks --------------------------------------------------------
+with tempfile.TemporaryDirectory() as tmp:
+    so = os.path.join(tmp, "liboracle_hits.so")
+    subprocess.run(["gcc", "-std=gnu11", "-O2", "-fPIC", "-shared", "-ffp-contract=off", os.path.join(ROOT, "tests", "oracle_hits.c"),
+                    "-o", so, "-lm"], check=True)
+    hits_lib = C.CDLL(so)
+    hits_lib.tcrt_oracle_primary_hits.restype = C.c_int
+    hits_lib.tcrt_oracle_primary_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                  C.c_void_p, C.c_void_p, C.c_void_p]
+    for name in V.NAMES:
+        s, cam = V.build(name)
+        flat, c = s.flatten(), cam.export()
+        ctx.upload_flat(flat, c)
+        cls = V.dispatch_class(ctx.scene_structures())
+        if cls != V.VARIANTS[name][3]:
+            print(f"{name}: dispatch class {cls}, expected {V.VARIANTS[name][3]}")
+            bad_total += 1
+        for d in V.DEPTHS:
+            tiled, untiled, (x0, x1) = V.frame_sizes(d)
+            bad = 0
+            for (w, h), band in ((tiled, (0, tiled[0])), (untiled, (0, untiled[0])), (tiled, (x0, x1))):
+                p = api.default_params(w, h, d)
+                img, st = ctx.render(p, *band)
+                ref, cnt = O.render(flat, c, p, *band)
+                bad += n_bad(img, ref) + counters_differ(st, cnt)
+            if d in V.LIST_DEPTHS:
+                w, h = V.list_frame_size(d)
+                p = api.default_params(w, h, d)
+                samples, cnt = O.render(flat, c, api.default_params(2 * w, 2 * h, d))
+                want = (samples[0::2, 0::2] + samples[0::2, 1::2] + samples[1::2, 0::2] + samples[1::2, 1::2]) / np.float32(4)
+                img, _, n, st = ctx.render_adaptive(p, 2, -1)
+                bad += n_bad(img, want) + counters_differ(st, cnt) + int(n != w * h)
+            f = fired()
+            bad_total += bad + len(f)
+            print(f"{name:9s} {str(cls):16s} d{d:<3d} cap {V.level_cap(d):3d}: mismatches {bad}, checks fired: {f or 'none'}",
+                  flush=True)
+        p = api.default_params(27, 17, 8)
+        got, _ = ctx.hit_buffers(p)
+        try:
+            assert_hits_equal(got, primary_hits(hits_lib, flat, c, p), name)
+            bad = 0
+        except AssertionError as e:
+            print(e)
+            bad = 1
+        f = fired()
+        bad_total += bad + len(f)
+        print(f"{name:9s} hit buffers 27x17: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
 print("CHECKED_OK" if bad_total == 0 else "CHECKED_FAIL")

@@ -99,6 +99,25 @@ public:
         const int xz[2] = {x, z};
         return rc_ = tcrt_pick(ctx_, &p, 1, xz, obj, dist, normal3);
     }
+    // what each ray sees (tcrt_trace_rays): rgb[3i..3i+2] is calculatePixel of rays[i] at level 0, with rs's depth and
+    // switches; the rays are traced with the origin and direction they hold (built by Camera::createEyeRay or Ray(o, d),
+    // which normalise), so rays[i] gives what the reference computes for it.  An invalid ray (tcrt.h) gets NaN.
+    int traceRays(const RenderSettings& rs, const std::vector<Ray>& rays, float* rgb, unsigned long long* n_invalid = NULL,
+                  tcrt_stats* stats = NULL) {
+        std::vector<float> o, d;
+        unpackRays(rays, o, d);
+        tcrt_params p = rs.params();
+        return rc_ = tcrt_trace_rays(ctx_, &p, rays.size(), o.data(), 0, d.data(), rgb, n_invalid, stats);
+    }
+    // the nearest hits of the rays (tcrt_intersect_rays): obj[i], dist[i], normal[3i..3i+2] as hitBuffers defines them
+    // (object -2 for an invalid ray); any pointer may be NULL, not all three
+    int intersectRays(const RenderSettings& rs, const std::vector<Ray>& rays, int* obj, float* dist, float* normal,
+                      unsigned long long* n_invalid = NULL, tcrt_stats* stats = NULL) {
+        std::vector<float> o, d;
+        unpackRays(rays, o, d);
+        tcrt_params p = rs.params();
+        return rc_ = tcrt_intersect_rays(ctx_, &p, rays.size(), o.data(), 0, d.data(), obj, dist, normal, n_invalid, stats);
+    }
     // init_log + printPixelsToLog (RayTracer.cpp:2022-2061,1574-1626)
     int printPixelsToLog(const char* path = LOG_FILE_NAME) {
         tcrt_params p = settings_.params();
@@ -108,6 +127,15 @@ public:
     tcrt_ctx* handle() { return ctx_; }
 
 private:
+    static void unpackRays(const std::vector<Ray>& rays, std::vector<float>& o, std::vector<float>& d) {
+        o.resize(rays.size() * 3);
+        d.resize(rays.size() * 3);
+        for (size_t i = 0; i < rays.size(); i++) {
+            const vector3d ro = rays[i].getOrigin(), rd = rays[i].getDirection();
+            o[3 * i] = ro.x; o[3 * i + 1] = ro.y; o[3 * i + 2] = ro.z;
+            d[3 * i] = rd.x; d[3 * i + 1] = rd.y; d[3 * i + 2] = rd.z;
+        }
+    }
     tcrt_ctx* ctx_;
     int rc_;
     double run_time_s_;

@@ -311,6 +311,51 @@ int tcrt_device_hit_buffers(tcrt_ctx* ctx, int device_slot, int** object, float*
                             size_t* n_pixels);
 int tcrt_pick(tcrt_ctx* ctx, const tcrt_params* params, int n, const int* xz, int* object, float* distance,
               float* normal);
+/* Ray batches: what caller-supplied rays see, and what they hit.  A batch is n rays; ray i has origin o_i =
+ * origins[3i..3i+2] (or origins[0..2] for every ray when shared_origin != 0) and direction d_i = directions[3i..3i+2],
+ * all float32.
+ *   - colour (tcrt_trace_rays): rgb[3i..3i+2] is what the reference's calculatePixel returns at level 0 for a Ray whose
+ *     stored origin and direction are exactly o_i and d_i, with the uploaded scene and params max_depth, shadows_on,
+ *     reflections_on, null_color and far_dist.  width, height and the camera are not read;
+ *   - nearest hit (tcrt_intersect_rays): object[i], distance[i], normal[3i..3i+2] with the definitions of
+ *     tcrt_hit_buffers applied to ray i (object index or -1; the reference's distance, negative inside a sphere, far_dist
+ *     on a miss; n2, or (+0, +0, +0) on a miss).  Only far_dist is read.  Any output pointer may be NULL, not all three.
+ * Directions are used as given, not normalised again: a Ray stores the direction its constructor has normalised, and
+ * vector3d::normalize is not idempotent to the bit.  A caller with raw directions (x, y, z) applies the reference's
+ * normalisation: len = sqrtf((x*x + y*y) + z*z), then x/len, y/len, z/len (binary32, no FMA, IEEE division and square root).
+ * A ray is traced only when it is valid: all six components finite, |o_k| <= 2^40, and s = (dx*dx + dy*dy) + dz*dz in
+ * binary32 without FMA satisfies |s - 1| <= 2^-21.  Every direction that normalisation makes of a vector whose squared
+ * length is a normal float passes (DESIGN.md 4.5).  An invalid ray is not traced and not counted as a ray: its colour
+ * is quiet NaN (0x7fc00000) in all three channels; its hit is object -2, distance NaN, normal NaN.  *n_invalid (may be
+ * NULL) returns their number; the call still succeeds.  The check runs on the device, in the kernel that traces the batch.
+ * A warp takes 32 consecutive rays: rays that are close in the batch should be close in space (e.g. 4 x 8 pixel tiles
+ * of a camera), or the walks of a warp diverge and the batch is slower (profiles/README.md 12).  The library does not sort.
+ * Host forms: inputs and outputs in pinned or pageable memory (identical results).  A multi-device ctx splits [0, n) into
+ * equal contiguous ranges, one per device.  The batch runs in pieces of at most 4 Mi rays round robin over the render
+ * streams: each piece's inputs are copied in (24 B per ray, 12 with a shared origin), traced by one launch, and its
+ * outputs copied out while later pieces trace.
+ * Device forms (_device): one device slot; every pointer must be device memory of that device (cudaPointerGetAttributes),
+ * else TCRT_ERR_INVALID; the caller has finished writing the inputs (e.g. synchronised its stream).
+ * All four calls are synchronous.  n = 0 launches nothing.  Errors: NULL ctx, params, inputs (n > 0) or outputs, or n
+ * whose byte count overflows: TCRT_ERR_INVALID; tcrt_trace_rays* with max_depth < 0: TCRT_ERR_INVALID, above
+ * TCRT_MAX_DEPTH: TCRT_ERR_UNSUPPORTED; before tcrt_upload_scene: TCRT_ERR_NO_SCENE.
+ * Stats: col_begin/col_end are each device's ray range [begin, end) (clipped to INT_MAX), rays_primary the valid rays,
+ * rays_shadow / rays_reflect as for frames (hits: 0), render_ms from the first input copy to the end of the last launch,
+ * d2h_ms the copy-back time not hidden behind the launches, gpu_launches the launches.
+ * Like hit buffers, these calls have buffers, queue heads and events of their own: they never change the last render,
+ * the multi-device cut or cost map, or a frame in flight, may run while two frames are in flight and do not count as one.
+ * tcrt_set_camera has no effect on them. */
+int tcrt_trace_rays(tcrt_ctx* ctx, const tcrt_params* params, size_t n, const float* origins, int shared_origin,
+                    const float* directions, float* rgb, unsigned long long* n_invalid, tcrt_stats* stats);
+int tcrt_intersect_rays(tcrt_ctx* ctx, const tcrt_params* params, size_t n, const float* origins, int shared_origin,
+                        const float* directions, int* object, float* distance, float* normal,
+                        unsigned long long* n_invalid, tcrt_stats* stats);
+int tcrt_trace_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* params, size_t n, const float* origins,
+                           int shared_origin, const float* directions, float* rgb, unsigned long long* n_invalid,
+                           tcrt_stats* stats);
+int tcrt_intersect_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* params, size_t n,
+                               const float* origins, int shared_origin, const float* directions, int* object,
+                               float* distance, float* normal, unsigned long long* n_invalid, tcrt_stats* stats);
 /* Cost-balanced column bands (replaces the equal z-bands of the reference's strategy 1,
  * RayTracer.cpp:904-906, whose load imbalance strategies 2-7 and PixelQueue were written to fix).
  * Renders a low-resolution copy of the frame on device slot 0 in which every finished pixel adds its

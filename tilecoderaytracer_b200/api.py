@@ -238,6 +238,28 @@ def plan_dead_paths(flat, params: TcrtParams) -> bool:
     return bool(prune.value)
 
 
+def normalize_like_reference(v) -> np.ndarray:
+    """vector3d::normalize in numpy float32, as a Ray's constructor applies it: len = sqrtf((x*x + y*y) + z*z), then three
+    IEEE divisions.  The ray-batch calls take directions as a Ray stores them; this turns raw directions (..., 3) into
+    those, bit for bit."""
+    a = np.asarray(v, dtype=np.float32)
+    x, y, z = a[..., 0], a[..., 1], a[..., 2]
+    with np.errstate(all="ignore"):
+        length = np.sqrt((x * x + y * y) + z * z)
+        return np.stack([x / length, y / length, z / length], axis=-1)
+
+
+def _ray_inputs(origins, directions):
+    """(n, origins, shared_origin, directions) as the ray-batch calls take them: float32, C-contiguous."""
+    d = np.asarray(directions)
+    assert d.dtype == np.float32 and d.ndim == 2 and d.shape[1] == 3 and d.flags["C_CONTIGUOUS"], "directions: (n, 3) float32"
+    o = np.asarray(origins)
+    assert o.dtype == np.float32 and o.flags["C_CONTIGUOUS"], "origins: float32, C-contiguous"
+    shared = o.shape == (3,)
+    assert shared or o.shape == d.shape, "origins: (n, 3), or (3,) for a shared origin"
+    return d.shape[0], o, int(shared), d
+
+
 class HostBuffer:
     """Pinned host memory (tcrt_alloc_host) viewed as a numpy array."""
 
@@ -501,6 +523,65 @@ class Context:
         self._ck(self._lib.tcrt_pick(self._h, C.byref(params), n, xz.ctypes.data_as(C.c_void_p), obj.ctypes.data_as(C.c_void_p),
                                      dist.ctypes.data_as(C.c_void_p), normal.ctypes.data_as(C.c_void_p)))
         return obj, dist, normal
+
+    def trace_rays(self, params: TcrtParams, origins, directions, out: Optional[np.ndarray] = None):
+        """What caller-supplied rays see (tcrt_trace_rays): origins (n, 3) float32, or (3,) for one origin shared by every
+        ray; directions (n, 3) float32, used as a Ray stores them (normalize_like_reference).  Returns (rgb (n, 3) float32,
+        n_invalid, RenderStats); an invalid ray's colour is NaN.  `out` (n, 3) float32 may be pinned or pageable."""
+        n, o, shared, d = _ray_inputs(origins, directions)
+        if out is None:
+            out = np.empty((n, 3), np.float32)
+        assert out.dtype == np.float32 and out.size == 3 * n and out.flags["C_CONTIGUOUS"], "out: (n, 3) float32"
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_trace_rays(self._h, C.byref(params), n, o.ctypes.data_as(C.c_void_p), shared,
+                                           d.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p), C.byref(bad),
+                                           C.byref(st)))
+        return out.reshape(n, 3), int(bad.value), RenderStats.from_c(st)
+
+    def intersect_rays(self, params: TcrtParams, origins, directions, out: Optional[dict] = None):
+        """The nearest hits of caller-supplied rays (tcrt_intersect_rays), inputs as in trace_rays: {"object" (n,) int32,
+        "distance" (n,) float32, "normal" (n, 3) float32} with the definitions of hit_buffers(); an invalid ray has object
+        -2, distance and normal NaN.  `out` maps some of these names to C-contiguous destinations (pinned or pageable);
+        only those are computed and returned.  Returns (dict, n_invalid, RenderStats)."""
+        n, o, shared, d = _ray_inputs(origins, directions)
+        if out is None:
+            out = {name: np.empty((n,) + tail, dtype) for name, dtype, tail in self.HIT_BUFFERS}
+        ptrs = []
+        for name, dtype, tail in self.HIT_BUFFERS:
+            a = out.get(name)
+            if a is not None:
+                assert a.dtype == dtype and a.size == n * int(np.prod(tail)) and a.flags["C_CONTIGUOUS"], name
+            ptrs.append(a.ctypes.data_as(C.c_void_p) if a is not None else None)
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_intersect_rays(self._h, C.byref(params), n, o.ctypes.data_as(C.c_void_p), shared,
+                                               d.ctypes.data_as(C.c_void_p), *ptrs, C.byref(bad), C.byref(st)))
+        res = {name: out[name].reshape((n,) + tail) for name, _, tail in self.HIT_BUFFERS if out.get(name) is not None}
+        return res, int(bad.value), RenderStats.from_c(st)
+
+    def trace_rays_device(self, params: TcrtParams, n: int, origins: int, directions: int, rgb: int,
+                          shared_origin: bool = False, slot: int = 0):
+        """trace_rays on device `slot` with device addresses (e.g. torch CUDA tensors' data_ptr()): origins 3n floats (3
+        when shared_origin), directions 3n floats, rgb 3n floats.  The inputs must be complete (synchronise the stream
+        that wrote them).  Returns (n_invalid, RenderStats)."""
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_trace_rays_device(self._h, slot, C.byref(params), n, C.c_void_p(origins), int(bool(shared_origin)),
+                                                  C.c_void_p(directions), C.c_void_p(rgb), C.byref(bad), C.byref(st)))
+        return int(bad.value), RenderStats.from_c(st)
+
+    def intersect_rays_device(self, params: TcrtParams, n: int, origins: int, directions: int, object: int = 0,
+                              distance: int = 0, normal: int = 0, shared_origin: bool = False, slot: int = 0):
+        """intersect_rays on device `slot` with device addresses as in trace_rays_device; 0 leaves an output out.
+        Returns (n_invalid, RenderStats)."""
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_intersect_rays_device(self._h, slot, C.byref(params), n, C.c_void_p(origins),
+                                                      int(bool(shared_origin)), C.c_void_p(directions),
+                                                      C.c_void_p(object or None), C.c_void_p(distance or None),
+                                                      C.c_void_p(normal or None), C.byref(bad), C.byref(st)))
+        return int(bad.value), RenderStats.from_c(st)
 
     def balance_columns(self, params: TcrtParams, n_bands: int) -> list[tuple[int, int]]:
         """Cost-balanced column bands of the frame (low-resolution pre-pass on device slot 0):

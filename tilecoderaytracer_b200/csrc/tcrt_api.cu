@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <limits.h>
 
 #include <math.h>
 
@@ -122,6 +123,21 @@ struct DeviceState {
     size_t ad_counts_cap = 0;
     int* ad_list = nullptr;
     size_t ad_list_cap = 0;
+    // ray batches (tcrt_trace_rays, tcrt_intersect_rays): per render stream the device scratch of one piece (its inputs,
+    // then its outputs) and the pinned staging of pageable inputs, allocated at first use; queue heads, counters and
+    // events of their own, so that a batch touches neither the last render nor a frame in flight.  The calls are
+    // synchronous: nothing else uses these while one runs.
+    float* ray_mem[kChunkStreams] = {};
+    size_t ray_mem_cap[kChunkStreams] = {};        // floats
+    float* ray_stage[kChunkStreams] = {};
+    size_t ray_stage_cap[kChunkStreams] = {};      // floats
+    unsigned char* ray_ctl = nullptr;              // 64 B per render stream: queue head @0, ray counters @8..31, invalid @32
+    unsigned long long* h_ray = nullptr;           // pinned copy of ray_ctl
+    cudaEvent_t ev_r0 = nullptr, ev_r1 = nullptr;  // first input copy / last launch done (render stream)
+    cudaEvent_t ev_rc = nullptr;                   // the last output copy is in host memory (copy stream)
+    cudaEvent_t ev_rk[kChunkStreams] = {};         // stream si's last piece has been traced
+    cudaEvent_t ev_rin[kChunkStreams] = {};        // stream si's input staging has been copied to the device
+    cudaEvent_t ev_rout[kChunkStreams] = {};       // stream si's output scratch has been copied out
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -258,6 +274,16 @@ void free_device(DeviceState& d) {
     cudaFree(d.ad_counts);
     cudaFree(d.ad_list);
     for (cudaEvent_t e : {d.ev_h0, d.ev_h1, d.ev_hc})
+        if (e) cudaEventDestroy(e);
+    for (int si = 0; si < kChunkStreams; si++) {
+        cudaFree(d.ray_mem[si]);
+        cudaFreeHost(d.ray_stage[si]);
+        for (cudaEvent_t e : {d.ev_rk[si], d.ev_rin[si], d.ev_rout[si]})
+            if (e) cudaEventDestroy(e);
+    }
+    cudaFree(d.ray_ctl);
+    cudaFreeHost(d.h_ray);
+    for (cudaEvent_t e : {d.ev_r0, d.ev_r1, d.ev_rc})
         if (e) cudaEventDestroy(e);
     cudaFreeHost(d.h_txt);
     cudaFreeHost(d.txt_stage);
@@ -2391,6 +2417,293 @@ int tcrt_pick(tcrt_ctx* ctx, const tcrt_params* p, int n, const int* xz, int* ob
     CK(ctx, cudaEventRecord(d.ev_h1, d.stream));
     CK(ctx, cudaEventSynchronize(d.ev_h1));
     return TCRT_OK;
+}
+
+}  // extern "C"
+
+// ---- ray batches (tcrt_trace_rays, tcrt_intersect_rays): the render and hit kernels' ray mode ---------------------------
+// Rays per piece: 4 Mi keeps every kernel index far inside int; a piece's scratch is 4 Mi * 11 words = 176 MB at most.
+constexpr size_t kRayPiece = (size_t)1 << 22;
+
+// The ray-batch events and control block of device d, created at first use.
+static int ensure_ray_state(tcrt_ctx* ctx, DeviceState& d) {
+    if (d.ray_ctl) return TCRT_OK;
+    for (int si = 0; si < kChunkStreams; si++) {
+        CK(ctx, cudaEventCreateWithFlags(&d.ev_rk[si], cudaEventDisableTiming));
+        CK(ctx, cudaEventCreateWithFlags(&d.ev_rin[si], cudaEventDisableTiming));
+        CK(ctx, cudaEventCreateWithFlags(&d.ev_rout[si], cudaEventDisableTiming));
+    }
+    CK(ctx, cudaEventCreate(&d.ev_r0));
+    CK(ctx, cudaEventCreate(&d.ev_r1));
+    CK(ctx, cudaEventCreate(&d.ev_rc));
+    CK(ctx, cudaHostAlloc((void**)&d.h_ray, 64 * kChunkStreams, cudaHostAllocPortable));
+    CK(ctx, cudaMalloc((void**)&d.ray_ctl, 64 * kChunkStreams));
+    return TCRT_OK;
+}
+
+// Pinned host memory of at least `need` floats in p (its contents are not kept).
+static int ensure_pinned(tcrt_ctx* ctx, float*& p, size_t& cap, size_t need) {
+    if (need <= cap && p) return TCRT_OK;
+    if (p) CK(ctx, cudaFreeHost(p));
+    p = nullptr;
+    cap = 0;
+    CK(ctx, cudaHostAlloc((void**)&p, need * sizeof(float), cudaHostAllocPortable));
+    cap = need;
+    return TCRT_OK;
+}
+
+// Is p device memory of device dev?
+static bool on_device(const void* p, int dev) {
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    return at.type == cudaMemoryTypeDevice && at.device == dev;
+}
+
+// One batch: [0, n) split into equal contiguous ranges, one per device (device forms: slot only), each traced in pieces of
+// at most kRayPiece rays round robin over the render streams.  A piece of a host form is: its inputs to the stream's scratch
+// (pinned ones straight, pageable ones through the stream's pinned staging), one launch, its outputs to the host on the copy
+// stream (pinned ones straight, pageable ones through stage_out).  A piece's outputs are sent once the next piece has been
+// queued, so a piece's copies overlap other pieces' launches; a stream's next piece waits for them before it reuses the
+// scratch.  Device forms launch on the caller's buffers directly.  out[0] rgb (colour) or object, out[1] distance,
+// out[2] normal (hits).
+static int rays_impl(tcrt_ctx* ctx, int slot, const tcrt_params* p, size_t n, const float* origins, int shared_origin,
+                     const float* dirs, bool hits, void* const out_in[3], unsigned long long* n_invalid, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
+    if (!p) return fail(ctx, TCRT_ERR_INVALID, "null params");
+    const bool device_form = slot >= 0;
+    if (device_form && slot >= (int)ctx->devs.size()) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", slot);
+    if (!hits && p->max_depth < 0) return fail(ctx, TCRT_ERR_INVALID, "max_depth %d < 0", p->max_depth);
+    char* out[3] = {static_cast<char*>(out_in[0]), static_cast<char*>(out_in[1]), static_cast<char*>(out_in[2])};
+    if (hits ? (!out[0] && !out[1] && !out[2]) : !out[0]) return fail(ctx, TCRT_ERR_INVALID, "no output");
+    if (n > 0 && (!origins || !dirs)) return fail(ctx, TCRT_ERR_INVALID, "null ray input");
+    if (n > SIZE_MAX / (6 * sizeof(float))) return fail(ctx, TCRT_ERR_INVALID, "%zu rays: byte count overflows", n);
+    if (!hits && p->max_depth > TCRT_MAX_DEPTH)
+        return fail(ctx, TCRT_ERR_UNSUPPORTED, "max_depth %d > TCRT_MAX_DEPTH %d", p->max_depth, TCRT_MAX_DEPTH);
+    if (device_form && n > 0) {
+        const int dev = ctx->devs[slot].dev;
+        const void* ptrs[5] = {origins, dirs, out[0], out[1], out[2]};
+        for (const void* q : ptrs)
+            if (q && !on_device(q, dev))
+                return fail(ctx, TCRT_ERR_INVALID, "pointer %p is not device memory of device %d (slot %d)", q, dev, slot);
+    }
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    const int nd = (int)ctx->devs.size();
+    const int d_begin = device_form ? slot : 0, d_end = device_form ? slot + 1 : nd;
+    std::vector<size_t> cut(nd + 1, 0);
+    for (int i = 0; i <= nd; i++)
+        cut[i] = device_form ? (i <= slot ? 0 : n) : n / nd * i + n % nd * i / nd;
+    // bytes per ray of each output
+    const int n_out = hits ? 3 : 1;
+    const size_t out_bytes[3] = {hits ? (size_t)4 : (size_t)12, 4, 12};
+    bool staged[3] = {false, false, false}, any_direct = false;
+    bool in_pageable[2] = {false, false};
+    if (!device_form && n > 0) {
+        for (int k = 0; k < n_out; k++) {
+            staged[k] = out[k] && host_pageable(out[k]);
+            any_direct = any_direct || (out[k] && !staged[k]);
+        }
+        in_pageable[0] = host_pageable(dirs);
+        in_pageable[1] = host_pageable(origins);
+    }
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (n_invalid) *n_invalid = 0;
+    auto stream_of = [](DeviceState& d, int si) { return si == 0 ? d.stream : d.chunk_stream[si - 1]; };
+    std::vector<int> used_streams(nd, 0), launches(nd, 0);
+    for (int i = d_begin; i < d_end; i++) {
+        DeviceState& d = ctx->devs[i];
+        const size_t r0 = cut[i], r1 = cut[i + 1];
+        if (r1 <= r0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        int rc = ensure_ray_state(ctx, d);
+        if (rc) return rc;
+        const size_t n_pieces = (r1 - r0 + kRayPiece - 1) / kRayPiece;
+        const int ns = ctx->one_stream ? 1 : (int)std::min<size_t>(kChunkStreams, n_pieces);
+        used_streams[i] = ns;
+        const size_t per = std::min(kRayPiece, r1 - r0);
+        // scratch: directions, origins, then the outputs (hits: object, distance, normal)
+        const size_t in_words = 3 * per + (shared_origin ? 3 : 3 * per);
+        const size_t all_out = hits ? 5 * per : 3 * per;
+        if (!device_form) {
+            for (int si = 0; si < ns; si++)
+                if ((rc = ensure(ctx, d.ray_mem[si], d.ray_mem_cap[si], in_words + all_out))) return rc;
+            if (in_pageable[0] || in_pageable[1])
+                for (int si = 0; si < ns; si++)
+                    if ((rc = ensure_pinned(ctx, d.ray_stage[si], d.ray_stage_cap[si], in_words))) return rc;
+        }
+        // on the render stream, behind whatever is queued there (a scene upload, frames in flight); the other render
+        // streams start behind it
+        CK(ctx, cudaMemsetAsync(d.ray_ctl, 0, 64 * ns, d.stream));
+        CK(ctx, cudaEventRecord(d.ev_r0, d.stream));
+        for (int si = 1; si < ns; si++) CK(ctx, cudaStreamWaitEvent(stream_of(d, si), d.ev_r0, 0));
+        // piece k: rays [r0 + k*per, ...) on stream k % ns
+        auto piece = [&](size_t k, size_t& a, size_t& cnt, int& si) {
+            a = r0 + k * per;
+            cnt = std::min(per, r1 - a);
+            si = (int)(k % (size_t)ns);
+        };
+        auto out_dev = [&](int si, size_t cnt, int k) -> float* {   // output k of a piece in the stream's scratch
+            float* base = d.ray_mem[si] + 3 * cnt + (shared_origin ? 3 : 3 * cnt);
+            return base + (k == 0 ? 0 : k == 1 ? cnt : 2 * cnt);
+        };
+        auto send_out = [&](size_t k) -> int {
+            size_t a, cnt;
+            int si;
+            piece(k, a, cnt, si);
+            if (any_direct) {
+                CK(ctx, cudaStreamWaitEvent(d.copy_stream, d.ev_rk[si], 0));
+                for (int b = 0; b < n_out; b++)
+                    if (out[b] && !staged[b])
+                        CK(ctx, cudaMemcpyAsync(out[b] + a * out_bytes[b], out_dev(si, cnt, b), cnt * out_bytes[b],
+                                                cudaMemcpyDeviceToHost, d.copy_stream));
+            }
+            for (int b = 0; b < n_out; b++) {
+                if (!staged[b]) continue;
+                CK(ctx, ensure_stage(d));
+                TxtPipe& pipe = copy_pipe_to(ctx, out[b]);
+                StageSlots slots;
+                const cudaError_t e = stage_out(pipe, d, slots, reinterpret_cast<const char*>(out_dev(si, cnt, b)),
+                                                cnt * out_bytes[b], a * out_bytes[b], d.ev_rk[si]);
+                slots.drain(pipe);
+                if (e != cudaSuccess || pipe.io_error)
+                    return fail(ctx, TCRT_ERR_CUDA, "staged copy-out of a ray batch: %s",
+                                e != cudaSuccess ? cudaGetErrorString(e) : "a chunk did not arrive");
+            }
+            CK(ctx, cudaEventRecord(d.ev_rout[si], d.copy_stream));
+            return TCRT_OK;
+        };
+        const size_t lag = (!device_form && ns > 1) ? 1 : 0;
+        for (size_t k = 0; k < n_pieces + lag; k++) {
+            if (k < n_pieces) {
+                size_t a, cnt;
+                int si;
+                piece(k, a, cnt, si);
+                const cudaStream_t ks = stream_of(d, si);
+                const float* o_src = origins + (shared_origin ? 0 : 3 * a);
+                const float* d_src = dirs + 3 * a;
+                void* dst[3] = {out[0], out[1], out[2]};
+                if (!device_form) {
+                    float* dd = d.ray_mem[si];
+                    float* od = dd + 3 * cnt;
+                    const size_t nd_f = 3 * cnt, no_f = shared_origin ? 3 : 3 * cnt;
+                    CK(ctx, cudaStreamWaitEvent(ks, d.ev_rout[si], 0));   // the scratch's last outputs have left
+                    if (in_pageable[0] || in_pageable[1]) {
+                        CK(ctx, cudaEventSynchronize(d.ev_rin[si]));        // so has the staging's last input
+                        float* st = d.ray_stage[si];
+                        if (in_pageable[0]) memcpy(st, d_src, nd_f * sizeof(float));
+                        if (in_pageable[1]) memcpy(st + nd_f, o_src, no_f * sizeof(float));
+                    }
+                    CK(ctx, cudaMemcpyAsync(dd, in_pageable[0] ? d.ray_stage[si] : d_src, nd_f * sizeof(float),
+                                            cudaMemcpyHostToDevice, ks));
+                    CK(ctx, cudaMemcpyAsync(od, in_pageable[1] ? d.ray_stage[si] + nd_f : o_src, no_f * sizeof(float),
+                                            cudaMemcpyHostToDevice, ks));
+                    CK(ctx, cudaEventRecord(d.ev_rin[si], ks));
+                    o_src = od;
+                    d_src = dd;
+                    // every output goes to the scratch; only the requested ones leave it
+                    for (int b = 0; b < n_out; b++) dst[b] = out_dev(si, cnt, b);
+                } else {
+                    for (int b = 0; b < n_out; b++)
+                        if (out[b]) dst[b] = out[b] + a * out_bytes[b];
+                }
+                unsigned char* ctl = d.ray_ctl + 64 * si;
+                CK(ctx, cudaMemsetAsync(ctl, 0, sizeof(unsigned int), ks));
+                RenderLaunch rl = band_launch(ctx, d, p, 0, 0, static_cast<float*>(dst[0]), reinterpret_cast<unsigned int*>(ctl));
+                rl.counters = reinterpret_cast<unsigned long long*>(ctl + 8);
+                rl.ray_invalid = reinterpret_cast<unsigned long long*>(ctl + 32);
+                rl.ray_o = o_src;
+                rl.ray_o_stride = shared_origin ? 0 : 3;
+                rl.ray_d = d_src;
+                rl.list_n = (int)cnt;
+                if (hits) {
+                    HitLaunch hl{};
+                    hl.rl = rl;
+                    hl.object = static_cast<int*>(dst[0]);
+                    hl.distance = static_cast<float*>(dst[1]);
+                    hl.normal = static_cast<float*>(dst[2]);
+                    CK(ctx, tcrt_launch_hits(hl, d.sm_count, ks));
+                } else {
+                    CK(ctx, tcrt_launch_render_rays(rl, d.sm_count, ks));
+                }
+                launches[i]++;
+                CK(ctx, cudaEventRecord(d.ev_rk[si], ks));
+            }
+            if (!device_form && k >= lag && (rc = send_out(k - lag))) return rc;
+        }
+        for (int si = 1; si < ns; si++) CK(ctx, cudaStreamWaitEvent(d.stream, d.ev_rk[si], 0));
+        CK(ctx, cudaEventRecord(d.ev_r1, d.stream));
+        CK(ctx, cudaMemcpyAsync(d.h_ray, d.ray_ctl, 64 * ns, cudaMemcpyDeviceToHost, d.stream));
+        if (!device_form) CK(ctx, cudaEventRecord(d.ev_rc, d.copy_stream));
+    }
+    unsigned long long bad = 0, n_launches = 0;
+    for (int i = d_begin; i < d_end; i++) {
+        DeviceState& d = ctx->devs[i];
+        if (stats) {
+            stats->col_begin[i] = (int)std::min<size_t>(cut[i], INT_MAX);
+            stats->col_end[i] = (int)std::min<size_t>(cut[i + 1], INT_MAX);
+        }
+        if (used_streams[i] == 0) continue;
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));
+        if (!device_form) CK(ctx, cudaEventSynchronize(d.ev_rc));
+        unsigned long long cnt[4] = {0, 0, 0, 0};   // primary, shadow, reflect, invalid
+        for (int si = 0; si < used_streams[i]; si++)
+            for (int c = 0; c < 4; c++) cnt[c] += d.h_ray[8 * si + 1 + c];
+        if (hits) cnt[0] = (cut[i + 1] - cut[i]) - cnt[3];
+        bad += cnt[3];
+        n_launches += (unsigned long long)launches[i];
+        if (stats) {
+            float ms = 0.f;
+            CK(ctx, cudaEventElapsedTime(&ms, d.ev_r0, d.ev_r1));
+            stats->render_ms[i] = ms;
+            if (!device_form) {
+                CK(ctx, cudaEventElapsedTime(&ms, d.ev_r1, d.ev_rc));
+                stats->d2h_ms[i] = std::max(ms, 0.f);   // copy time not hidden behind the kernels
+            }
+            stats->rays_primary[i] = cnt[0];
+            stats->rays_shadow[i] = cnt[1];
+            stats->rays_reflect[i] = cnt[2];
+        }
+    }
+    if (stats) {
+        stats->n_devices = nd;
+        stats->gpu_launches = n_launches;
+    }
+    if (n_invalid) *n_invalid = bad;
+    return TCRT_OK;
+}
+
+extern "C" {
+
+int tcrt_trace_rays(tcrt_ctx* ctx, const tcrt_params* p, size_t n, const float* origins, int shared_origin,
+                    const float* directions, float* rgb, unsigned long long* n_invalid, tcrt_stats* stats) {
+    void* out[3] = {rgb, nullptr, nullptr};
+    return rays_impl(ctx, -1, p, n, origins, shared_origin, directions, false, out, n_invalid, stats);
+}
+
+int tcrt_intersect_rays(tcrt_ctx* ctx, const tcrt_params* p, size_t n, const float* origins, int shared_origin,
+                        const float* directions, int* object, float* distance, float* normal,
+                        unsigned long long* n_invalid, tcrt_stats* stats) {
+    void* out[3] = {object, distance, normal};
+    return rays_impl(ctx, -1, p, n, origins, shared_origin, directions, true, out, n_invalid, stats);
+}
+
+int tcrt_trace_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* p, size_t n, const float* origins,
+                           int shared_origin, const float* directions, float* rgb, unsigned long long* n_invalid,
+                           tcrt_stats* stats) {
+    if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
+    void* out[3] = {rgb, nullptr, nullptr};
+    return rays_impl(ctx, device_slot, p, n, origins, shared_origin, directions, false, out, n_invalid, stats);
+}
+
+int tcrt_intersect_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* p, size_t n, const float* origins,
+                               int shared_origin, const float* directions, int* object, float* distance, float* normal,
+                               unsigned long long* n_invalid, tcrt_stats* stats) {
+    if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
+    void* out[3] = {object, distance, normal};
+    return rays_impl(ctx, device_slot, p, n, origins, shared_origin, directions, true, out, n_invalid, stats);
 }
 
 }  // extern "C"

@@ -122,13 +122,27 @@ struct RenderLaunch {
     // queue position q traces sample 1 + q % (ss*ss-1) of frame pixel list[q / (ss*ss-1)] (x*H + z of the W x H frame)
     // into out[3q..3q+2] (list_to_sample, tcrt_render_common.cuh).  Band mode ignores these.
     const int* list;
-    int list_n;              // queue positions: list entries * (ss*ss - 1)
+    int list_n;              // queue positions: list entries * (ss*ss - 1); in ray mode the rays of the launch
     int list_ss;
+    // ray mode (tcrt_launch_render_rays, ray batches): queue position q traces the caller's ray q — origin
+    // ray_o[ray_o_stride*q ..], direction ray_d[3q ..] — into out[3q..3q+2], x0 == 0 and the camera unused.  A ray that
+    // fails the validity rule of tcrt.h (ray_from_batch, tcrt_render_common.cuh) is not traced: out gets quiet NaNs and
+    // *ray_invalid counts it.  The other modes ignore these.
+    const float* ray_o;
+    int ray_o_stride;        // 3, or 0: one origin shared by every ray
+    const float* ray_d;
+    unsigned long long* ray_invalid;
 };
+
+// What a render launch traces: the pixels of a band, the samples of a pixel list, or a batch of caller-supplied rays.
+// A compile-time parameter of the render kernel bodies (one kernel per mode keeps each bounce loop in the instruction cache).
+enum RenderMode { kModeBand = 0, kModeList = 1, kModeRays = 2 };
 
 // Primary-hit launch (tcrt_hits.cu): rl describes the frame, the band [x0, x1) and the scene; out of rl the kernel uses the
 // camera, width, height, x0, x1, far_dist, queue and n_objects.  Band mode (xz == nullptr): every pixel of the band, x-major
 // like frames.  List mode: entry i is pixel (xz[2i], xz[2i+1]) of the frame (rl.x0 == 0), and output i is its hit.
+// Ray mode (rl.ray_d != nullptr): output i is the hit of ray i of the batch, rl.list_n rays, with rl's ray fields as in
+// render ray mode; an invalid ray gets object -2, distance and normal NaN.  Each output pointer may be nullptr there.
 struct HitLaunch {
     RenderLaunch rl;
     const int* xz;
@@ -165,9 +179,12 @@ cudaError_t tcrt_launch_render_wave(const RenderLaunch& rl, int fm, int sm_count
 size_t tcrt_render_max_smem();
 // kernel for scenes whose spheres sit in a uniform grid (tcrt_render_grid.cu); smem = bytes of the staged blob
 cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream,
-                                    bool list = false);
+                                    RenderMode mode = kModeBand);
 // list-mode render launch (adaptive frames, RenderLaunch::list): the render or grid kernel's list-mode twin, one launch
 cudaError_t tcrt_launch_render_list(const RenderLaunch& rl, int sm_count, cudaStream_t stream);
+// ray-mode render launch (ray batches, RenderLaunch::ray_*): the render or grid kernel's ray-mode twin, one launch of
+// rl.list_n rays; nothing when there are none
+cudaError_t tcrt_launch_render_rays(const RenderLaunch& rl, int sm_count, cudaStream_t stream);
 // experimental task-pool kernel for sphere-BVH scenes (tcrt_render_pool.cu, developer builds only); smem_scene = bytes of the staged blob
 cudaError_t tcrt_launch_render_pool(const RenderLaunch& rl, int fm, int sm_count, size_t smem_scene, cudaStream_t stream);
 // n random (a.xyz, b) cases: div3 (shared-reciprocal division of the render kernel) vs __fdiv_rn; *bad += mismatches

@@ -8,7 +8,7 @@
 // A kernel of its own rather than an output of the render kernels: their bounce loop has to fit the instruction cache
 // (DESIGN.md §4.4), and a primary hit needs none of it — no light loop, no level stack, no refill.  One sweep per pixel.
 // Scenes with a sphere grid walk the sphere BVH, which is always built alongside the grid and finds the same nearest hit
-// (DESIGN.md §4.5).
+// (DESIGN.md §4.5); its per-ray fattening covers rays from any origin, so ray batches (tcrt_intersect_rays) walk it too.
 #include "tcrt_render_common.cuh"
 
 namespace {
@@ -34,18 +34,32 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
     sm.idx = reinterpret_cast<const int*>(base + sc.idx_off);
 
     const unsigned lane = threadIdx.x & 31u;
-    const unsigned total = hl.xz != nullptr ? (unsigned)hl.n_list : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const bool rays = rl.ray_d != nullptr;
+    const unsigned total = rays ? (unsigned)rl.list_n
+                                : hl.xz != nullptr ? (unsigned)hl.n_list : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    unsigned n_invalid = 0;
     for (;;) {
         // one claim = 32 queue positions: one 4x8 tile of the band (BVH walks of a warp stay coherent), or 32 list entries
+        // or rays
         unsigned q0 = 0;
         if (lane == 0) q0 = atomicAdd(rl.queue, 32u);
         q0 = __shfl_sync(kFull, q0, 0);
         if (q0 >= total) break;
         const unsigned q = q0 + lane;
-        const bool active = q < total;
+        bool active = q < total;
         int xc = 0, z = 0;
         V3 O = mk(0.f, 0.f, 0.f), D = mk(1.f, 0.f, 0.f);
-        if (active) {
+        if (active && rays) {
+            // the caller's ray; an invalid one gets the markers and takes no part in the sweep
+            if (!ray_from_batch(rl, (int)q, O, D)) {
+                const float nan = __uint_as_float(0x7fc00000u);
+                if (hl.object) hl.object[q] = -2;
+                if (hl.distance) hl.distance[q] = nan;
+                if (hl.normal) hl.normal[3 * (size_t)q] = hl.normal[3 * (size_t)q + 1] = hl.normal[3 * (size_t)q + 2] = nan;
+                active = false;
+                ++n_invalid;
+            }
+        } else if (active) {
             if (hl.xz != nullptr) {      // list mode: rl.x0 == 0, the pairs were range-checked by the host
                 xc = __ldg(hl.xz + 2 * (size_t)q);
                 z = __ldg(hl.xz + 2 * (size_t)q + 1);
@@ -86,14 +100,20 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
                     n2 = xyz(__ldg(sc.obj_normals + 6 * obj + (den < 0.0f ? 0 : 3) + 1));
                 }
             }
-            const size_t pix = hl.xz != nullptr ? (size_t)q : (size_t)xc * rl.height + z;
+            const size_t pix = (rays || hl.xz != nullptr) ? (size_t)q : (size_t)xc * rl.height + z;
             TCRT_CHECK(pix < total, kChkPixel);
-            hl.object[pix] = obj;
-            hl.distance[pix] = dist;
-            hl.normal[3 * pix + 0] = n2.x;
-            hl.normal[3 * pix + 1] = n2.y;
-            hl.normal[3 * pix + 2] = n2.z;
+            if (hl.object) hl.object[pix] = obj;   // only ray batches may leave an output out
+            if (hl.distance) hl.distance[pix] = dist;
+            if (hl.normal) {
+                hl.normal[3 * pix + 0] = n2.x;
+                hl.normal[3 * pix + 1] = n2.y;
+                hl.normal[3 * pix + 2] = n2.z;
+            }
         }
+    }
+    if (rays) {
+        const unsigned n = __reduce_add_sync(kFull, n_invalid);
+        if (lane == 0 && n != 0) atomicAdd(rl.ray_invalid, (unsigned long long)n);
     }
 }
 
@@ -125,14 +145,15 @@ cudaError_t tcrt_launch_hits(const HitLaunch& hl_in, int sm_count, cudaStream_t 
     RenderLaunch& rl = hl.rl;
     const size_t smem = (size_t)std::max(1, rl.scene.blob_f4 - rl.scene.stage_off) * sizeof(float4);
     if (smem > tcrt_render_max_smem()) return cudaErrorInvalidValue;
-    const unsigned total = hl.xz != nullptr ? (unsigned)hl.n_list : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = rl.ray_d != nullptr ? (unsigned)rl.list_n
+                           : hl.xz != nullptr ? (unsigned)hl.n_list : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     if (total == 0) return cudaSuccess;
     // persistent grid, sized as tcrt_launch_render sizes the render kernel's, but no more CTAs than there are claims
     int ctas_per_sm = (rl.scene.bvh_sph != nullptr && rl.scene.n_fin == 0) ? kMinBlocksBvh : kMinBlocks;
     while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;
     const long long need = ((long long)total + kBlock - 1) / kBlock;
     const int grid = (int)std::min<long long>((long long)sm_count * ctas_per_sm, need);
-    rl.tiled = (hl.xz == nullptr && (rl.x1 - rl.x0) % TCRT_TILE_W == 0 && rl.height % TCRT_TILE_H == 0) ? 1 : 0;
+    rl.tiled = (hl.xz == nullptr && rl.ray_d == nullptr && (rl.x1 - rl.x0) % TCRT_TILE_W == 0 && rl.height % TCRT_TILE_H == 0) ? 1 : 0;
     rl.row_order = nullptr;
     const int sb = rl.scene.bvh_sph == nullptr ? 0 : 1;
     const int fm = rl.scene.bvh_fin != nullptr ? 2 : (rl.scene.n_fin == 0 ? 0 : (rl.scene.n_clu > 0 ? 1 : 3));

@@ -37,9 +37,10 @@
 
 namespace {
 
-// The kernel body.  LIST = false: the pixels of the band [rl.x0, rl.x1) (render_kernel).  LIST = true: the samples of a
-// pixel list (render_list_kernel, adaptive frames; RenderLaunch::list): only the refill block and the output slot differ.
-template <int CAP, int SBVH, int FM, bool LIST>
+// The kernel body.  MODE kModeBand: the pixels of the band [rl.x0, rl.x1) (render_kernel).  kModeList: the samples of a
+// pixel list (render_list_kernel, adaptive frames; RenderLaunch::list).  kModeRays: the caller's rays (render_rays_kernel,
+// ray batches; RenderLaunch::ray_*).  Only the refill block, the output slot and the invalid-ray count differ.
+template <int CAP, int SBVH, int FM, int MODE>
 __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
     extern __shared__ float4 smem4[];
     const DeviceScene& sc = rl.scene;
@@ -61,7 +62,7 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
 
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned total = LIST ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = MODE != kModeBand ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     const V3 null_color = mk(rl.null_r, rl.null_g, rl.null_b);
 
     float stack[CAP * 7];   // per level: local rgb, k, object rgb (local memory, touched only on reflective hits)
@@ -75,6 +76,7 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
     ln.D = mk(1.f, 0.f, 0.f);
     // ray counters: per WARP (ballot + popc keeps them in uniform registers, not in every lane's)
     unsigned n_primary = 0, n_shadow = 0, n_reflect = 0;
+    unsigned n_invalid = 0;        // ray mode: rays refused by the validity rule
     unsigned wcur = 0, wend = 0;   // the warp's claimed chunk of pixel ids
     bool exhausted = false;
 
@@ -99,15 +101,34 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
             }
             unsigned avail = wend - wcur;
             unsigned rank = __popc(idle & lt_mask);
+            bool refused = false;
             if (ln.pix < 0 && rank < avail) {
-                int xc, z;
                 TCRT_CHECK(wcur + rank < total, kChkQueue);
-                if (LIST) list_to_sample(rl, (int)(wcur + rank), xc, z);
-                else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
-                TCRT_CHECK(xc >= 0 && xc < rl.x1 - rl.x0 && z >= 0 && z < rl.height, kChkQueue);
-                ln.pix = LIST ? (int)(wcur + rank) : xc * rl.height + z;
-                ln.level = 0;
-                primary_ray(rl, xc, z, ln.O, ln.D);
+                if (MODE == kModeRays) {
+                    // the caller's ray; an invalid one gets the NaN marker and leaves the lane idle for the next ray
+                    const int q = (int)(wcur + rank);
+                    if (ray_from_batch(rl, q, ln.O, ln.D)) {
+                        ln.pix = q;
+                        ln.level = 0;
+                    } else {
+                        float* o = rl.out + 3 * (size_t)q;
+                        o[0] = o[1] = o[2] = __uint_as_float(0x7fc00000u);
+                        refused = true;
+                    }
+                } else {
+                    int xc, z;
+                    if (MODE == kModeList) list_to_sample(rl, (int)(wcur + rank), xc, z);
+                    else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
+                    TCRT_CHECK(xc >= 0 && xc < rl.x1 - rl.x0 && z >= 0 && z < rl.height, kChkQueue);
+                    ln.pix = MODE == kModeList ? (int)(wcur + rank) : xc * rl.height + z;
+                    ln.level = 0;
+                    primary_ray(rl, xc, z, ln.O, ln.D);
+                }
+            }
+            if (MODE == kModeRays) {
+                const unsigned n_refused = (unsigned)__popc(__ballot_sync(kFull, refused));
+                n_primary -= n_refused;
+                n_invalid += n_refused;
             }
             n_primary += min((unsigned)__popc(idle), avail);
             wcur += min((unsigned)__popc(idle), avail);
@@ -298,7 +319,7 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
                 o[1] = tail.y;
                 o[2] = tail.z;
                 // cost estimate for the band balancer's pre-pass: bounces of this pixel, per column
-                if (!LIST && rl.col_cost != nullptr) {
+                if (MODE == kModeBand && rl.col_cost != nullptr) {
                     const int xc = ln.pix / rl.height;
                     atomicAdd(rl.col_cost + xc, (unsigned)(ln.level + 1));
                     atomicAdd(rl.col_cost + (rl.x1 - rl.x0) + (ln.pix - xc * rl.height), (unsigned)(ln.level + 1));
@@ -314,17 +335,23 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
         atomicAdd(rl.counters + 0, (unsigned long long)n_primary);
         atomicAdd(rl.counters + 1, (unsigned long long)n_shadow);
         atomicAdd(rl.counters + 2, (unsigned long long)n_reflect);
+        if (MODE == kModeRays && n_invalid != 0) atomicAdd(rl.ray_invalid, (unsigned long long)n_invalid);
     }
 }
 
 template <int CAP, int SBVH, int FM>
 __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_kernel(const __grid_constant__ RenderLaunch rl) {
-    render_body<CAP, SBVH, FM, false>(rl);
+    render_body<CAP, SBVH, FM, kModeBand>(rl);
 }
 
 template <int CAP, int SBVH, int FM>
 __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_list_kernel(const __grid_constant__ RenderLaunch rl) {
-    render_body<CAP, SBVH, FM, true>(rl);
+    render_body<CAP, SBVH, FM, kModeList>(rl);
+}
+
+template <int CAP, int SBVH, int FM>
+__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_rays_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_body<CAP, SBVH, FM, kModeRays>(rl);
 }
 
 template <int CAP, int SBVH, int FM>
@@ -348,21 +375,22 @@ cudaError_t launch_cap(const RenderLaunch& rl, int grid, size_t smem, cudaStream
     return cudaErrorInvalidValue;
 }
 
-template <int CAP, int SBVH, int FM>
+// the list- and ray-mode twins (kModeList, kModeRays)
+template <int CAP, int SBVH, int FM, int MODE>
 cudaError_t launch_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
-    cudaError_t e = cudaFuncSetAttribute(render_list_kernel<CAP, SBVH, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
+    const auto kernel = MODE == kModeRays ? render_rays_kernel<CAP, SBVH, FM> : render_list_kernel<CAP, SBVH, FM>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    render_list_kernel<CAP, SBVH, FM><<<grid, kBlock, smem, stream>>>(rl);
+    kernel<<<grid, kBlock, smem, stream>>>(rl);
     return cudaGetLastError();
 }
 
-template <int CAP>
+template <int CAP, int MODE>
 cudaError_t launch_list_cap(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
     const int sb = rl.scene.bvh_sph == nullptr ? 0 : 1;
     const int fm = rl.scene.bvh_fin != nullptr ? 2 : (rl.scene.n_fin == 0 ? 0 : (rl.scene.n_clu > 0 ? 1 : 3));
 #define TCRT_CASE(SB, FMV) \
-    if (sb == SB && fm == FMV) return launch_list_one<CAP, SB, FMV>(rl, grid, smem, stream);
+    if (sb == SB && fm == FMV) return launch_list_one<CAP, SB, FMV, MODE>(rl, grid, smem, stream);
     TCRT_CASE(0, 0) TCRT_CASE(0, 1) TCRT_CASE(0, 2) TCRT_CASE(0, 3)
     TCRT_CASE(1, 0) TCRT_CASE(1, 1) TCRT_CASE(1, 2) TCRT_CASE(1, 3)
 #undef TCRT_CASE
@@ -524,9 +552,11 @@ cudaError_t tcrt_launch_render(const RenderLaunch& rl_in, int sm_count, cudaStre
     return e;
 }
 
-// List mode (adaptive frames): the same kernels with the list refill, grid-sized and dispatched as tcrt_launch_render
-// does, never the developer builds' pool or wavefront paths.  One launch; nothing when the list is empty.
-cudaError_t tcrt_launch_render_list(const RenderLaunch& rl_in, int sm_count, cudaStream_t stream) {
+// List mode (adaptive frames) and ray mode (ray batches): the same kernels with the list or ray refill, grid-sized and
+// dispatched as tcrt_launch_render does, never the developer builds' pool or wavefront paths.  One launch; nothing when
+// the list is empty.
+template <int MODE>
+static cudaError_t launch_twin(const RenderLaunch& rl_in, int sm_count, cudaStream_t stream) {
     RenderLaunch rl = rl_in;
     if (rl.list_n <= 0) return cudaSuccess;
     const size_t smem = (size_t)std::max(1, rl.scene.blob_f4 - rl.scene.stage_off) * sizeof(float4);
@@ -537,15 +567,23 @@ cudaError_t tcrt_launch_render_list(const RenderLaunch& rl_in, int sm_count, cud
     rl.col_cost = nullptr;
     rl.refill_min = 32;
     if (rl.scene.grid_cells != nullptr && rl.scene.bvh_sph != nullptr && (fm == 0 || fm == 3))
-        return tcrt_launch_render_grid(rl, fm, sm_count, smem, stream, true);
+        return tcrt_launch_render_grid(rl, fm, sm_count, smem, stream, (RenderMode)MODE);
     int ctas_per_sm = (rl.scene.bvh_sph != nullptr && rl.scene.n_fin == 0) ? kMinBlocksBvh : kMinBlocks;
     while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;
     // persistent grid, but no more CTAs than there are claims of 32 queue positions per warp
     const long long need = ((long long)rl.list_n + kBlock - 1) / kBlock;
     const int grid = (int)std::min<long long>((long long)sm_count * ctas_per_sm, need);
     const int levels = rl.max_depth + 1;
-    if (levels <= 8) return launch_list_cap<8>(rl, grid, smem, stream);
-    if (levels <= 16) return launch_list_cap<16>(rl, grid, smem, stream);
-    if (levels <= 64) return launch_list_cap<64>(rl, grid, smem, stream);
-    return launch_list_cap<256>(rl, grid, smem, stream);
+    if (levels <= 8) return launch_list_cap<8, MODE>(rl, grid, smem, stream);
+    if (levels <= 16) return launch_list_cap<16, MODE>(rl, grid, smem, stream);
+    if (levels <= 64) return launch_list_cap<64, MODE>(rl, grid, smem, stream);
+    return launch_list_cap<256, MODE>(rl, grid, smem, stream);
+}
+
+cudaError_t tcrt_launch_render_list(const RenderLaunch& rl, int sm_count, cudaStream_t stream) {
+    return launch_twin<kModeList>(rl, sm_count, stream);
+}
+
+cudaError_t tcrt_launch_render_rays(const RenderLaunch& rl, int sm_count, cudaStream_t stream) {
+    return launch_twin<kModeRays>(rl, sm_count, stream);
 }

@@ -37,9 +37,10 @@ constexpr int kZeroShift = 20;
 constexpr int kDead = 7 << kZeroShift;
 static_assert(TCRT_MAX_DEPTH < kLevelMask, "levels and level records have to fit their fields");
 
-// The kernel body.  LIST = false: the pixels of the band (render_grid_kernel); LIST = true: the samples of a pixel list
-// (render_grid_list_kernel, adaptive frames; RenderLaunch::list): only the refill block and the output slot differ.
-template <int CAP, int FM, bool LIST>
+// The kernel body.  MODE kModeBand: the pixels of the band (render_grid_kernel); kModeList: the samples of a pixel list
+// (render_grid_list_kernel, adaptive frames; RenderLaunch::list); kModeRays: the caller's rays (render_grid_rays_kernel,
+// ray batches; RenderLaunch::ray_*).  Only the refill block, the output slot and the invalid-ray count differ.
+template <int CAP, int FM, int MODE>
 __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
     extern __shared__ float4 smem4[];
     const DeviceScene& sc = rl.scene;
@@ -60,7 +61,7 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
 
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned total = LIST ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = MODE != kModeBand ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     const V3 null_color = mk(rl.null_r, rl.null_g, rl.null_b);
 
     float stack[CAP * 7];   // per level: local rgb, k, object rgb (local memory, touched only on reflective hits)
@@ -73,6 +74,7 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
     ln.O = mk(0.f, 0.f, 0.f);
     ln.D = mk(1.f, 0.f, 0.f);
     unsigned n_primary = 0, n_shadow = 0, n_reflect = 0;
+    unsigned n_invalid = 0;        // ray mode: rays refused by the validity rule
     unsigned wcur = 0, wend = 0;   // the warp's claimed tile of pixel ids
     bool exhausted = false;
 
@@ -93,14 +95,33 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
             }
             const unsigned avail = wend - wcur;
             const unsigned rank = __popc(idle & lt_mask);
+            bool refused = false;
             if (ln.pix < 0 && rank < avail) {
-                int xc, z;
                 TCRT_CHECK(wcur + rank < total, kChkQueue);
-                if (LIST) list_to_sample(rl, (int)(wcur + rank), xc, z);
-                else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
-                ln.pix = LIST ? (int)(wcur + rank) : xc * rl.height + z;
-                ln.level = 0;
-                primary_ray(rl, xc, z, ln.O, ln.D);
+                if (MODE == kModeRays) {
+                    // the caller's ray; an invalid one gets the NaN marker and leaves the lane idle for the next ray
+                    const int q = (int)(wcur + rank);
+                    if (ray_from_batch(rl, q, ln.O, ln.D)) {
+                        ln.pix = q;
+                        ln.level = 0;
+                    } else {
+                        float* o = rl.out + 3 * (size_t)q;
+                        o[0] = o[1] = o[2] = __uint_as_float(0x7fc00000u);
+                        refused = true;
+                    }
+                } else {
+                    int xc, z;
+                    if (MODE == kModeList) list_to_sample(rl, (int)(wcur + rank), xc, z);
+                    else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
+                    ln.pix = MODE == kModeList ? (int)(wcur + rank) : xc * rl.height + z;
+                    ln.level = 0;
+                    primary_ray(rl, xc, z, ln.O, ln.D);
+                }
+            }
+            if (MODE == kModeRays) {
+                const unsigned n_refused = (unsigned)__popc(__ballot_sync(kFull, refused));
+                n_primary -= n_refused;
+                n_invalid += n_refused;
             }
             n_primary += min((unsigned)__popc(idle), avail);
             wcur += min((unsigned)__popc(idle), avail);
@@ -419,7 +440,7 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                 o[1] = tail.y;
                 o[2] = tail.z;
                 // cost estimate for the band balancer's pre-pass: bounces of this pixel, per column
-                if (!LIST && rl.col_cost != nullptr) {
+                if (MODE == kModeBand && rl.col_cost != nullptr) {
                     const int xc = ln.pix / rl.height;
                     const unsigned bounces = (unsigned)((ln.level & kLevelMask) + 1);
                     atomicAdd(rl.col_cost + xc, bounces);
@@ -436,17 +457,23 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
         atomicAdd(rl.counters + 0, (unsigned long long)n_primary);
         atomicAdd(rl.counters + 1, (unsigned long long)n_shadow);
         atomicAdd(rl.counters + 2, (unsigned long long)n_reflect);
+        if (MODE == kModeRays && n_invalid != 0) atomicAdd(rl.ray_invalid, (unsigned long long)n_invalid);
     }
 }
 
 template <int CAP, int FM>
 __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_kernel(const __grid_constant__ RenderLaunch rl) {
-    render_grid_body<CAP, FM, false>(rl);
+    render_grid_body<CAP, FM, kModeBand>(rl);
 }
 
 template <int CAP, int FM>
 __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_list_kernel(const __grid_constant__ RenderLaunch rl) {
-    render_grid_body<CAP, FM, true>(rl);
+    render_grid_body<CAP, FM, kModeList>(rl);
+}
+
+template <int CAP, int FM>
+__global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_rays_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_grid_body<CAP, FM, kModeRays>(rl);
 }
 
 template <int CAP, int FM>
@@ -457,17 +484,20 @@ cudaError_t launch_grid_one(const RenderLaunch& rl, int grid, size_t smem, cudaS
     return cudaGetLastError();
 }
 
+// the list- and ray-mode twins
 template <int CAP, int FM>
-cudaError_t launch_grid_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
-    cudaError_t e = cudaFuncSetAttribute(render_grid_list_kernel<CAP, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+cudaError_t launch_grid_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream, RenderMode mode) {
+    const auto kernel = mode == kModeRays ? render_grid_rays_kernel<CAP, FM> : render_grid_list_kernel<CAP, FM>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    render_grid_list_kernel<CAP, FM><<<grid, kGridBlock, smem, stream>>>(rl);
+    kernel<<<grid, kGridBlock, smem, stream>>>(rl);
     return cudaGetLastError();
 }
 
 template <int CAP>
-cudaError_t launch_grid_cap(const RenderLaunch& rl, int fm, int grid, size_t smem, cudaStream_t stream, bool list) {
-    if (list) return fm == 0 ? launch_grid_list_one<CAP, 0>(rl, grid, smem, stream) : launch_grid_list_one<CAP, 3>(rl, grid, smem, stream);
+cudaError_t launch_grid_cap(const RenderLaunch& rl, int fm, int grid, size_t smem, cudaStream_t stream, RenderMode mode) {
+    if (mode != kModeBand)
+        return fm == 0 ? launch_grid_list_one<CAP, 0>(rl, grid, smem, stream, mode) : launch_grid_list_one<CAP, 3>(rl, grid, smem, stream, mode);
     return fm == 0 ? launch_grid_one<CAP, 0>(rl, grid, smem, stream) : launch_grid_one<CAP, 3>(rl, grid, smem, stream);
 }
 
@@ -499,15 +529,16 @@ extern "C" int tcrt_dev_lane_stats_grid(unsigned long long* out16, int reset) {
 #endif
 
 // fm: 0 no finite planes, 3 a handful swept linearly; rl.scene.grid_cells != nullptr (tcrt_upload_scene built a grid).
-// list: the list-mode kernels (tcrt_launch_render_list), with no more CTAs than there are claims.
-cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream, bool list) {
+// mode kModeList / kModeRays: the list- or ray-mode kernels (tcrt_launch_render_list / _rays), with no more CTAs than
+// there are claims.
+cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream, RenderMode mode) {
     int ctas_per_sm = kGridMinBlocks;
     while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;
     int grid = sm_count * ctas_per_sm;
-    if (list) grid = (int)std::min<long long>(grid, ((long long)rl.list_n + kGridBlock - 1) / kGridBlock);
+    if (mode != kModeBand) grid = (int)std::min<long long>(grid, ((long long)rl.list_n + kGridBlock - 1) / kGridBlock);
     const int levels = rl.max_depth + 1;
-    if (levels <= 8) return launch_grid_cap<8>(rl, fm, grid, smem, stream, list);
-    if (levels <= 16) return launch_grid_cap<16>(rl, fm, grid, smem, stream, list);
-    if (levels <= 64) return launch_grid_cap<64>(rl, fm, grid, smem, stream, list);
-    return launch_grid_cap<256>(rl, fm, grid, smem, stream, list);
+    if (levels <= 8) return launch_grid_cap<8>(rl, fm, grid, smem, stream, mode);
+    if (levels <= 16) return launch_grid_cap<16>(rl, fm, grid, smem, stream, mode);
+    if (levels <= 64) return launch_grid_cap<64>(rl, fm, grid, smem, stream, mode);
+    return launch_grid_cap<256>(rl, fm, grid, smem, stream, mode);
 }

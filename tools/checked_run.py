@@ -4,7 +4,8 @@ library — every index range-checked, the level stack poisoned and checked for 
 every frame with the oracle bit for bit, and reports the check flags (0 = nothing fired).  Then the same for every
 dispatch class of tests/test_kernel_variants.py at the boundary depths of each level stack: band kernels (a tiled and an
 untiled frame, a band from an odd column), list kernels (adaptive frames refining every pixel) and hit kernels.  The
-flags are read from each translation unit that launches a kernel: render, grid and hits.
+flags are read from each translation unit that launches a kernel: render, grid and hits.  Last, a ray batch of valid and
+invalid rays on a grid scene and a BVH scene, traced and intersected, against tests/oracle_rays.c.
 usage: python -c "from tilecoderaytracer_b200 import build; build.build_lib(defines=('TCRT_CHECKED',), out=LIB)"
        TCRT_LIB=LIB python tools/checked_run.py"""
 import ctypes as C
@@ -114,4 +115,44 @@ with tempfile.TemporaryDirectory() as tmp:
         f = fired()
         bad_total += bad + len(f)
         print(f"{name:9s} hit buffers 27x17: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
+
+# ---- ray batches: valid and invalid rays mixed, through the render / grid kernels' ray mode and the hit kernel's -----------
+import test_ray_batches as R  # noqa: E402
+
+with tempfile.TemporaryDirectory() as tmp:
+    so = os.path.join(tmp, "liboracle_rays.so")
+    subprocess.run(["gcc", "-std=gnu11", "-O2", "-fPIC", "-shared", "-ffp-contract=off", os.path.join(ROOT, "tests", "oracle_rays.c"),
+                    "-o", so, "-lm"], check=True)
+    rl = C.CDLL(so)
+    rl.tcrt_oracle_trace_rays.restype = rl.tcrt_oracle_intersect_rays.restype = C.c_int
+    rl.tcrt_oracle_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                          C.POINTER(C.c_ulonglong), C.POINTER(O.OracleCounters)]
+    rl.tcrt_oracle_intersect_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_ulonglong)]
+    ox, dx, valid = R.crafted_rays()
+    for name, grid in (("synth256", True), ("default", False)):
+        cam = api.Camera()
+        sc = api.Scene().build(name, cam)
+        ctx.upload(sc, cam)
+        flat = sc.flatten()
+        o, d, _ = R.eye_rays(cam.export(), 48, 40, "shuffle")
+        o = np.concatenate([o, ox[~valid], o[:7]])
+        d = np.concatenate([d, dx[~valid], d[:7]])
+        bad = int(ctx.scene_structures()["grid_cells"] > 0) != int(grid)
+        for depth in (0, 8, 50):
+            p = api.default_params(1, 1, depth)
+            got, n_inv, st = ctx.trace_rays(p, o, d)
+            want, w_inv, cnt = R.oracle_trace(rl, flat, p, o, d)
+            bad += n_bad(got.reshape(-1, 1, 3), want.reshape(-1, 1, 3)) + counters_differ(st, cnt) + int(n_inv != w_inv)
+            h, h_inv, _ = ctx.intersect_rays(p, o, d)
+            want_h, _ = R.oracle_hits(rl, flat, p, o, d)
+            try:
+                R.assert_hits_equal(h, want_h, name)
+            except AssertionError as e:
+                print(e)
+                bad += 1
+        f = fired()
+        bad_total += bad + len(f)
+        print(f"ray batch {name:9s} {len(o)} rays ({int((~valid).sum())} invalid), d0/8/50: mismatches {bad}, "
+              f"checks fired: {f or 'none'}", flush=True)
 print("CHECKED_OK" if bad_total == 0 else "CHECKED_FAIL")

@@ -118,6 +118,25 @@ public:
         tcrt_params p = rs.params();
         return rc_ = tcrt_intersect_rays(ctx_, &p, rays.size(), o.data(), 0, d.data(), obj, dist, normal, n_invalid, stats);
     }
+    // inShadeCollisionDetection(rays[i], tmax[i]) (tcrt_occluded_rays): occluded[i] = 1 when a non-light object is hit
+    // nearer than tmax[i], else 0; 0xFF for an invalid ray or tmax (tcrt.h).  tmax.size() must equal rays.size().
+    int occludedRays(const std::vector<Ray>& rays, const std::vector<float>& tmax, unsigned char* occluded,
+                     unsigned long long* n_invalid = NULL, tcrt_stats* stats = NULL) {
+        if (tmax.size() != rays.size()) return rc_ = TCRT_ERR_INVALID;
+        std::vector<float> o, d;
+        unpackRays(rays, o, d);
+        return rc_ = tcrt_occluded_rays(ctx_, rays.size(), o.data(), 0, d.data(), tmax.data(), occluded, n_invalid, stats);
+    }
+    // inShade(points[i], light l) for every light (tcrt_occluded_lights): occluded[i * n_lights + l], lights in increasing
+    // object index; 0xFF for an invalid pair (tcrt.h)
+    int occludedLights(const std::vector<vector3d>& points, unsigned char* occluded, unsigned long long* n_invalid = NULL,
+                       tcrt_stats* stats = NULL) {
+        std::vector<float> p(points.size() * 3);
+        for (size_t i = 0; i < points.size(); i++) {
+            p[3 * i] = points[i].x; p[3 * i + 1] = points[i].y; p[3 * i + 2] = points[i].z;
+        }
+        return rc_ = tcrt_occluded_lights(ctx_, points.size(), p.data(), occluded, n_invalid, stats);
+    }
     // init_log + printPixelsToLog (RayTracer.cpp:2022-2061,1574-1626)
     int printPixelsToLog(const char* path = LOG_FILE_NAME) {
         tcrt_params p = settings_.params();

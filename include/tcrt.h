@@ -356,6 +356,40 @@ int tcrt_trace_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* pa
 int tcrt_intersect_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* params, size_t n,
                                const float* origins, int shared_origin, const float* directions, int* object,
                                float* distance, float* normal, unsigned long long* n_invalid, tcrt_stats* stats);
+/* Occlusion queries: the reference's shadow test (inShadeCollisionDetection, RayTracer.cpp:709-739) for caller-supplied
+ * rays, and its inShade (:743-771) for caller-supplied points against every light.  Neither takes tcrt_params: the shadow
+ * test reads none of them (not far_dist, shadows_on or max_depth).
+ *   - rays (tcrt_occluded_rays): origins and directions as for the ray batches above (per ray or shared origin, used as a
+ *     Ray stores them, the same validity rule), plus a limit tmax[i] per ray.  occluded[i] = 1 when some object that is
+ *     not a light has a reference collision at distance d < tmax_i (strict), else 0.  tmax = +inf is allowed.  A sphere's
+ *     distance is negative when the origin is inside it, so an origin inside a non-light sphere is always occluded.
+ *   - points (tcrt_occluded_lights): points[3i..3i+2], n points; occluded[i * n_lights + l] for every light l in the order
+ *     of tcrt_scene.light_obj (increasing object index).  The value is what inShade(P_i, light l) returns, with the
+ *     reference's arithmetic: dir = L - P, dist = sqrtf((dx*dx + dy*dy) + dz*dz), lr = dir / dist (three IEEE
+ *     divisions), then the test above along lr with limit dist.  A scene without lights is success: nothing is written.
+ * An answer of 0xFF marks an invalid ray or pair, which is not traced: a ray that fails the batch rule, or whose tmax is
+ * NaN or <= 0; a pair whose point fails the origin rule (finite, |p_k| <= 2^40; the point's whole row), or whose lr fails
+ * the direction rule (|s - 1| <= 2^-21).  The latter happens only when P is at the light or within about 1e-19 of it,
+ * where the reference would answer "not in shade" (its 0/0 compares false); like the ray batches' rule, this is a
+ * deliberate deviation.  *n_invalid (may be NULL) counts invalid rays, or invalid (point, light) pairs.
+ * Host forms: inputs and outputs in pinned or pageable memory.  A multi-device ctx splits [0, n) into equal contiguous
+ * ranges of rays or points.  Pieces of at most 4 Mi rays (28 B of input each, 16 with a shared origin) or 4 Mi (point,
+ * light) pairs (12 B of input per point, n_lights bytes of output), at least one point, round robin over the render
+ * streams.  Device forms (_device) as for the ray batches.  All four calls are synchronous; n = 0 launches nothing.
+ * Errors: NULL ctx, inputs (n > 0) or output, or a byte count that overflows: TCRT_ERR_INVALID; before tcrt_upload_scene:
+ * TCRT_ERR_NO_SCENE.  Stats: col_begin/col_end each device's range of rays or points, rays_shadow the tests traced (valid
+ * rays or valid pairs), rays_primary and rays_reflect 0, render_ms, d2h_ms and gpu_launches as for the ray batches.  They
+ * never change the last render, the writers, the multi-device cut or cost map, or a frame in flight, and ignore
+ * tcrt_set_camera. */
+int tcrt_occluded_rays(tcrt_ctx* ctx, size_t n, const float* origins, int shared_origin, const float* directions,
+                       const float* tmax, unsigned char* occluded, unsigned long long* n_invalid, tcrt_stats* stats);
+int tcrt_occluded_lights(tcrt_ctx* ctx, size_t n, const float* points, unsigned char* occluded,
+                         unsigned long long* n_invalid, tcrt_stats* stats);
+int tcrt_occluded_rays_device(tcrt_ctx* ctx, int device_slot, size_t n, const float* origins, int shared_origin,
+                              const float* directions, const float* tmax, unsigned char* occluded,
+                              unsigned long long* n_invalid, tcrt_stats* stats);
+int tcrt_occluded_lights_device(tcrt_ctx* ctx, int device_slot, size_t n, const float* points, unsigned char* occluded,
+                                unsigned long long* n_invalid, tcrt_stats* stats);
 /* Cost-balanced column bands (replaces the equal z-bands of the reference's strategy 1,
  * RayTracer.cpp:904-906, whose load imbalance strategies 2-7 and PixelQueue were written to fix).
  * Renders a low-resolution copy of the frame on device slot 0 in which every finished pixel adds its

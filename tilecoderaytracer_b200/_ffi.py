@@ -125,6 +125,14 @@ SIGNATURES = {
     "tcrt_intersect_rays_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(TcrtParams), C.c_size_t, C.c_void_p, C.c_int,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_ulonglong),
                                              C.POINTER(TcrtStats)]),
+    "tcrt_occluded_rays": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
+    "tcrt_occluded_lights": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(C.c_ulonglong),
+                                       C.POINTER(TcrtStats)]),
+    "tcrt_occluded_rays_device": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
+    "tcrt_occluded_lights_device": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p,
+                                              C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),
     "tcrt_bands_from_costs": (C.c_int, [C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),

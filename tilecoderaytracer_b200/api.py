@@ -312,6 +312,7 @@ class Context:
 
     def upload_flat(self, flat: TcrtScene, cam: TcrtCamera) -> None:
         self._ck(self._lib.tcrt_upload_scene(self._h, C.byref(flat), C.byref(cam)))
+        self._n_lights = int(flat.n_lights)
 
     def scene_structures(self) -> dict:
         """Which pruning structures the uploaded scene got (tcrt_scene_structures)."""
@@ -581,6 +582,62 @@ class Context:
                                                       int(bool(shared_origin)), C.c_void_p(directions),
                                                       C.c_void_p(object or None), C.c_void_p(distance or None),
                                                       C.c_void_p(normal or None), C.byref(bad), C.byref(st)))
+        return int(bad.value), RenderStats.from_c(st)
+
+    def occluded_rays(self, origins, directions, tmax, out: Optional[np.ndarray] = None):
+        """The reference's shadow test of caller-supplied rays (tcrt_occluded_rays): origins and directions as in
+        trace_rays, tmax (n,) float32 per ray (+inf allowed).  Returns (occluded (n,) uint8, n_invalid, RenderStats): 1 when
+        a non-light object is hit at a distance < tmax, 0 if not, 0xFF for an invalid ray or tmax (NaN or <= 0).  `out` (n,)
+        uint8 may be pinned or pageable."""
+        n, o, shared, d = _ray_inputs(origins, directions)
+        t = np.asarray(tmax)
+        assert t.dtype == np.float32 and t.shape == (n,) and t.flags["C_CONTIGUOUS"], "tmax: (n,) float32"
+        if out is None:
+            out = np.empty(n, np.uint8)
+        assert out.dtype == np.uint8 and out.size == n and out.flags["C_CONTIGUOUS"], "out: (n,) uint8"
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_occluded_rays(self._h, n, o.ctypes.data_as(C.c_void_p), shared, d.ctypes.data_as(C.c_void_p),
+                                              t.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p), C.byref(bad),
+                                              C.byref(st)))
+        return out.reshape(n), int(bad.value), RenderStats.from_c(st)
+
+    def occluded_lights(self, points, out: Optional[np.ndarray] = None):
+        """inShade of caller-supplied points against every light (tcrt_occluded_lights): points (n, 3) float32.  Returns
+        (occluded (n, n_lights) uint8, lights in the order of the scene's light_obj, n_invalid (pairs), RenderStats); 0xFF
+        marks a point outside the origin rule or one at (within ~1e-19 of) the light.  `out` (n, n_lights) uint8 may be
+        pinned or pageable."""
+        pts = np.asarray(points)
+        assert pts.dtype == np.float32 and pts.ndim == 2 and pts.shape[1] == 3 and pts.flags["C_CONTIGUOUS"], "points: (n, 3) float32"
+        n, n_lights = pts.shape[0], getattr(self, "_n_lights", 0)
+        if out is None:
+            out = np.empty((n, n_lights), np.uint8)
+        assert out.dtype == np.uint8 and out.size == n * n_lights and out.flags["C_CONTIGUOUS"], "out: (n, n_lights) uint8"
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_occluded_lights(self._h, n, pts.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p),
+                                                C.byref(bad), C.byref(st)))
+        return out.reshape(n, n_lights), int(bad.value), RenderStats.from_c(st)
+
+    def occluded_rays_device(self, n: int, origins: int, directions: int, tmax: int, occluded: int,
+                             shared_origin: bool = False, slot: int = 0):
+        """occluded_rays on device `slot` with device addresses (e.g. torch CUDA tensors' data_ptr()): origins 3n floats
+        (3 when shared_origin), directions 3n floats, tmax n floats, occluded n bytes.  The inputs must be complete.
+        Returns (n_invalid, RenderStats)."""
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_occluded_rays_device(self._h, slot, n, C.c_void_p(origins), int(bool(shared_origin)),
+                                                     C.c_void_p(directions), C.c_void_p(tmax), C.c_void_p(occluded),
+                                                     C.byref(bad), C.byref(st)))
+        return int(bad.value), RenderStats.from_c(st)
+
+    def occluded_lights_device(self, n: int, points: int, occluded: int, slot: int = 0):
+        """occluded_lights on device `slot` with device addresses: points 3n floats, occluded n * n_lights bytes.
+        Returns (n_invalid, RenderStats)."""
+        bad = C.c_ulonglong(0)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_occluded_lights_device(self._h, slot, n, C.c_void_p(points), C.c_void_p(occluded),
+                                                       C.byref(bad), C.byref(st)))
         return int(bad.value), RenderStats.from_c(st)
 
     def balance_columns(self, params: TcrtParams, n_bands: int) -> list[tuple[int, int]]:

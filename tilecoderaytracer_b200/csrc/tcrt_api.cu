@@ -2462,91 +2462,118 @@ static bool on_device(const void* p, int dev) {
     return at.type == cudaMemoryTypeDevice && at.device == dev;
 }
 
-// One batch: [0, n) split into equal contiguous ranges, one per device (device forms: slot only), each traced in pieces of
-// at most kRayPiece rays round robin over the render streams.  A piece of a host form is: its inputs to the stream's scratch
-// (pinned ones straight, pageable ones through the stream's pinned staging), one launch, its outputs to the host on the copy
-// stream (pinned ones straight, pageable ones through stage_out).  A piece's outputs are sent once the next piece has been
-// queued, so a piece's copies overlap other pieces' launches; a stream's next piece waits for them before it reuses the
-// scratch.  Device forms launch on the caller's buffers directly.  out[0] rgb (colour) or object, out[1] distance,
-// out[2] normal (hits).
-static int rays_impl(tcrt_ctx* ctx, int slot, const tcrt_params* p, size_t n, const float* origins, int shared_origin,
-                     const float* dirs, bool hits, void* const out_in[3], unsigned long long* n_invalid, tcrt_stats* stats) {
+// What a batch computes: the colour of each ray (render kernels' ray mode), its nearest hit (hit kernel's ray mode),
+// whether it is occluded before its limit, or whether each point is occluded from each light (occlusion kernel).
+enum BatchKind { kBatchColour, kBatchHits, kBatchOccRays, kBatchOccPoints };
+
+// One batch: [0, n) split into equal contiguous ranges, one per device (device forms: slot only), each run in pieces round
+// robin over the render streams: at most kRayPiece rays, or (points) kRayPiece (point, light) pairs and at least one point.
+// A piece of a host form is: its inputs to the stream's scratch (pinned ones straight, pageable ones through the stream's
+// pinned staging), one launch, its outputs to the host on the copy stream (pinned ones straight, pageable ones through
+// stage_out).  A piece's outputs are sent once the next piece has been queued, so a piece's copies overlap other pieces'
+// launches; a stream's next piece waits for them before it reuses the scratch.  Device forms launch on the caller's buffers
+// directly.  Inputs: directions (rays) or points, origins (rays), tmax (occluded rays).  out[0] rgb (colour), object (hits)
+// or the occlusion bytes, out[1] distance, out[2] normal (hits).  p: params of the colour and hit kinds, nullptr otherwise.
+static int rays_impl(tcrt_ctx* ctx, int slot, BatchKind kind, const tcrt_params* p, size_t n, const float* origins,
+                     int shared_origin, const float* dirs, const float* tmax, void* const out_in[3],
+                     unsigned long long* n_invalid, tcrt_stats* stats) {
     if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
-    if (!p) return fail(ctx, TCRT_ERR_INVALID, "null params");
+    const bool hits = kind == kBatchHits, occ = kind == kBatchOccRays || kind == kBatchOccPoints;
+    const bool points = kind == kBatchOccPoints;
+    if (!occ && !p) return fail(ctx, TCRT_ERR_INVALID, "null params");
     const bool device_form = slot >= 0;
     if (device_form && slot >= (int)ctx->devs.size()) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", slot);
-    if (!hits && p->max_depth < 0) return fail(ctx, TCRT_ERR_INVALID, "max_depth %d < 0", p->max_depth);
+    if (kind == kBatchColour && p->max_depth < 0) return fail(ctx, TCRT_ERR_INVALID, "max_depth %d < 0", p->max_depth);
     char* out[3] = {static_cast<char*>(out_in[0]), static_cast<char*>(out_in[1]), static_cast<char*>(out_in[2])};
     if (hits ? (!out[0] && !out[1] && !out[2]) : !out[0]) return fail(ctx, TCRT_ERR_INVALID, "no output");
-    if (n > 0 && (!origins || !dirs)) return fail(ctx, TCRT_ERR_INVALID, "null ray input");
+    if (n > 0 && (points ? !dirs : (!origins || !dirs || (kind == kBatchOccRays && !tmax))))
+        return fail(ctx, TCRT_ERR_INVALID, "null ray input");
     if (n > SIZE_MAX / (6 * sizeof(float))) return fail(ctx, TCRT_ERR_INVALID, "%zu rays: byte count overflows", n);
-    if (!hits && p->max_depth > TCRT_MAX_DEPTH)
+    if (kind == kBatchColour && p->max_depth > TCRT_MAX_DEPTH)
         return fail(ctx, TCRT_ERR_UNSUPPORTED, "max_depth %d > TCRT_MAX_DEPTH %d", p->max_depth, TCRT_MAX_DEPTH);
     if (device_form && n > 0) {
         const int dev = ctx->devs[slot].dev;
-        const void* ptrs[5] = {origins, dirs, out[0], out[1], out[2]};
+        const void* ptrs[6] = {origins, dirs, tmax, out[0], out[1], out[2]};
         for (const void* q : ptrs)
             if (q && !on_device(q, dev))
                 return fail(ctx, TCRT_ERR_INVALID, "pointer %p is not device memory of device %d (slot %d)", q, dev, slot);
     }
     if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    // output bytes per point (a scene without lights: nothing to answer, nothing launched)
+    const size_t n_lights = points ? (size_t)ctx->devs[0].ds.n_lights : 1;
+    if (n_lights > 0 && n > SIZE_MAX / n_lights)
+        return fail(ctx, TCRT_ERR_INVALID, "%zu points x %zu lights: byte count overflows", n, n_lights);
+    tcrt_params occ_params;   // read by band_launch only; the occlusion kernel reads none of it
+    if (occ) {
+        tcrt_default_params(&occ_params);
+        p = &occ_params;
+    }
     const int nd = (int)ctx->devs.size();
     const int d_begin = device_form ? slot : 0, d_end = device_form ? slot + 1 : nd;
     std::vector<size_t> cut(nd + 1, 0);
     for (int i = 0; i <= nd; i++)
         cut[i] = device_form ? (i <= slot ? 0 : n) : n / nd * i + n % nd * i / nd;
-    // bytes per ray of each output
+    // inputs, in the order of the scratch: directions or points (3 floats per item), origins (3 per item, or 3 in all when
+    // shared), tmax (1 per item)
+    const int n_in = kind == kBatchOccRays ? 3 : points ? 1 : 2;
+    const float* in_src[3] = {dirs, origins, tmax};
+    auto in_words = [&](int k, size_t cnt) -> size_t { return k == 1 ? (shared_origin ? 3 : 3 * cnt) : (k == 0 ? 3 : 1) * cnt; };
+    // bytes per item of each output
     const int n_out = hits ? 3 : 1;
-    const size_t out_bytes[3] = {hits ? (size_t)4 : (size_t)12, 4, 12};
+    const size_t out_bytes[3] = {hits ? (size_t)4 : occ ? n_lights : (size_t)12, 4, 12};
+    const size_t item_out = out_bytes[0] + (hits ? out_bytes[1] + out_bytes[2] : 0);
     bool staged[3] = {false, false, false}, any_direct = false;
-    bool in_pageable[2] = {false, false};
+    bool in_pageable[3] = {false, false, false}, any_pageable = false;
     if (!device_form && n > 0) {
         for (int k = 0; k < n_out; k++) {
             staged[k] = out[k] && host_pageable(out[k]);
             any_direct = any_direct || (out[k] && !staged[k]);
         }
-        in_pageable[0] = host_pageable(dirs);
-        in_pageable[1] = host_pageable(origins);
+        for (int k = 0; k < n_in; k++) any_pageable = any_pageable || (in_pageable[k] = host_pageable(in_src[k]));
     }
     if (stats) memset(stats, 0, sizeof(*stats));
     if (n_invalid) *n_invalid = 0;
     auto stream_of = [](DeviceState& d, int si) { return si == 0 ? d.stream : d.chunk_stream[si - 1]; };
     std::vector<int> used_streams(nd, 0), launches(nd, 0);
+    const size_t piece_items = std::max<size_t>(1, kRayPiece / std::max<size_t>(1, n_lights));
     for (int i = d_begin; i < d_end; i++) {
         DeviceState& d = ctx->devs[i];
         const size_t r0 = cut[i], r1 = cut[i + 1];
-        if (r1 <= r0) continue;
+        if (r1 <= r0 || n_lights == 0) continue;
         CK(ctx, cudaSetDevice(d.dev));
         int rc = ensure_ray_state(ctx, d);
         if (rc) return rc;
-        const size_t n_pieces = (r1 - r0 + kRayPiece - 1) / kRayPiece;
+        const size_t n_pieces = (r1 - r0 + piece_items - 1) / piece_items;
         const int ns = ctx->one_stream ? 1 : (int)std::min<size_t>(kChunkStreams, n_pieces);
         used_streams[i] = ns;
-        const size_t per = std::min(kRayPiece, r1 - r0);
-        // scratch: directions, origins, then the outputs (hits: object, distance, normal)
-        const size_t in_words = 3 * per + (shared_origin ? 3 : 3 * per);
-        const size_t all_out = hits ? 5 * per : 3 * per;
+        const size_t per = std::min(piece_items, r1 - r0);
+        // scratch: the inputs, then the outputs (hits: object, distance, normal)
+        auto all_in = [&](size_t cnt) {
+            size_t w = 0;
+            for (int k = 0; k < n_in; k++) w += in_words(k, cnt);
+            return w;
+        };
         if (!device_form) {
             for (int si = 0; si < ns; si++)
-                if ((rc = ensure(ctx, d.ray_mem[si], d.ray_mem_cap[si], in_words + all_out))) return rc;
-            if (in_pageable[0] || in_pageable[1])
+                if ((rc = ensure(ctx, d.ray_mem[si], d.ray_mem_cap[si], all_in(per) + (per * item_out + 3) / 4))) return rc;
+            if (any_pageable)
                 for (int si = 0; si < ns; si++)
-                    if ((rc = ensure_pinned(ctx, d.ray_stage[si], d.ray_stage_cap[si], in_words))) return rc;
+                    if ((rc = ensure_pinned(ctx, d.ray_stage[si], d.ray_stage_cap[si], all_in(per)))) return rc;
         }
         // on the render stream, behind whatever is queued there (a scene upload, frames in flight); the other render
         // streams start behind it
         CK(ctx, cudaMemsetAsync(d.ray_ctl, 0, 64 * ns, d.stream));
         CK(ctx, cudaEventRecord(d.ev_r0, d.stream));
         for (int si = 1; si < ns; si++) CK(ctx, cudaStreamWaitEvent(stream_of(d, si), d.ev_r0, 0));
-        // piece k: rays [r0 + k*per, ...) on stream k % ns
+        // piece k: items [r0 + k*per, ...) on stream k % ns
         auto piece = [&](size_t k, size_t& a, size_t& cnt, int& si) {
             a = r0 + k * per;
             cnt = std::min(per, r1 - a);
             si = (int)(k % (size_t)ns);
         };
-        auto out_dev = [&](int si, size_t cnt, int k) -> float* {   // output k of a piece in the stream's scratch
-            float* base = d.ray_mem[si] + 3 * cnt + (shared_origin ? 3 : 3 * cnt);
-            return base + (k == 0 ? 0 : k == 1 ? cnt : 2 * cnt);
+        auto out_dev = [&](int si, size_t cnt, int k) -> char* {   // output k of a piece in the stream's scratch
+            char* base = reinterpret_cast<char*>(d.ray_mem[si] + all_in(cnt));
+            return base + (k == 0 ? 0 : k == 1 ? cnt * out_bytes[0] : cnt * (out_bytes[0] + out_bytes[1]));
         };
         auto send_out = [&](size_t k) -> int {
             size_t a, cnt;
@@ -2564,8 +2591,8 @@ static int rays_impl(tcrt_ctx* ctx, int slot, const tcrt_params* p, size_t n, co
                 CK(ctx, ensure_stage(d));
                 TxtPipe& pipe = copy_pipe_to(ctx, out[b]);
                 StageSlots slots;
-                const cudaError_t e = stage_out(pipe, d, slots, reinterpret_cast<const char*>(out_dev(si, cnt, b)),
-                                                cnt * out_bytes[b], a * out_bytes[b], d.ev_rk[si]);
+                const cudaError_t e = stage_out(pipe, d, slots, out_dev(si, cnt, b), cnt * out_bytes[b], a * out_bytes[b],
+                                                d.ev_rk[si]);
                 slots.drain(pipe);
                 if (e != cudaSuccess || pipe.io_error)
                     return fail(ctx, TCRT_ERR_CUDA, "staged copy-out of a ray batch: %s",
@@ -2581,27 +2608,23 @@ static int rays_impl(tcrt_ctx* ctx, int slot, const tcrt_params* p, size_t n, co
                 int si;
                 piece(k, a, cnt, si);
                 const cudaStream_t ks = stream_of(d, si);
-                const float* o_src = origins + (shared_origin ? 0 : 3 * a);
-                const float* d_src = dirs + 3 * a;
+                const float* src[3];
+                for (int b = 0; b < n_in; b++)
+                    src[b] = in_src[b] + (b == 1 && shared_origin ? 0 : in_words(b, a));
                 void* dst[3] = {out[0], out[1], out[2]};
                 if (!device_form) {
-                    float* dd = d.ray_mem[si];
-                    float* od = dd + 3 * cnt;
-                    const size_t nd_f = 3 * cnt, no_f = shared_origin ? 3 : 3 * cnt;
                     CK(ctx, cudaStreamWaitEvent(ks, d.ev_rout[si], 0));   // the scratch's last outputs have left
-                    if (in_pageable[0] || in_pageable[1]) {
-                        CK(ctx, cudaEventSynchronize(d.ev_rin[si]));        // so has the staging's last input
-                        float* st = d.ray_stage[si];
-                        if (in_pageable[0]) memcpy(st, d_src, nd_f * sizeof(float));
-                        if (in_pageable[1]) memcpy(st + nd_f, o_src, no_f * sizeof(float));
+                    if (any_pageable) CK(ctx, cudaEventSynchronize(d.ev_rin[si]));   // so has the staging's last input
+                    size_t off = 0;
+                    for (int b = 0; b < n_in; b++) {
+                        const size_t w = in_words(b, cnt);
+                        if (in_pageable[b]) memcpy(d.ray_stage[si] + off, src[b], w * sizeof(float));
+                        CK(ctx, cudaMemcpyAsync(d.ray_mem[si] + off, in_pageable[b] ? d.ray_stage[si] + off : src[b],
+                                                w * sizeof(float), cudaMemcpyHostToDevice, ks));
+                        src[b] = d.ray_mem[si] + off;
+                        off += w;
                     }
-                    CK(ctx, cudaMemcpyAsync(dd, in_pageable[0] ? d.ray_stage[si] : d_src, nd_f * sizeof(float),
-                                            cudaMemcpyHostToDevice, ks));
-                    CK(ctx, cudaMemcpyAsync(od, in_pageable[1] ? d.ray_stage[si] + nd_f : o_src, no_f * sizeof(float),
-                                            cudaMemcpyHostToDevice, ks));
                     CK(ctx, cudaEventRecord(d.ev_rin[si], ks));
-                    o_src = od;
-                    d_src = dd;
                     // every output goes to the scratch; only the requested ones leave it
                     for (int b = 0; b < n_out; b++) dst[b] = out_dev(si, cnt, b);
                 } else {
@@ -2610,14 +2633,24 @@ static int rays_impl(tcrt_ctx* ctx, int slot, const tcrt_params* p, size_t n, co
                 }
                 unsigned char* ctl = d.ray_ctl + 64 * si;
                 CK(ctx, cudaMemsetAsync(ctl, 0, sizeof(unsigned int), ks));
-                RenderLaunch rl = band_launch(ctx, d, p, 0, 0, static_cast<float*>(dst[0]), reinterpret_cast<unsigned int*>(ctl));
+                RenderLaunch rl = band_launch(ctx, d, p, 0, 0, occ ? nullptr : static_cast<float*>(dst[0]),
+                                              reinterpret_cast<unsigned int*>(ctl));
                 rl.counters = reinterpret_cast<unsigned long long*>(ctl + 8);
                 rl.ray_invalid = reinterpret_cast<unsigned long long*>(ctl + 32);
-                rl.ray_o = o_src;
-                rl.ray_o_stride = shared_origin ? 0 : 3;
-                rl.ray_d = d_src;
                 rl.list_n = (int)cnt;
-                if (hits) {
+                if (!points) {
+                    rl.ray_o = src[1];
+                    rl.ray_o_stride = shared_origin ? 0 : 3;
+                    rl.ray_d = src[0];
+                }
+                if (occ) {
+                    OccLaunch ol{};
+                    ol.rl = rl;
+                    ol.tmax = points ? nullptr : src[2];
+                    ol.points = points ? src[0] : nullptr;
+                    ol.out = static_cast<unsigned char*>(dst[0]);
+                    CK(ctx, tcrt_launch_occlusion(ol, d.sm_count, ks));
+                } else if (hits) {
                     HitLaunch hl{};
                     hl.rl = rl;
                     hl.object = static_cast<int*>(dst[0]);
@@ -2680,14 +2713,14 @@ extern "C" {
 int tcrt_trace_rays(tcrt_ctx* ctx, const tcrt_params* p, size_t n, const float* origins, int shared_origin,
                     const float* directions, float* rgb, unsigned long long* n_invalid, tcrt_stats* stats) {
     void* out[3] = {rgb, nullptr, nullptr};
-    return rays_impl(ctx, -1, p, n, origins, shared_origin, directions, false, out, n_invalid, stats);
+    return rays_impl(ctx, -1, kBatchColour, p, n, origins, shared_origin, directions, nullptr, out, n_invalid, stats);
 }
 
 int tcrt_intersect_rays(tcrt_ctx* ctx, const tcrt_params* p, size_t n, const float* origins, int shared_origin,
                         const float* directions, int* object, float* distance, float* normal,
                         unsigned long long* n_invalid, tcrt_stats* stats) {
     void* out[3] = {object, distance, normal};
-    return rays_impl(ctx, -1, p, n, origins, shared_origin, directions, true, out, n_invalid, stats);
+    return rays_impl(ctx, -1, kBatchHits, p, n, origins, shared_origin, directions, nullptr, out, n_invalid, stats);
 }
 
 int tcrt_trace_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* p, size_t n, const float* origins,
@@ -2695,7 +2728,7 @@ int tcrt_trace_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* p,
                            tcrt_stats* stats) {
     if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
     void* out[3] = {rgb, nullptr, nullptr};
-    return rays_impl(ctx, device_slot, p, n, origins, shared_origin, directions, false, out, n_invalid, stats);
+    return rays_impl(ctx, device_slot, kBatchColour, p, n, origins, shared_origin, directions, nullptr, out, n_invalid, stats);
 }
 
 int tcrt_intersect_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* p, size_t n, const float* origins,
@@ -2703,7 +2736,35 @@ int tcrt_intersect_rays_device(tcrt_ctx* ctx, int device_slot, const tcrt_params
                                unsigned long long* n_invalid, tcrt_stats* stats) {
     if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
     void* out[3] = {object, distance, normal};
-    return rays_impl(ctx, device_slot, p, n, origins, shared_origin, directions, true, out, n_invalid, stats);
+    return rays_impl(ctx, device_slot, kBatchHits, p, n, origins, shared_origin, directions, nullptr, out, n_invalid, stats);
+}
+
+int tcrt_occluded_rays(tcrt_ctx* ctx, size_t n, const float* origins, int shared_origin, const float* directions,
+                       const float* tmax, unsigned char* occluded, unsigned long long* n_invalid, tcrt_stats* stats) {
+    void* out[3] = {occluded, nullptr, nullptr};
+    return rays_impl(ctx, -1, kBatchOccRays, nullptr, n, origins, shared_origin, directions, tmax, out, n_invalid, stats);
+}
+
+int tcrt_occluded_lights(tcrt_ctx* ctx, size_t n, const float* points, unsigned char* occluded,
+                         unsigned long long* n_invalid, tcrt_stats* stats) {
+    void* out[3] = {occluded, nullptr, nullptr};
+    return rays_impl(ctx, -1, kBatchOccPoints, nullptr, n, nullptr, 0, points, nullptr, out, n_invalid, stats);
+}
+
+int tcrt_occluded_rays_device(tcrt_ctx* ctx, int device_slot, size_t n, const float* origins, int shared_origin,
+                              const float* directions, const float* tmax, unsigned char* occluded,
+                              unsigned long long* n_invalid, tcrt_stats* stats) {
+    if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
+    void* out[3] = {occluded, nullptr, nullptr};
+    return rays_impl(ctx, device_slot, kBatchOccRays, nullptr, n, origins, shared_origin, directions, tmax, out, n_invalid,
+                     stats);
+}
+
+int tcrt_occluded_lights_device(tcrt_ctx* ctx, int device_slot, size_t n, const float* points, unsigned char* occluded,
+                                unsigned long long* n_invalid, tcrt_stats* stats) {
+    if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
+    void* out[3] = {occluded, nullptr, nullptr};
+    return rays_impl(ctx, device_slot, kBatchOccPoints, nullptr, n, nullptr, 0, points, nullptr, out, n_invalid, stats);
 }
 
 }  // extern "C"

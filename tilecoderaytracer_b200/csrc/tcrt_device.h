@@ -152,6 +152,19 @@ struct HitLaunch {
     float* normal;     // 3 per pixel: its normal ray's direction ((0,0,0) on a miss)
 };
 
+// Occlusion launch (tcrt_hits.cu, tcrt_occluded_rays / tcrt_occluded_lights): the shadow test of inShadeCollisionDetection
+// for rl.list_n items.  Out of rl the kernel uses the scene, queue, counters[1] (tests traced), ray_invalid (invalid rays or
+// pairs) and n_objects.  Rays mode (points == nullptr): item q is ray q of rl's ray fields (render ray mode) with limit
+// tmax[q], answered in out[q].  Points mode: item q is the point points[3q..3q+2], tested against every light l of the
+// scene along the reference's inShade construction, answered in out[q * n_lights + l].  An answer is 1 (occluded), 0, or
+// 0xFF for an invalid ray or pair.
+struct OccLaunch {
+    RenderLaunch rl;
+    const float* tmax;
+    const float* points;
+    unsigned char* out;
+};
+
 // host builder of the box clusters (tcrt_cluster.cpp).  Face f = 2*axis + k; an absent face has
 // c = NaN and plane = -1; `plane` indexes the caller's list.
 struct TcrtBoxCluster {
@@ -192,6 +205,8 @@ cudaError_t tcrt_launch_div3_check(unsigned long long n, unsigned seed, unsigned
 
 // primary-hit buffers and picks (tcrt_hits.cu): one launch, nothing when there are no pixels
 cudaError_t tcrt_launch_hits(const HitLaunch& hl, int sm_count, cudaStream_t stream);
+// occlusion queries (tcrt_hits.cu): one launch, nothing when there are no items
+cudaError_t tcrt_launch_occlusion(const OccLaunch& ol, int sm_count, cudaStream_t stream);
 
 // txt formatter (tcrt_format.cu)
 // fixed path: 31-byte lines; general path: per-pixel lengths -> two-level exclusive scan

@@ -1,4 +1,5 @@
-// tcrt_hits.cu — primary-hit buffers (tcrt_hit_buffers) and picking (tcrt_pick).
+// tcrt_hits.cu — primary-hit buffers (tcrt_hit_buffers), picking (tcrt_pick), and the ray-batch queries that need no
+// bounce loop: nearest hits (tcrt_intersect_rays) and occlusion (tcrt_occluded_rays, tcrt_occluded_lights).
 //
 // Per pixel, what the reference computes at level 0 of calculatePixel (RayTracer.cpp:448-638): the winner of
 // getCollision (:50-89), that winner's distance, and the direction of the normal ray of its CollisionObject
@@ -13,13 +14,8 @@
 
 namespace {
 
-template <int SBVH, int FM>
-__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) hits_kernel(const __grid_constant__ HitLaunch hl) {
-    extern __shared__ float4 smem4[];
-    const RenderLaunch& rl = hl.rl;
-    const DeviceScene& sc = rl.scene;
-    // ---- stage the sweep blob, as render_kernel does (the BVH-covered spheres in front of stage_off stay global) ----
-    const int stage_off = SBVH ? sc.stage_off : 0;
+// Stage the sweep blob, as render_kernel does (the BVH-covered spheres in front of stage_off stay global), and view it.
+__device__ __forceinline__ Sm stage_blob(const DeviceScene& sc, float4* smem4, int stage_off) {
     const int n_stage = sc.blob_f4 - stage_off;
     for (int i = threadIdx.x; i < n_stage; i += kBlock) smem4[i] = __ldg(sc.blob + stage_off + i);
     __syncthreads();
@@ -32,6 +28,16 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
     sm.clu = base + sc.clu_off;
     sm.cslot = reinterpret_cast<const int*>(base + sc.cslot_off);
     sm.idx = reinterpret_cast<const int*>(base + sc.idx_off);
+    return sm;
+}
+
+template <int SBVH, int FM>
+__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) hits_kernel(const __grid_constant__ HitLaunch hl) {
+    extern __shared__ float4 smem4[];
+    const RenderLaunch& rl = hl.rl;
+    const DeviceScene& sc = rl.scene;
+    const int stage_off = SBVH ? sc.stage_off : 0;
+    const Sm sm = stage_blob(sc, smem4, stage_off);
 
     const unsigned lane = threadIdx.x & 31u;
     const bool rays = rl.ray_d != nullptr;
@@ -117,6 +123,86 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
     }
 }
 
+// Occlusion queries (tcrt_occluded_rays / tcrt_occluded_lights): inShadeCollisionDetection (RayTracer.cpp:709-739) of a
+// caller's ray with its own limit, or inShade (:743-771) of a caller's point against every light.  The any-hit walk is
+// the render kernel's sweep_shadow; claims and staging are hits_kernel's.  A lane with nothing to ask (past the end, an
+// invalid ray or pair) enters the warp-synchronous walks as a lane that wants no answer.
+template <int SBVH, int FM>
+__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) occlusion_kernel(const __grid_constant__ OccLaunch ol) {
+    extern __shared__ float4 smem4[];
+    const RenderLaunch& rl = ol.rl;
+    const DeviceScene& sc = rl.scene;
+    const Sm sm = stage_blob(sc, smem4, SBVH ? sc.stage_off : 0);
+
+    const unsigned lane = threadIdx.x & 31u;
+    const bool points = ol.points != nullptr;
+    const unsigned total = (unsigned)rl.list_n;
+    unsigned n_invalid = 0, n_tests = 0;
+    for (;;) {
+        unsigned q0 = 0;
+        if (lane == 0) q0 = atomicAdd(rl.queue, 32u);
+        q0 = __shfl_sync(kFull, q0, 0);
+        if (q0 >= total) break;
+        const unsigned q = q0 + lane;
+        const bool active = q < total;
+        if (!points) {
+            // the caller's ray and limit; no shell shortcut (mask 0): the far end of the segment is not a light
+            V3 O = mk(0.f, 0.f, 0.f), D = mk(1.f, 0.f, 0.f);
+            float tmax = 1.0f;
+            bool want = false;
+            if (active) {
+                const float t = __ldg(ol.tmax + q);
+                want = ray_from_batch(rl, (int)q, O, D) && t > 0.0f;   // NaN and t <= 0 fail
+                if (want) tmax = t;
+                else ol.out[q] = 0xFF;
+            }
+            const bool occl = sweep_shadow<SBVH, FM>(sm, sc, O, D, tmax, 0u, !want);
+            if (want) ol.out[q] = occl ? 1 : 0;
+            n_tests += want ? 1u : 0u;
+            n_invalid += (active && !want) ? 1u : 0u;
+        } else {
+            // the point: the origin rule of ray batches
+            V3 P = mk(0.f, 0.f, 0.f);
+            bool ok = false;
+            if (active) {
+                const float* pp = ol.points + 3 * (size_t)q;
+                P = mk(__ldg(pp), __ldg(pp + 1), __ldg(pp + 2));
+                const float big = 1099511627776.0f;   // 2^40; NaN fails
+                ok = fabsf(P.x) <= big && fabsf(P.y) <= big && fabsf(P.z) <= big;
+                if (!ok) P = mk(0.f, 0.f, 0.f);
+            }
+            for (int l = 0; l < sc.n_lights; ++l) {   // warp-uniform: the light's shell mask is the warp's
+                const float4 lp = sm.light[2 * l];
+                const float4 lc = sm.light[2 * l + 1];
+                // inShade (:743-752), as the render kernel's light loop builds it: dir = L - P, |dir|, Ray(P, dir)
+                // normalises with the same length
+                const V3 dir = xyz(lp) - P;
+                const float dist = __fsqrt_rn(dir.x * dir.x + dir.y * dir.y + dir.z * dir.z);
+                const V3 lr = div3(dir, dist);
+                // the direction rule of ray batches; fails only within ~1e-19 of the light (0/0 at it)
+                const float s = __fadd_rn(__fadd_rn(__fmul_rn(lr.x, lr.x), __fmul_rn(lr.y, lr.y)), __fmul_rn(lr.z, lr.z));
+                const bool want = ok && fabsf(s - 1.0f) <= 4.76837158203125e-07f;
+                const bool occl = sweep_shadow<SBVH, FM>(sm, sc, P, lr, dist, __float_as_uint(lc.w), !want);
+                if (active) ol.out[(size_t)q * (unsigned)sc.n_lights + l] = want ? (occl ? 1 : 0) : 0xFF;
+                n_tests += want ? 1u : 0u;
+                n_invalid += (active && !want) ? 1u : 0u;
+            }
+        }
+    }
+    const unsigned t = __reduce_add_sync(kFull, n_tests);
+    const unsigned n = __reduce_add_sync(kFull, n_invalid);
+    if (lane == 0 && t != 0) atomicAdd(rl.counters + 1, (unsigned long long)t);
+    if (lane == 0 && n != 0) atomicAdd(rl.ray_invalid, (unsigned long long)n);
+}
+
+template <int SBVH, int FM>
+cudaError_t launch_occlusion_one(const OccLaunch& ol, int grid, size_t smem, cudaStream_t stream) {
+    cudaError_t e = cudaFuncSetAttribute(occlusion_kernel<SBVH, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    occlusion_kernel<SBVH, FM><<<grid, kBlock, smem, stream>>>(ol);
+    return cudaGetLastError();
+}
+
 template <int SBVH, int FM>
 cudaError_t launch_hits_one(const HitLaunch& hl, int grid, size_t smem, cudaStream_t stream) {
     cudaError_t e = cudaFuncSetAttribute(hits_kernel<SBVH, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -140,25 +226,50 @@ extern "C" int tcrt_dev_hits_check_flags(unsigned int* flags, int reset) {
 }
 #endif
 
-cudaError_t tcrt_launch_hits(const HitLaunch& hl_in, int sm_count, cudaStream_t stream) {
-    HitLaunch hl = hl_in;
-    RenderLaunch& rl = hl.rl;
-    const size_t smem = (size_t)std::max(1, rl.scene.blob_f4 - rl.scene.stage_off) * sizeof(float4);
-    if (smem > tcrt_render_max_smem()) return cudaErrorInvalidValue;
-    const unsigned total = rl.ray_d != nullptr ? (unsigned)rl.list_n
-                           : hl.xz != nullptr ? (unsigned)hl.n_list : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
-    if (total == 0) return cudaSuccess;
-    // persistent grid, sized as tcrt_launch_render sizes the render kernel's, but no more CTAs than there are claims
+// The launch shape of the hit and occlusion kernels: staged bytes, a persistent grid sized as tcrt_launch_render sizes the
+// render kernel's but with no more CTAs than `total` items need, and the dispatch class.  false: the blob does not fit.
+static bool launch_shape(const RenderLaunch& rl, unsigned total, int sm_count, size_t& smem, int& grid, int& sb, int& fm) {
+    smem = (size_t)std::max(1, rl.scene.blob_f4 - rl.scene.stage_off) * sizeof(float4);
+    if (smem > tcrt_render_max_smem()) return false;
     int ctas_per_sm = (rl.scene.bvh_sph != nullptr && rl.scene.n_fin == 0) ? kMinBlocksBvh : kMinBlocks;
     while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;
     const long long need = ((long long)total + kBlock - 1) / kBlock;
-    const int grid = (int)std::min<long long>((long long)sm_count * ctas_per_sm, need);
+    grid = (int)std::min<long long>((long long)sm_count * ctas_per_sm, need);
+    sb = rl.scene.bvh_sph == nullptr ? 0 : 1;
+    fm = rl.scene.bvh_fin != nullptr ? 2 : (rl.scene.n_fin == 0 ? 0 : (rl.scene.n_clu > 0 ? 1 : 3));
+    return true;
+}
+
+cudaError_t tcrt_launch_hits(const HitLaunch& hl_in, int sm_count, cudaStream_t stream) {
+    HitLaunch hl = hl_in;
+    RenderLaunch& rl = hl.rl;
+    const unsigned total = rl.ray_d != nullptr ? (unsigned)rl.list_n
+                           : hl.xz != nullptr ? (unsigned)hl.n_list : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    size_t smem;
+    int grid, sb, fm;
+    if (!launch_shape(rl, total, sm_count, smem, grid, sb, fm)) return cudaErrorInvalidValue;
+    if (total == 0) return cudaSuccess;
     rl.tiled = (hl.xz == nullptr && rl.ray_d == nullptr && (rl.x1 - rl.x0) % TCRT_TILE_W == 0 && rl.height % TCRT_TILE_H == 0) ? 1 : 0;
     rl.row_order = nullptr;
-    const int sb = rl.scene.bvh_sph == nullptr ? 0 : 1;
-    const int fm = rl.scene.bvh_fin != nullptr ? 2 : (rl.scene.n_fin == 0 ? 0 : (rl.scene.n_clu > 0 ? 1 : 3));
 #define TCRT_CASE(SB, FMV) \
     if (sb == SB && fm == FMV) return launch_hits_one<SB, FMV>(hl, grid, smem, stream);
+    TCRT_CASE(0, 0) TCRT_CASE(0, 1) TCRT_CASE(0, 2) TCRT_CASE(0, 3)
+    TCRT_CASE(1, 0) TCRT_CASE(1, 1) TCRT_CASE(1, 2) TCRT_CASE(1, 3)
+#undef TCRT_CASE
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t tcrt_launch_occlusion(const OccLaunch& ol_in, int sm_count, cudaStream_t stream) {
+    OccLaunch ol = ol_in;
+    const unsigned total = (unsigned)ol.rl.list_n;
+    size_t smem;
+    int grid, sb, fm;
+    if (!launch_shape(ol.rl, total, sm_count, smem, grid, sb, fm)) return cudaErrorInvalidValue;
+    if (total == 0) return cudaSuccess;
+    ol.rl.tiled = 0;
+    ol.rl.row_order = nullptr;
+#define TCRT_CASE(SB, FMV) \
+    if (sb == SB && fm == FMV) return launch_occlusion_one<SB, FMV>(ol, grid, smem, stream);
     TCRT_CASE(0, 0) TCRT_CASE(0, 1) TCRT_CASE(0, 2) TCRT_CASE(0, 3)
     TCRT_CASE(1, 0) TCRT_CASE(1, 1) TCRT_CASE(1, 2) TCRT_CASE(1, 3)
 #undef TCRT_CASE

@@ -5,7 +5,9 @@ every frame with the oracle bit for bit, and reports the check flags (0 = nothin
 dispatch class of tests/test_kernel_variants.py at the boundary depths of each level stack: band kernels (a tiled and an
 untiled frame, a band from an odd column), list kernels (adaptive frames refining every pixel) and hit kernels.  The
 flags are read from each translation unit that launches a kernel: render, grid and hits.  Last, a ray batch of valid and
-invalid rays on a grid scene and a BVH scene, traced and intersected, against tests/oracle_rays.c.
+invalid rays on a grid scene and a BVH scene, traced and intersected, against tests/oracle_rays.c, and the occlusion queries
+(points against every light, rays with their limits) on a grid scene, BVH scenes and box-cluster scenes against
+tests/oracle_occlusion.c.
 usage: python -c "from tilecoderaytracer_b200 import build; build.build_lib(defines=('TCRT_CHECKED',), out=LIB)"
        TCRT_LIB=LIB python tools/checked_run.py"""
 import ctypes as C
@@ -155,4 +157,44 @@ with tempfile.TemporaryDirectory() as tmp:
         bad_total += bad + len(f)
         print(f"ray batch {name:9s} {len(o)} rays ({int((~valid).sum())} invalid), d0/8/50: mismatches {bad}, "
               f"checks fired: {f or 'none'}", flush=True)
+
+# ---- occlusion queries: points against every light and rays with their limits, through the occlusion kernel ---------------
+import test_occlusion as Q  # noqa: E402
+
+with tempfile.TemporaryDirectory() as tmp:
+    so = os.path.join(tmp, "liboracle_occlusion.so")
+    subprocess.run(["gcc", "-std=gnu11", "-O2", "-fPIC", "-shared", "-ffp-contract=off", os.path.join(ROOT, "tests", "oracle_occlusion.c"),
+                    "-o", so, "-lm"], check=True)
+    ql = C.CDLL(so)
+    ull = C.POINTER(C.c_ulonglong)
+    ql.tcrt_oracle_occluded_rays.restype = ql.tcrt_oracle_occluded_lights.restype = ql.tcrt_oracle_shadow_origins.restype = C.c_int
+    ql.tcrt_oracle_occluded_rays.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, ull, ull]
+    ql.tcrt_oracle_occluded_lights.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, ull, ull]
+    ql.tcrt_oracle_shadow_origins.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+    for name, want_cls in (("synth256", ("grid", 1, 0)), ("random:24:200", ("render", 1, 2)), ("boxes:3:14", ("render", 0, 2)),
+                           ("default", ("render", 0, 1)), ("sb1_fm1", ("render", 1, 1))):
+        if name in V.VARIANTS:
+            sc, cam = V.build(name)
+        else:
+            cam = api.Camera()
+            sc = api.Scene().build(name, cam)
+        flat, c = sc.flatten(), cam.export()
+        ctx.upload_flat(flat, c)
+        bad = int(V.dispatch_class(ctx.scene_structures()) != want_cls)
+        rng = np.random.default_rng(5)
+        pts = Q.scene_points(ctx, ql, flat, c, rng)
+        o, d, t, _, _ = Q.scene_rays(ctx, ql, flat, c, rng)
+        o = np.concatenate([o, ox])
+        d = np.concatenate([d, dx])
+        t = np.concatenate([t, np.full(len(ox), np.float32(np.nan))])
+        got, g_bad, st = ctx.occluded_lights(pts)
+        want, w_bad, w_tests = Q.oracle_lights(ql, flat, pts)
+        bad += int((got != want).any(-1).sum()) + int(g_bad != w_bad) + int(st.rays_shadow != w_tests)
+        got, g_bad, st = ctx.occluded_rays(o, d, t)
+        want, w_bad, w_tests = Q.oracle_rays(ql, flat, o, d, t)
+        bad += int((got != want).sum()) + int(g_bad != w_bad) + int(st.rays_shadow != w_tests)
+        f = fired()
+        bad_total += bad + len(f)
+        print(f"occlusion {name:14s} {str(want_cls):16s} {len(pts)} points x {flat.n_lights} lights, {len(o)} rays: "
+              f"mismatches {bad}, checks fired: {f or 'none'}", flush=True)
 print("CHECKED_OK" if bad_total == 0 else "CHECKED_FAIL")

@@ -124,7 +124,10 @@ typedef struct tcrt_params {
     int shadows_on;     /* SHADOWS_ON */
     int reflections_on; /* REFLECTIONS_ON */
     float null_color[3];/* NULL_COLOR (0.75,0.75,0.75): miss / recursion cap */
-    float far_dist;     /* FLOAT_MAX_VALUE 65535: hits at or beyond are invisible */
+    float far_dist;     /* FLOAT_MAX_VALUE 65535: hits at or beyond are invisible.  Any value is
+                         * accepted and rendered like the reference: +inf sees every hit; at
+                         * far_dist <= 0 only a sphere around the ray's origin (its distance is
+                         * negative) can still be hit; -inf and NaN hide everything. */
 } tcrt_params;
 
 /* Fills the reference's shipped values: 500x504, depth 50, shadows+reflections on,

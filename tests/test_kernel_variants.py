@@ -140,8 +140,63 @@ def _spheres(s, centres, radius):
             .setReflectiveFactor(1.0).setDiffuseFactor(.3).setSpecularFactor(.6)
 
 
-def _scene(enclosure, spheres, big):
-    s = api.Scene()
+class _PlacedRef:
+    """A SceneObjectRef of a placed scene: a checkerboard's cell width and height are lengths."""
+
+    def __init__(self, ref, scale):
+        self._ref, self._scale = ref, scale
+
+    def __getattr__(self, name):
+        return getattr(self._ref, name)
+
+    def setCheckerBoard(self, light, dark, width, height):
+        self._ref.setCheckerBoard(light, dark, width * self._scale, height * self._scale)
+        return self
+
+
+class Placed:
+    """An api.Scene built with every point x mapped to scale * x + shift (in double, rounded once to float by the API):
+    radii, box dimensions and checker cells are multiplied by scale; normal and horizontal vectors stay.  It has the
+    Scene calls the builders use."""
+
+    def __init__(self, scene, scale, shift):
+        self.scene, self.scale, self.shift = scene, float(scale), np.asarray(shift, float)
+
+    def point(self, v):
+        return _pt(self.scale * np.asarray(v, float) + self.shift)
+
+    def _ref(self, ref):
+        return _PlacedRef(ref, self.scale)
+
+    def addSphere(self, origin, radius):
+        return self._ref(self.scene.addSphere(self.point(origin), radius * self.scale))
+
+    def addInfinitePlane(self, origin, normal, horizontal):
+        return self._ref(self.scene.addInfinitePlane(self.point(origin), normal, horizontal))
+
+    def addFinitePlaneCorners(self, origin, vertical_corner, horizontal_corner):
+        return self._ref(self.scene.addFinitePlaneCorners(self.point(origin), self.point(vertical_corner),
+                                                          self.point(horizontal_corner)))
+
+    def makeSceneBox(self, origin, dims):
+        return [self._ref(r) for r in self.scene.makeSceneBox(self.point(origin), _pt(self.scale * np.asarray(dims, float)))]
+
+    def camera(self, cam):
+        """The exported camera of `cam` under the same map."""
+        c = cam.export()
+        for name in ("eye", "screen_origin"):
+            v = self.point(getattr(c, name)[:])
+            for k in range(3):
+                getattr(c, name)[k] = v[k]
+        for name in ("screen_width", "screen_height", "screen_halfwidth", "screen_halfheight"):
+            setattr(c, name, getattr(c, name) * self.scale)
+        return c
+
+
+def _scene(enclosure, spheres, big, place=None):
+    """(Scene, Camera) of a builder; with place = (scale, shift): (Scene, exported camera) of it placed by Placed."""
+    scene = api.Scene()
+    s = scene if place is None else Placed(scene, *place)
     _lights(s, enclosure)
     if enclosure == "infinite":
         _infinite_faces(s)
@@ -155,7 +210,9 @@ def _scene(enclosure, spheres, big):
         _spheres(s, LATTICE, .3)
     if big:
         _spheres(s, [BIG[0]], BIG[1])
-    return s, api.Camera()
+    if place is None:
+        return scene, api.Camera()
+    return scene, s.camera(api.Camera())
 
 
 # name -> (enclosure, spheres, one big sphere, the class the dispatcher must pick).  A class is ("render", SBVH, FM) for
@@ -176,10 +233,11 @@ VARIANTS = {
 NAMES = list(VARIANTS)
 
 
-def build(name):
-    """(Scene, Camera) of a variant; keep the Scene alive while its flatten() is in use."""
+def build(name, place=None):
+    """(Scene, Camera) of a variant, or (Scene, exported camera) placed at place = (scale, shift); keep the Scene alive
+    while its flatten() is in use."""
     enclosure, spheres, big, _ = VARIANTS[name]
-    return _scene(enclosure, spheres, big)
+    return _scene(enclosure, spheres, big, place)
 
 
 def dispatch_class(st):

@@ -191,7 +191,9 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                 const float tn = fmaxf(fmaxf(fminf(ax, bx), fminf(ay, by)), fminf(az, bz));
                 const float tf = fminf(fminf(fmaxf(ax, bx), fmaxf(ay, by)), fmaxf(az, bz));
                 const float t0 = fmaxf(tn, 0.0f);
-                walking = walking && (tf >= t0) && (t0 <= best);
+                // a far_dist <= 0 (or NaN) still lets a sphere around the origin win with its negative distance: that
+                // sphere is registered in the origin's cell, the first one visited, and the exit test stops after it
+                walking = walking && (tf >= t0) && (t0 <= fmaxf(best, 0.0f));
                 int cx = 0, cy = 0, cz = 0;
                 float tmx = 0.f, tmy = 0.f, tmz = 0.f;
                 const float dtx = sc.grid_cell[0] * fabsf(ix), dty = sc.grid_cell[1] * fabsf(iy), dtz = sc.grid_cell[2] * fabsf(iz);

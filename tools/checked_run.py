@@ -118,6 +118,35 @@ with tempfile.TemporaryDirectory() as tmp:
         bad_total += bad + len(f)
         print(f"{name:9s} hit buffers 27x17: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
 
+# ---- the placed scenes of tests/test_scene_placement.py: every class moved and rescaled, the lattices at the grid's tightest
+# offset, and every far_dist on the grid scene with the camera inside a sphere ---------------------------------------------------
+import test_scene_placement as P  # noqa: E402
+
+for pid, name in P.CASES:
+    s, flat, c = P.build_placed(pid, name)
+    ctx.upload_flat(flat, c)
+    bad = int(V.dispatch_class(ctx.scene_structures()) != P.expected_class(pid, name))
+    for d in P.DEPTHS:
+        p = P.placed_params(pid, name, *P.frame_size(d), d)
+        img, st = ctx.render(p)
+        ref, cnt = O.render(flat, c, p)
+        bad += n_bad(img, ref) + counters_differ(st, cnt)
+    f = fired()
+    bad_total += bad + len(f)
+    print(f"placed {pid:12s} {name:9s} d{P.DEPTHS}: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
+s, c = P.inside_sphere_scene()
+flat = s.flatten()
+ctx.upload_flat(flat, c)
+bad = 0
+for far in P.FAR_DISTS:
+    p = P.far_params(32, 24, 4, far)
+    img, st = ctx.render(p)
+    ref, cnt = O.render(flat, c, p)
+    bad += n_bad(img, ref) + counters_differ(st, cnt)
+f = fired()
+bad_total += bad + len(f)
+print(f"inside_sphere at {len(P.FAR_DISTS)} far_dist values: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
+
 # ---- ray batches: valid and invalid rays mixed, through the render / grid kernels' ray mode and the hit kernel's -----------
 import test_ray_batches as R  # noqa: E402
 

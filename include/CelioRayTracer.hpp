@@ -236,11 +236,14 @@ public:
     sdecimal32 getScreenWidth() const { return screen_width; }
     sdecimal32 getScreeHeight() const { return screen_height; }
     void setSceneTwoMirrors();                  // Camera.cpp:42-69
+    // the pose arithmetic of Camera.cpp:22-38: screen centre so, screen x axis horiz, view direction outward (neither
+    // normalised); vertical = horiz x outward, all three normalised, the eye one unit behind the screen.  The screen size
+    // is kept (another field of view: edit the exported tcrt_camera's screen_* fields, halfwidth = width / 2).
+    void aim(vector3d so, vector3d horiz, vector3d outward);
     // what the kernels read for primary-ray generation
     void exportTo(tcrt_camera* out) const;
 
 private:
-    void aim(vector3d so, vector3d horiz, vector3d outward);
     sdecimal32 screen_width, screen_height, screen_halfwidth, screen_halfheight;
     vector3d screen_origin, vector_outwards, vector_vertical, vector_horizontal;
     sdecimal32 eye_distance;

@@ -137,6 +137,18 @@ public:
         }
         return rc_ = tcrt_occluded_lights(ctx_, points.size(), p.data(), occluded, n_invalid, stats);
     }
+    // the scene from every camera of `cameras` in one call (tcrt_render_views): view v is exactly render(rs, ...) after
+    // the scene's camera is set to cameras[v], stacked view-major, rgb[((v*W + x)*H + z)*3 + c]; rgb8 (may be NULL, and
+    // rgb may be NULL when it is not) the same quantised to 8 bits.  The last render and the scene's camera are not
+    // touched.  Not for rs.samples != 1.
+    int renderViews(const RenderSettings& rs, const std::vector<Camera>& cameras, float* rgb, unsigned char* rgb8 = NULL,
+                    tcrt_stats* stats = NULL) {
+        if (rs.samples != 1) return rc_ = TCRT_ERR_UNSUPPORTED;
+        std::vector<tcrt_camera> c(cameras.size());
+        for (size_t i = 0; i < cameras.size(); i++) cameras[i].exportTo(&c[i]);
+        tcrt_params p = rs.params();
+        return rc_ = tcrt_render_views(ctx_, &p, (int)cameras.size(), c.data(), rgb, rgb8, stats);
+    }
     // init_log + printPixelsToLog (RayTracer.cpp:2022-2061,1574-1626)
     int printPixelsToLog(const char* path = LOG_FILE_NAME) {
         tcrt_params p = settings_.params();

@@ -105,7 +105,9 @@ typedef struct tcrt_scene {
     const float* textures;
 } tcrt_scene;
 
-/* Camera (Camera.h:20-39, Camera.cpp:9-40): everything createEyeRay (Camera.cpp:71-84) reads. */
+/* Camera (Camera.h:20-39, Camera.cpp:9-40): everything createEyeRay (Camera.cpp:71-84) reads.  A pose is built the
+ * reference's way by Camera::aim (tcrt_hcamera_aim); another field of view is an edit of the four screen_* fields, with
+ * screen_halfwidth = screen_width / 2 and screen_halfheight = screen_height / 2 as the reference sets them. */
 typedef struct tcrt_camera {
     float eye[3];           /* eye_origin */
     float screen_origin[3];
@@ -393,6 +395,37 @@ int tcrt_occluded_rays_device(tcrt_ctx* ctx, int device_slot, size_t n, const fl
                               unsigned long long* n_invalid, tcrt_stats* stats);
 int tcrt_occluded_lights_device(tcrt_ctx* ctx, int device_slot, size_t n, const float* points, unsigned char* occluded,
                                 unsigned long long* n_invalid, tcrt_stats* stats);
+/* Multi-view frames: one scene seen from a batch of cameras in one call (stereo pairs, cube-map faces, turntables,
+ * thumbnails).  View v is exactly the frame tcrt_render returns for params after tcrt_set_camera(ctx, &cameras[v]), bit
+ * for bit, every pixel: NaN payloads of degenerate cameras, every far_dist, switch and depth the frame path accepts.
+ * cameras is host memory, n_views of them; no camera is validated, as with tcrt_set_camera.
+ * Layout: the views are stacked view-major, each x-major like frames: rgb[((v*W + x)*H + z)*3 + c].  Equivalently the
+ * stack is the x-major array of one (n_views*W) x H frame whose global column v*W + x is column x of view v.  rgb8 holds
+ * q(c) of the same floats (the quant8 of the 8-bit frames above) in the same order.  Either output may be NULL, not both.
+ * The image rows (top row first) of view v are a[v].transpose(1, 0, 2)[::-1].
+ * The ctx camera is neither read nor changed.  Like the ray batches, the call has buffers, queue heads and events of its
+ * own: it never changes the last render (tcrt_download, tcrt_device_frame, the writers), the multi-device cut or cost map,
+ * or a frame in flight, may run while two frames are in flight and does not count as one.  It is queued on the render
+ * stream behind whatever is there (so it sees a scene uploaded just before it) and is synchronous.
+ * The camera table (64 B per view) is copied to each device once per call.  The global columns run in pieces of at most
+ * 4 Mi pixels, whole columns, on multiples of 4 columns when W % 4 == 0, round robin over the render streams; each piece
+ * is one launch (4x8-pixel tiles when its width is a multiple of 4 and H of 8), plus one quantisation launch for rgb8,
+ * and its outputs are copied out while later pieces render.  Supersampled and adaptive views and per-view hit buffers do
+ * not exist.
+ * Host form (tcrt_render_views): pinned or pageable destinations, identical results.  A multi-device ctx splits the
+ * global columns [0, n_views*W) into equal contiguous ranges, cut on multiples of 4 when W % 4 == 0.
+ * Device form (_device): one device slot; every non-NULL output must be device memory of that slot's device, else
+ * TCRT_ERR_INVALID.
+ * n_views = 0 succeeds and launches nothing.  Errors: NULL ctx or params, NULL cameras with n_views > 0, both outputs
+ * NULL, n_views < 0 or bad params: TCRT_ERR_INVALID; max_depth above TCRT_MAX_DEPTH, or n_views*W above INT_MAX:
+ * TCRT_ERR_UNSUPPORTED; before tcrt_upload_scene: TCRT_ERR_NO_SCENE.
+ * Stats: col_begin/col_end each device's range of global columns; rays_* as for frames, summed over the views; render_ms
+ * from the first launch to the end of the last one; d2h_ms the copy time not hidden behind the launches; gpu_launches
+ * every launch, the quantisation launches included. */
+int tcrt_render_views(tcrt_ctx* ctx, const tcrt_params* params, int n_views, const tcrt_camera* cameras, float* rgb,
+                      unsigned char* rgb8, tcrt_stats* stats);
+int tcrt_render_views_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* params, int n_views,
+                             const tcrt_camera* cameras, float* rgb, unsigned char* rgb8, tcrt_stats* stats);
 /* Cost-balanced column bands (replaces the equal z-bands of the reference's strategy 1,
  * RayTracer.cpp:904-906, whose load imbalance strategies 2-7 and PixelQueue were written to fix).
  * Renders a low-resolution copy of the frame on device slot 0 in which every finished pixel adds its

@@ -21,6 +21,10 @@ void tcrt_hscene_free(tcrt_hscene* s);
 tcrt_hcamera* tcrt_hcamera_new(void);                              /* Camera::Camera() */
 void tcrt_hcamera_free(tcrt_hcamera* c);
 void tcrt_hcamera_set_two_mirrors(tcrt_hcamera* c);                /* Camera::setSceneTwoMirrors() */
+/* Camera::aim: the reference's pose arithmetic (Camera.cpp:22-38) for the screen centre screen_origin3, the screen's x
+ * axis horizontal3 and the viewing direction outwards3 (neither need be normalised): vertical = horizontal x outwards,
+ * then all three normalised, the eye one unit behind the screen.  The screen size is kept. */
+void tcrt_hcamera_aim(tcrt_hcamera* c, const float* screen_origin3, const float* horizontal3, const float* outwards3);
 void tcrt_hcamera_export(const tcrt_hcamera* c, tcrt_camera* out);
 /* Camera::createEyeRay(dx, dy): origin and normalised direction */
 void tcrt_hcamera_eye_ray(const tcrt_hcamera* c, float dx_percent, float dy_percent, float* origin3, float* dir3);

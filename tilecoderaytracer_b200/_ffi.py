@@ -133,6 +133,10 @@ SIGNATURES = {
                                             C.c_void_p, C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
     "tcrt_occluded_lights_device": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p,
                                               C.POINTER(C.c_ulonglong), C.POINTER(TcrtStats)]),
+    "tcrt_render_views": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.POINTER(TcrtStats)]),
+    "tcrt_render_views_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(TcrtParams), C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.POINTER(TcrtStats)]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),
     "tcrt_bands_from_costs": (C.c_int, [C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),
@@ -158,6 +162,7 @@ SIGNATURES = {
     "tcrt_hcamera_set_two_mirrors": (None, [C.c_void_p]),
     "tcrt_hcamera_export": (None, [C.c_void_p, C.POINTER(TcrtCamera)]),
     "tcrt_hcamera_eye_ray": (None, [C.c_void_p, C.c_float, C.c_float, c_float_p, c_float_p]),
+    "tcrt_hcamera_aim": (None, [C.c_void_p, c_float_p, c_float_p, c_float_p]),
     "tcrt_hscene_build": (C.c_int, [C.c_void_p, C.c_void_p, C.c_char_p]),
     "tcrt_hscene_load_text": (C.c_int, [C.c_void_p, C.c_void_p, C.c_char_p, C.c_char_p, C.c_size_t]),
     "tcrt_hscene_add_sphere": (C.c_int, [C.c_void_p, c_float_p, C.c_float]),

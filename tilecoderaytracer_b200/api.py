@@ -40,6 +40,15 @@ class Camera:
     def setSceneTwoMirrors(self) -> None:
         self._lib.tcrt_hcamera_set_two_mirrors(self._h)
 
+    def aim(self, screen_origin: Sequence[float], horizontal: Sequence[float], outwards: Sequence[float]) -> "Camera":
+        """Camera::aim, the reference's pose arithmetic (Camera.cpp:22-38): the screen's centre at screen_origin, its
+        x axis along horizontal, the view along outwards, vertical = horizontal x outwards (before either is
+        normalised), then all three normalised and the eye one unit behind the screen.  The screen size is kept; for
+        another field of view edit screen_width / screen_height of export() with halfwidth = width / 2 and halfheight =
+        height / 2, as the reference sets them.  Returns self."""
+        self._lib.tcrt_hcamera_aim(self._h, _f3(screen_origin), _f3(horizontal), _f3(outwards))
+        return self
+
     def createEyeRay(self, dx_percent: float, dy_percent: float):
         o = (C.c_float * 3)()
         d = (C.c_float * 3)()
@@ -50,6 +59,14 @@ class Camera:
         cam = TcrtCamera()
         self._lib.tcrt_hcamera_export(self._h, C.byref(cam))
         return cam
+
+
+def _camera_table(cameras) -> C.Array:
+    """A contiguous tcrt_camera array of Camera objects and / or TcrtCamera structs."""
+    cams = [c.export() if isinstance(c, Camera) else c for c in cameras]
+    for c in cams:
+        assert isinstance(c, TcrtCamera), "cameras: Camera or TcrtCamera"
+    return (TcrtCamera * len(cams))(*cams)
 
 
 class SceneObjectRef:
@@ -560,6 +577,42 @@ class Context:
                                                d.ctypes.data_as(C.c_void_p), *ptrs, C.byref(bad), C.byref(st)))
         res = {name: out[name].reshape((n,) + tail) for name, _, tail in self.HIT_BUFFERS if out.get(name) is not None}
         return res, int(bad.value), RenderStats.from_c(st)
+
+    def render_views(self, params: TcrtParams, cameras, out: Optional[np.ndarray] = None):
+        """One scene from a batch of cameras (tcrt_render_views): view v is exactly render(params) after
+        set_camera(cameras[v]).  cameras: a sequence of Camera or TcrtCamera.  Returns ((V, W, H, 3) float32, RenderStats);
+        the stack is x-major like frames, image rows of view v are a[v].transpose(1, 0, 2)[::-1].  `out` may be pinned or
+        pageable.  The ctx camera, the last render and frames in flight are untouched."""
+        cams = _camera_table(cameras)
+        V, W, H = len(cams), params.width, params.height
+        if out is None:
+            out = np.empty((V, W, H, 3), np.float32)
+        assert out.dtype == np.float32 and out.size == V * W * H * 3 and out.flags["C_CONTIGUOUS"], "out: (V, W, H, 3) float32"
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_views(self._h, C.byref(params), V, C.cast(cams, C.c_void_p),
+                                             out.ctypes.data_as(C.c_void_p), None, C.byref(st)))
+        return out.reshape(V, W, H, 3), RenderStats.from_c(st)
+
+    def render_views_rgb8(self, params: TcrtParams, cameras, out: Optional[np.ndarray] = None):
+        """render_views() quantised on the GPU (tcrt.h's q(c)): ((V, W, H, 3) uint8, RenderStats)."""
+        cams = _camera_table(cameras)
+        V, W, H = len(cams), params.width, params.height
+        if out is None:
+            out = np.empty((V, W, H, 3), np.uint8)
+        assert out.dtype == np.uint8 and out.size == V * W * H * 3 and out.flags["C_CONTIGUOUS"], "out: (V, W, H, 3) uint8"
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_views(self._h, C.byref(params), V, C.cast(cams, C.c_void_p), None,
+                                             out.ctypes.data_as(C.c_void_p), C.byref(st)))
+        return out.reshape(V, W, H, 3), RenderStats.from_c(st)
+
+    def render_views_device(self, params: TcrtParams, cameras, rgb: int = 0, rgb8: int = 0, slot: int = 0) -> RenderStats:
+        """render_views on device `slot` into device addresses (e.g. torch CUDA tensors' data_ptr()): rgb V*W*H*3 floats,
+        rgb8 V*W*H*3 bytes; 0 leaves an output out (not both).  Returns RenderStats."""
+        cams = _camera_table(cameras)
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_render_views_device(self._h, slot, C.byref(params), len(cams), C.cast(cams, C.c_void_p),
+                                                    C.c_void_p(rgb or None), C.c_void_p(rgb8 or None), C.byref(st)))
+        return RenderStats.from_c(st)
 
     def trace_rays_device(self, params: TcrtParams, n: int, origins: int, directions: int, rgb: int,
                           shared_origin: bool = False, slot: int = 0):

@@ -32,6 +32,9 @@ void tcrt_hscene_free(tcrt_hscene* s) {
 tcrt_hcamera* tcrt_hcamera_new(void) { return new tcrt_hcamera(); }
 void tcrt_hcamera_free(tcrt_hcamera* c) { delete c; }
 void tcrt_hcamera_set_two_mirrors(tcrt_hcamera* c) { if (c) c->cam.setSceneTwoMirrors(); }
+void tcrt_hcamera_aim(tcrt_hcamera* c, const float* so, const float* h, const float* o) {
+    if (c && so && h && o) c->cam.aim(v3(so), v3(h), v3(o));
+}
 void tcrt_hcamera_export(const tcrt_hcamera* c, tcrt_camera* out) { if (c && out) c->cam.exportTo(out); }
 void tcrt_hcamera_eye_ray(const tcrt_hcamera* c, float dx, float dy, float* o3, float* d3) {
     Ray* r = c->cam.createEyeRay(dx, dy);

@@ -138,6 +138,10 @@ struct DeviceState {
     cudaEvent_t ev_rk[kChunkStreams] = {};         // stream si's last piece has been traced
     cudaEvent_t ev_rin[kChunkStreams] = {};        // stream si's input staging has been copied to the device
     cudaEvent_t ev_rout[kChunkStreams] = {};       // stream si's output scratch has been copied out
+    // multi-view frames (tcrt_render_views): the call's camera table, copied in once per call; the pieces use the ray
+    // batches' scratch, queue heads, counters and events above
+    tcrt_camera* view_cams = nullptr;
+    size_t view_cams_cap = 0;                      // cameras
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -283,6 +287,7 @@ void free_device(DeviceState& d) {
     }
     cudaFree(d.ray_ctl);
     cudaFreeHost(d.h_ray);
+    cudaFree(d.view_cams);
     for (cudaEvent_t e : {d.ev_r0, d.ev_r1, d.ev_rc})
         if (e) cudaEventDestroy(e);
     cudaFreeHost(d.h_txt);
@@ -2463,8 +2468,9 @@ static bool on_device(const void* p, int dev) {
 }
 
 // What a batch computes: the colour of each ray (render kernels' ray mode), its nearest hit (hit kernel's ray mode),
-// whether it is occluded before its limit, or whether each point is occluded from each light (occlusion kernel).
-enum BatchKind { kBatchColour, kBatchHits, kBatchOccRays, kBatchOccPoints };
+// whether it is occluded before its limit, whether each point is occluded from each light (occlusion kernel), or the
+// columns of a stack of views (render kernels' views mode; an item is one global column of height pixels).
+enum BatchKind { kBatchColour, kBatchHits, kBatchOccRays, kBatchOccPoints, kBatchViews };
 
 // One batch: [0, n) split into equal contiguous ranges, one per device (device forms: slot only), each run in pieces round
 // robin over the render streams: at most kRayPiece rays, or (points) kRayPiece (point, light) pairs and at least one point.
@@ -2474,22 +2480,29 @@ enum BatchKind { kBatchColour, kBatchHits, kBatchOccRays, kBatchOccPoints };
 // launches; a stream's next piece waits for them before it reuses the scratch.  Device forms launch on the caller's buffers
 // directly.  Inputs: directions (rays) or points, origins (rays), tmax (occluded rays).  out[0] rgb (colour), object (hits)
 // or the occlusion bytes, out[1] distance, out[2] normal (hits).  p: params of the colour and hit kinds, nullptr otherwise.
+// Views: n = n_views * width global columns; the only input is the camera table `cams` (n / width cameras, copied once per
+// device to its view_cams before the first piece); out[0] rgb, out[1] rgb8, either may be nullptr.  Pieces are at most
+// kRayPiece pixels, whole columns, multiples of 4 columns when width % 4 == 0 (and the pieces hold at least 4), and so is
+// the cut between devices.  A piece is one views launch into the float scratch (device form: into rgb in place, or the
+// scratch when only rgb8 is requested), then for rgb8 one quantisation launch on the same stream.
 static int rays_impl(tcrt_ctx* ctx, int slot, BatchKind kind, const tcrt_params* p, size_t n, const float* origins,
                      int shared_origin, const float* dirs, const float* tmax, void* const out_in[3],
-                     unsigned long long* n_invalid, tcrt_stats* stats) {
+                     unsigned long long* n_invalid, tcrt_stats* stats, const tcrt_camera* cams = nullptr) {
     if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
     const bool hits = kind == kBatchHits, occ = kind == kBatchOccRays || kind == kBatchOccPoints;
-    const bool points = kind == kBatchOccPoints;
+    const bool points = kind == kBatchOccPoints, views = kind == kBatchViews;
     if (!occ && !p) return fail(ctx, TCRT_ERR_INVALID, "null params");
     const bool device_form = slot >= 0;
     if (device_form && slot >= (int)ctx->devs.size()) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", slot);
     if (kind == kBatchColour && p->max_depth < 0) return fail(ctx, TCRT_ERR_INVALID, "max_depth %d < 0", p->max_depth);
     char* out[3] = {static_cast<char*>(out_in[0]), static_cast<char*>(out_in[1]), static_cast<char*>(out_in[2])};
-    if (hits ? (!out[0] && !out[1] && !out[2]) : !out[0]) return fail(ctx, TCRT_ERR_INVALID, "no output");
-    if (n > 0 && (points ? !dirs : (!origins || !dirs || (kind == kBatchOccRays && !tmax))))
-        return fail(ctx, TCRT_ERR_INVALID, "null ray input");
+    if (hits ? (!out[0] && !out[1] && !out[2]) : views ? (!out[0] && !out[1]) : !out[0])
+        return fail(ctx, TCRT_ERR_INVALID, "no output");
+    if (n > 0 && (views ? !cams : points ? !dirs : (!origins || !dirs || (kind == kBatchOccRays && !tmax))))
+        return fail(ctx, TCRT_ERR_INVALID, views ? "null cameras" : "null ray input");
+    if (views && !valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
     if (n > SIZE_MAX / (6 * sizeof(float))) return fail(ctx, TCRT_ERR_INVALID, "%zu rays: byte count overflows", n);
-    if (kind == kBatchColour && p->max_depth > TCRT_MAX_DEPTH)
+    if ((kind == kBatchColour || views) && p->max_depth > TCRT_MAX_DEPTH)
         return fail(ctx, TCRT_ERR_UNSUPPORTED, "max_depth %d > TCRT_MAX_DEPTH %d", p->max_depth, TCRT_MAX_DEPTH);
     if (device_form && n > 0) {
         const int dev = ctx->devs[slot].dev;
@@ -2510,18 +2523,21 @@ static int rays_impl(tcrt_ctx* ctx, int slot, BatchKind kind, const tcrt_params*
     }
     const int nd = (int)ctx->devs.size();
     const int d_begin = device_form ? slot : 0, d_end = device_form ? slot + 1 : nd;
+    // views: devices and pieces are cut on multiples of 4 columns when the views' width is (whole 4x8 tiles)
+    const size_t unit = views && p->width % TCRT_TILE_W == 0 ? TCRT_TILE_W : 1;
     std::vector<size_t> cut(nd + 1, 0);
     for (int i = 0; i <= nd; i++)
-        cut[i] = device_form ? (i <= slot ? 0 : n) : n / nd * i + n % nd * i / nd;
+        cut[i] = device_form ? (i <= slot ? 0 : n) : (n / unit / nd * i + n / unit % nd * i / nd) * unit;
     // inputs, in the order of the scratch: directions or points (3 floats per item), origins (3 per item, or 3 in all when
-    // shared), tmax (1 per item)
-    const int n_in = kind == kBatchOccRays ? 3 : points ? 1 : 2;
+    // shared), tmax (1 per item); views have none (their camera table is copied once, not per piece)
+    const int n_in = views ? 0 : kind == kBatchOccRays ? 3 : points ? 1 : 2;
     const float* in_src[3] = {dirs, origins, tmax};
     auto in_words = [&](int k, size_t cnt) -> size_t { return k == 1 ? (shared_origin ? 3 : 3 * cnt) : (k == 0 ? 3 : 1) * cnt; };
     // bytes per item of each output
-    const int n_out = hits ? 3 : 1;
-    const size_t out_bytes[3] = {hits ? (size_t)4 : occ ? n_lights : (size_t)12, 4, 12};
-    const size_t item_out = out_bytes[0] + (hits ? out_bytes[1] + out_bytes[2] : 0);
+    const int n_out = hits ? 3 : views ? 2 : 1;
+    const size_t col_px = views ? (size_t)p->height : 1;   // pixels per item
+    const size_t out_bytes[3] = {hits ? (size_t)4 : occ ? n_lights : 12 * col_px, views ? 3 * col_px : 4, 12};
+    const size_t item_out = out_bytes[0] + (hits ? out_bytes[1] + out_bytes[2] : views ? out_bytes[1] : 0);
     bool staged[3] = {false, false, false}, any_direct = false;
     bool in_pageable[3] = {false, false, false}, any_pageable = false;
     if (!device_form && n > 0) {
@@ -2535,7 +2551,8 @@ static int rays_impl(tcrt_ctx* ctx, int slot, BatchKind kind, const tcrt_params*
     if (n_invalid) *n_invalid = 0;
     auto stream_of = [](DeviceState& d, int si) { return si == 0 ? d.stream : d.chunk_stream[si - 1]; };
     std::vector<int> used_streams(nd, 0), launches(nd, 0);
-    const size_t piece_items = std::max<size_t>(1, kRayPiece / std::max<size_t>(1, n_lights));
+    size_t piece_items = std::max<size_t>(1, kRayPiece / std::max<size_t>(1, n_lights) / col_px);
+    if (piece_items >= unit) piece_items -= piece_items % unit;
     for (int i = d_begin; i < d_end; i++) {
         DeviceState& d = ctx->devs[i];
         const size_t r0 = cut[i], r1 = cut[i + 1];
@@ -2559,9 +2576,17 @@ static int rays_impl(tcrt_ctx* ctx, int slot, BatchKind kind, const tcrt_params*
             if (any_pageable)
                 for (int si = 0; si < ns; si++)
                     if ((rc = ensure_pinned(ctx, d.ray_stage[si], d.ray_stage_cap[si], all_in(per)))) return rc;
+        } else if (views && !out[0]) {   // rgb8 only: the floats go to the scratch
+            for (int si = 0; si < ns; si++)
+                if ((rc = ensure(ctx, d.ray_mem[si], d.ray_mem_cap[si], per * col_px * 3))) return rc;
         }
         // on the render stream, behind whatever is queued there (a scene upload, frames in flight); the other render
         // streams start behind it
+        if (views) {
+            const size_t n_cams = n / (size_t)p->width;
+            if ((rc = ensure(ctx, d.view_cams, d.view_cams_cap, n_cams))) return rc;
+            CK(ctx, cudaMemcpyAsync(d.view_cams, cams, n_cams * sizeof(tcrt_camera), cudaMemcpyHostToDevice, d.stream));
+        }
         CK(ctx, cudaMemsetAsync(d.ray_ctl, 0, 64 * ns, d.stream));
         CK(ctx, cudaEventRecord(d.ev_r0, d.stream));
         for (int si = 1; si < ns; si++) CK(ctx, cudaStreamWaitEvent(stream_of(d, si), d.ev_r0, 0));
@@ -2650,6 +2675,17 @@ static int rays_impl(tcrt_ctx* ctx, int slot, BatchKind kind, const tcrt_params*
                     ol.points = points ? src[0] : nullptr;
                     ol.out = static_cast<unsigned char*>(dst[0]);
                     CK(ctx, tcrt_launch_occlusion(ol, d.sm_count, ks));
+                } else if (views) {
+                    // pixel (xc, z) of the piece is global column a + xc
+                    rl.x0 = (int)a;
+                    rl.x1 = (int)(a + cnt);
+                    rl.out = dst[0] ? static_cast<float*>(dst[0]) : d.ray_mem[si];
+                    rl.view_cams = d.view_cams;
+                    CK(ctx, tcrt_launch_render_views(rl, d.sm_count, ks));
+                    if (out[1]) {
+                        CK(ctx, tcrt_launch_quantize8(rl.out, cnt * col_px, static_cast<unsigned char*>(dst[1]), ks));
+                        launches[i]++;
+                    }
                 } else if (hits) {
                     HitLaunch hl{};
                     hl.rl = rl;
@@ -2765,6 +2801,35 @@ int tcrt_occluded_lights_device(tcrt_ctx* ctx, int device_slot, size_t n, const 
     if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
     void* out[3] = {occluded, nullptr, nullptr};
     return rays_impl(ctx, device_slot, kBatchOccPoints, nullptr, n, nullptr, 0, points, nullptr, out, n_invalid, stats);
+}
+
+}  // extern "C"
+
+// Multi-view frames: the n_views * width global columns of the stacked views as a batch of kind kBatchViews.
+static int views_impl(tcrt_ctx* ctx, int slot, const tcrt_params* p, int n_views, const tcrt_camera* cams, float* rgb,
+                      unsigned char* rgb8, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null ctx");
+    if (!p) return fail(ctx, TCRT_ERR_INVALID, "null params");
+    if (n_views < 0) return fail(ctx, TCRT_ERR_INVALID, "n_views %d < 0", n_views);
+    if (!valid_params(p)) return fail(ctx, TCRT_ERR_INVALID, "bad params");
+    if ((long long)n_views * p->width > INT_MAX)
+        return fail(ctx, TCRT_ERR_UNSUPPORTED, "%d views of width %d: more than INT_MAX columns", n_views, p->width);
+    void* out[3] = {rgb, rgb8, nullptr};
+    return rays_impl(ctx, slot, kBatchViews, p, (size_t)n_views * (size_t)p->width, nullptr, 0, nullptr, nullptr, out,
+                     nullptr, stats, cams);
+}
+
+extern "C" {
+
+int tcrt_render_views(tcrt_ctx* ctx, const tcrt_params* p, int n_views, const tcrt_camera* cameras, float* rgb,
+                      unsigned char* rgb8, tcrt_stats* stats) {
+    return views_impl(ctx, -1, p, n_views, cameras, rgb, rgb8, stats);
+}
+
+int tcrt_render_views_device(tcrt_ctx* ctx, int device_slot, const tcrt_params* p, int n_views, const tcrt_camera* cameras,
+                             float* rgb, unsigned char* rgb8, tcrt_stats* stats) {
+    if (device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
+    return views_impl(ctx, device_slot, p, n_views, cameras, rgb, rgb8, stats);
 }
 
 }  // extern "C"

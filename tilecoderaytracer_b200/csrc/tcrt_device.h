@@ -132,11 +132,16 @@ struct RenderLaunch {
     int ray_o_stride;        // 3, or 0: one origin shared by every ray
     const float* ray_d;
     unsigned long long* ray_invalid;
+    // views mode (tcrt_launch_render_views, multi-view frames): band mode over the global columns [x0, x1) of a stack of
+    // views, each width x height; global column g is column g % width of view g / width, whose primary rays take their
+    // camera from view_cams[g / width] instead of cam (view_ray, tcrt_render_common.cuh).  The other modes ignore it.
+    const tcrt_camera* view_cams;
 };
 
-// What a render launch traces: the pixels of a band, the samples of a pixel list, or a batch of caller-supplied rays.
-// A compile-time parameter of the render kernel bodies (one kernel per mode keeps each bounce loop in the instruction cache).
-enum RenderMode { kModeBand = 0, kModeList = 1, kModeRays = 2 };
+// What a render launch traces: the pixels of a band, the samples of a pixel list, a batch of caller-supplied rays, or the
+// pixels of a band of stacked views.  A compile-time parameter of the render kernel bodies (one kernel per mode keeps each
+// bounce loop in the instruction cache).
+enum RenderMode { kModeBand = 0, kModeList = 1, kModeRays = 2, kModeViews = 3 };
 
 // Primary-hit launch (tcrt_hits.cu): rl describes the frame, the band [x0, x1) and the scene; out of rl the kernel uses the
 // camera, width, height, x0, x1, far_dist, queue and n_objects.  Band mode (xz == nullptr): every pixel of the band, x-major
@@ -198,6 +203,9 @@ cudaError_t tcrt_launch_render_list(const RenderLaunch& rl, int sm_count, cudaSt
 // ray-mode render launch (ray batches, RenderLaunch::ray_*): the render or grid kernel's ray-mode twin, one launch of
 // rl.list_n rays; nothing when there are none
 cudaError_t tcrt_launch_render_rays(const RenderLaunch& rl, int sm_count, cudaStream_t stream);
+// views-mode render launch (multi-view frames, RenderLaunch::view_cams): the render or grid kernel's views-mode twin over
+// the global columns [rl.x0, rl.x1), 4x8 tiles where the band allows them; one launch, nothing when the band is empty
+cudaError_t tcrt_launch_render_views(const RenderLaunch& rl, int sm_count, cudaStream_t stream);
 // experimental task-pool kernel for sphere-BVH scenes (tcrt_render_pool.cu, developer builds only); smem_scene = bytes of the staged blob
 cudaError_t tcrt_launch_render_pool(const RenderLaunch& rl, int fm, int sm_count, size_t smem_scene, cudaStream_t stream);
 // n random (a.xyz, b) cases: div3 (shared-reciprocal division of the render kernel) vs __fdiv_rn; *bad += mismatches

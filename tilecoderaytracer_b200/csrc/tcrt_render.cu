@@ -39,7 +39,9 @@ namespace {
 
 // The kernel body.  MODE kModeBand: the pixels of the band [rl.x0, rl.x1) (render_kernel).  kModeList: the samples of a
 // pixel list (render_list_kernel, adaptive frames; RenderLaunch::list).  kModeRays: the caller's rays (render_rays_kernel,
-// ray batches; RenderLaunch::ray_*).  Only the refill block, the output slot and the invalid-ray count differ.
+// ray batches; RenderLaunch::ray_*).  kModeViews: band mode over the global columns of a stack of views whose primary rays
+// take their camera from a table (render_views_kernel, multi-view frames; RenderLaunch::view_cams).  Only the refill
+// block, the output slot and the invalid-ray count differ.
 template <int CAP, int SBVH, int FM, int MODE>
 __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
     extern __shared__ float4 smem4[];
@@ -62,7 +64,8 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
 
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned total = MODE != kModeBand ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = (MODE == kModeList || MODE == kModeRays) ? (unsigned)rl.list_n
+                                                                   : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     const V3 null_color = mk(rl.null_r, rl.null_g, rl.null_b);
 
     float stack[CAP * 7];   // per level: local rgb, k, object rgb (local memory, touched only on reflective hits)
@@ -122,7 +125,8 @@ __device__ __forceinline__ void render_body(const RenderLaunch& rl) {
                     TCRT_CHECK(xc >= 0 && xc < rl.x1 - rl.x0 && z >= 0 && z < rl.height, kChkQueue);
                     ln.pix = MODE == kModeList ? (int)(wcur + rank) : xc * rl.height + z;
                     ln.level = 0;
-                    primary_ray(rl, xc, z, ln.O, ln.D);
+                    if (MODE == kModeViews) view_ray(rl, xc, z, ln.O, ln.D);
+                    else primary_ray(rl, xc, z, ln.O, ln.D);
                 }
             }
             if (MODE == kModeRays) {
@@ -355,6 +359,11 @@ __global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kM
 }
 
 template <int CAP, int SBVH, int FM>
+__global__ void __launch_bounds__(kBlock, (SBVH && FM == 0) ? kMinBlocksBvh : kMinBlocks) render_views_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_body<CAP, SBVH, FM, kModeViews>(rl);
+}
+
+template <int CAP, int SBVH, int FM>
 cudaError_t launch_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
     cudaError_t e = cudaFuncSetAttribute(render_kernel<CAP, SBVH, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)smem);
@@ -375,10 +384,12 @@ cudaError_t launch_cap(const RenderLaunch& rl, int grid, size_t smem, cudaStream
     return cudaErrorInvalidValue;
 }
 
-// the list- and ray-mode twins (kModeList, kModeRays)
+// the list-, ray- and views-mode twins (kModeList, kModeRays, kModeViews)
 template <int CAP, int SBVH, int FM, int MODE>
 cudaError_t launch_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
-    const auto kernel = MODE == kModeRays ? render_rays_kernel<CAP, SBVH, FM> : render_list_kernel<CAP, SBVH, FM>;
+    const auto kernel = MODE == kModeViews ? render_views_kernel<CAP, SBVH, FM>
+                        : MODE == kModeRays ? render_rays_kernel<CAP, SBVH, FM>
+                                            : render_list_kernel<CAP, SBVH, FM>;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kernel<<<grid, kBlock, smem, stream>>>(rl);
@@ -552,17 +563,19 @@ cudaError_t tcrt_launch_render(const RenderLaunch& rl_in, int sm_count, cudaStre
     return e;
 }
 
-// List mode (adaptive frames) and ray mode (ray batches): the same kernels with the list or ray refill, grid-sized and
-// dispatched as tcrt_launch_render does, never the developer builds' pool or wavefront paths.  One launch; nothing when
-// the list is empty.
+// List mode (adaptive frames), ray mode (ray batches) and views mode (multi-view frames): the same kernels with the list,
+// ray or views refill, grid-sized and dispatched as tcrt_launch_render does, never the developer builds' pool or wavefront
+// paths.  One launch; nothing when the list is empty.  Views launches keep the band's 4x8 tiles (eye rays in x-major
+// order trace 8-16 % slower than in tile order, profiles/README.md 12); the list is their band's pixels.
 template <int MODE>
 static cudaError_t launch_twin(const RenderLaunch& rl_in, int sm_count, cudaStream_t stream) {
     RenderLaunch rl = rl_in;
+    if (MODE == kModeViews) rl.list_n = rl.x1 > rl.x0 ? (rl.x1 - rl.x0) * rl.height : 0;
     if (rl.list_n <= 0) return cudaSuccess;
     const size_t smem = (size_t)std::max(1, rl.scene.blob_f4 - rl.scene.stage_off) * sizeof(float4);
     if (smem > tcrt_render_max_smem()) return cudaErrorInvalidValue;
     const int fm = finite_mode(rl.scene);
-    rl.tiled = 0;
+    rl.tiled = MODE == kModeViews && (rl.x1 - rl.x0) % TCRT_TILE_W == 0 && rl.height % TCRT_TILE_H == 0 ? 1 : 0;
     rl.row_order = nullptr;
     rl.col_cost = nullptr;
     rl.refill_min = 32;
@@ -586,4 +599,8 @@ cudaError_t tcrt_launch_render_list(const RenderLaunch& rl, int sm_count, cudaSt
 
 cudaError_t tcrt_launch_render_rays(const RenderLaunch& rl, int sm_count, cudaStream_t stream) {
     return launch_twin<kModeRays>(rl, sm_count, stream);
+}
+
+cudaError_t tcrt_launch_render_views(const RenderLaunch& rl, int sm_count, cudaStream_t stream) {
+    return launch_twin<kModeViews>(rl, sm_count, stream);
 }

@@ -39,7 +39,8 @@ static_assert(TCRT_MAX_DEPTH < kLevelMask, "levels and level records have to fit
 
 // The kernel body.  MODE kModeBand: the pixels of the band (render_grid_kernel); kModeList: the samples of a pixel list
 // (render_grid_list_kernel, adaptive frames; RenderLaunch::list); kModeRays: the caller's rays (render_grid_rays_kernel,
-// ray batches; RenderLaunch::ray_*).  Only the refill block, the output slot and the invalid-ray count differ.
+// ray batches; RenderLaunch::ray_*); kModeViews: the pixels of a band of stacked views (render_grid_views_kernel,
+// multi-view frames; RenderLaunch::view_cams).  Only the refill block, the output slot and the invalid-ray count differ.
 template <int CAP, int FM, int MODE>
 __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
     extern __shared__ float4 smem4[];
@@ -61,7 +62,8 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
 
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned total = MODE != kModeBand ? (unsigned)rl.list_n : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
+    const unsigned total = (MODE == kModeList || MODE == kModeRays) ? (unsigned)rl.list_n
+                                                                   : (unsigned)(rl.x1 - rl.x0) * (unsigned)rl.height;
     const V3 null_color = mk(rl.null_r, rl.null_g, rl.null_b);
 
     float stack[CAP * 7];   // per level: local rgb, k, object rgb (local memory, touched only on reflective hits)
@@ -115,7 +117,8 @@ __device__ __forceinline__ void render_grid_body(const RenderLaunch& rl) {
                     else queue_to_pixel(rl, (int)(wcur + rank), xc, z);
                     ln.pix = MODE == kModeList ? (int)(wcur + rank) : xc * rl.height + z;
                     ln.level = 0;
-                    primary_ray(rl, xc, z, ln.O, ln.D);
+                    if (MODE == kModeViews) view_ray(rl, xc, z, ln.O, ln.D);
+                    else primary_ray(rl, xc, z, ln.O, ln.D);
                 }
             }
             if (MODE == kModeRays) {
@@ -479,6 +482,11 @@ __global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_rays_k
 }
 
 template <int CAP, int FM>
+__global__ void __launch_bounds__(kGridBlock, kGridMinBlocks) render_grid_views_kernel(const __grid_constant__ RenderLaunch rl) {
+    render_grid_body<CAP, FM, kModeViews>(rl);
+}
+
+template <int CAP, int FM>
 cudaError_t launch_grid_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream) {
     cudaError_t e = cudaFuncSetAttribute(render_grid_kernel<CAP, FM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -486,10 +494,12 @@ cudaError_t launch_grid_one(const RenderLaunch& rl, int grid, size_t smem, cudaS
     return cudaGetLastError();
 }
 
-// the list- and ray-mode twins
+// the list-, ray- and views-mode twins
 template <int CAP, int FM>
 cudaError_t launch_grid_list_one(const RenderLaunch& rl, int grid, size_t smem, cudaStream_t stream, RenderMode mode) {
-    const auto kernel = mode == kModeRays ? render_grid_rays_kernel<CAP, FM> : render_grid_list_kernel<CAP, FM>;
+    const auto kernel = mode == kModeViews ? render_grid_views_kernel<CAP, FM>
+                        : mode == kModeRays ? render_grid_rays_kernel<CAP, FM>
+                                            : render_grid_list_kernel<CAP, FM>;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kernel<<<grid, kGridBlock, smem, stream>>>(rl);
@@ -531,8 +541,8 @@ extern "C" int tcrt_dev_lane_stats_grid(unsigned long long* out16, int reset) {
 #endif
 
 // fm: 0 no finite planes, 3 a handful swept linearly; rl.scene.grid_cells != nullptr (tcrt_upload_scene built a grid).
-// mode kModeList / kModeRays: the list- or ray-mode kernels (tcrt_launch_render_list / _rays), with no more CTAs than
-// there are claims.
+// mode kModeList / kModeRays / kModeViews: the list-, ray- or views-mode kernels (tcrt_launch_render_list / _rays /
+// _views; rl.list_n = the launch's queue positions), with no more CTAs than there are claims.
 cudaError_t tcrt_launch_render_grid(const RenderLaunch& rl, int fm, int sm_count, size_t smem, cudaStream_t stream, RenderMode mode) {
     int ctas_per_sm = kGridMinBlocks;
     while (ctas_per_sm > 1 && (smem + 1024) * ctas_per_sm > 220 * 1024) --ctas_per_sm;

@@ -7,7 +7,8 @@ untiled frame, a band from an odd column), list kernels (adaptive frames refinin
 flags are read from each translation unit that launches a kernel: render, grid and hits.  Last, a ray batch of valid and
 invalid rays on a grid scene and a BVH scene, traced and intersected, against tests/oracle_rays.c, and the occlusion queries
 (points against every light, rays with their limits) on a grid scene, BVH scenes and box-cluster scenes against
-tests/oracle_occlusion.c.
+tests/oracle_occlusion.c, and multi-view frames on a grid scene, a BVH scene and a box-cluster scene, with a piece
+boundary inside a view.
 usage: python -c "from tilecoderaytracer_b200 import build; build.build_lib(defines=('TCRT_CHECKED',), out=LIB)"
        TCRT_LIB=LIB python tools/checked_run.py"""
 import ctypes as C
@@ -226,4 +227,34 @@ with tempfile.TemporaryDirectory() as tmp:
         bad_total += bad + len(f)
         print(f"occlusion {name:14s} {str(want_cls):16s} {len(pts)} points x {flat.n_lights} lights, {len(o)} rays: "
               f"mismatches {bad}, checks fired: {f or 'none'}", flush=True)
+
+# ---- multi-view frames: the render / grid kernels' views mode, against the oracle on small views and against set_camera +
+# render on views of several pieces (3 x 1500 x 1024: pieces of 4096 columns, a boundary inside view 2) ------------------------
+import test_views as MV  # noqa: E402
+
+for name, want_cls in (("synth256", ("grid", 1, 0)), ("random:24:200", ("render", 1, 2)), ("boxes:3:14", ("render", 0, 2))):
+    cam = api.Camera()
+    sc = api.Scene().build(name, cam)
+    flat, c = sc.flatten(), cam.export()
+    ctx.upload_flat(flat, c)
+    bad = int(V.dispatch_class(ctx.scene_structures()) != want_cls)
+    cams = MV.three_views(c)
+    for depth in (0, 8, 50):
+        for (w, h), oracle in (((48, 40), True), ((13, 11), True), ((1500, 1024), False)):
+            p = api.default_params(w, h, depth)
+            got, st = ctx.render_views(p, cams)
+            got = got.copy()
+            if oracle:
+                for v, cv in enumerate(cams):
+                    ref, cnt = O.render(flat, cv, p)
+                    bad += n_bad(got[v], ref)
+            else:
+                want, cnt = MV.per_view(ctx, p, cams)
+                bad += n_bad(got.reshape(-1, 1, 3), want.reshape(-1, 1, 3)) + int(MV._counters(st) != cnt)
+                bad += int(st.gpu_launches != 2)
+                ctx.set_camera(c)
+    f = fired()
+    bad_total += bad + len(f)
+    print(f"views {name:14s} {str(want_cls):16s} 3 views of 48x40, 13x11 and 1500x1024, d0/8/50: mismatches {bad}, "
+          f"checks fired: {f or 'none'}", flush=True)
 print("CHECKED_OK" if bad_total == 0 else "CHECKED_FAIL")

@@ -52,6 +52,9 @@ public:
         camera.exportTo(&c);
         return rc_ = tcrt_upload_scene(ctx_, &s, &c);
     }
+    // moving spheres (tcrt_update_spheres): geom[4*i .. 4*i+3] = centre xyz and radius*radius of sphere i, in the order of
+    // the scene given to setScene; the scene stays resident, the GPU refits its structures
+    int updateSpheres(const float* geom, tcrt_stats* stats = NULL) { return rc_ = tcrt_update_spheres(ctx_, geom, stats); }
     // the pixel loop (RayTracer.cpp:911-923): pixels[x][z] -> pixels_xmajor[(x*H + z)*3 + c]; with rs.samples > 1 each
     // pixel is the mean of rs.samples x rs.samples samples (tcrt_render_columns_ss), with rs.contrast >= 0 only the pixels
     // at contrast edges (tcrt_render_columns_adaptive)

@@ -192,6 +192,35 @@ int tcrt_plan_grid_cells(const tcrt_scene* scene, const float* points, int n_poi
  * Bad params: TCRT_ERR_INVALID; max_depth above TCRT_MAX_DEPTH: TCRT_ERR_UNSUPPORTED, as for renders. */
 int tcrt_plan_dead_paths(const tcrt_scene* scene, const tcrt_params* params, int* prune);
 
+/* Moving spheres (multi-frame mode, SURVEY §8f): new centres and radii for every sphere of the resident scene, applied on
+ * the devices without rebuilding the scene.  sphere_geom holds n_spheres x (centre x y z, radius_squared) float32, in the
+ * layout and sphere order of tcrt_scene.sphere_geom of the last tcrt_upload_scene.
+ * After the call every call that reads the scene (frames in every form, async frames, hit buffers, tcrt_pick, ray
+ * batches, occlusion queries, multi-view frames, tcrt_balance_columns) returns, bit for bit, what it returns after
+ * tcrt_upload_scene of the uploaded scene with sphere_geom replaced by the input and each sphere's obj_origin row
+ * replaced by its new centre (for a light sphere: the light's position).  Planes, materials, textures, lights and counts
+ * are unchanged.
+ * The sphere BVH keeps its topology and has its boxes refitted; the sphere grid keeps its origin, cell size and
+ * dimensions and has its cells registered again.  The grid is dropped (tcrt_scene_structures info[1] = 0; the sphere-BVH
+ * kernel serves the scene) when a sphere's widened box leaves the grid's box or the registrations break the builder's
+ * rules (more than 8 per sphere, more than 24 in one cell); it stays dropped until the next tcrt_upload_scene, which is
+ * also how to re-optimise a scene that has drifted far.
+ * Validation: every centre component and radius_squared finite, radius_squared >= 0; otherwise TCRT_ERR_INVALID and the
+ * scene is unchanged on every device (the device form checks on the device before anything is written).  Before any
+ * upload: TCRT_ERR_NO_SCENE.  A scene without spheres: TCRT_OK, nothing launched.
+ * Ordering: the update is queued on each device's render stream, like an upload: frames queued before it see the old
+ * spheres, calls made after it the new ones.  The call is synchronous: with frames in flight it returns once they have
+ * finished.  It invalidates the balanced cut and cost map, makes the next tcrt_upload_scene rebuild even an unchanged
+ * scene, and leaves the last render, the writers and tcrt_device_frame alone.
+ * stats (may be NULL): render_ms per device is the update's device time, gpu_launches its launches (a library scan or
+ * sort counts as one), no rays.
+ * tcrt_update_spheres_device: sphere_geom is device memory of device_slot's device (e.g. a torch CUDA tensor written by a
+ * physics step), 16-byte aligned (the rows are read as float4), complete when the call is made; other devices of the ctx
+ * get a device-to-device copy.  A pointer that is not device memory of that device, or not 16-byte aligned:
+ * TCRT_ERR_INVALID, nothing launched.  The host form takes any float-aligned pointer. */
+int tcrt_update_spheres(tcrt_ctx* ctx, const float* sphere_geom, tcrt_stats* stats);
+int tcrt_update_spheres_device(tcrt_ctx* ctx, int device_slot, const float* sphere_geom, tcrt_stats* stats);
+
 /* ---- render (replaces the pixel loop RayTracer.cpp:911-923) ----------------------- */
 /* Whole image -> host_rgb[width*height*3], x-major, z fastest, (r,g,b) float32: the layout
  * of the reference's pixels[W][H] (RayTracer.h:44).  stats may be NULL.  host_rgb may be pinned (tcrt_alloc_host,

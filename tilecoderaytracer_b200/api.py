@@ -255,6 +255,18 @@ def plan_dead_paths(flat, params: TcrtParams) -> bool:
     return bool(prune.value)
 
 
+def sphere_geom(centres, radii) -> np.ndarray:
+    """The (n, 4) float32 rows Context.update_spheres takes: centre x y z, radius_squared, with radius_squared formed as
+    SceneSphere(o, r) forms it — r * r in binary32."""
+    c = np.asarray(centres, dtype=np.float32).reshape(-1, 3)
+    r = np.asarray(radii, dtype=np.float32).reshape(-1)
+    assert r.shape[0] == c.shape[0], "one radius per centre"
+    out = np.empty((c.shape[0], 4), np.float32)
+    out[:, :3] = c
+    out[:, 3] = r * r
+    return out
+
+
 def normalize_like_reference(v) -> np.ndarray:
     """vector3d::normalize in numpy float32, as a Ray's constructor applies it: len = sqrtf((x*x + y*y) + z*z), then three
     IEEE divisions.  The ray-batch calls take directions as a Ray stores them; this turns raw directions (..., 3) into
@@ -758,6 +770,25 @@ class Context:
     def write_bin(self, params: TcrtParams, path: str) -> None:
         """The last render as raw float32 ("TCRTBIN1" header + pixels[W][H] order)."""
         self._ck(self._lib.tcrt_write_bin(self._h, C.byref(params), path.encode()))
+
+    def update_spheres(self, geom) -> RenderStats:
+        """Moving spheres (tcrt_update_spheres): new (centre, radius_squared) rows, (n_spheres, 4) float32 in the order of
+        the uploaded scene's sphere_geom (sphere_geom() forms them).  Every later call sees the scene uploaded with these
+        spheres (and light spheres' positions at their new centres), bit for bit; the BVH is refitted and the grid
+        re-registered on the GPU.  Waits for frames in flight.  Returns RenderStats (render_ms: the update's device time)."""
+        g = np.asarray(geom)
+        assert g.dtype == np.float32 and g.ndim == 2 and g.shape[1] == 4 and g.flags["C_CONTIGUOUS"], "geom: (n, 4) float32"
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_update_spheres(self._h, g.ctypes.data_as(C.c_void_p), C.byref(st)))
+        return RenderStats.from_c(st)
+
+    def update_spheres_device(self, ptr: int, slot: int = 0) -> RenderStats:
+        """update_spheres from device memory of device `slot` (e.g. a torch CUDA tensor's data_ptr(), n_spheres x 4
+        float32, 16-byte aligned, complete when called); the other devices of the context get a device-to-device copy.  A
+        pointer that is not 16-byte aligned raises TcrtError (TCRT_ERR_INVALID)."""
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_update_spheres_device(self._h, slot, C.c_void_p(ptr or None), C.byref(st)))
+        return RenderStats.from_c(st)
 
     def set_camera(self, cam: TcrtCamera) -> None:
         """Multi-frame mode: new camera, same resident scene."""

@@ -142,6 +142,24 @@ struct DeviceState {
     // batches' scratch, queue heads, counters and events above
     tcrt_camera* view_cams = nullptr;
     size_t view_cams_cap = 0;                      // cameras
+    // sphere updates (tcrt_update_spheres): the upload's maps (slot_of, light_sph, levels, level_start) for the upload
+    // numbered upd_serial, the input when it does not already live on this device, what the launches reduce (pinned copy
+    // in h_upd_back), the spheres' boxes, and the grid's registration buffers — whose item list the scene then reads.
+    // The call is synchronous: nothing else uses these while one runs.
+    unsigned long long upd_serial = 0;
+    int* upd_maps = nullptr;
+    size_t upd_maps_cap = 0;                       // ints
+    float4* upd_geom = nullptr;
+    size_t upd_geom_cap = 0;
+    unsigned char* upd_back = nullptr;
+    size_t upd_back_cap = 0;
+    unsigned char* h_upd_back = nullptr;
+    size_t h_upd_back_cap = 0;
+    float* upd_boxes = nullptr;
+    size_t upd_boxes_cap = 0;                      // floats
+    unsigned char* upd_grid = nullptr;
+    size_t upd_grid_cap = 0;
+    cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;  // around the update's launches (render stream)
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -155,6 +173,99 @@ struct DeadPathBound {
     double leaf = 0.0;     // |tail| of a light hit or of a non-reflective hit (local)
     double obj = 0.0;      // largest |object colour| component, textures included
     double kref = 0.0;     // largest reflective factor
+};
+
+// ---- the per-launch scalars of the pruning structures (DeviceScene), from the bounds of what they hold -----------------
+// Shared by the upload (plan_scene_blob) and by sphere updates (tcrt_update_spheres), which reduce the spheres' part of
+// the bounds on the device and keep the planes' part from the upload.
+struct SceneBounds {
+    double sph_lo[3] = {1e300, 1e300, 1e300}, sph_hi[3] = {-1e300, -1e300, -1e300};   // boxes of the boxed spheres
+    double pl_lo[3] = {1e300, 1e300, 1e300}, pl_hi[3] = {-1e300, -1e300, -1e300};     // finite-plane boxes, box clusters
+    float rmin = INFINITY;                                                              // smallest radius in the sphere BVH
+};
+
+// bvh_rmin, bvh_c*, bvh_r2, bvh_cmax, clu_c*, clu_rbig, and grid_k2_max when the scene has a grid (grid_margin set)
+void scene_scalars(const SceneBounds& b, bool sph_bvh, bool clusters, bool grid, DeviceScene& ds) {
+    double blo[3], bhi[3];
+    for (int k = 0; k < 3; k++) {
+        blo[k] = std::min(b.sph_lo[k], b.pl_lo[k]);
+        bhi[k] = std::max(b.sph_hi[k], b.pl_hi[k]);
+    }
+    ds.bvh_rmin = sph_bvh ? b.rmin * 0.999f : 1.f;
+    ds.clu_cx = ds.clu_cy = ds.clu_cz = ds.clu_rbig = 0.f;
+    ds.bvh_cx = ds.bvh_cy = ds.bvh_cz = ds.bvh_r2 = ds.bvh_cmax = 0.f;
+    if (clusters) {
+        double r1 = 0.0, cmax = 0.0;
+        for (int k = 0; k < 3; k++) {
+            r1 += 0.5 * (bhi[k] - blo[k]);
+            cmax = std::max(cmax, std::max(fabs(blo[k]), fabs(bhi[k])));
+        }
+        ds.clu_cx = (float)(0.5 * (blo[0] + bhi[0]));
+        ds.clu_cy = (float)(0.5 * (blo[1] + bhi[1]));
+        ds.clu_cz = (float)(0.5 * (blo[2] + bhi[2]));
+        ds.clu_rbig = (float)((r1 + cmax) * 1.001 + 1e-6);
+    }
+    if (ds.n_sph_bvh || ds.n_fin_bvh) {   // (a BVH that exists covers its prefix)
+        double c[3], r2 = 0.0, cmax = 0.0;
+        for (int k = 0; k < 3; k++) {
+            if (!(blo[k] <= bhi[k])) blo[k] = bhi[k] = 0.0;
+            c[k] = 0.5 * (blo[k] + bhi[k]);
+            r2 += 0.25 * (bhi[k] - blo[k]) * (bhi[k] - blo[k]);
+            cmax = std::max(cmax, std::max(fabs(blo[k]), fabs(bhi[k])));
+        }
+        ds.bvh_cx = (float)c[0]; ds.bvh_cy = (float)c[1]; ds.bvh_cz = (float)c[2];
+        ds.bvh_r2 = (float)(r2 * 1.001 + 1e-6);
+        ds.bvh_cmax = (float)(cmax * 1.001);
+    }
+    if (grid) {
+        // the far-origin test without fatten()'s square root: m(k2) = (sqrt(rmin^2 + k2 E) - rmin) 1.001 + 1e-6 rmin grows
+        // with k2, so m <= margin is a bound on k2 (solved in double, 0.1 % below: fewer rays on the grid is always sound)
+        const double rmin = ds.bvh_rmin, t = ((double)ds.grid_margin - 1e-6 * rmin) / 1.001;
+        const double k2 = t > 0.0 ? (t * t + 2.0 * t * rmin) / (double)TCRT_SPH_E : 0.0;
+        ds.grid_k2_max = (float)(0.999 * k2);
+    }
+}
+
+// The two light-table rows of a light at og: (position, intensity) (material colour, mask), what the light loop reads
+// (RayTracer.cpp:540-563).  Shadow rays end at the light.  A cluster whose faces all lie on its hull ("shell": a room)
+// cannot be crossed by a segment whose two ends are strictly inside the hull; whether the light is (with twice the
+// kernel's per-ray margin) is a constant: bit c of the mask.  Needs ds.clu_* (scene_scalars).
+void light_rows(const float* og, float intensity, const float* colour, const std::vector<TcrtBoxCluster>& clusters,
+                const DeviceScene& ds, float4* rows) {
+    unsigned inside_mask = 0u;
+    for (int c = 0; c < (int)clusters.size() && c < 32; c++) {
+        const TcrtBoxCluster& b = clusters[c];
+        bool shell = true, inside = true;
+        for (int f = 0; f < 6; f++)
+            if (b.plane[f] >= 0 && b.c[f] != b.lo[f / 2] && b.c[f] != b.hi[f / 2]) shell = false;
+        const double l1 = fabs((double)og[0] - ds.clu_cx) + fabs((double)og[1] - ds.clu_cy) +
+                          fabs((double)og[2] - ds.clu_cz) + ds.clu_rbig;
+        const double ml = 2.0 * 4e-6 * l1;   // 2 x TCRT_CLU_K x l1, see tcrt_render.cu clu_ray
+        for (int k = 0; k < 3; k++)
+            if (!((double)og[k] > (double)b.lo[k] + ml && (double)og[k] < (double)b.hi[k] - ml)) inside = false;
+        if (shell && inside) inside_mask |= 1u << c;
+    }
+    rows[0] = make_float4(og[0], og[1], og[2], intensity);
+    float4 lc = make_float4(colour[0], colour[1], colour[2], 0.f);
+    memcpy(&lc.w, &inside_mask, 4);
+    rows[1] = lc;
+}
+
+// What a sphere update needs of the upload: where each sphere lives in the blob, the planes' constants, the BVH's levels,
+// the grid's registration arithmetic and the lights.
+struct UpdatePlan {
+    int n_spheres = 0;
+    std::vector<int> slot_of;            // sphere i (tcrt_scene order) -> its slot in the blob's sphere array (inverse of ps)
+    int n_boxed = 0;                     // slots [0, n_boxed): the spheres the upload boxed into the bounds
+    double ext_fixed = 1.0;              // max(1, |finite-plane origins|)
+    SceneBounds bounds;                  // its plane part
+    std::vector<int> levels, level_start;   // the sphere BVH's inner nodes, level by level from the root
+    std::vector<TcrtBoxCluster> clusters;
+    TcrtSphereGrid grid;                 // lo_d, cell_d, reg_margin_d, dims (no cells or items)
+    size_t n_cells = 0;
+    std::vector<float> light_og, light_col, light_int;   // 3, 3, 1 per light, as uploaded
+    std::vector<int> light_sph;          // sphere index of each light sphere, in light order
+    std::vector<int> light_of_sph;       // the light each of those is
 };
 
 }  // namespace
@@ -203,6 +314,10 @@ struct tcrt_ctx {
     size_t scene_off[9] = {};       // surface, material, normals, frame, tex, bvh_s, bvh_f, grid cells, grid items
     bool scene_bvh_s = false, scene_bvh_f = false, scene_grid = false;
     DeadPathBound scene_dead;
+    UpdatePlan scene_upd;           // what tcrt_update_spheres needs of the last upload
+    unsigned long long scene_serial = 0;   // bumped by every new blob (DeviceState::upd_serial)
+    float4* upd_stage = nullptr;    // pinned: the input of tcrt_update_spheres, then the light rows it rewrites
+    size_t upd_stage_cap = 0;       // float4s
 };
 
 namespace {
@@ -288,6 +403,14 @@ void free_device(DeviceState& d) {
     cudaFree(d.ray_ctl);
     cudaFreeHost(d.h_ray);
     cudaFree(d.view_cams);
+    cudaFree(d.upd_maps);
+    cudaFree(d.upd_geom);
+    cudaFree(d.upd_back);
+    cudaFreeHost(d.h_upd_back);
+    cudaFree(d.upd_boxes);
+    cudaFree(d.upd_grid);
+    for (cudaEvent_t e : {d.ev_u0, d.ev_u1})
+        if (e) cudaEventDestroy(e);
     for (cudaEvent_t e : {d.ev_r0, d.ev_r1, d.ev_rc})
         if (e) cudaEventDestroy(e);
     cudaFreeHost(d.h_txt);
@@ -473,6 +596,7 @@ void tcrt_destroy(tcrt_ctx* ctx) {
     for (auto& d : ctx->devs) free_device(d);
     if (ctx->host_text) cudaFreeHost(ctx->host_text);
     if (ctx->scene_stage) cudaFreeHost(ctx->scene_stage);
+    if (ctx->upd_stage) cudaFreeHost(ctx->upd_stage);
     delete ctx;
 }
 
@@ -483,6 +607,7 @@ struct SceneBlob {
     DeviceScene ds{};
     size_t off[9] = {};          // surface, material, normals, frame, tex, bvh_s, bvh_f, grid cells, grid items
     bool grid = false, bvh_s = false, bvh_f = false;
+    UpdatePlan upd;
     std::string err;
 };
 static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out);
@@ -655,28 +780,29 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
     std::vector<TcrtBoxCluster> clusters;
     ds.n_fin_gen = ds.n_fin_nl;
     ds.n_arect = 0;
-    ds.clu_cx = ds.clu_cy = ds.clu_cz = ds.clu_rbig = 0.f;
     ds.bvh_sph_root = ds.bvh_fin_root = 0;
     ds.n_sph_bvh = ds.n_fin_bvh = 0;
-    ds.bvh_cx = ds.bvh_cy = ds.bvh_cz = ds.bvh_r2 = ds.bvh_cmax = 0.f;
-    ds.bvh_rmin = 1.f;
+    UpdatePlan& upd = out.upd;
+    SceneBounds& bounds = upd.bounds;
     {
         double ext = 1.0;
-        for (int i = 0; i < s->n_spheres; i++)
-            for (int k = 0; k < 3; k++) ext = std::max(ext, fabs((double)s->sphere_geom[4 * i + k]));
         for (int i = 0; i < s->n_fin_planes; i++)
             for (int k = 0; k < 3; k++) ext = std::max(ext, fabs((double)s->fin_geom[16 * i + 12 + k]));
+        upd.ext_fixed = ext;
+        for (int i = 0; i < s->n_spheres; i++)
+            for (int k = 0; k < 3; k++) ext = std::max(ext, fabs((double)s->sphere_geom[4 * i + k]));
         if (!std::isfinite(ext)) ext = 1e30;
         const double margin = 1e-5 * ext;
         std::vector<float> boxes_s, boxes_f;
         std::vector<int> ord;
-        double blo[3] = {1e300, 1e300, 1e300}, bhi[3] = {-1e300, -1e300, -1e300};
-        auto grow = [&](const float* bx) {
+        auto grow_into = [](double* lo, double* hi, const float* bx) {
             for (int k = 0; k < 3; k++) {
-                if (std::isfinite(bx[k])) blo[k] = std::min(blo[k], (double)bx[k]);
-                if (std::isfinite(bx[3 + k])) bhi[k] = std::max(bhi[k], (double)bx[3 + k]);
+                if (std::isfinite(bx[k])) lo[k] = std::min(lo[k], (double)bx[k]);
+                if (std::isfinite(bx[3 + k])) hi[k] = std::max(hi[k], (double)bx[3 + k]);
             }
         };
+        auto grow_sph = [&](const float* bx) { grow_into(bounds.sph_lo, bounds.sph_hi, bx); };
+        auto grow = [&](const float* bx) { grow_into(bounds.pl_lo, bounds.pl_hi, bx); };
         if (ds.n_sph_nl >= kSphereBvhMin) {
             // Tiny spheres would force a large per-ray fattening on everything (see `fatten`): the
             // (at most 16) spheres below half the median radius stay in the linear part.
@@ -693,9 +819,10 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
             float rmin = INFINITY;
             for (int k = 0; k < nb; k++) {
                 sphere_box(s->sphere_geom + 4 * in[k], margin, &boxes_s[6 * k]);
-                grow(&boxes_s[6 * k]);
+                grow_sph(&boxes_s[6 * k]);
                 rmin = std::min(rmin, sqrtf(s->sphere_geom[4 * in[k] + 3]));
             }
+            upd.n_boxed = nb;
             ds.bvh_sph_root = tcrt_build_bvh(boxes_s, nb, ord, bvh_s, &bvh_depth_s);
             std::vector<int> np;
             for (int k = 0; k < nb; k++) np.push_back(in[ord[k]]);
@@ -703,7 +830,7 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
             np.insert(np.end(), ps.begin() + ds.n_sph_nl, ps.end());
             ps.swap(np);
             ds.n_sph_bvh = nb;
-            ds.bvh_rmin = rmin * 0.999f;
+            bounds.rmin = rmin;
             // a uniform grid over the same spheres (leaf order), when they are even enough for one (tcrt_bvh.cpp)
             if (!bvh_s.empty()) {
                 std::vector<float> leaf_boxes(6 * (size_t)nb);
@@ -716,7 +843,6 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
             if (bvh_s.empty()) {
                 ds.n_sph_bvh = 0;
                 ds.bvh_sph_root = 0;
-                ds.bvh_rmin = 1.f;
                 bvh_depth_s = 0;
             }
         }
@@ -759,29 +885,6 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
                 }
             }
         }
-        if (!clusters.empty()) {
-            double r1 = 0.0, cmax = 0.0;
-            for (int k = 0; k < 3; k++) {
-                r1 += 0.5 * (bhi[k] - blo[k]);
-                cmax = std::max(cmax, std::max(fabs(blo[k]), fabs(bhi[k])));
-            }
-            ds.clu_cx = (float)(0.5 * (blo[0] + bhi[0]));
-            ds.clu_cy = (float)(0.5 * (blo[1] + bhi[1]));
-            ds.clu_cz = (float)(0.5 * (blo[2] + bhi[2]));
-            ds.clu_rbig = (float)((r1 + cmax) * 1.001 + 1e-6);
-        }
-        if (!bvh_s.empty() || !bvh_f.empty() || ds.n_sph_bvh || ds.n_fin_bvh) {
-            double c[3], r2 = 0.0, cmax = 0.0;
-            for (int k = 0; k < 3; k++) {
-                if (!(blo[k] <= bhi[k])) blo[k] = bhi[k] = 0.0;
-                c[k] = 0.5 * (blo[k] + bhi[k]);
-                r2 += 0.25 * (bhi[k] - blo[k]) * (bhi[k] - blo[k]);
-                cmax = std::max(cmax, std::max(fabs(blo[k]), fabs(bhi[k])));
-            }
-            ds.bvh_cx = (float)c[0]; ds.bvh_cy = (float)c[1]; ds.bvh_cz = (float)c[2];
-            ds.bvh_r2 = (float)(r2 * 1.001 + 1e-6);
-            ds.bvh_cmax = (float)(cmax * 1.001);
-        }
     }
 
     ds.fin_off = ds.n_sph;
@@ -810,6 +913,17 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
     const size_t off_bvh_f = off_bvh_s + bvh_s.size();
     // the grid serves the kernels without finite-plane structures (FM 0 / 3); elsewhere the sphere BVH alone
     has_grid = has_grid && !bvh_s.empty() && bvh_f.empty() && clusters.empty();
+    if (has_grid) {
+        for (int k = 0; k < 3; k++) {
+            ds.grid_lo[k] = grid.lo[k];
+            ds.grid_cell[k] = grid.cell[k];
+            ds.grid_hi[k] = grid.lo[k] + grid.cell[k] * (float)grid.dims[k];
+            ds.grid_inv_cell[k] = 1.0f / grid.cell[k];
+            ds.grid_dims[k] = grid.dims[k];
+        }
+        ds.grid_margin = grid.reg_margin;
+    }
+    scene_scalars(bounds, !bvh_s.empty(), !clusters.empty(), has_grid, ds);
     const size_t off_grid_cells = off_bvh_f + bvh_f.size();
     const size_t n_grid_cells = has_grid ? grid.cell_start.size() - 1 : 0;
     const size_t off_grid_items = off_grid_cells + 2 * n_grid_cells;
@@ -847,29 +961,8 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
     }
     for (int l = 0; l < ds.n_lights; l++) {
         const int lo = s->light_obj[l];
-        const float* og = s->obj_origin + 4 * lo;
-        const float* sf = s->obj_surface + 4 * lo;
-        // Shadow rays end at the light.  A cluster whose faces all lie on its hull ("shell": a room)
-        // cannot be crossed by a segment whose two ends are strictly inside the hull; whether the
-        // light is (with twice the kernel's per-ray margin) is a constant: bit c of the mask.
-        unsigned inside_mask = 0u;
-        for (int c = 0; c < ds.n_clu && c < 32; c++) {
-            const TcrtBoxCluster& b = clusters[c];
-            bool shell = true, inside = true;
-            for (int f = 0; f < 6; f++)
-                if (b.plane[f] >= 0 && b.c[f] != b.lo[f / 2] && b.c[f] != b.hi[f / 2]) shell = false;
-            const double l1 = fabs((double)og[0] - ds.clu_cx) + fabs((double)og[1] - ds.clu_cy) +
-                              fabs((double)og[2] - ds.clu_cz) + ds.clu_rbig;
-            const double ml = 2.0 * 4e-6 * l1;   // 2 x TCRT_CLU_K x l1, see tcrt_render.cu clu_ray
-            for (int k = 0; k < 3; k++)
-                if (!((double)og[k] > (double)b.lo[k] + ml && (double)og[k] < (double)b.hi[k] - ml)) inside = false;
-            if (shell && inside) inside_mask |= 1u << c;
-        }
-        // (position, intensity) (material colour, mask): what the light loop reads, RayTracer.cpp:540-563
-        host[ds.light_off + 2 * l] = make_float4(og[0], og[1], og[2], s->obj_material[4 * lo + 2]);
-        float4 lc = make_float4(sf[0], sf[1], sf[2], 0.f);
-        memcpy(&lc.w, &inside_mask, 4);
-        host[ds.light_off + 2 * l + 1] = lc;
+        light_rows(s->obj_origin + 4 * lo, s->obj_material[4 * lo + 2], s->obj_surface + 4 * lo, clusters, ds,
+                   &host[ds.light_off + 2 * l]);
     }
     for (int i = 0; i < n; i++) {
         host[off_surface + i] = f4(s->obj_surface + 4 * i);
@@ -910,20 +1003,46 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
             memcpy(&host[off_grid_cells + 2 * c + 1], &meta, sizeof(meta));
         }
         memcpy(&host[off_grid_items], grid.items.data(), grid.items.size() * sizeof(int));
-        for (int k = 0; k < 3; k++) {
-            ds.grid_lo[k] = grid.lo[k];
-            ds.grid_cell[k] = grid.cell[k];
-            ds.grid_hi[k] = grid.lo[k] + grid.cell[k] * (float)grid.dims[k];
-            ds.grid_inv_cell[k] = 1.0f / grid.cell[k];
-            ds.grid_dims[k] = grid.dims[k];
+    }
+
+    // what a sphere update needs (tcrt_update_spheres)
+    upd.n_spheres = ds.n_sph;
+    upd.slot_of.assign(ds.n_sph, 0);
+    for (int k = 0; k < ds.n_sph; k++) upd.slot_of[ps[k]] = k;
+    upd.level_start.assign(1, 0);
+    std::vector<int> level;
+    if (!bvh_s.empty()) level.push_back(0);   // the root: the builder's first node
+    while (!level.empty()) {
+        upd.levels.insert(upd.levels.end(), level.begin(), level.end());
+        upd.level_start.push_back((int)upd.levels.size());
+        std::vector<int> next;
+        for (int node : level) {
+            int ref[2];
+            memcpy(ref, &bvh_s[4 * (size_t)node + 3], sizeof ref);   // (child0, child1, -, -)
+            for (int r : ref)
+                if (r >= 0) next.push_back(r);
         }
-        ds.grid_margin = grid.reg_margin;
-        // the far-origin test without fatten()'s square root: m(k2) = (sqrt(rmin^2 + k2 E) - rmin) 1.001 + 1e-6 rmin grows
-        // with k2, so m <= margin is a bound on k2 (solved in double, 0.1 % below: fewer rays on the grid is always sound)
-        {
-            const double rmin = ds.bvh_rmin, t = ((double)grid.reg_margin - 1e-6 * rmin) / 1.001;
-            const double k2 = t > 0.0 ? (t * t + 2.0 * t * rmin) / (double)TCRT_SPH_E : 0.0;
-            ds.grid_k2_max = (float)(0.999 * k2);
+        level.swap(next);
+    }
+    upd.clusters = clusters;
+    if (has_grid) {
+        upd.grid = grid;
+        upd.grid.cell_start.clear();
+        upd.grid.items.clear();
+        upd.n_cells = n_grid_cells;
+    }
+    std::vector<int> sph_of_obj(n, -1);   // the sphere whose centre an object's origin is (the last, should several share one)
+    for (int i = 0; i < s->n_spheres; i++) sph_of_obj[s->sphere_obj[i]] = i;
+    for (int l = 0; l < ds.n_lights; l++) {
+        const int lo = s->light_obj[l];
+        for (int k = 0; k < 3; k++) {
+            upd.light_og.push_back(s->obj_origin[4 * lo + k]);
+            upd.light_col.push_back(s->obj_surface[4 * lo + k]);
+        }
+        upd.light_int.push_back(s->obj_material[4 * lo + 2]);
+        if (sph_of_obj[lo] >= 0) {
+            upd.light_sph.push_back(sph_of_obj[lo]);
+            upd.light_of_sph.push_back(l);
         }
     }
 
@@ -970,6 +1089,8 @@ static int build_scene_blob(tcrt_ctx* ctx, const tcrt_scene* s) {
     ctx->scene_bvh_s = b.bvh_s;
     ctx->scene_bvh_f = b.bvh_f;
     ctx->scene_dead = dead_path_bound(s);
+    ctx->scene_upd = std::move(b.upd);
+    ctx->scene_serial++;
     return TCRT_OK;
 }
 
@@ -3251,6 +3372,237 @@ int tcrt_write_txt_band(tcrt_ctx* ctx, const tcrt_params* p, const char* path, d
                                                "gather the bands and use tcrt_write_txt");
     if (!closed || io_error) return fail(ctx, TCRT_ERR_IO, "short write to %s", path);
     return TCRT_OK;
+}
+
+}  // extern "C"
+
+// ---- moving spheres (tcrt_update_spheres) ------------------------------------------------------------------------------------
+// The spheres of the resident scene take new centres and radii on every device, in place: tcrt_update.cu scatters them into
+// the blob, refits the sphere BVH and re-registers the sphere grid; the host then recomputes what the launches take by
+// value (scene_scalars) and the light rows (light_rows) from one small read-back, with the upload's own code.  Planes,
+// materials, textures and counts stay.  DESIGN.md §4.3, §4.5.
+
+// bytes of device memory from `off` on, rounded so that the next piece starts 256-byte aligned
+static size_t carve(size_t& off, size_t bytes) {
+    const size_t at = off;
+    off += (bytes + 255) & ~(size_t)255;
+    return at;
+}
+
+static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* stats) {
+    if (!ctx || !geom) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    const int nd = (int)ctx->devs.size();
+    int src_dev = -1;
+    if (slot >= 0) {
+        if (slot >= nd) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range (have %d)", slot, nd);
+        src_dev = ctx->devs[slot].dev;
+        if (!on_device(geom, src_dev)) return fail(ctx, TCRT_ERR_INVALID, "sphere_geom is not device memory of slot %d's device", slot);
+        if (reinterpret_cast<uintptr_t>(geom) % 16 != 0)   // the launches read it as float4
+            return fail(ctx, TCRT_ERR_INVALID, "sphere_geom is not 16-byte aligned");
+    }
+    if (stats) {
+        memset(stats, 0, sizeof(*stats));
+        stats->n_devices = nd;
+    }
+    const UpdatePlan& up = ctx->scene_upd;
+    const int n = up.n_spheres;
+    if (n == 0) return TCRT_OK;
+    const DeviceScene& ds0 = ctx->scene_ds;
+    const bool grid = ctx->scene_grid;
+    const int n_bvh = ds0.n_sph_bvh, n_ls = (int)up.light_sph.size(), n_levels = (int)up.level_start.size() - 1;
+    const unsigned cap = 8u * (unsigned)n_bvh;
+    const size_t back_bytes = sizeof(UpdateBack) + 12 * (size_t)n_ls;
+    const size_t stage_f4 = std::max((size_t)n, 2 * (size_t)ds0.n_lights);
+    if (stage_f4 > ctx->upd_stage_cap) {
+        if (ctx->upd_stage) cudaFreeHost(ctx->upd_stage);
+        ctx->upd_stage = nullptr;
+        ctx->upd_stage_cap = 0;
+        CK(ctx, cudaHostAlloc((void**)&ctx->upd_stage, stage_f4 * sizeof(float4), cudaHostAllocPortable));
+        ctx->upd_stage_cap = stage_f4;
+    }
+    if (slot < 0) memcpy(ctx->upd_stage, geom, (size_t)n * sizeof(float4));
+    int launches = 0;
+    std::vector<int*> items(nd, nullptr);
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));   // frames queued before the call finish with the old scene
+        if (!d.ev_u0) CK(ctx, cudaEventCreate(&d.ev_u0));
+        if (!d.ev_u1) CK(ctx, cudaEventCreate(&d.ev_u1));
+        // the upload's maps, once per upload
+        const size_t n_maps = (size_t)n + n_ls + up.levels.size() + up.level_start.size();
+        int rc = ensure(ctx, d.upd_maps, d.upd_maps_cap, n_maps);
+        if (rc) return rc;
+        if (d.upd_serial != ctx->scene_serial) {
+            std::vector<int> maps(up.slot_of);
+            maps.insert(maps.end(), up.light_sph.begin(), up.light_sph.end());
+            maps.insert(maps.end(), up.levels.begin(), up.levels.end());
+            maps.insert(maps.end(), up.level_start.begin(), up.level_start.end());
+            CK(ctx, cudaMemcpy(d.upd_maps, maps.data(), maps.size() * sizeof(int), cudaMemcpyHostToDevice));
+            d.upd_serial = ctx->scene_serial;
+        }
+        if ((rc = ensure(ctx, d.upd_back, d.upd_back_cap, back_bytes))) return rc;
+        if (back_bytes > d.h_upd_back_cap) {
+            if (d.h_upd_back) cudaFreeHost(d.h_upd_back);
+            d.h_upd_back = nullptr;
+            d.h_upd_back_cap = 0;
+            CK(ctx, cudaHostAlloc((void**)&d.h_upd_back, back_bytes, cudaHostAllocPortable));
+            d.h_upd_back_cap = back_bytes;
+        }
+        if ((rc = ensure(ctx, d.upd_boxes, d.upd_boxes_cap, 6 * (size_t)std::max(up.n_boxed, 1)))) return rc;
+        UpdateLaunch ul{};
+        size_t grid_bytes = 0, tmp_bytes = 0, o_cnt = 0, o_off = 0, o_keys = 0, o_vals = 0, o_keys2 = 0, o_sorted = 0, o_items = 0, o_cc = 0,
+               o_cs = 0, o_tmp = 0;
+        if (grid) {
+            tmp_bytes = tcrt_update_tmp_bytes(cap, n_bvh, (int)up.n_cells);
+            o_cnt = carve(grid_bytes, 8 * ((size_t)n_bvh + 1));
+            o_off = carve(grid_bytes, 8 * ((size_t)n_bvh + 1));
+            o_keys = carve(grid_bytes, 4 * (size_t)cap);
+            o_vals = carve(grid_bytes, 4 * (size_t)cap);
+            o_keys2 = carve(grid_bytes, 4 * (size_t)cap);
+            o_sorted = carve(grid_bytes, 4 * (size_t)cap);
+            o_items = carve(grid_bytes, 4 * (size_t)cap);
+            o_cc = carve(grid_bytes, 4 * (up.n_cells + 1));
+            o_cs = carve(grid_bytes, 4 * (up.n_cells + 1));
+            o_tmp = carve(grid_bytes, tmp_bytes);
+            // the item list the scene may be reading moves only when the buffer grows (the render stream is idle here)
+            if ((rc = ensure(ctx, d.upd_grid, d.upd_grid_cap, grid_bytes))) return rc;
+            unsigned char* g = d.upd_grid;
+            ul.grid = 1;
+            for (int k = 0; k < 3; k++) {
+                ul.glo[k] = up.grid.lo_d[k];
+                ul.gcell[k] = up.grid.cell_d[k];
+                ul.gdims[k] = up.grid.dims[k];
+            }
+            ul.gmargin = up.grid.reg_margin_d;
+            ul.n_cells = (int)up.n_cells;
+            ul.cap = cap;
+            ul.reg_count = reinterpret_cast<unsigned long long*>(g + o_cnt);
+            ul.reg_off = reinterpret_cast<unsigned long long*>(g + o_off);
+            ul.keys = reinterpret_cast<unsigned*>(g + o_keys);
+            ul.vals = reinterpret_cast<unsigned*>(g + o_vals);
+            ul.keys2 = reinterpret_cast<unsigned*>(g + o_keys2);
+            ul.sorted = reinterpret_cast<unsigned*>(g + o_sorted);
+            ul.items = reinterpret_cast<int*>(g + o_items);
+            ul.cell_count = reinterpret_cast<unsigned*>(g + o_cc);
+            ul.cell_start = reinterpret_cast<unsigned*>(g + o_cs);
+            ul.cells = d.scene_mem + ctx->scene_off[7];
+            ul.tmp = g + o_tmp;
+            ul.tmp_bytes = tmp_bytes;
+            items[i] = ul.items;
+        }
+        // the input on this device
+        const float4* src = reinterpret_cast<const float4*>(geom);
+        if (slot < 0 || d.dev != src_dev) {
+            if ((rc = ensure(ctx, d.upd_geom, d.upd_geom_cap, (size_t)n))) return rc;
+            if (slot < 0)
+                CK(ctx, cudaMemcpyAsync(d.upd_geom, ctx->upd_stage, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, d.stream));
+            else
+                CK(ctx, cudaMemcpyPeerAsync(d.upd_geom, d.dev, geom, src_dev, (size_t)n * sizeof(float4), d.stream));
+            src = d.upd_geom;
+        }
+        ul.geom = src;
+        ul.n = n;
+        ul.slot_of = d.upd_maps;
+        ul.spheres = d.scene_mem;
+        ul.n_boxed = up.n_boxed;
+        ul.n_bvh = n_bvh;
+        ul.ext_fixed = up.ext_fixed;
+        ul.light_sph = d.upd_maps + n;
+        ul.n_light_sph = n_ls;
+        ul.back = reinterpret_cast<UpdateBack*>(d.upd_back);
+        ul.boxes = d.upd_boxes;
+        if (ctx->scene_bvh_s) {
+            ul.nodes = d.scene_mem + ctx->scene_off[5];
+            ul.levels = d.upd_maps + n + n_ls;
+            ul.level_start = ul.levels + up.levels.size();
+            ul.n_levels = n_levels;
+        }
+        CK(ctx, cudaEventRecord(d.ev_u0, d.stream));
+        CK(ctx, tcrt_launch_update_spheres(ul, d.sm_count, d.stream, &launches));
+        CK(ctx, cudaEventRecord(d.ev_u1, d.stream));
+        CK(ctx, cudaMemcpyAsync(d.h_upd_back, d.upd_back, back_bytes, cudaMemcpyDeviceToHost, d.stream));
+    }
+    bool invalid = false;
+    for (auto& d : ctx->devs) {
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));
+        invalid = invalid || reinterpret_cast<const UpdateBack*>(d.h_upd_back)->invalid != 0;
+    }
+    if (invalid)   // no launch after the check wrote anything: the scene is unchanged
+        return fail(ctx, TCRT_ERR_INVALID, "sphere_geom holds a centre or radius_squared that is not finite, or radius_squared < 0");
+
+    // the scalars and the light rows, with the upload's code (every device reduced the same values)
+    const UpdateBack& b = *reinterpret_cast<const UpdateBack*>(ctx->devs[0].h_upd_back);
+    auto unkey = [](unsigned key) {
+        const unsigned u = (key & 0x80000000u) ? (key & 0x7fffffffu) : ~key;
+        float f;
+        memcpy(&f, &u, 4);
+        return f;
+    };
+    SceneBounds bounds = up.bounds;
+    for (int k = 0; k < 3; k++) {
+        if (b.lo_key[k]) bounds.sph_lo[k] = unkey(~b.lo_key[k]);
+        if (b.hi_key[k]) bounds.sph_hi[k] = unkey(b.hi_key[k]);
+    }
+    if (n_bvh > 0) {
+        const unsigned r2 = ~b.r2min_key;
+        float r2f;
+        memcpy(&r2f, &r2, 4);
+        bounds.rmin = sqrtf(r2f);
+    }
+    const bool keep_grid = grid && !b.grid_out && !b.grid_full;
+    DeviceScene ds = ds0;
+    scene_scalars(bounds, ctx->scene_bvh_s, !up.clusters.empty(), keep_grid, ds);
+    const float* centres = reinterpret_cast<const float*>(&b + 1);
+    std::vector<float> og(up.light_og);
+    for (int j = 0; j < n_ls; j++)
+        for (int k = 0; k < 3; k++) og[3 * up.light_of_sph[j] + k] = centres[3 * j + k];
+    for (int l = 0; l < ds.n_lights; l++)
+        light_rows(&og[3 * l], up.light_int[l], &up.light_col[3 * l], up.clusters, ds, ctx->upd_stage + 2 * l);
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        CK(ctx, cudaSetDevice(d.dev));
+        if (ds.n_lights > 0)
+            CK(ctx, cudaMemcpyAsync(d.scene_mem + ds.light_off, ctx->upd_stage, 2 * (size_t)ds.n_lights * sizeof(float4),
+                                    cudaMemcpyHostToDevice, d.stream));
+        DeviceScene& dd = d.ds;
+        dd.bvh_cx = ds.bvh_cx; dd.bvh_cy = ds.bvh_cy; dd.bvh_cz = ds.bvh_cz;
+        dd.bvh_r2 = ds.bvh_r2; dd.bvh_rmin = ds.bvh_rmin; dd.bvh_cmax = ds.bvh_cmax;
+        dd.clu_cx = ds.clu_cx; dd.clu_cy = ds.clu_cy; dd.clu_cz = ds.clu_cz; dd.clu_rbig = ds.clu_rbig;
+        dd.grid_k2_max = ds.grid_k2_max;
+        dd.grid_items = keep_grid ? items[i] : nullptr;
+        if (!keep_grid) dd.grid_cells = nullptr;
+    }
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));
+        if (stats) {
+            float ms = 0.f;
+            CK(ctx, cudaEventElapsedTime(&ms, d.ev_u0, d.ev_u1));
+            stats->render_ms[i] = ms;
+        }
+    }
+    if (stats) stats->gpu_launches = (unsigned long long)launches;
+    ctx->scene_ds = ds;
+    ctx->scene_grid = keep_grid;
+    ctx->scene_key.clear();        // the staged blob no longer matches the devices: the next upload rebuilds
+    ctx->cut_valid = false;
+    ctx->costs_valid = false;
+    return TCRT_OK;
+}
+
+extern "C" {
+
+int tcrt_update_spheres(tcrt_ctx* ctx, const float* sphere_geom, tcrt_stats* stats) {
+    return update_impl(ctx, -1, sphere_geom, stats);
+}
+
+int tcrt_update_spheres_device(tcrt_ctx* ctx, int device_slot, const float* sphere_geom, tcrt_stats* stats) {
+    if (ctx && device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
+    return update_impl(ctx, device_slot, sphere_geom, stats);
 }
 
 }  // extern "C"

@@ -263,7 +263,10 @@ bool tcrt_build_sphere_grid(const std::vector<float>& boxes, int n, TcrtSphereGr
         g.lo[k] = (float)lo[k];
         g.cell[k] = (float)cs[k];
         g.dims[k] = dims[k];
+        g.lo_d[k] = lo[k];
+        g.cell_d[k] = cs[k];
     }
+    g.reg_margin_d = margin;
     g.reg_margin = (float)(0.5 * margin);     // what a ray's fattening may be: half of what the registration allowed for
     return true;
 }

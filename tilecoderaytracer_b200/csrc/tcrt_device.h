@@ -88,6 +88,11 @@ struct TcrtSphereGrid {
     float reg_margin = 0.f;             // a ray whose fattening is below this may use the grid
     std::vector<int> cell_start;        // dims[0]*dims[1]*dims[2] + 1
     std::vector<int> items;             // sphere slots (leaf order), cell by cell
+    // the registration's own arithmetic (double): a sphere's box, widened by reg_margin_d, is registered in the cells
+    // floor((box - reg_margin_d - lo_d) / cell_d) .. floor((box + reg_margin_d - lo_d) / cell_d), clamped to the grid
+    double lo_d[3] = {0, 0, 0};
+    double cell_d[3] = {1, 1, 1};
+    double reg_margin_d = 0.0;
 };
 bool tcrt_build_sphere_grid(const std::vector<float>& boxes, int n, TcrtSphereGrid& g);
 #endif
@@ -169,6 +174,61 @@ struct OccLaunch {
     const float* points;
     unsigned char* out;
 };
+
+// Sphere updates (tcrt_update.cu, tcrt_update_spheres): the resident scene's spheres take new geometry in place; the
+// sphere BVH is refitted and the sphere grid re-registered.  What the launches reduce for the host, in `back`:
+struct UpdateBack {
+    unsigned invalid;            // != 0: a centre component or radius_squared is not finite, or radius_squared < 0
+    unsigned ext_bits;           // max |centre component| over every sphere (float bits)
+    unsigned r2min_key;          // ~bits of the smallest radius_squared over the BVH's spheres (atomicMax of the inverse)
+    unsigned grid_out;           // != 0: a registered sphere's widened box leaves the grid's box
+    unsigned grid_full;          // != 0: more than 8 registrations per sphere, or more than 24 in one cell
+    unsigned lo_key[3];          // ~order key of the smallest box coordinate per axis over the boxed spheres (0: none)
+    unsigned hi_key[3];          // order key of the largest one (0: none)
+    unsigned pad[5];
+    // then 3 floats per light sphere (UpdateLaunch::light_sph): its new centre
+};
+struct UpdateLaunch {
+    const float4* geom;          // n x (centre, radius_squared), in the order of tcrt_scene.sphere_geom
+    int n;
+    const int* slot_of;          // sphere i -> its slot in the blob's sphere array
+    float4* spheres;             // the blob's sphere array
+    int n_boxed;                 // slots [0, n_boxed) have boxes that count in the bounds
+    int n_bvh;                   // slots [0, n_bvh) are the sphere BVH's leaves (0: no BVH)
+    double ext_fixed;            // max(1, |finite-plane origins|), kept from the upload
+    const int* light_sph;        // n_light_sph sphere indices whose centres go back to the host
+    int n_light_sph;
+    UpdateBack* back;            // zeroed before the launches
+    float* boxes;                // 6 per boxed slot (lo xyz, hi xyz)
+    // sphere BVH: inner nodes level by level from the root (levels[level_start[l] .. level_start[l + 1]))
+    float4* nodes;
+    const int* levels;
+    const int* level_start;
+    int n_levels;
+    // sphere grid (grid == 0: none, or dropped): the builder's registration arithmetic, tcrt_build_sphere_grid
+    int grid;
+    double glo[3], gcell[3], gmargin;
+    int gdims[3];
+    int n_cells;
+    unsigned cap;                // room for registrations: 8 per grid sphere
+    unsigned long long* reg_count;   // n_bvh + 1: registrations per sphere, then their exclusive scan in reg_off
+    unsigned long long* reg_off;
+    unsigned* keys;              // cap (cell, slot) pairs, then sorted by cell into keys2 / sorted (scratch)
+    unsigned* vals;
+    unsigned* keys2;
+    unsigned* sorted;
+    int* items;                  // the grid's item list the scene reads: `sorted`, copied by the last launch after the checks
+    unsigned* cell_count;        // n_cells + 1, then the exclusive scan in cell_start
+    unsigned* cell_start;
+    float4* cells;               // the blob's cell records
+    void* tmp;                   // CUB scratch, tcrt_update_tmp_bytes
+    size_t tmp_bytes;
+};
+// bytes of CUB scratch the grid re-registration needs
+size_t tcrt_update_tmp_bytes(unsigned cap, int n_bvh, int n_cells);
+// the whole update on one stream: validate and reduce, scatter and box, refit, re-register (nothing written to the scene
+// when the input is invalid); *launches += kernels launched
+cudaError_t tcrt_launch_update_spheres(const UpdateLaunch& ul, int sm_count, cudaStream_t stream, int* launches);
 
 // host builder of the box clusters (tcrt_cluster.cpp).  Face f = 2*axis + k; an absent face has
 // c = NaN and plane = -1; `plane` indexes the caller's list.

@@ -55,6 +55,34 @@ public:
     // moving spheres (tcrt_update_spheres): geom[4*i .. 4*i+3] = centre xyz and radius*radius of sphere i, in the order of
     // the scene given to setScene; the scene stays resident, the GPU refits its structures
     int updateSpheres(const float* geom, tcrt_stats* stats = NULL) { return rc_ = tcrt_update_spheres(ctx_, geom, stats); }
+    // material edits (tcrt_update_materials, tcrt_update_textures): `scene` is the scene given to setScene, edited with the
+    // ObjMaterial / SceneObject setters; the colour, factors, intensity and texture id of objects[0 .. n) and every checker
+    // row are sent.  A scene whose counts, lights or number of textures differ from the uploaded one: TCRT_ERR_INVALID
+    // (that takes setScene).  stats: of the objects' rows.
+    int updateMaterials(const Scene& scene, const int* objects, int n, tcrt_stats* stats = NULL) {
+        SceneFlattener f;
+        scene.flatten(f);
+        if (f.n_objects != flat_.n_objects || f.sphere_obj.size() != flat_.sphere_obj.size() ||
+            f.fin_obj.size() != flat_.fin_obj.size() || f.inf_obj.size() != flat_.inf_obj.size() ||
+            f.light_obj != flat_.light_obj || f.textures.size() != flat_.textures.size() || n < 0 || (n > 0 && !objects))
+            return rc_ = TCRT_ERR_INVALID;
+        std::vector<float> surface(4 * (size_t)n), material(4 * (size_t)n);
+        std::vector<int> texture(n);
+        for (int i = 0; i < n; i++) {
+            const int o = objects[i];
+            if (o < 0 || o >= f.n_objects) return rc_ = TCRT_ERR_INVALID;
+            for (int k = 0; k < 4; k++) {
+                surface[4 * i + k] = f.obj_surface[4 * o + k];
+                material[4 * i + k] = f.obj_material[4 * o + k];
+            }
+            texture[i] = f.obj_info[4 * o + 3];
+        }
+        if (n > 0 && (rc_ = tcrt_update_materials(ctx_, n, objects, surface.data(), material.data(), texture.data(), stats)))
+            return rc_;
+        std::vector<int> ids(f.textures.size() / 8);
+        for (size_t t = 0; t < ids.size(); t++) ids[t] = (int)t;
+        return rc_ = ids.empty() ? TCRT_OK : tcrt_update_textures(ctx_, (int)ids.size(), ids.data(), f.textures.data(), NULL);
+    }
     // the pixel loop (RayTracer.cpp:911-923): pixels[x][z] -> pixels_xmajor[(x*H + z)*3 + c]; with rs.samples > 1 each
     // pixel is the mean of rs.samples x rs.samples samples (tcrt_render_columns_ss), with rs.contrast >= 0 only the pixels
     // at contrast edges (tcrt_render_columns_adaptive)

@@ -221,6 +221,32 @@ int tcrt_plan_dead_paths(const tcrt_scene* scene, const tcrt_params* params, int
 int tcrt_update_spheres(tcrt_ctx* ctx, const float* sphere_geom, tcrt_stats* stats);
 int tcrt_update_spheres_device(tcrt_ctx* ctx, int device_slot, const float* sphere_geom, tcrt_stats* stats);
 
+/* Material edits (multi-frame mode): new colours, shading factors, light intensities, texture ids and checker rows for
+ * objects of the resident scene, written on the devices without rebuilding the scene.
+ * tcrt_update_materials: objects[i] is an object index of the last tcrt_upload_scene; its new rows are surface[4i ..]
+ * (colour r g b, diffuse_factor: the layout of tcrt_scene.obj_surface), material[4i ..] (specular, reflective,
+ * intensity, w: the layout of obj_material, w ignored) and texture[i] (a texture id in [-1, n_textures)).  Any of
+ * surface, material and texture may be NULL, which leaves that part of every listed object unchanged; all three NULL is
+ * TCRT_ERR_INVALID.  tcrt_update_textures: textures[i] is a texture id, rows[8i ..] its new checker row in the layout of
+ * tcrt_scene.textures.
+ * After either call every call that reads the scene (frames in every form, async frames, multi-view frames, ray batches,
+ * tcrt_balance_columns) returns, bit for bit, what it returns after tcrt_upload_scene of the uploaded scene (with the
+ * spheres of any tcrt_update_spheres since) with those rows replaced.  Hit buffers, tcrt_pick and the occlusion queries
+ * do not read materials.  Float values are not checked, as the upload does not check them: NaN, inf, -0 and negative
+ * factors render as the reference renders them.  Which objects are lights and how many textures there are stay as
+ * uploaded: making an object a light, or giving it a new checker, needs tcrt_upload_scene.
+ * Validation: an object or texture index out of range, an index listed twice in one call, a texture id out of range,
+ * n < 0 or a NULL array with n > 0: TCRT_ERR_INVALID, and nothing changes on any device.  Before any upload:
+ * TCRT_ERR_NO_SCENE.  n == 0: TCRT_OK, nothing launched.
+ * Ordering, as for tcrt_update_spheres: the edit is queued on each device's render stream (frames queued before it see
+ * the old materials), the call returns once frames in flight have finished, it invalidates the balanced cut and cost
+ * map, makes the next tcrt_upload_scene rebuild even an unchanged scene, and leaves the last render, the writers and
+ * tcrt_device_frame alone.
+ * stats (may be NULL): render_ms per device is the edit's device time, gpu_launches its launches, no rays. */
+int tcrt_update_materials(tcrt_ctx* ctx, int n, const int* objects, const float* surface, const float* material,
+                          const int* texture, tcrt_stats* stats);
+int tcrt_update_textures(tcrt_ctx* ctx, int n, const int* textures, const float* rows, tcrt_stats* stats);
+
 /* ---- render (replaces the pixel loop RayTracer.cpp:911-923) ----------------------- */
 /* Whole image -> host_rgb[width*height*3], x-major, z fastest, (r,g,b) float32: the layout
  * of the reference's pixels[W][H] (RayTracer.h:44).  stats may be NULL.  host_rgb may be pinned (tcrt_alloc_host,

@@ -139,6 +139,9 @@ SIGNATURES = {
                                            C.c_void_p, C.POINTER(TcrtStats)]),
     "tcrt_update_spheres": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(TcrtStats)]),
     "tcrt_update_spheres_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(TcrtStats)]),
+    "tcrt_update_materials": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.POINTER(TcrtStats)]),
+    "tcrt_update_textures": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(TcrtStats)]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),
     "tcrt_bands_from_costs": (C.c_int, [C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),

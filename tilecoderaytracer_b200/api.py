@@ -267,6 +267,22 @@ def sphere_geom(centres, radii) -> np.ndarray:
     return out
 
 
+def material_rows(flat, objects):
+    """The (surface, material, texture) rows of `objects` in a flattened scene, as Context.update_materials takes them:
+    (n, 4) float32 (colour rgb, diffuse), (n, 4) float32 (specular, reflective, intensity, 0) and (n,) int32 texture ids.
+    Edit a host Scene with the reference's setters, flatten it, and send the rows of the objects that changed."""
+    idx = np.asarray(objects, dtype=np.int64).reshape(-1)
+    n = flat.n_objects
+    assert ((idx >= 0) & (idx < n)).all(), "object index out of range"
+    if n == 0:
+        return np.zeros((0, 4), np.float32), np.zeros((0, 4), np.float32), np.zeros(0, np.int32)
+    surface = np.ctypeslib.as_array(flat.obj_surface, (n * 4,)).reshape(n, 4)
+    material = np.ctypeslib.as_array(flat.obj_material, (n * 4,)).reshape(n, 4)
+    info = np.ctypeslib.as_array(flat.obj_info, (n * 4,)).reshape(n, 4)
+    return (np.ascontiguousarray(surface[idx], np.float32), np.ascontiguousarray(material[idx], np.float32),
+            np.ascontiguousarray(info[idx, 3], np.int32))
+
+
 def normalize_like_reference(v) -> np.ndarray:
     """vector3d::normalize in numpy float32, as a Ray's constructor applies it: len = sqrtf((x*x + y*y) + z*z), then three
     IEEE divisions.  The ray-batch calls take directions as a Ray stores them; this turns raw directions (..., 3) into
@@ -788,6 +804,35 @@ class Context:
         pointer that is not 16-byte aligned raises TcrtError (TCRT_ERR_INVALID)."""
         st = TcrtStats()
         self._ck(self._lib.tcrt_update_spheres_device(self._h, slot, C.c_void_p(ptr or None), C.byref(st)))
+        return RenderStats.from_c(st)
+
+    def update_materials(self, objects, surface=None, material=None, texture=None) -> RenderStats:
+        """Material edits (tcrt_update_materials): new rows for the listed objects of the resident scene — surface (n, 4)
+        float32 (colour rgb, diffuse), material (n, 4) float32 (specular, reflective, intensity, ignored), texture (n,)
+        int32 ids in [-1, n_textures) — each None to leave that part alone (material_rows() forms them).  Every later
+        call sees the uploaded scene with those rows replaced, bit for bit.  Which objects are lights and the number of
+        textures stay.  Waits for frames in flight.  Returns RenderStats (render_ms: the edit's device time)."""
+        obj = np.ascontiguousarray(objects, dtype=np.int32).reshape(-1)
+        n = obj.shape[0]
+
+        parts = [None if a is None else np.asarray(a) for a in (surface, material, texture)]
+        for a, dtype, shape in zip(parts, (np.float32, np.float32, np.int32), ((n, 4), (n, 4), (n,))):
+            assert a is None or (a.dtype == dtype and a.shape == shape and a.flags["C_CONTIGUOUS"]), \
+                f"{shape} {np.dtype(dtype).name}"
+        ptrs = [None if a is None else C.c_void_p(a.ctypes.data) for a in parts]
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_update_materials(self._h, n, obj.ctypes.data_as(C.c_void_p), *ptrs, C.byref(st)))
+        return RenderStats.from_c(st)
+
+    def update_textures(self, ids, rows) -> RenderStats:
+        """Checker edits (tcrt_update_textures): rows (n, 8) float32 (light rgb, width, dark rgb, height) for the texture
+        ids `ids` of the resident scene, the layout of the flattened scene's textures."""
+        t = np.ascontiguousarray(ids, dtype=np.int32).reshape(-1)
+        r = np.asarray(rows)
+        assert r.dtype == np.float32 and r.shape == (t.shape[0], 8) and r.flags["C_CONTIGUOUS"], "rows: (n, 8) float32"
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_update_textures(self._h, t.shape[0], t.ctypes.data_as(C.c_void_p),
+                                                r.ctypes.data_as(C.c_void_p), C.byref(st)))
         return RenderStats.from_c(st)
 
     def set_camera(self, cam: TcrtCamera) -> None:

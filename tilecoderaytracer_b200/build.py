@@ -34,7 +34,7 @@ NVCC_FLAGS = [
 CXX_FLAGS = ["-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-Wall"]
 INCLUDES = ["-I", os.path.join(ROOT, "include"), "-I", os.path.join(ROOT, "scenes")]
 
-CUDA_SOURCES = ["tcrt_render.cu", "tcrt_render_grid.cu", "tcrt_render_wave.cu", "tcrt_render_pool.cu", "tcrt_hits.cu", "tcrt_adaptive.cu", "tcrt_update.cu", "tcrt_format.cu", "tcrt_api.cu", "tcrt_bvh.cpp", "tcrt_cluster.cpp"]
+CUDA_SOURCES = ["tcrt_render.cu", "tcrt_render_grid.cu", "tcrt_render_wave.cu", "tcrt_render_pool.cu", "tcrt_hits.cu", "tcrt_adaptive.cu", "tcrt_update.cu", "tcrt_materials.cu", "tcrt_format.cu", "tcrt_api.cu", "tcrt_bvh.cpp", "tcrt_cluster.cpp"]
 HOST_SOURCES = ["host_scene.cpp", "host_capi.cpp"]
 
 

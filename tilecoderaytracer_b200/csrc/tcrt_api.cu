@@ -159,7 +159,13 @@ struct DeviceState {
     size_t upd_boxes_cap = 0;                      // floats
     unsigned char* upd_grid = nullptr;
     size_t upd_grid_cap = 0;
-    cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;  // around the update's launches (render stream)
+    cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;  // around the update's launches (render stream), or a material edit's
+    // material edits (tcrt_update_materials): the object -> light map of the upload numbered mat_serial, and the records
+    unsigned long long mat_serial = 0;
+    int* mat_light_of = nullptr;
+    size_t mat_light_of_cap = 0;                   // ints
+    MaterialRecord* mat_rec = nullptr;
+    size_t mat_rec_cap = 0;
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -268,6 +274,31 @@ struct UpdatePlan {
     std::vector<int> light_of_sph;       // the light each of those is
 };
 
+// What material edits (tcrt_update_materials, tcrt_update_textures) need of the last upload: a host copy of the scene's
+// materials, with every edit merged in, and which light each object is.
+struct MaterialShadow {
+    std::vector<float> surface, material;   // obj_surface, obj_material
+    std::vector<int> info;                  // obj_info: is_light and texture id are what the materials read
+    std::vector<float> textures;
+    std::vector<int> light_obj;
+    std::vector<int> light_of;              // object index -> its light, -1 for the other objects
+    int n_objects() const { return (int)(surface.size() / 4); }
+    int n_textures() const { return (int)(textures.size() / 8); }
+    // the parts of the scene dead_path_bound reads
+    tcrt_scene view() const {
+        tcrt_scene s{};
+        s.n_objects = n_objects();
+        s.n_lights = (int)light_obj.size();
+        s.n_textures = n_textures();
+        s.obj_surface = surface.data();
+        s.obj_material = material.data();
+        s.obj_info = info.data();
+        s.light_obj = light_obj.data();
+        s.textures = textures.data();
+        return s;
+    }
+};
+
 }  // namespace
 
 static void destroy_copy_pipe(tcrt_ctx* ctx);
@@ -315,8 +346,10 @@ struct tcrt_ctx {
     bool scene_bvh_s = false, scene_bvh_f = false, scene_grid = false;
     DeadPathBound scene_dead;
     UpdatePlan scene_upd;           // what tcrt_update_spheres needs of the last upload
-    unsigned long long scene_serial = 0;   // bumped by every new blob (DeviceState::upd_serial)
-    float4* upd_stage = nullptr;    // pinned: the input of tcrt_update_spheres, then the light rows it rewrites
+    MaterialShadow scene_mat;       // what tcrt_update_materials and tcrt_update_textures need of it
+    unsigned long long scene_serial = 0;   // bumped by every new blob (DeviceState::upd_serial, mat_serial)
+    float4* upd_stage = nullptr;    // pinned: the input of tcrt_update_spheres, then the light rows it rewrites; the
+                                    // packed records of a material edit
     size_t upd_stage_cap = 0;       // float4s
 };
 
@@ -409,6 +442,8 @@ void free_device(DeviceState& d) {
     cudaFreeHost(d.h_upd_back);
     cudaFree(d.upd_boxes);
     cudaFree(d.upd_grid);
+    cudaFree(d.mat_light_of);
+    cudaFree(d.mat_rec);
     for (cudaEvent_t e : {d.ev_u0, d.ev_u1})
         if (e) cudaEventDestroy(e);
     for (cudaEvent_t e : {d.ev_r0, d.ev_r1, d.ev_rc})
@@ -1090,6 +1125,17 @@ static int build_scene_blob(tcrt_ctx* ctx, const tcrt_scene* s) {
     ctx->scene_bvh_f = b.bvh_f;
     ctx->scene_dead = dead_path_bound(s);
     ctx->scene_upd = std::move(b.upd);
+    {
+        const int n = s->n_objects;
+        MaterialShadow& m = ctx->scene_mat;
+        m.surface.assign(s->obj_surface, s->obj_surface + 4 * (size_t)n);
+        m.material.assign(s->obj_material, s->obj_material + 4 * (size_t)n);
+        m.info.assign(s->obj_info, s->obj_info + 4 * (size_t)n);
+        m.textures.assign(s->textures, s->textures + 8 * (size_t)s->n_textures);
+        m.light_obj.assign(s->light_obj, s->light_obj + s->n_lights);
+        m.light_of.assign(n, -1);
+        for (int l = 0; l < s->n_lights; l++) m.light_of[s->light_obj[l]] = l;
+    }
     ctx->scene_serial++;
     return TCRT_OK;
 }
@@ -3389,6 +3435,17 @@ static size_t carve(size_t& off, size_t bytes) {
     return at;
 }
 
+// ctx->upd_stage with room for `f4` float4s
+static int ensure_upd_stage(tcrt_ctx* ctx, size_t f4) {
+    if (f4 <= ctx->upd_stage_cap) return TCRT_OK;
+    if (ctx->upd_stage) cudaFreeHost(ctx->upd_stage);
+    ctx->upd_stage = nullptr;
+    ctx->upd_stage_cap = 0;
+    CK(ctx, cudaHostAlloc((void**)&ctx->upd_stage, f4 * sizeof(float4), cudaHostAllocPortable));
+    ctx->upd_stage_cap = f4;
+    return TCRT_OK;
+}
+
 static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* stats) {
     if (!ctx || !geom) return fail(ctx, TCRT_ERR_INVALID, "null argument");
     if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
@@ -3413,14 +3470,7 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
     const int n_bvh = ds0.n_sph_bvh, n_ls = (int)up.light_sph.size(), n_levels = (int)up.level_start.size() - 1;
     const unsigned cap = 8u * (unsigned)n_bvh;
     const size_t back_bytes = sizeof(UpdateBack) + 12 * (size_t)n_ls;
-    const size_t stage_f4 = std::max((size_t)n, 2 * (size_t)ds0.n_lights);
-    if (stage_f4 > ctx->upd_stage_cap) {
-        if (ctx->upd_stage) cudaFreeHost(ctx->upd_stage);
-        ctx->upd_stage = nullptr;
-        ctx->upd_stage_cap = 0;
-        CK(ctx, cudaHostAlloc((void**)&ctx->upd_stage, stage_f4 * sizeof(float4), cudaHostAllocPortable));
-        ctx->upd_stage_cap = stage_f4;
-    }
+    if (int rc = ensure_upd_stage(ctx, std::max((size_t)n, 2 * (size_t)ds0.n_lights))) return rc;
     if (slot < 0) memcpy(ctx->upd_stage, geom, (size_t)n * sizeof(float4));
     int launches = 0;
     std::vector<int*> items(nd, nullptr);
@@ -3603,6 +3653,147 @@ int tcrt_update_spheres(tcrt_ctx* ctx, const float* sphere_geom, tcrt_stats* sta
 int tcrt_update_spheres_device(tcrt_ctx* ctx, int device_slot, const float* sphere_geom, tcrt_stats* stats) {
     if (ctx && device_slot < 0) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range", device_slot);
     return update_impl(ctx, device_slot, sphere_geom, stats);
+}
+
+}  // extern "C"
+
+// ---- material edits (tcrt_update_materials, tcrt_update_textures) ------------------------------------------------------------
+// New colours, shading factors, intensities, texture ids and checker rows for the resident scene.  The host checks the input
+// against its copy of the materials (ctx->scene_mat) before anything changes, merges it in and packs full rows;
+// tcrt_materials.cu scatters them on every device.  The dead-path bound is the only host state derived from materials, and
+// it is recomputed from the copy.  DESIGN.md §4.3.
+
+// The n records packed in ctx->upd_stage -> every device: one copy and one scatter launch each, on the render stream after
+// the frames queued before the call.
+static int send_material_records(tcrt_ctx* ctx, int n, tcrt_stats* stats) {
+    const MaterialShadow& m = ctx->scene_mat;
+    const int nd = (int)ctx->devs.size();
+    int launches = 0;
+    for (auto& d : ctx->devs) {
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));   // frames queued before the call finish with the old materials
+        if (!d.ev_u0) CK(ctx, cudaEventCreate(&d.ev_u0));
+        if (!d.ev_u1) CK(ctx, cudaEventCreate(&d.ev_u1));
+        int rc = ensure(ctx, d.mat_light_of, d.mat_light_of_cap, std::max(m.light_of.size(), (size_t)1));
+        if (rc) return rc;
+        if (d.mat_serial != ctx->scene_serial) {   // the map, once per upload
+            CK(ctx, cudaMemcpy(d.mat_light_of, m.light_of.data(), m.light_of.size() * sizeof(int), cudaMemcpyHostToDevice));
+            d.mat_serial = ctx->scene_serial;
+        }
+        if ((rc = ensure(ctx, d.mat_rec, d.mat_rec_cap, (size_t)n))) return rc;
+        CK(ctx, cudaMemcpyAsync(d.mat_rec, ctx->upd_stage, (size_t)n * sizeof(MaterialRecord), cudaMemcpyHostToDevice, d.stream));
+        MaterialLaunch ml{};
+        ml.rec = d.mat_rec;
+        ml.n = n;
+        ml.surface = d.scene_mem + ctx->scene_off[0];
+        ml.material = d.scene_mem + ctx->scene_off[1];
+        ml.textures = d.scene_mem + ctx->scene_off[4];
+        ml.lights = d.scene_mem + ctx->scene_ds.light_off;
+        ml.light_of = d.mat_light_of;
+        CK(ctx, cudaEventRecord(d.ev_u0, d.stream));
+        CK(ctx, tcrt_launch_material_edit(ml, d.stream, &launches));
+        CK(ctx, cudaEventRecord(d.ev_u1, d.stream));
+    }
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));
+        if (stats) {
+            float ms = 0.f;
+            CK(ctx, cudaEventElapsedTime(&ms, d.ev_u0, d.ev_u1));
+            stats->render_ms[i] = ms;
+        }
+    }
+    if (stats) stats->gpu_launches = (unsigned long long)launches;
+    const tcrt_scene view = m.view();
+    ctx->scene_dead = dead_path_bound(&view);
+    ctx->scene_key.clear();        // the staged blob no longer matches the devices: the next upload rebuilds
+    ctx->cut_valid = false;        // bounce counts follow the reflective factors and the dead paths
+    ctx->costs_valid = false;
+    return TCRT_OK;
+}
+
+static void clear_stats(tcrt_ctx* ctx, tcrt_stats* stats) {
+    if (!stats) return;
+    memset(stats, 0, sizeof(*stats));
+    stats->n_devices = (int)ctx->devs.size();
+}
+
+extern "C" {
+
+int tcrt_update_materials(tcrt_ctx* ctx, int n, const int* objects, const float* surface, const float* material,
+                          const int* texture, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (n < 0) return fail(ctx, TCRT_ERR_INVALID, "n = %d is negative", n);
+    if (!surface && !material && !texture) return fail(ctx, TCRT_ERR_INVALID, "surface, material and texture are all NULL");
+    if (n > 0 && !objects) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    MaterialShadow& m = ctx->scene_mat;
+    const int n_obj = m.n_objects(), n_tex = m.n_textures();
+    std::vector<char> seen(n_obj, 0);
+    for (int i = 0; i < n; i++) {
+        const int o = objects[i];
+        if (o < 0 || o >= n_obj) return fail(ctx, TCRT_ERR_INVALID, "object index %d out of range (have %d)", o, n_obj);
+        if (seen[o]) return fail(ctx, TCRT_ERR_INVALID, "object %d is listed twice", o);
+        seen[o] = 1;
+        if (texture && (texture[i] < -1 || texture[i] >= n_tex))
+            return fail(ctx, TCRT_ERR_INVALID, "texture id %d out of range (have %d)", texture[i], n_tex);
+    }
+    clear_stats(ctx, stats);
+    if (n == 0) return TCRT_OK;
+    if (int rc = ensure_upd_stage(ctx, sizeof(MaterialRecord) / sizeof(float4) * (size_t)n)) return rc;
+    MaterialRecord* rec = reinterpret_cast<MaterialRecord*>(ctx->upd_stage);
+    UpdatePlan& up = ctx->scene_upd;
+    for (int i = 0; i < n; i++) {
+        const int o = objects[i];
+        float* sf = &m.surface[4 * (size_t)o];
+        float* mt = &m.material[4 * (size_t)o];
+        if (surface) memcpy(sf, surface + 4 * (size_t)i, 4 * sizeof(float));
+        if (material) memcpy(mt, material + 4 * (size_t)i, 3 * sizeof(float));   // w is not a material
+        if (texture) m.info[4 * (size_t)o + 3] = texture[i];
+        rec[i] = MaterialRecord{};
+        rec[i].a = make_float4(sf[0], sf[1], sf[2], sf[3]);
+        rec[i].b = make_float4(mt[0], mt[1], mt[2], mt[3]);
+        rec[i].target = o;
+        rec[i].tex = m.info[4 * (size_t)o + 3];
+        const int l = m.light_of[o];
+        if (l >= 0) {   // tcrt_update_spheres rewrites every light row from these
+            for (int k = 0; k < 3; k++) up.light_col[3 * l + k] = sf[k];
+            up.light_int[l] = mt[2];
+        }
+    }
+    return send_material_records(ctx, n, stats);
+}
+
+int tcrt_update_textures(tcrt_ctx* ctx, int n, const int* textures, const float* rows, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (n < 0) return fail(ctx, TCRT_ERR_INVALID, "n = %d is negative", n);
+    if (n > 0 && (!textures || !rows)) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    MaterialShadow& m = ctx->scene_mat;
+    const int n_tex = m.n_textures();
+    std::vector<char> seen(n_tex, 0);
+    for (int i = 0; i < n; i++) {
+        const int t = textures[i];
+        if (t < 0 || t >= n_tex) return fail(ctx, TCRT_ERR_INVALID, "texture id %d out of range (have %d)", t, n_tex);
+        if (seen[t]) return fail(ctx, TCRT_ERR_INVALID, "texture %d is listed twice", t);
+        seen[t] = 1;
+    }
+    clear_stats(ctx, stats);
+    if (n == 0) return TCRT_OK;
+    if (int rc = ensure_upd_stage(ctx, sizeof(MaterialRecord) / sizeof(float4) * (size_t)n)) return rc;
+    MaterialRecord* rec = reinterpret_cast<MaterialRecord*>(ctx->upd_stage);
+    for (int i = 0; i < n; i++) {
+        const int t = textures[i];
+        const float* row = rows + 8 * (size_t)i;
+        memcpy(&m.textures[8 * (size_t)t], row, 8 * sizeof(float));
+        rec[i] = MaterialRecord{};
+        rec[i].a = make_float4(row[0], row[1], row[2], row[3]);
+        rec[i].b = make_float4(row[4], row[5], row[6], row[7]);
+        rec[i].target = ~t;
+        rec[i].tex = -1;
+    }
+    return send_material_records(ctx, n, stats);
 }
 
 }  // extern "C"

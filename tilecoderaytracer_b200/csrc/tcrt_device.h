@@ -230,6 +230,27 @@ size_t tcrt_update_tmp_bytes(unsigned cap, int n_bvh, int n_cells);
 // when the input is invalid); *launches += kernels launched
 cudaError_t tcrt_launch_update_spheres(const UpdateLaunch& ul, int sm_count, cudaStream_t stream, int* launches);
 
+// Material edits (tcrt_materials.cu, tcrt_update_materials / tcrt_update_textures): one packed record per edited object or
+// checker row, full rows from the host's copy of the materials.
+struct MaterialRecord {
+    float4 a;                    // object: (colour rgb, diffuse); checker: (light rgb, width)
+    float4 b;                    // object: (specular, reflective, intensity, -); checker: (dark rgb, height)
+    int target;                  // object index, or ~texture id for a checker row
+    int tex;                     // object: its texture id (-1: none)
+    int pad[2];
+};
+struct MaterialLaunch {
+    const MaterialRecord* rec;
+    int n;
+    float4* surface;             // the blob's obj_surface, obj_material and texture tables, and its light table
+    float4* material;
+    float4* textures;
+    float4* lights;
+    const int* light_of;         // object index -> its light (-1: not a light), uploaded once per upload
+};
+// the scatter launch (nothing when n == 0); *launches += kernels launched
+cudaError_t tcrt_launch_material_edit(const MaterialLaunch& ml, cudaStream_t stream, int* launches);
+
 // host builder of the box clusters (tcrt_cluster.cpp).  Face f = 2*axis + k; an absent face has
 // c = NaN and plane = -1; `plane` indexes the caller's list.
 struct TcrtBoxCluster {

@@ -8,7 +8,7 @@ flags are read from each translation unit that launches a kernel: render, grid a
 invalid rays on a grid scene and a BVH scene, traced and intersected, against tests/oracle_rays.c, and the occlusion queries
 (points against every light, rays with their limits) on a grid scene, BVH scenes and box-cluster scenes against
 tests/oracle_occlusion.c, and multi-view frames on a grid scene, a BVH scene and a box-cluster scene, with a piece
-boundary inside a view.
+boundary inside a view, and one scene of every dispatch class after a material edit (tests/test_material_edits.py).
 usage: python -c "from tilecoderaytracer_b200 import build; build.build_lib(defines=('TCRT_CHECKED',), out=LIB)"
        TCRT_LIB=LIB python tools/checked_run.py"""
 import ctypes as C
@@ -257,4 +257,24 @@ for name, want_cls in (("synth256", ("grid", 1, 0)), ("random:24:200", ("render"
     bad_total += bad + len(f)
     print(f"views {name:14s} {str(want_cls):16s} 3 views of 48x40, 13x11 and 1500x1024, d0/8/50: mismatches {bad}, "
           f"checks fired: {f or 'none'}", flush=True)
+
+# ---- material edits: one edited scene per dispatch class (a third of the objects and every checker row), against the oracle
+import test_material_edits as ME  # noqa: E402
+
+for name in V.NAMES:
+    sc, cam = V.build(name)
+    flat, c = sc.flatten(), cam.export()
+    ctx.upload_flat(flat, c)
+    e = ME.random_edit(flat, np.random.default_rng(7))
+    e.apply(ctx)
+    edited = e.flat(flat)
+    bad = int(V.dispatch_class(ctx.scene_structures()) != V.VARIANTS[name][3])
+    for d in (0, 8):
+        p = api.default_params(27, 17, d)
+        img, st = ctx.render(p)
+        ref, cnt = O.render(edited, c, p)
+        bad += n_bad(img, ref) + int(counters_differ(st, cnt))
+    f = fired()
+    bad_total += bad + len(f)
+    print(f"material edit {name:9s} 27x17 d0/8: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
 print("CHECKED_OK" if bad_total == 0 else "CHECKED_FAIL")

@@ -83,6 +83,30 @@ public:
         for (size_t t = 0; t < ids.size(); t++) ids[t] = (int)t;
         return rc_ = ids.empty() ? TCRT_OK : tcrt_update_textures(ctx_, (int)ids.size(), ids.data(), f.textures.data(), NULL);
     }
+    // moving planes (tcrt_update_planes): `moved` is a scene built in the object order of the scene given to setScene, with
+    // some planes constructed elsewhere; the geometry, normals and origin of objects[0 .. n) are sent.  A scene whose
+    // counts, object types or lights differ from the uploaded one, or an object that is not a plane: TCRT_ERR_INVALID
+    // (that takes setScene).
+    int updatePlanes(const Scene& moved, const int* objects, int n, tcrt_stats* stats = NULL) {
+        SceneFlattener f;
+        moved.flatten(f);
+        if (f.n_objects != flat_.n_objects || f.sphere_obj.size() != flat_.sphere_obj.size() ||
+            f.fin_obj.size() != flat_.fin_obj.size() || f.inf_obj.size() != flat_.inf_obj.size() ||
+            f.light_obj != flat_.light_obj || n < 0 || (n > 0 && !objects))
+            return rc_ = TCRT_ERR_INVALID;
+        for (int o = 0; o < f.n_objects; o++)
+            if (f.obj_info[4 * o] != flat_.obj_info[4 * o]) return rc_ = TCRT_ERR_INVALID;
+        std::vector<float> geom(16 * (size_t)n), normals(8 * (size_t)n), origin(4 * (size_t)n);
+        for (int i = 0; i < n; i++) {
+            const int o = objects[i];
+            if (o < 0 || o >= f.n_objects || f.obj_info[4 * o] == TCRT_SPHERE) return rc_ = TCRT_ERR_INVALID;
+            const std::vector<float>& rows = f.obj_info[4 * o] == TCRT_FINITE_PLANE ? f.fin_geom : f.inf_geom;
+            for (int k = 0; k < 16; k++) geom[16 * i + k] = rows[16 * (size_t)f.obj_info[4 * o + 1] + k];
+            for (int k = 0; k < 8; k++) normals[8 * i + k] = f.obj_normals[8 * (size_t)o + k];
+            for (int k = 0; k < 4; k++) origin[4 * i + k] = f.obj_origin[4 * (size_t)o + k];
+        }
+        return rc_ = tcrt_update_planes(ctx_, n, objects, geom.data(), normals.data(), origin.data(), stats);
+    }
     // the pixel loop (RayTracer.cpp:911-923): pixels[x][z] -> pixels_xmajor[(x*H + z)*3 + c]; with rs.samples > 1 each
     // pixel is the mean of rs.samples x rs.samples samples (tcrt_render_columns_ss), with rs.contrast >= 0 only the pixels
     // at contrast edges (tcrt_render_columns_adaptive)

@@ -199,7 +199,7 @@ int tcrt_plan_dead_paths(const tcrt_scene* scene, const tcrt_params* params, int
  * batches, occlusion queries, multi-view frames, tcrt_balance_columns) returns, bit for bit, what it returns after
  * tcrt_upload_scene of the uploaded scene with sphere_geom replaced by the input and each sphere's obj_origin row
  * replaced by its new centre (for a light sphere: the light's position).  Planes, materials, textures, lights and counts
- * are unchanged.
+ * are unchanged (planes move with tcrt_update_planes, materials with tcrt_update_materials).
  * The sphere BVH keeps its topology and has its boxes refitted; the sphere grid keeps its origin, cell size and
  * dimensions and has its cells registered again.  The grid is dropped (tcrt_scene_structures info[1] = 0; the sphere-BVH
  * kernel serves the scene) when a sphere's widened box leaves the grid's box or the registrations break the builder's
@@ -246,6 +246,35 @@ int tcrt_update_spheres_device(tcrt_ctx* ctx, int device_slot, const float* sphe
 int tcrt_update_materials(tcrt_ctx* ctx, int n, const int* objects, const float* surface, const float* material,
                           const int* texture, tcrt_stats* stats);
 int tcrt_update_textures(tcrt_ctx* ctx, int n, const int* textures, const float* rows, tcrt_stats* stats);
+
+/* Moving planes (multi-frame mode): new geometry for finite and infinite planes of the resident scene — a box, a door or
+ * a wall dragged in an editor, a room opened or a floor tilted by an animation — written on the devices without rebuilding
+ * the scene.  objects[i] is the object index of a finite or an infinite plane of the last tcrt_upload_scene; its new rows
+ * are geom[16i ..] (the layout of tcrt_scene.fin_geom or inf_geom, by the object's type), normals[8i ..] (its obj_normals
+ * row: facing normal, then reverse normal) and origin[4i ..] (its obj_origin row: SceneObject::origin, for a light the
+ * light's position; for a plane built from three corners the far corner, which geom does not determine).
+ * After the call every call that reads the scene (frames in every form, async frames, multi-view frames, hit buffers,
+ * tcrt_pick, ray batches, occlusion queries, tcrt_balance_columns) returns, bit for bit, what it returns after
+ * tcrt_upload_scene of the uploaded scene (with the sphere updates and material edits since) with those three rows of
+ * each listed object replaced.  Float values are not checked, as the upload does not check them: NaN, inf and
+ * degenerate planes render as the reference renders them.  Counts, object types, which objects are lights, materials and
+ * textures stay as uploaded; spheres move with tcrt_update_spheres.
+ * The finite-plane BVH keeps its topology and has its boxes refitted; a box cluster keeps its members and gets the hull
+ * of their new rectangles.  The clusters are dropped (tcrt_scene_structures info[3] = info[4] = 0; the linear sweep takes
+ * their rectangles) when a member is no longer an axis-aligned rectangle with its face's normal axis; they stay dropped
+ * until the next tcrt_upload_scene, which is also how to re-optimise a scene that has drifted far.  When the moved planes
+ * raise the scene's extent, the spheres' boxes are widened in the same call, which may drop the sphere grid as
+ * tcrt_update_spheres does.
+ * Validation: an object index out of range, one that is a sphere, one listed twice, n < 0 or a NULL array with n > 0:
+ * TCRT_ERR_INVALID, and nothing changes on any device.  Before any upload: TCRT_ERR_NO_SCENE.  n == 0: TCRT_OK, nothing
+ * launched.
+ * Ordering, as for tcrt_update_spheres: the update is queued on each device's render stream (frames queued before it see
+ * the old planes), the call returns once frames in flight have finished, it invalidates the balanced cut and cost map,
+ * makes the next tcrt_upload_scene rebuild even an unchanged scene, and leaves the last render, the writers and
+ * tcrt_device_frame alone.
+ * stats (may be NULL): render_ms per device is the update's device time, gpu_launches its launches, no rays. */
+int tcrt_update_planes(tcrt_ctx* ctx, int n, const int* objects, const float* geom, const float* normals,
+                       const float* origin, tcrt_stats* stats);
 
 /* ---- render (replaces the pixel loop RayTracer.cpp:911-923) ----------------------- */
 /* Whole image -> host_rgb[width*height*3], x-major, z fastest, (r,g,b) float32: the layout

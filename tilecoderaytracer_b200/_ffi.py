@@ -142,6 +142,8 @@ SIGNATURES = {
     "tcrt_update_materials": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.POINTER(TcrtStats)]),
     "tcrt_update_textures": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(TcrtStats)]),
+    "tcrt_update_planes": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.POINTER(TcrtStats)]),
     "tcrt_flush_l2": (C.c_int, [C.c_void_p]),
     "tcrt_balance_columns": (C.c_int, [C.c_void_p, C.POINTER(TcrtParams), C.c_int, C.POINTER(C.c_int)]),
     "tcrt_bands_from_costs": (C.c_int, [C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),

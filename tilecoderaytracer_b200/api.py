@@ -283,6 +283,30 @@ def material_rows(flat, objects):
             np.ascontiguousarray(info[idx, 3], np.int32))
 
 
+def plane_rows(flat, objects):
+    """The (geom, normals, origin) rows of the planes `objects` in a flattened scene, as Context.update_planes takes them:
+    (n, 16) float32 in the layout of fin_geom or inf_geom by each object's type, (n, 8) float32 obj_normals rows (facing,
+    then reverse normal) and (n, 4) float32 obj_origin rows.  Build the moved planes with the reference's constructors in a
+    scene of the same object order, flatten it, and send the rows of the planes that moved."""
+    idx = np.asarray(objects, dtype=np.int64).reshape(-1)
+    n = flat.n_objects
+    assert ((idx >= 0) & (idx < n)).all(), "object index out of range"
+    geom = np.zeros((len(idx), 16), np.float32)
+    if n == 0:
+        return geom, np.zeros((0, 8), np.float32), np.zeros((0, 4), np.float32)
+    info = np.ctypeslib.as_array(flat.obj_info, (n * 4,)).reshape(n, 4)
+    tables = {}
+    for kind, rows, count in ((1, "fin_geom", flat.n_fin_planes), (2, "inf_geom", flat.n_inf_planes)):
+        if count:
+            tables[kind] = np.ctypeslib.as_array(getattr(flat, rows), (count * 16,)).reshape(count, 16)
+    for i, o in enumerate(idx):
+        assert info[o, 0] in tables, f"object {o} is not a plane"
+        geom[i] = tables[info[o, 0]][info[o, 1]]
+    normals = np.ctypeslib.as_array(flat.obj_normals, (n * 8,)).reshape(n, 8)
+    origin = np.ctypeslib.as_array(flat.obj_origin, (n * 4,)).reshape(n, 4)
+    return (geom, np.ascontiguousarray(normals[idx], np.float32), np.ascontiguousarray(origin[idx], np.float32))
+
+
 def normalize_like_reference(v) -> np.ndarray:
     """vector3d::normalize in numpy float32, as a Ray's constructor applies it: len = sqrtf((x*x + y*y) + z*z), then three
     IEEE divisions.  The ray-batch calls take directions as a Ray stores them; this turns raw directions (..., 3) into
@@ -833,6 +857,22 @@ class Context:
         st = TcrtStats()
         self._ck(self._lib.tcrt_update_textures(self._h, t.shape[0], t.ctypes.data_as(C.c_void_p),
                                                 r.ctypes.data_as(C.c_void_p), C.byref(st)))
+        return RenderStats.from_c(st)
+
+    def update_planes(self, objects, geom, normals, origin) -> RenderStats:
+        """Moving planes (tcrt_update_planes): new rows for the listed finite and infinite planes of the resident scene —
+        geom (n, 16) float32 (the fin_geom / inf_geom layout by type), normals (n, 8) float32, origin (n, 4) float32 —
+        as plane_rows() forms them.  Every later call sees the uploaded scene with those rows replaced, bit for bit; the
+        finite-plane BVH and the box clusters follow on the GPU.  Counts, types, lights and materials stay.  Waits for
+        frames in flight.  Returns RenderStats (render_ms: the update's device time)."""
+        obj = np.ascontiguousarray(objects, dtype=np.int32).reshape(-1)
+        n = obj.shape[0]
+        parts = [np.asarray(a) for a in (geom, normals, origin)]
+        for a, width in zip(parts, (16, 8, 4)):
+            assert a.dtype == np.float32 and a.shape == (n, width) and a.flags["C_CONTIGUOUS"], f"({n}, {width}) float32"
+        st = TcrtStats()
+        self._ck(self._lib.tcrt_update_planes(self._h, n, obj.ctypes.data_as(C.c_void_p),
+                                              *[C.c_void_p(a.ctypes.data) for a in parts], C.byref(st)))
         return RenderStats.from_c(st)
 
     def set_camera(self, cam: TcrtCamera) -> None:

@@ -166,6 +166,15 @@ struct DeviceState {
     size_t mat_light_of_cap = 0;                   // ints
     MaterialRecord* mat_rec = nullptr;
     size_t mat_rec_cap = 0;
+    // plane updates (tcrt_update_planes): the finite-plane BVH's levels of the upload numbered pl_serial, its leaf boxes,
+    // and the records
+    unsigned long long pl_serial = 0;
+    int* pl_levels = nullptr;
+    size_t pl_levels_cap = 0;                      // ints
+    float* pl_boxes = nullptr;
+    size_t pl_boxes_cap = 0;                       // floats
+    PlaneRecord* pl_rec = nullptr;
+    size_t pl_rec_cap = 0;
 };
 
 struct TxtPipe;      // worker threads of the .txt writer and of the staged copy-out (defined with the writer)
@@ -257,22 +266,96 @@ void light_rows(const float* og, float intensity, const float* colour, const std
     rows[1] = lc;
 }
 
+// The four blob rows of a box cluster (layout: tcrt_device.h)
+void cluster_rows(const TcrtBoxCluster& b, float4* rows) {
+    rows[0] = make_float4(b.lo[0], b.hi[0], b.lo[1], b.hi[1]);
+    int present = 0;
+    for (int f = 0; f < 6; f++) present |= (b.plane[f] >= 0) << f;
+    float4 b1 = make_float4(b.lo[2], b.hi[2], 0.f, 0.f);
+    memcpy(&b1.z, &present, 4);
+    rows[1] = b1;
+    rows[2] = make_float4(b.c[0], b.c[1], b.c[2], b.c[3]);
+    rows[3] = make_float4(b.c[4], b.c[5], 0.f, 0.f);
+}
+
+// The six obj_normals rows of an object from its (facing, reverse) normals n8: per side the normal n1 the collision
+// returns, n2 = normalize(n1) of Ray(point, normal) (Ray.h:21-25) and N = normalize(n2) of the specular term
+// (RayTracer.cpp:565-566) — constants of the plane, evaluated with the reference's arithmetic (sqrtf, three divisions;
+// this TU is built with -ffp-contract=off).  Shared by the upload and by plane updates, which must agree to the bit.
+void normal_rows(const float* n8, float4* rows) {
+    for (int side = 0; side < 2; side++) {
+        float v[3] = {n8[4 * side], n8[4 * side + 1], n8[4 * side + 2]};
+        for (int rep = 0; rep < 3; rep++) {
+            rows[3 * side + rep] = make_float4(v[0], v[1], v[2], 0.f);
+            volatile float len = sqrtf(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);   // vector3d.h:57-74
+            v[0] = v[0] / len;
+            v[1] = v[1] / len;
+            v[2] = v[2] / len;
+        }
+    }
+}
+
 // What a sphere update needs of the upload: where each sphere lives in the blob, the planes' constants, the BVH's levels,
-// the grid's registration arithmetic and the lights.
+// the grid's registration arithmetic and the lights.  Plane updates (tcrt_update_planes) keep it current: it describes
+// the resident scene, not only the upload.
 struct UpdatePlan {
     int n_spheres = 0;
     std::vector<int> slot_of;            // sphere i (tcrt_scene order) -> its slot in the blob's sphere array (inverse of ps)
     int n_boxed = 0;                     // slots [0, n_boxed): the spheres the upload boxed into the bounds
     double ext_fixed = 1.0;              // max(1, |finite-plane origins|)
-    SceneBounds bounds;                  // its plane part
+    double ext_sph = 0.0;                // max |sphere centre component|, of the upload or the last sphere update
+    double ext_sph_box = 1.0;            // the ext the resident sphere boxes were built with
+    double ext_fin_box = 1.0;            // the smallest ext a resident finite-plane box was built with
+    SceneBounds bounds;                  // the spheres' part and the planes' part
     std::vector<int> levels, level_start;   // the sphere BVH's inner nodes, level by level from the root
     std::vector<TcrtBoxCluster> clusters;
     TcrtSphereGrid grid;                 // lo_d, cell_d, reg_margin_d, dims (no cells or items)
     size_t n_cells = 0;
-    std::vector<float> light_og, light_col, light_int;   // 3, 3, 1 per light, as uploaded
+    std::vector<float> light_og, light_col, light_int;   // 3, 3, 1 per light, current
     std::vector<int> light_sph;          // sphere index of each light sphere, in light order
     std::vector<int> light_of_sph;       // the light each of those is
+    // planes (tcrt_update_planes): the blob's finite-plane rows by slot, each object's plane slot, the finite-plane BVH's
+    // leaf boxes (6 per slot of its prefix) and inner levels, and the layout of the rows an update writes
+    std::vector<float> fin_rows;         // 16 per finite-plane slot, as in the blob
+    std::vector<int> fin_slot_of_obj, inf_slot_of_obj;   // object -> its finite / infinite plane slot, -1 for others
+    std::vector<float> fin_boxes;
+    std::vector<int> fin_levels, fin_level_start;
+    size_t off_normals = 0, off_frame = 0;   // float4 offsets of obj_normals and inf_frame in the blob
 };
+
+// a box (lo xyz, hi xyz) into bounds lo, hi: its finite coordinates
+void grow_into(double* lo, double* hi, const float* bx) {
+    for (int k = 0; k < 3; k++) {
+        if (std::isfinite(bx[k])) lo[k] = std::min(lo[k], (double)bx[k]);
+        if (std::isfinite(bx[3 + k])) hi[k] = std::max(hi[k], (double)bx[3 + k]);
+    }
+}
+
+// ext of the upload's boxes (plan_scene_blob), from its finite-plane part and its sphere part; update_ext in tcrt_update.cu
+double scene_ext(double ext_fixed, double ext_sph) {
+    const double ext = fmax(ext_fixed, ext_sph);
+    return std::isfinite(ext) ? ext : 1e30;
+}
+
+// the level lists of a BVH's inner nodes from the root (tcrt_bvh.cpp: node 0), as the refit launch walks them
+void bvh_levels(const std::vector<float4>& nodes, std::vector<int>& levels, std::vector<int>& level_start) {
+    levels.clear();
+    level_start.assign(1, 0);
+    std::vector<int> level;
+    if (!nodes.empty()) level.push_back(0);
+    while (!level.empty()) {
+        levels.insert(levels.end(), level.begin(), level.end());
+        level_start.push_back((int)levels.size());
+        std::vector<int> next;
+        for (int node : level) {
+            int ref[2];
+            memcpy(ref, &nodes[4 * (size_t)node + 3], sizeof ref);   // (child0, child1, -, -)
+            for (int r : ref)
+                if (r >= 0) next.push_back(r);
+        }
+        level.swap(next);
+    }
+}
 
 // What material edits (tcrt_update_materials, tcrt_update_textures) need of the last upload: a host copy of the scene's
 // materials, with every edit merged in, and which light each object is.
@@ -444,6 +527,9 @@ void free_device(DeviceState& d) {
     cudaFree(d.upd_grid);
     cudaFree(d.mat_light_of);
     cudaFree(d.mat_rec);
+    cudaFree(d.pl_levels);
+    cudaFree(d.pl_boxes);
+    cudaFree(d.pl_rec);
     for (cudaEvent_t e : {d.ev_u0, d.ev_u1})
         if (e) cudaEventDestroy(e);
     for (cudaEvent_t e : {d.ev_r0, d.ev_r1, d.ev_rc})
@@ -825,17 +911,13 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
             for (int k = 0; k < 3; k++) ext = std::max(ext, fabs((double)s->fin_geom[16 * i + 12 + k]));
         upd.ext_fixed = ext;
         for (int i = 0; i < s->n_spheres; i++)
-            for (int k = 0; k < 3; k++) ext = std::max(ext, fabs((double)s->sphere_geom[4 * i + k]));
+            for (int k = 0; k < 3; k++) upd.ext_sph = std::max(upd.ext_sph, fabs((double)s->sphere_geom[4 * i + k]));
+        ext = std::max(ext, upd.ext_sph);
         if (!std::isfinite(ext)) ext = 1e30;
+        upd.ext_sph_box = upd.ext_fin_box = ext;
         const double margin = 1e-5 * ext;
         std::vector<float> boxes_s, boxes_f;
         std::vector<int> ord;
-        auto grow_into = [](double* lo, double* hi, const float* bx) {
-            for (int k = 0; k < 3; k++) {
-                if (std::isfinite(bx[k])) lo[k] = std::min(lo[k], (double)bx[k]);
-                if (std::isfinite(bx[3 + k])) hi[k] = std::max(hi[k], (double)bx[3 + k]);
-            }
-        };
         auto grow_sph = [&](const float* bx) { grow_into(bounds.sph_lo, bounds.sph_hi, bx); };
         auto grow = [&](const float* bx) { grow_into(bounds.pl_lo, bounds.pl_hi, bx); };
         if (ds.n_sph_nl >= kSphereBvhMin) {
@@ -892,6 +974,11 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
             for (int k = 0; k < ds.n_fin_nl; k++) np[k] = pf[ord[k]];
             pf.swap(np);
             ds.n_fin_bvh = ds.n_fin_nl;
+            if (!bvh_f.empty()) {   // the leaf boxes by slot, for plane updates
+                upd.fin_boxes.resize(6 * (size_t)ds.n_fin_nl);
+                for (int k = 0; k < ds.n_fin_nl; k++)
+                    memcpy(&upd.fin_boxes[6 * (size_t)k], &boxes_f[6 * (size_t)ord[k]], 6 * sizeof(float));
+            }
         }
         // Axis-aligned finite planes (every makeSceneBox face) are swept through box clusters instead
         // of one by one (tcrt_cluster.cpp); with a finite-plane BVH the BVH covers them.
@@ -983,14 +1070,7 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
         int* cslot = reinterpret_cast<int*>(&host[ds.cslot_off]);
         for (int c = 0; c < ds.n_clu; c++) {
             const TcrtBoxCluster& b = clusters[c];
-            host[ds.clu_off + 4 * c + 0] = make_float4(b.lo[0], b.hi[0], b.lo[1], b.hi[1]);
-            int present = 0;
-            for (int f = 0; f < 6; f++) present |= (b.plane[f] >= 0) << f;
-            float4 b1 = make_float4(b.lo[2], b.hi[2], 0.f, 0.f);
-            memcpy(&b1.z, &present, 4);
-            host[ds.clu_off + 4 * c + 1] = b1;
-            host[ds.clu_off + 4 * c + 2] = make_float4(b.c[0], b.c[1], b.c[2], b.c[3]);
-            host[ds.clu_off + 4 * c + 3] = make_float4(b.c[4], b.c[5], 0.f, 0.f);
+            cluster_rows(b, &host[ds.clu_off + 4 * c]);
             for (int f = 0; f < 6; f++) cslot[6 * c + f] = b.plane[f];
         }
     }
@@ -1006,21 +1086,7 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
         if (is_light(i)) flags |= (int)0x80000000u;
         memcpy(&m.w, &flags, sizeof(float));   // bit pattern, read back with __float_as_int
         host[off_material + i] = m;
-        // per side (facing, reverse): the normal n1 the collision returns, n2 = normalize(n1) of
-        // Ray(point, normal) (Ray.h:21-25) and N = normalize(n2) of the specular term
-        // (RayTracer.cpp:565-566) — constants of the plane, evaluated here with the reference's
-        // arithmetic (sqrtf, three divisions; this TU is built with -ffp-contract=off)
-        for (int side = 0; side < 2; side++) {
-            float v[3] = {s->obj_normals[8 * i + 4 * side], s->obj_normals[8 * i + 4 * side + 1],
-                          s->obj_normals[8 * i + 4 * side + 2]};
-            for (int rep = 0; rep < 3; rep++) {
-                host[off_normals + 6 * i + 3 * side + rep] = make_float4(v[0], v[1], v[2], 0.f);
-                volatile float len = sqrtf(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);   // vector3d.h:57-74
-                v[0] = v[0] / len;
-                v[1] = v[1] / len;
-                v[2] = v[2] / len;
-            }
-        }
+        normal_rows(s->obj_normals + 8 * (size_t)i, &host[off_normals + 6 * (size_t)i]);
     }
     for (int t = 0; t < s->n_textures; t++) {
         host[off_tex + 2 * t] = f4(s->textures + 8 * t);
@@ -1044,21 +1110,16 @@ static int plan_scene_blob(const tcrt_scene* s, SceneBlob& out) {
     upd.n_spheres = ds.n_sph;
     upd.slot_of.assign(ds.n_sph, 0);
     for (int k = 0; k < ds.n_sph; k++) upd.slot_of[ps[k]] = k;
-    upd.level_start.assign(1, 0);
-    std::vector<int> level;
-    if (!bvh_s.empty()) level.push_back(0);   // the root: the builder's first node
-    while (!level.empty()) {
-        upd.levels.insert(upd.levels.end(), level.begin(), level.end());
-        upd.level_start.push_back((int)upd.levels.size());
-        std::vector<int> next;
-        for (int node : level) {
-            int ref[2];
-            memcpy(ref, &bvh_s[4 * (size_t)node + 3], sizeof ref);   // (child0, child1, -, -)
-            for (int r : ref)
-                if (r >= 0) next.push_back(r);
-        }
-        level.swap(next);
-    }
+    bvh_levels(bvh_s, upd.levels, upd.level_start);
+    bvh_levels(bvh_f, upd.fin_levels, upd.fin_level_start);
+    upd.fin_rows.resize(16 * (size_t)ds.n_fin);
+    for (int k = 0; k < ds.n_fin; k++) memcpy(&upd.fin_rows[16 * (size_t)k], s->fin_geom + 16 * (size_t)pf[k], 16 * sizeof(float));
+    upd.fin_slot_of_obj.assign(n, -1);
+    upd.inf_slot_of_obj.assign(n, -1);
+    for (int k = 0; k < ds.n_fin; k++) upd.fin_slot_of_obj[s->fin_obj[pf[k]]] = k;
+    for (int k = 0; k < ds.n_inf; k++) upd.inf_slot_of_obj[s->inf_obj[pi[k]]] = k;
+    upd.off_normals = off_normals;
+    upd.off_frame = off_frame;
     upd.clusters = clusters;
     if (has_grid) {
         upd.grid = grid;
@@ -3446,34 +3507,38 @@ static int ensure_upd_stage(tcrt_ctx* ctx, size_t f4) {
     return TCRT_OK;
 }
 
-static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* stats) {
-    if (!ctx || !geom) return fail(ctx, TCRT_ERR_INVALID, "null argument");
-    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+// What the sphere launches leave for the host: the spheres' part of the bounds, whether the grid stays, the max |centre
+// component| they reduced, the lights' positions, and per device the grid's item list and the launches' device time.
+struct SpherePass {
+    SceneBounds bounds;
+    bool keep_grid = false;
+    double ext_sph = 0.0;
+    std::vector<float> og;
+    std::vector<int*> items;
+    std::vector<float> ms;
+    bool invalid = false;        // a resident sphere is not finite (a rebox): nothing was written
+};
+
+// The sphere update's launches on every device, after the frames queued before the call, and their read-back.  rebox: the
+// resident spheres stay where they are and are boxed again with the ext of ext_fixed (a plane update that raised it); geom
+// is then unused.  Nothing of the scene changes when the input is invalid.
+static int sphere_pass(tcrt_ctx* ctx, int slot, const float* geom, bool rebox, double ext_fixed, SpherePass& out,
+                       int* launches) {
     const int nd = (int)ctx->devs.size();
-    int src_dev = -1;
-    if (slot >= 0) {
-        if (slot >= nd) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range (have %d)", slot, nd);
-        src_dev = ctx->devs[slot].dev;
-        if (!on_device(geom, src_dev)) return fail(ctx, TCRT_ERR_INVALID, "sphere_geom is not device memory of slot %d's device", slot);
-        if (reinterpret_cast<uintptr_t>(geom) % 16 != 0)   // the launches read it as float4
-            return fail(ctx, TCRT_ERR_INVALID, "sphere_geom is not 16-byte aligned");
-    }
-    if (stats) {
-        memset(stats, 0, sizeof(*stats));
-        stats->n_devices = nd;
-    }
+    const int src_dev = slot >= 0 ? ctx->devs[slot].dev : -1;
     const UpdatePlan& up = ctx->scene_upd;
     const int n = up.n_spheres;
-    if (n == 0) return TCRT_OK;
     const DeviceScene& ds0 = ctx->scene_ds;
     const bool grid = ctx->scene_grid;
     const int n_bvh = ds0.n_sph_bvh, n_ls = (int)up.light_sph.size(), n_levels = (int)up.level_start.size() - 1;
     const unsigned cap = 8u * (unsigned)n_bvh;
     const size_t back_bytes = sizeof(UpdateBack) + 12 * (size_t)n_ls;
     if (int rc = ensure_upd_stage(ctx, std::max((size_t)n, 2 * (size_t)ds0.n_lights))) return rc;
-    if (slot < 0) memcpy(ctx->upd_stage, geom, (size_t)n * sizeof(float4));
-    int launches = 0;
-    std::vector<int*> items(nd, nullptr);
+    if (slot < 0 && !rebox) memcpy(ctx->upd_stage, geom, (size_t)n * sizeof(float4));
+    out.items.assign(nd, nullptr);
+    out.ms.assign(nd, 0.f);
+    // the maps: slot_of, light_sph, levels, level_start, then for a rebox the identity and the light spheres' slots
+    const size_t o_ident = (size_t)n + n_ls + up.levels.size() + up.level_start.size();
     for (int i = 0; i < nd; i++) {
         DeviceState& d = ctx->devs[i];
         CK(ctx, cudaSetDevice(d.dev));
@@ -3481,7 +3546,7 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
         if (!d.ev_u0) CK(ctx, cudaEventCreate(&d.ev_u0));
         if (!d.ev_u1) CK(ctx, cudaEventCreate(&d.ev_u1));
         // the upload's maps, once per upload
-        const size_t n_maps = (size_t)n + n_ls + up.levels.size() + up.level_start.size();
+        const size_t n_maps = o_ident + (size_t)n + n_ls;
         int rc = ensure(ctx, d.upd_maps, d.upd_maps_cap, n_maps);
         if (rc) return rc;
         if (d.upd_serial != ctx->scene_serial) {
@@ -3489,6 +3554,8 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
             maps.insert(maps.end(), up.light_sph.begin(), up.light_sph.end());
             maps.insert(maps.end(), up.levels.begin(), up.levels.end());
             maps.insert(maps.end(), up.level_start.begin(), up.level_start.end());
+            for (int k = 0; k < n; k++) maps.push_back(k);
+            for (int j = 0; j < n_ls; j++) maps.push_back(up.slot_of[up.light_sph[j]]);
             CK(ctx, cudaMemcpy(d.upd_maps, maps.data(), maps.size() * sizeof(int), cudaMemcpyHostToDevice));
             d.upd_serial = ctx->scene_serial;
         }
@@ -3540,11 +3607,11 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
             ul.cells = d.scene_mem + ctx->scene_off[7];
             ul.tmp = g + o_tmp;
             ul.tmp_bytes = tmp_bytes;
-            items[i] = ul.items;
+            out.items[i] = ul.items;
         }
-        // the input on this device
-        const float4* src = reinterpret_cast<const float4*>(geom);
-        if (slot < 0 || d.dev != src_dev) {
+        // the input on this device (a rebox reads the blob's spheres in place: slot i is row i)
+        const float4* src = rebox ? d.scene_mem : reinterpret_cast<const float4*>(geom);
+        if (!rebox && (slot < 0 || d.dev != src_dev)) {
             if ((rc = ensure(ctx, d.upd_geom, d.upd_geom_cap, (size_t)n))) return rc;
             if (slot < 0)
                 CK(ctx, cudaMemcpyAsync(d.upd_geom, ctx->upd_stage, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, d.stream));
@@ -3554,12 +3621,12 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
         }
         ul.geom = src;
         ul.n = n;
-        ul.slot_of = d.upd_maps;
+        ul.slot_of = rebox ? d.upd_maps + o_ident : d.upd_maps;
         ul.spheres = d.scene_mem;
         ul.n_boxed = up.n_boxed;
         ul.n_bvh = n_bvh;
-        ul.ext_fixed = up.ext_fixed;
-        ul.light_sph = d.upd_maps + n;
+        ul.ext_fixed = ext_fixed;
+        ul.light_sph = rebox ? d.upd_maps + o_ident + n : d.upd_maps + n;
         ul.n_light_sph = n_ls;
         ul.back = reinterpret_cast<UpdateBack*>(d.upd_back);
         ul.boxes = d.upd_boxes;
@@ -3570,20 +3637,24 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
             ul.n_levels = n_levels;
         }
         CK(ctx, cudaEventRecord(d.ev_u0, d.stream));
-        CK(ctx, tcrt_launch_update_spheres(ul, d.sm_count, d.stream, &launches));
+        CK(ctx, tcrt_launch_update_spheres(ul, d.sm_count, d.stream, launches));
         CK(ctx, cudaEventRecord(d.ev_u1, d.stream));
         CK(ctx, cudaMemcpyAsync(d.h_upd_back, d.upd_back, back_bytes, cudaMemcpyDeviceToHost, d.stream));
     }
     bool invalid = false;
-    for (auto& d : ctx->devs) {
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
         CK(ctx, cudaSetDevice(d.dev));
         CK(ctx, cudaStreamSynchronize(d.stream));
+        CK(ctx, cudaEventElapsedTime(&out.ms[i], d.ev_u0, d.ev_u1));
         invalid = invalid || reinterpret_cast<const UpdateBack*>(d.h_upd_back)->invalid != 0;
     }
+    out.invalid = invalid;
+    if (invalid && rebox) return TCRT_OK;   // the upload does not check spheres; their boxes stay as they are
     if (invalid)   // no launch after the check wrote anything: the scene is unchanged
         return fail(ctx, TCRT_ERR_INVALID, "sphere_geom holds a centre or radius_squared that is not finite, or radius_squared < 0");
 
-    // the scalars and the light rows, with the upload's code (every device reduced the same values)
+    // the bounds and the light positions (every device reduced the same values)
     const UpdateBack& b = *reinterpret_cast<const UpdateBack*>(ctx->devs[0].h_upd_back);
     auto unkey = [](unsigned key) {
         const unsigned u = (key & 0x80000000u) ? (key & 0x7fffffffu) : ~key;
@@ -3591,7 +3662,8 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
         memcpy(&f, &u, 4);
         return f;
     };
-    SceneBounds bounds = up.bounds;
+    SceneBounds& bounds = out.bounds;
+    bounds = up.bounds;
     for (int k = 0; k < 3; k++) {
         if (b.lo_key[k]) bounds.sph_lo[k] = unkey(~b.lo_key[k]);
         if (b.hi_key[k]) bounds.sph_hi[k] = unkey(b.hi_key[k]);
@@ -3602,42 +3674,78 @@ static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* s
         memcpy(&r2f, &r2, 4);
         bounds.rmin = sqrtf(r2f);
     }
-    const bool keep_grid = grid && !b.grid_out && !b.grid_full;
-    DeviceScene ds = ds0;
-    scene_scalars(bounds, ctx->scene_bvh_s, !up.clusters.empty(), keep_grid, ds);
+    float ext_sph;
+    memcpy(&ext_sph, &b.ext_bits, 4);
+    out.ext_sph = ext_sph;
+    out.keep_grid = grid && !b.grid_out && !b.grid_full;
     const float* centres = reinterpret_cast<const float*>(&b + 1);
-    std::vector<float> og(up.light_og);
+    out.og = up.light_og;
     for (int j = 0; j < n_ls; j++)
-        for (int k = 0; k < 3; k++) og[3 * up.light_of_sph[j] + k] = centres[3 * j + k];
+        for (int k = 0; k < 3; k++) out.og[3 * up.light_of_sph[j] + k] = centres[3 * j + k];
+    return TCRT_OK;
+}
+
+// The per-launch scalars of ds into every device's scene, and the grid as the sphere launches left it
+static void set_scalars(tcrt_ctx* ctx, const DeviceScene& ds, bool keep_grid, const std::vector<int*>& items) {
+    for (size_t i = 0; i < ctx->devs.size(); i++) {
+        DeviceScene& dd = ctx->devs[i].ds;
+        dd.bvh_cx = ds.bvh_cx; dd.bvh_cy = ds.bvh_cy; dd.bvh_cz = ds.bvh_cz;
+        dd.bvh_r2 = ds.bvh_r2; dd.bvh_rmin = ds.bvh_rmin; dd.bvh_cmax = ds.bvh_cmax;
+        dd.clu_cx = ds.clu_cx; dd.clu_cy = ds.clu_cy; dd.clu_cz = ds.clu_cz; dd.clu_rbig = ds.clu_rbig;
+        dd.grid_k2_max = ds.grid_k2_max;
+        if (!items.empty()) dd.grid_items = keep_grid ? items[i] : nullptr;
+        if (!keep_grid) dd.grid_cells = nullptr;
+    }
+}
+
+static int update_impl(tcrt_ctx* ctx, int slot, const float* geom, tcrt_stats* stats) {
+    if (!ctx || !geom) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    const int nd = (int)ctx->devs.size();
+    if (slot >= 0) {
+        if (slot >= nd) return fail(ctx, TCRT_ERR_INVALID, "device slot %d out of range (have %d)", slot, nd);
+        const int src_dev = ctx->devs[slot].dev;
+        if (!on_device(geom, src_dev)) return fail(ctx, TCRT_ERR_INVALID, "sphere_geom is not device memory of slot %d's device", slot);
+        if (reinterpret_cast<uintptr_t>(geom) % 16 != 0)   // the launches read it as float4
+            return fail(ctx, TCRT_ERR_INVALID, "sphere_geom is not 16-byte aligned");
+    }
+    if (stats) {
+        memset(stats, 0, sizeof(*stats));
+        stats->n_devices = nd;
+    }
+    UpdatePlan& up = ctx->scene_upd;
+    if (up.n_spheres == 0) return TCRT_OK;
+    int launches = 0;
+    SpherePass sp;
+    if (int rc = sphere_pass(ctx, slot, geom, false, up.ext_fixed, sp, &launches)) return rc;
+
+    // the scalars and the light rows, with the upload's code
+    DeviceScene ds = ctx->scene_ds;
+    scene_scalars(sp.bounds, ctx->scene_bvh_s, !up.clusters.empty(), sp.keep_grid, ds);
     for (int l = 0; l < ds.n_lights; l++)
-        light_rows(&og[3 * l], up.light_int[l], &up.light_col[3 * l], up.clusters, ds, ctx->upd_stage + 2 * l);
+        light_rows(&sp.og[3 * l], up.light_int[l], &up.light_col[3 * l], up.clusters, ds, ctx->upd_stage + 2 * l);
     for (int i = 0; i < nd; i++) {
         DeviceState& d = ctx->devs[i];
         CK(ctx, cudaSetDevice(d.dev));
         if (ds.n_lights > 0)
             CK(ctx, cudaMemcpyAsync(d.scene_mem + ds.light_off, ctx->upd_stage, 2 * (size_t)ds.n_lights * sizeof(float4),
                                     cudaMemcpyHostToDevice, d.stream));
-        DeviceScene& dd = d.ds;
-        dd.bvh_cx = ds.bvh_cx; dd.bvh_cy = ds.bvh_cy; dd.bvh_cz = ds.bvh_cz;
-        dd.bvh_r2 = ds.bvh_r2; dd.bvh_rmin = ds.bvh_rmin; dd.bvh_cmax = ds.bvh_cmax;
-        dd.clu_cx = ds.clu_cx; dd.clu_cy = ds.clu_cy; dd.clu_cz = ds.clu_cz; dd.clu_rbig = ds.clu_rbig;
-        dd.grid_k2_max = ds.grid_k2_max;
-        dd.grid_items = keep_grid ? items[i] : nullptr;
-        if (!keep_grid) dd.grid_cells = nullptr;
     }
+    set_scalars(ctx, ds, sp.keep_grid, sp.items);
     for (int i = 0; i < nd; i++) {
         DeviceState& d = ctx->devs[i];
         CK(ctx, cudaSetDevice(d.dev));
         CK(ctx, cudaStreamSynchronize(d.stream));
-        if (stats) {
-            float ms = 0.f;
-            CK(ctx, cudaEventElapsedTime(&ms, d.ev_u0, d.ev_u1));
-            stats->render_ms[i] = ms;
-        }
+        if (stats) stats->render_ms[i] = sp.ms[i];
     }
     if (stats) stats->gpu_launches = (unsigned long long)launches;
+    // what a later plane update starts from
+    up.bounds = sp.bounds;
+    up.light_og = sp.og;
+    up.ext_sph = sp.ext_sph;
+    up.ext_sph_box = scene_ext(up.ext_fixed, sp.ext_sph);
     ctx->scene_ds = ds;
-    ctx->scene_grid = keep_grid;
+    ctx->scene_grid = sp.keep_grid;
     ctx->scene_key.clear();        // the staged blob no longer matches the devices: the next upload rebuilds
     ctx->cut_valid = false;
     ctx->costs_valid = false;
@@ -3797,3 +3905,205 @@ int tcrt_update_textures(tcrt_ctx* ctx, int n, const int* textures, const float*
 }
 
 }  // extern "C"
+
+// ---- moving planes (tcrt_update_planes) --------------------------------------------------------------------------------------
+// New rows for finite and infinite planes of the resident scene.  Planes are few (every finite plane is staged in shared
+// memory), so the host plans from its copy of the finite-plane rows (UpdatePlan) with the upload's own code: plane and
+// normal rows, the finite-plane BVH's leaf boxes (fin_box), the clusters' hulls (tcrt_refit_box_cluster) or their drop,
+// the light table (light_rows) and the per-launch scalars (scene_scalars).  tcrt_update.cu scatters the rows and refits
+// the finite-plane BVH.  When the new plane origins raise ext above the ext the resident sphere boxes were built with, the
+// sphere update's launches box the resident spheres again first.  DESIGN.md §4.3, §4.5.
+
+extern "C" int tcrt_update_planes(tcrt_ctx* ctx, int n, const int* objects, const float* geom, const float* normals,
+                                  const float* origin, tcrt_stats* stats) {
+    if (!ctx) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (n < 0) return fail(ctx, TCRT_ERR_INVALID, "n = %d is negative", n);
+    if (n > 0 && (!objects || !geom || !normals || !origin)) return fail(ctx, TCRT_ERR_INVALID, "null argument");
+    if (!ctx->has_scene) return fail(ctx, TCRT_ERR_NO_SCENE, "tcrt_upload_scene has not been called");
+    UpdatePlan& up = ctx->scene_upd;
+    const int n_obj = ctx->n_objects;
+    std::vector<char> seen(n_obj, 0);
+    for (int i = 0; i < n; i++) {
+        const int o = objects[i];
+        if (o < 0 || o >= n_obj) return fail(ctx, TCRT_ERR_INVALID, "object index %d out of range (have %d)", o, n_obj);
+        if (up.fin_slot_of_obj[o] < 0 && up.inf_slot_of_obj[o] < 0)
+            return fail(ctx, TCRT_ERR_INVALID, "object %d is a sphere (tcrt_update_spheres moves spheres)", o);
+        if (seen[o]) return fail(ctx, TCRT_ERR_INVALID, "object %d is listed twice", o);
+        seen[o] = 1;
+    }
+    clear_stats(ctx, stats);
+    if (n == 0) return TCRT_OK;
+    const int nd = (int)ctx->devs.size();
+    const MaterialShadow& mat = ctx->scene_mat;
+    DeviceScene ds = ctx->scene_ds;
+
+    // the rows of the moved planes, into the host's copy and the records
+    std::vector<PlaneRecord> rec;
+    auto put = [&](size_t dst, float4 v) {
+        PlaneRecord r{};
+        r.v = v;
+        r.dst = (int)dst;
+        rec.push_back(r);
+    };
+    auto f4 = [](const float* p) { return make_float4(p[0], p[1], p[2], p[3]); };
+    std::vector<int> moved_fin;   // finite-plane slots of the moved non-light planes
+    for (int i = 0; i < n; i++) {
+        const int o = objects[i];
+        const float* g = geom + 16 * (size_t)i;
+        const int fs = up.fin_slot_of_obj[o], is = up.inf_slot_of_obj[o];
+        if (fs >= 0) {
+            memcpy(&up.fin_rows[16 * (size_t)fs], g, 16 * sizeof(float));
+            for (int j = 0; j < 4; j++) put((size_t)ds.fin_off + 4 * (size_t)fs + j, f4(g + 4 * j));
+            if (fs < ds.n_fin_nl) moved_fin.push_back(fs);
+        } else {
+            put((size_t)ds.inf_off + is, f4(g));
+            for (int j = 0; j < 3; j++) put(up.off_frame + 3 * (size_t)is + j, f4(g + 4 * (j + 1)));
+        }
+        float4 nr[6];
+        normal_rows(normals + 8 * (size_t)i, nr);
+        for (int k = 0; k < 6; k++) put(up.off_normals + 6 * (size_t)o + k, nr[k]);
+        const int l = mat.light_of[o];
+        if (l >= 0)
+            for (int k = 0; k < 3; k++) up.light_og[3 * (size_t)l + k] = origin[4 * (size_t)i + k];
+    }
+
+    // ext of the moved scene: its finite-plane origins and the spheres' extent of the last read-back
+    double ext_fixed = 1.0;
+    for (int k = 0; k < ds.n_fin; k++)
+        for (int c = 0; c < 3; c++) ext_fixed = std::max(ext_fixed, fabs((double)up.fin_rows[16 * (size_t)k + 12 + c]));
+    const double ext = scene_ext(ext_fixed, up.ext_sph);
+
+    // the planes' part of the bounds: the finite-plane BVH's leaf boxes and the clusters' hulls
+    SceneBounds bounds = up.bounds;
+    for (int k = 0; k < 3; k++) {
+        bounds.pl_lo[k] = 1e300;
+        bounds.pl_hi[k] = -1e300;
+    }
+    const int nb = ctx->scene_bvh_f ? ds.n_fin_bvh : 0;
+    if (nb > 0) {
+        // every resident box at least as wide as the upload of the moved scene makes it: all of them again when ext grew
+        const double margin = 1e-5 * ext;
+        if (ext > up.ext_fin_box) {
+            for (int k = 0; k < nb; k++) fin_box(&up.fin_rows[16 * (size_t)k], margin, &up.fin_boxes[6 * (size_t)k]);
+            up.ext_fin_box = ext;
+        } else {
+            for (int k : moved_fin)
+                if (k < nb) fin_box(&up.fin_rows[16 * (size_t)k], margin, &up.fin_boxes[6 * (size_t)k]);
+            up.ext_fin_box = std::min(up.ext_fin_box, ext);
+        }
+        for (int k = 0; k < nb; k++) grow_into(bounds.pl_lo, bounds.pl_hi, &up.fin_boxes[6 * (size_t)k]);
+    }
+    std::vector<TcrtBoxCluster> clusters = up.clusters;
+    for (TcrtBoxCluster& c : clusters)
+        if (!tcrt_refit_box_cluster(up.fin_rows.data(), c)) {
+            // a member left its face's axis: no cluster until the next upload.  The rectangles already sit after the
+            // generic planes, so the linear sweep over [0, n_fin_nl) takes them (FM 3).
+            clusters.clear();
+            ds.n_clu = 0;
+            ds.n_arect = 0;
+            ds.n_fin_gen = ds.n_fin_nl;
+            break;
+        }
+    for (int c = 0; c < (int)clusters.size(); c++) {
+        grow_into(bounds.pl_lo, bounds.pl_hi, clusters[c].lo);   // lo[3], hi[3] are contiguous: a 6-float box
+        float4 rows[4];
+        cluster_rows(clusters[c], rows);
+        for (int j = 0; j < 4; j++) put((size_t)ds.clu_off + 4 * (size_t)c + j, rows[j]);
+    }
+
+    // the spheres boxed again when ext grew past the ext of their boxes (a lower ext keeps the wider boxes, still sound)
+    int launches = 0;
+    SpherePass sp;
+    bool rebox = up.n_boxed > 0 && ext > up.ext_sph_box;
+    if (rebox) {
+        if (int rc = sphere_pass(ctx, -1, nullptr, true, ext_fixed, sp, &launches)) return rc;
+        rebox = !sp.invalid;
+    }
+    if (rebox) {
+        for (int k = 0; k < 3; k++) {
+            bounds.sph_lo[k] = sp.bounds.sph_lo[k];
+            bounds.sph_hi[k] = sp.bounds.sph_hi[k];
+        }
+        bounds.rmin = sp.bounds.rmin;
+    }
+    const bool keep_grid = rebox ? sp.keep_grid : ctx->scene_grid;
+
+    // the scalars and every light row, with the upload's code
+    scene_scalars(bounds, ctx->scene_bvh_s, !clusters.empty(), keep_grid, ds);
+    for (int l = 0; l < ds.n_lights; l++) {
+        float4 rows[2];
+        light_rows(&up.light_og[3 * (size_t)l], up.light_int[l], &up.light_col[3 * (size_t)l], clusters, ds, rows);
+        put((size_t)ds.light_off + 2 * (size_t)l, rows[0]);
+        put((size_t)ds.light_off + 2 * (size_t)l + 1, rows[1]);
+    }
+
+    // every device: the records (and the leaf boxes), one scatter launch, the refit
+    const size_t rec_f4 = rec.size() * (sizeof(PlaneRecord) / sizeof(float4));
+    const int n_levels = nb > 0 ? (int)up.fin_level_start.size() - 1 : 0;
+    if (int rc = ensure_upd_stage(ctx, rec_f4 + (6 * (size_t)nb + 3) / 4)) return rc;
+    memcpy(ctx->upd_stage, rec.data(), rec.size() * sizeof(PlaneRecord));
+    float* boxes_stage = reinterpret_cast<float*>(ctx->upd_stage + rec_f4);
+    if (nb > 0) memcpy(boxes_stage, up.fin_boxes.data(), 6 * (size_t)nb * sizeof(float));
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));   // frames queued before the call finish with the old planes
+        if (!d.ev_u0) CK(ctx, cudaEventCreate(&d.ev_u0));
+        if (!d.ev_u1) CK(ctx, cudaEventCreate(&d.ev_u1));
+        int rc = ensure(ctx, d.pl_rec, d.pl_rec_cap, rec.size());
+        if (rc) return rc;
+        CK(ctx, cudaMemcpyAsync(d.pl_rec, ctx->upd_stage, rec.size() * sizeof(PlaneRecord), cudaMemcpyHostToDevice, d.stream));
+        PlaneLaunch pl{};
+        pl.rec = d.pl_rec;
+        pl.n = (int)rec.size();
+        pl.scene = d.scene_mem;
+        if (n_levels > 0) {
+            const size_t n_lv = up.fin_levels.size() + up.fin_level_start.size();
+            if ((rc = ensure(ctx, d.pl_levels, d.pl_levels_cap, n_lv))) return rc;
+            if (d.pl_serial != ctx->scene_serial) {   // the levels, once per upload
+                std::vector<int> lv(up.fin_levels);
+                lv.insert(lv.end(), up.fin_level_start.begin(), up.fin_level_start.end());
+                CK(ctx, cudaMemcpy(d.pl_levels, lv.data(), lv.size() * sizeof(int), cudaMemcpyHostToDevice));
+                d.pl_serial = ctx->scene_serial;
+            }
+            if ((rc = ensure(ctx, d.pl_boxes, d.pl_boxes_cap, 6 * (size_t)nb))) return rc;
+            if ((rc = ensure(ctx, d.upd_back, d.upd_back_cap, sizeof(UpdateBack)))) return rc;
+            CK(ctx, cudaMemcpyAsync(d.pl_boxes, boxes_stage, 6 * (size_t)nb * sizeof(float), cudaMemcpyHostToDevice, d.stream));
+            pl.boxes = d.pl_boxes;
+            pl.nodes = d.scene_mem + ctx->scene_off[6];
+            pl.levels = d.pl_levels;
+            pl.level_start = d.pl_levels + up.fin_levels.size();
+            pl.n_levels = n_levels;
+            pl.back = reinterpret_cast<UpdateBack*>(d.upd_back);
+        }
+        CK(ctx, cudaEventRecord(d.ev_u0, d.stream));
+        CK(ctx, tcrt_launch_update_planes(pl, d.stream, &launches));
+        CK(ctx, cudaEventRecord(d.ev_u1, d.stream));
+    }
+    set_scalars(ctx, ds, keep_grid, rebox ? sp.items : std::vector<int*>());
+    for (int i = 0; i < nd; i++) {
+        DeviceState& d = ctx->devs[i];
+        d.ds.n_clu = ds.n_clu;
+        d.ds.n_arect = ds.n_arect;
+        d.ds.n_fin_gen = ds.n_fin_gen;
+        CK(ctx, cudaSetDevice(d.dev));
+        CK(ctx, cudaStreamSynchronize(d.stream));
+        if (stats) {
+            float ms = 0.f;
+            CK(ctx, cudaEventElapsedTime(&ms, d.ev_u0, d.ev_u1));
+            stats->render_ms[i] = ms + (rebox ? sp.ms[i] : 0.f);
+        }
+    }
+    if (stats) stats->gpu_launches = (unsigned long long)launches;
+    // what later updates start from
+    up.ext_fixed = ext_fixed;
+    if (rebox) up.ext_sph_box = ext;
+    up.bounds = bounds;
+    up.clusters.swap(clusters);
+    ctx->scene_ds = ds;
+    ctx->scene_grid = keep_grid;
+    ctx->scene_key.clear();        // the staged blob no longer matches the devices: the next upload rebuilds
+    ctx->cut_valid = false;
+    ctx->costs_valid = false;
+    return TCRT_OK;
+}

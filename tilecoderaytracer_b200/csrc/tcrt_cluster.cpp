@@ -166,3 +166,26 @@ void tcrt_build_box_clusters(const float* fin_geom, const std::vector<int>& plan
         out.push_back(o);
     }
 }
+
+bool tcrt_refit_box_cluster(const float* fin_slots, TcrtBoxCluster& c) {
+    // the builder's hull of the members' rectangles (contained, not necessarily tight: DESIGN.md §4.5 "Moving planes")
+    double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    float face[6];
+    for (int f = 0; f < 6; f++) {
+        face[f] = NAN;
+        if (c.plane[f] < 0) continue;
+        ARect r;
+        if (!classify(fin_slots + 16 * (size_t)c.plane[f], c.plane[f], r) || r.axis != f / 2) return false;
+        for (int k = 0; k < 3; k++) {
+            lo[k] = std::min(lo[k], r.lo[k]);
+            hi[k] = std::max(hi[k], r.hi[k]);
+        }
+        face[f] = r.c;
+    }
+    for (int k = 0; k < 3; k++) {
+        c.lo[k] = round_down(lo[k]);
+        c.hi[k] = round_up(hi[k]);
+    }
+    memcpy(c.c, face, sizeof face);
+    return true;
+}

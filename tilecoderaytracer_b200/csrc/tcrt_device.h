@@ -251,6 +251,30 @@ struct MaterialLaunch {
 // the scatter launch (nothing when n == 0); *launches += kernels launched
 cudaError_t tcrt_launch_material_edit(const MaterialLaunch& ml, cudaStream_t stream, int* launches);
 
+// Moving planes (tcrt_update_planes, tcrt_update.cu): the host plans every row the upload would write for the moved scene
+// (plane rows, normal rows, cluster records, light rows) and sends them as packed records; one scatter launch writes them
+// into the blob, then the finite-plane BVH is refitted from the leaf boxes with the sphere update's refit launch.
+struct PlaneRecord {
+    float4 v;
+    int dst;                     // float4 offset of the row in the device's scene allocation
+    int pad[3];
+};
+struct PlaneLaunch {
+    const PlaneRecord* rec;
+    int n;
+    float4* scene;               // the device's scene allocation (DeviceState::scene_mem)
+    // finite-plane BVH (n_levels == 0: none): leaf boxes, 6 per slot (lo xyz, hi xyz), its nodes and inner levels from the
+    // root (levels[level_start[l] .. level_start[l + 1]))
+    const float* boxes;
+    float4* nodes;
+    const int* levels;
+    const int* level_start;
+    int n_levels;
+    UpdateBack* back;            // zeroed scratch the refit launch checks (`invalid`)
+};
+// the scatter launch and the refit (nothing when there is nothing to write); *launches += kernels launched
+cudaError_t tcrt_launch_update_planes(const PlaneLaunch& pl, cudaStream_t stream, int* launches);
+
 // host builder of the box clusters (tcrt_cluster.cpp).  Face f = 2*axis + k; an absent face has
 // c = NaN and plane = -1; `plane` indexes the caller's list.
 struct TcrtBoxCluster {
@@ -263,6 +287,10 @@ struct TcrtBoxCluster {
 // arect_of_plane[i] != 0 when planes[i] is axis-aligned and therefore owned by a cluster.
 void tcrt_build_box_clusters(const float* fin_geom, const std::vector<int>& planes, std::vector<int>& arect_of_plane,
                              std::vector<TcrtBoxCluster>& out);
+// Moving planes: the hull and face coordinates of cluster c recomputed from its members' rows (fin_slots: 16 floats per
+// finite-plane slot; c.plane holds slots) with the builder's arithmetic.  false, c unchanged, when a member no longer
+// classifies as an axis-aligned rectangle with the normal axis of its face.
+bool tcrt_refit_box_cluster(const float* fin_slots, TcrtBoxCluster& c);
 #endif
 
 // render kernels (tcrt_render.cu).  wave_mem / wave_bytes: scratch for the wavefront path (tcrt_render_wave.cu), which

@@ -1,5 +1,6 @@
 // tcrt_update.cu — moving spheres (tcrt_update_spheres): the resident scene's spheres take new centres and radii in place,
-// and the pruning structures follow them on the device, without the host's sort, SAH build and grid search.
+// and the pruning structures follow them on the device, without the host's sort, SAH build and grid search.  Moving planes
+// (tcrt_update_planes) scatter the rows the host planned and refit the finite-plane BVH with the same refit launch.
 //
 // Every structure only decides WHICH primitives a ray tests; the tests themselves are the reference's arithmetic
 // (DESIGN.md §4.5).  So a BVH keeps its topology and leaf order and only has its boxes refitted around the moved spheres,
@@ -194,6 +195,14 @@ __global__ void __launch_bounds__(kUpdBlock) update_cells_kernel(const UpdateLau
     reinterpret_cast<int4*>(ul.cells)[2 * c + 1] = meta;
 }
 
+// Moving planes (tcrt_update_planes): every row the host planned for the moved scene, written into the blob
+__global__ void __launch_bounds__(kUpdBlock) plane_scatter_kernel(const PlaneLaunch pl) {
+    const int i = blockIdx.x * kUpdBlock + threadIdx.x;
+    if (i >= pl.n) return;
+    const PlaneRecord r = pl.rec[i];
+    pl.scene[r.dst] = r.v;
+}
+
 int key_bits(int n_cells) {   // bits of the keys 0 .. n_cells (n_cells: the tail's key)
     int b = 1;
     while ((1u << b) <= (unsigned)n_cells && b < 32) b++;
@@ -242,5 +251,26 @@ cudaError_t tcrt_launch_update_spheres(const UpdateLaunch& ul, int sm_count, cud
     if (e != cudaSuccess) return e;
     update_cells_kernel<<<(std::max<unsigned>(ul.cap, (unsigned)ul.n_cells) + kUpdBlock - 1) / kUpdBlock, kUpdBlock, 0, stream>>>(ul);
     *launches += 5;   // the scans and the sort count as one launch each
+    return cudaGetLastError();
+}
+
+cudaError_t tcrt_launch_update_planes(const PlaneLaunch& pl, cudaStream_t stream, int* launches) {
+    if (pl.n > 0) {
+        plane_scatter_kernel<<<(pl.n + kUpdBlock - 1) / kUpdBlock, kUpdBlock, 0, stream>>>(pl);
+        *launches += 1;
+    }
+    if (pl.n_levels > 0) {   // the finite-plane BVH, refitted like the sphere BVH from its leaves' boxes (slots = leaf order)
+        UpdateLaunch ul{};
+        ul.back = pl.back;
+        ul.boxes = const_cast<float*>(pl.boxes);   // read only
+        ul.nodes = pl.nodes;
+        ul.levels = pl.levels;
+        ul.level_start = pl.level_start;
+        ul.n_levels = pl.n_levels;
+        cudaError_t e = cudaMemsetAsync(pl.back, 0, sizeof(UpdateBack), stream);
+        if (e != cudaSuccess) return e;
+        update_refit_kernel<<<1, kRefitBlock, 0, stream>>>(ul);
+        *launches += 1;
+    }
     return cudaGetLastError();
 }

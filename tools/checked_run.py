@@ -8,7 +8,8 @@ flags are read from each translation unit that launches a kernel: render, grid a
 invalid rays on a grid scene and a BVH scene, traced and intersected, against tests/oracle_rays.c, and the occlusion queries
 (points against every light, rays with their limits) on a grid scene, BVH scenes and box-cluster scenes against
 tests/oracle_occlusion.c, and multi-view frames on a grid scene, a BVH scene and a box-cluster scene, with a piece
-boundary inside a view, and one scene of every dispatch class after a material edit (tests/test_material_edits.py).
+boundary inside a view, one scene of every dispatch class after a material edit (tests/test_material_edits.py), and one
+scene of every dispatch class after its planes moved, with a cluster drop (tests/test_plane_updates.py).
 usage: python -c "from tilecoderaytracer_b200 import build; build.build_lib(defines=('TCRT_CHECKED',), out=LIB)"
        TCRT_LIB=LIB python tools/checked_run.py"""
 import ctypes as C
@@ -277,4 +278,28 @@ for name in V.NAMES:
     f = fired()
     bad_total += bad + len(f)
     print(f"material edit {name:9s} 27x17 d0/8: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
+
+# ---- moving planes: the moves of tests/test_plane_updates.py in every dispatch class, and a room's cluster drop
+import test_plane_updates as PU  # noqa: E402
+
+for name in V.NAMES:
+    rec, cam = PU.build(name)
+    flat, c = rec.scene.flatten(), cam.export()
+    ctx.upload_flat(flat, c)
+    steps = [(w, calls) for w, calls, _ in PU.variant_moves(name, rec, flat, np.random.default_rng(7))]
+    if V.VARIANTS[name][0] == "room":
+        steps += PU.cluster_drop_moves(rec, flat)[:1]
+    bad = 0
+    for what, calls in steps:
+        mv = PU.Move.of(calls)
+        mv.apply(ctx)
+        flat = mv.flat(flat)
+        for d in (0, 8):
+            p = api.default_params(27, 17, d)
+            img, st = ctx.render(p)
+            ref, cnt = O.render(flat, c, p)
+            bad += n_bad(img, ref) + int(counters_differ(st, cnt))
+    f = fired()
+    bad_total += bad + len(f)
+    print(f"plane update {name:9s} {len(steps)} moves, 27x17 d0/8: mismatches {bad}, checks fired: {f or 'none'}", flush=True)
 print("CHECKED_OK" if bad_total == 0 else "CHECKED_FAIL")
